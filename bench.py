@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — reads/sec of the sgcount match-and-count path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1], the configuration the metric is quoted on): Brunello-
 shaped synthetic library (77 441 x 20 bp, seed 0xB2000002), one sample of 50 M x 75 bp reads,
@@ -100,6 +100,15 @@ def bench_config(world: int, reads_per_gpu: int) -> dict:
 
 def library_fasta(lib_arr) -> bytes:
     return b"".join(b">lib.%d\n%s\n" % (i, lib_arr[i].tobytes()) for i in range(len(lib_arr)))
+
+
+def dump_outputs(out_dir, counts, total, matched):
+    """--dump-outputs: what Counter.finish() handed back after the last timed step, so that two
+    builds can be compared output for output on the same seeded sample.  float64 holds every count
+    exactly (all are below 2**53); the three arrays hold (N_GUIDES + 2) x 8 bytes."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in (("counts", counts), ("total_reads", [total]), ("matched_reads", [matched])):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(arr, dtype=np.float64))
 
 
 # ---------------------------------------------------------------------------------------------
@@ -809,6 +818,8 @@ def run_gpu(args):
     last = (args.steps - 1) % n_buf
     state, counter = states[last], counters[last]
     counts_last, total_last, matched_last = counter.finish()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, counts_last, total_last, matched_last)
     value = world * n_reads * args.steps / (total_ms * 1e-3)
     headline_plan = (counter.launch_info().replicas, counter.launch_info().hot_guides)
 
@@ -1120,7 +1131,14 @@ def main():
     ap.add_argument("--config-reps", type=int, default=3)
     ap.add_argument("--config-scale", type=float, default=1.0,
                     help="development only: fraction of the reads of configs 3-5 (reported as scaled_to)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's per-guide counts, total and matched reads to DIR/<name>.npy "
+                         "(float64; the GPU arm only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the GPU arm; the reference arm counts a host-dependent number of reads")
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
         run_reference(args)

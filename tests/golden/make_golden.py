@@ -1,8 +1,8 @@
 #!/usr/bin/env python3
 """Derives the config-1 golden fixtures from the reference's example data.
 
-Run in the build container only (it reads /root/reference/example, which does not exist on
-the GPU box):   python tests/golden/make_golden.py
+Run with the example/ directory of the reference's source tree (the tests read only the
+committed outputs):   python tests/golden/make_golden.py <sgcount source>/example
 
 Outputs, all under tests/golden/:
   example/<name>.gz          the example FASTA/FASTQ records re-serialised (id, seq, +, qual)
@@ -21,8 +21,8 @@ import hashlib
 import json
 import os
 import shutil
+import sys
 
-SRC = "/root/reference/example"
 DST = os.path.join(os.path.dirname(os.path.abspath(__file__)), "example")
 
 FASTQ = ["sequence", "zero.sequence", "diff.sequence", "offset", "offset_clipped"]
@@ -46,16 +46,19 @@ def write_gz(path, records):
 
 
 def main():
+    if len(sys.argv) != 2:
+        raise SystemExit("usage: make_golden.py <reference example directory>")
+    src = sys.argv[1]
     os.makedirs(DST, exist_ok=True)
-    lib = read_records(os.path.join(SRC, "library.fasta.gz"))
+    lib = read_records(os.path.join(src, "library.fasta.gz"))
     write_gz(os.path.join(DST, "library.fasta.gz"), lib)
-    shutil.copyfile(os.path.join(SRC, "g2s.txt"), os.path.join(DST, "g2s.txt"))
+    shutil.copyfile(os.path.join(src, "g2s.txt"), os.path.join(DST, "g2s.txt"))
     seq_to_alias = {r[1].decode(): r[0][1:].decode() for r in lib}
     aliases = [r[0][1:].decode() for r in lib]
 
     expected = {"library": {"n": len(lib), "k": K, "aliases": aliases}, "offset": OFFSET, "fixtures": {}}
     for name in FASTQ:
-        recs = read_records(os.path.join(SRC, name + ".fastq.gz"))
+        recs = read_records(os.path.join(src, name + ".fastq.gz"))
         write_gz(os.path.join(DST, name + ".fastq.gz"), recs)
         counts = {a: 0 for a in aliases}
         labelled = clipped = 0
