@@ -258,6 +258,22 @@ int sgc_fastq_stream_submit(sgc_fastq_stream*, const uint8_t* gz, const uint64_t
 int sgc_fastq_stream_submit_range(sgc_fastq_stream*, const uint8_t* gz, const uint64_t* block_begin,
                                   const uint32_t* block_isize, uint32_t n_blocks, uint32_t head_skip,
                                   uint32_t tail_skip, int self_contained);
+/* ONE gzip member that is not BGZF (what gzip and pigz write): the whole file, gz[0 .. n_bytes) in
+ * host memory, inflated, framed and counted on the device, once per stream, then
+ * sgc_fastq_stream_finish.  One DEFLATE stream is decoded in parallel by speculation: candidate
+ * dynamic-Huffman block starts every 32 KiB of compressed input, a decode without output from each
+ * to the next that links the true block boundaries from the member's first block on, then every
+ * linked piece decoded into 16-bit symbols whose references to the unknown 32 KiB in front of it
+ * are resolved afterwards.  The compressed member stays on the device; the text goes in waves (the
+ * limits of the BGZF waves), about 3 bytes of device memory per byte of text in a wave.  When the
+ * boundaries cannot be followed to the member's end (blocks other than dynamic Huffman codes over
+ * long stretches, damage), the trailer does not end the file (a second member) or ISIZE / CRC-32
+ * disagree, it fails with SGC_ERR_GZIP, and with SGC_ERR_FASTQ_FORMAT as sgc_fastq_stream_submit
+ * does; the caller then counts the file on the host. */
+int sgc_fastq_stream_submit_member(sgc_fastq_stream*, const uint8_t* gz, uint64_t n_bytes);
+/* After sgc_fastq_stream_submit_member: candidate pieces, pieces on the chain of true block
+ * boundaries, candidates the chain ran past. */
+int sgc_fastq_stream_member_stats(const sgc_fastq_stream*, uint64_t* pieces, uint64_t* chain, uint64_t* absorbed);
 int sgc_fastq_stream_finish(sgc_fastq_stream*, uint64_t* n_records);
 
 /* Statistics of the last sgc_counter_submit_device call, for benchmarking. */

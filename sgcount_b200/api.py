@@ -393,7 +393,7 @@ def bgzf_blocks(blob: bytes):
 
 
 class FastqStream:
-    """sgc_fastq_stream: BGZF blocks of a FASTQ inflated, framed and counted on the device.
+    """sgc_fastq_stream: BGZF blocks of a FASTQ (or one single-member gzip file) inflated, framed and counted on the device.
     read_len > 0: fixed-length reads, `counter` created with the span Offset of span_geometry();
     read_len == 0: reads of any length, `counter` an ordinary counter."""
 
@@ -417,6 +417,19 @@ class FastqStream:
         assert len(begin) == len(isize) + 1
         check(_cabi.load().sgc_fastq_stream_submit(self._ptr, blob.ctypes.data, begin.ctypes.data, isize.ctypes.data, len(isize)))
         self._counter._result = None
+
+    def submit_member(self, blob: np.ndarray) -> None:
+        """a whole single-member gzip file (uint8), decoded in parallel pieces on the device; call once,
+        then finish().  SgcError(ERR_GZIP) when the device declines it (count it on the host instead)"""
+        blob = np.ascontiguousarray(blob, dtype=np.uint8)
+        check(_cabi.load().sgc_fastq_stream_submit_member(self._ptr, blob.ctypes.data, len(blob)))
+        self._counter._result = None
+
+    def member_stats(self) -> tuple:
+        """(candidate pieces, pieces on the chain of block boundaries, candidates run past) of submit_member"""
+        v = [C.c_uint64() for _ in range(3)]
+        check(_cabi.load().sgc_fastq_stream_member_stats(self._ptr, *[C.byref(x) for x in v]))
+        return tuple(int(x.value) for x in v)
 
     def finish(self) -> int:
         n = C.c_uint64()

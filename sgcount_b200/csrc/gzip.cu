@@ -22,6 +22,9 @@
 // complete record are carried in front of the next wave's text.  Only fixed-length 4-line FASTQ
 // takes this path (the head of the sample, which the host reads for the offset detector, says so);
 // anything irregular is reported and the caller counts the sample through the host path instead.
+#include <stdio.h>
+#include <stdlib.h>
+
 #include <algorithm>
 #include <map>
 #include <mutex>
@@ -267,6 +270,148 @@ __global__ void tail_restore_kernel(uint8_t* __restrict__ text, const StreamStat
     text[kHeadroom - tail + i] = tail_buf[i];
 }
 
+// ---- one gzip member (not BGZF) decoded in pieces: the steps of inflate_core.h "ONE member in pieces" ----
+// Candidate piece starts: one warp per nominal boundary c_j = j * piece bytes (j >= 1), its lanes probing
+// consecutive bit offsets; the first that passes wins (or ~0: none before c_{j+1}).
+__global__ void __launch_bounds__(kInflateThreads) member_find_kernel(const uint8_t* __restrict__ gz, uint64_t n_gz,
+                                                                     uint64_t piece, uint32_t n_bounds, uint64_t* __restrict__ cand) {
+  extern __shared__ uint16_t sm[];
+  const uint32_t j = 1 + blockIdx.x * (kInflateThreads / 32) + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (j >= n_bounds) return;  // (whole warps)
+  DeviceSymbols symbols;
+  const DeviceTables t{sm + threadIdx.x, &symbols};
+  const uint64_t lo = j * piece * 8, hi = min((uint64_t)(j + 1) * piece, n_gz) * 8;
+  uint64_t found = ~0ull;
+  for (uint64_t base = lo; base < hi; base += 32) {
+    const uint64_t bit = base + lane;
+    const bool ok = bit < hi && inflate::probe_block_start(gz, (size_t)n_gz, bit, t, inflate::kProbeTrial);
+    const uint32_t votes = __ballot_sync(0xffffffffu, ok);
+    if (votes) {
+      found = base + (uint64_t)(__ffs((int)votes) - 1);
+      break;
+    }
+  }
+  if (lane == 0) cand[j] = found;
+}
+
+// what the boundary pass learns about a piece (inflate::piece_boundary)
+struct PieceMeta {
+  uint64_t end_bit, out_len;
+  uint32_t next;
+  int32_t status;
+};
+__global__ void __launch_bounds__(kInflateThreads) member_boundary_kernel(const uint8_t* __restrict__ gz, uint64_t n_gz,
+                                                                         const uint64_t* __restrict__ starts, uint32_t n,
+                                                                         PieceMeta* __restrict__ meta) {
+  extern __shared__ uint16_t sm[];
+  const uint32_t j = blockIdx.x * kInflateThreads + threadIdx.x;
+  if (j >= n) return;
+  DeviceSymbols symbols;
+  const DeviceTables t{sm + threadIdx.x, &symbols};
+  PieceMeta m{0, 0, 0, 0};
+  m.status = inflate::piece_boundary(gz, (size_t)n_gz, starts, n, j, inflate::kMaxAbsorb, t, &m.next, &m.end_bit, &m.out_len);
+  meta[j] = m;
+}
+
+// a piece of the chain in the current wave: where its bits start and end, where its text goes
+// (offset within the wave's text) and how far before its start a match may reach
+struct WavePiece {
+  uint64_t start_bit, end_bit, off, reach;
+};
+__global__ void __launch_bounds__(kInflateThreads) member_decode_kernel(const uint8_t* __restrict__ gz, uint64_t n_gz,
+                                                                       const WavePiece* __restrict__ wp, uint32_t n,
+                                                                       uint16_t* __restrict__ sym, StreamState* st) {
+  extern __shared__ uint16_t sm[];
+  const uint32_t i = blockIdx.x * kInflateThreads + threadIdx.x;
+  if (i >= n) return;
+  DeviceSymbols symbols;
+  const DeviceTables t{sm + threadIdx.x, &symbols};
+  const WavePiece p = wp[i];
+  const uint64_t len = wp[i + 1].off - p.off;
+  inflate::MarkSink sink{sym + p.off, 0, len, p.reach};
+  uint64_t e = 0;
+  bool fin = false;
+  int rc = inflate::inflate_piece(gz, (size_t)n_gz, p.start_bit, p.end_bit, t, sink, [&](uint64_t b) { return b >= p.end_bit; },
+                                  &e, &fin);
+  if (rc == inflate::kOk && (e != p.end_bit || sink.op != len)) rc = 100;
+  if (rc != inflate::kOk) {
+    const unsigned int prev = atomicMin(&st->bad_block, i);
+    if (i < prev) st->bad_status = rc;
+  }
+}
+
+// byte x of the wave's text from its symbol: a marker names a byte of the 32 KiB in front of the
+// piece, which is either earlier text of this wave or the end of the previous waves (`window`)
+__device__ __forceinline__ uint8_t member_resolve(uint16_t s, uint64_t piece_off, const uint8_t* text, const uint8_t* window) {
+  if (s < 256) return (uint8_t)s;
+  const int64_t g = (int64_t)piece_off - (int64_t)inflate::kWindow + (int64_t)(s - 256);
+  return g >= 0 ? text[g] : window[inflate::kWindow + g];
+}
+
+// The last 32 KiB (or all) of every piece, piece after piece: each depends on the 32 KiB in front of
+// its piece, which the pieces before resolved.  The only sequential step: one block, 32 bytes a thread.
+constexpr int kWindowThreads = 1024;
+__global__ void __launch_bounds__(kWindowThreads) member_window_kernel(const uint16_t* __restrict__ sym,
+                                                                      const WavePiece* __restrict__ wp, uint32_t n,
+                                                                      uint8_t* text, const uint8_t* __restrict__ window) {
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint64_t a = wp[i].off, b = wp[i + 1].off;
+    const uint64_t lo = b - a > inflate::kWindow ? b - inflate::kWindow : a;
+    const uint64_t x0 = lo + (uint64_t)threadIdx.x * 32;
+    uint16_t s[32];
+#pragma unroll
+    for (int k = 0; k < 32; ++k) s[k] = x0 + k < b ? sym[x0 + k] : 0;
+    uint8_t v[32];
+#pragma unroll
+    for (int k = 0; k < 32; ++k) v[k] = x0 + k < b ? member_resolve(s[k], a, text, window) : 0;
+#pragma unroll
+    for (int k = 0; k < 32; ++k)
+      if (x0 + k < b) text[x0 + k] = v[k];
+    __syncthreads();  // (the next piece reads these bytes)
+  }
+}
+
+// everything else, every piece side by side (its window is resolved)
+__global__ void __launch_bounds__(256) member_resolve_kernel(const uint16_t* __restrict__ sym, const WavePiece* __restrict__ wp,
+                                                            uint8_t* text, const uint8_t* __restrict__ window) {
+  const uint64_t a = wp[blockIdx.x].off, b = wp[blockIdx.x + 1].off;
+  if (b - a <= inflate::kWindow) return;
+  const uint64_t end = b - inflate::kWindow;
+  for (uint64_t x = a + threadIdx.x; x < end; x += blockDim.x) text[x] = member_resolve(sym[x], a, text, window);
+}
+
+// CRC-32 of every piece's text, one warp each (joined on the host across pieces and waves)
+__global__ void __launch_bounds__(kCrcWarps * 32) member_crc_kernel(const WavePiece* __restrict__ wp, uint32_t n,
+                                                                   const uint8_t* __restrict__ text, uint32_t* __restrict__ crc_out) {
+  __shared__ uint32_t table[256];
+  table[threadIdx.x] = inflate::crc_table_entry(threadIdx.x);
+  __syncthreads();
+  const uint32_t i = blockIdx.x * kCrcWarps + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (i >= n) return;
+  const uint8_t* d = text + wp[i].off;
+  const size_t len = (size_t)(wp[i + 1].off - wp[i].off);
+  const size_t c = inflate::crc_piece_len(len), first = len - 31 * c;
+  const size_t at = lane == 0 ? 0 : first + (lane - 1) * c;
+  uint32_t crc = inflate::crc_bytes(d + at, lane == 0 ? first : c, [&](uint32_t k) { return table[k]; });
+  uint32_t p = inflate::crc_x8n(c);
+#pragma unroll
+  for (int s = 1; s < 32; s *= 2) {
+    const uint32_t other = __shfl_down_sync(0xffffffffu, crc, s);
+    if ((lane & (2 * s - 1)) == 0) crc = inflate::crc_multmodp(p, crc) ^ other;
+    p = inflate::crc_multmodp(p, p);
+  }
+  if (lane == 0) crc_out[i] = crc;
+}
+
+// the 32 KiB in front of the next wave: the end of this wave's text, preceded by the old window
+__global__ void member_window_save_kernel(const uint8_t* __restrict__ text, uint64_t n_text, const uint8_t* __restrict__ old_window,
+                                          uint8_t* __restrict__ new_window) {
+  for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < inflate::kWindow; k += gridDim.x * blockDim.x) {
+    const int64_t p = (int64_t)n_text - (int64_t)inflate::kWindow + k;
+    new_window[k] = p >= 0 ? text[p] : old_window[inflate::kWindow + p];
+  }
+}
+
 // Device scratch of the ingest streams comes from one memory pool per device whose unused memory stays
 // cached, through the stream-ordered allocator.  cudaFree waits for ALL work on the device and cudaMalloc
 // queues up behind it: with several samples in flight on one device (the CLI runs four) every sample that
@@ -349,6 +494,16 @@ struct sgc_fastq_stream {
   std::vector<uint64_t> h_begin, h_outoff;
   uint64_t blocks_total = 0, records_total = 0;
   bool failed = false;
+  // one member in pieces (sgc_fastq_stream_submit_member)
+  uint16_t* d_sym = nullptr;
+  uint8_t* d_window[2] = {nullptr, nullptr};
+  uint64_t* d_cand = nullptr;
+  PieceMeta* d_meta = nullptr;
+  WavePiece* d_wave = nullptr;
+  uint32_t* d_crc = nullptr;
+  size_t sym_cap = 0, cand_cap = 0, meta_cap = 0, wave_cap = 0, crc_cap = 0;
+  uint64_t member_pieces = 0, member_chain = 0, member_absorbed = 0;
+  bool member_submitted = false;
 };
 
 namespace {
@@ -434,8 +589,16 @@ void sgc::fastq_stream_release(sgc_fastq_stream* s) {
   s->counter = nullptr;
   s->failed = true;  // nothing more can be submitted
   for (void* p : {(void*)s->d_state, (void*)s->d_gz, (void*)s->d_text, (void*)s->d_spans, (void*)s->d_tail, (void*)s->d_seq_start,
-                  (void*)s->d_seq_end, (void*)s->d_begin, (void*)s->d_outoff, (void*)s->d_counts, (void*)s->d_first, (void*)s->d_sums})
+                  (void*)s->d_seq_end, (void*)s->d_begin, (void*)s->d_outoff, (void*)s->d_counts, (void*)s->d_first, (void*)s->d_sums,
+                  (void*)s->d_sym, (void*)s->d_window[0], (void*)s->d_window[1], (void*)s->d_cand, (void*)s->d_meta,
+                  (void*)s->d_wave, (void*)s->d_crc})
     scratch_free(p, s->pool, s->stream);
+  s->d_sym = nullptr;
+  s->d_window[0] = s->d_window[1] = nullptr;
+  s->d_cand = nullptr;
+  s->d_meta = nullptr;
+  s->d_wave = nullptr;
+  s->d_crc = nullptr;
   s->d_state = nullptr;
   s->d_gz = s->d_text = s->d_spans = s->d_tail = nullptr;
   s->d_seq_start = s->d_seq_end = nullptr;
@@ -474,6 +637,9 @@ int sgc_fastq_stream_create(sgc_counter* counter, uint32_t read_len, uint32_t sp
   SGC_CUDA_TRY(cudaMemcpyAsync(s->d_state, &st0, sizeof st0, cudaMemcpyHostToDevice, s->stream));
   SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
   SGC_CUDA_TRY(cudaFuncSetAttribute(inflate_blocks_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kInflateSmem));
+  SGC_CUDA_TRY(cudaFuncSetAttribute(member_find_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kInflateSmem));
+  SGC_CUDA_TRY(cudaFuncSetAttribute(member_boundary_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kInflateSmem));
+  SGC_CUDA_TRY(cudaFuncSetAttribute(member_decode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kInflateSmem));
   counter->fastq_streams.push_back(s);
   cleanup.s = nullptr;
   *out = s;
@@ -553,6 +719,151 @@ int sgc_fastq_stream_finish(sgc_fastq_stream* s, uint64_t* n_records) {
     }
   }
   if (n_records) *n_records = s->records_total;
+  return SGC_OK;
+}
+
+int sgc_fastq_stream_submit_member(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes) {
+  if (!s || !gz) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
+  if (s->failed || !s->counter) return set_error(SGC_ERR_INVALID_ARG, "the stream has failed or its counter is gone");
+  if (s->member_submitted || s->blocks_total)
+    return set_error(SGC_ERR_INVALID_ARG, "a gzip member goes to a fresh stream, once");
+  s->member_submitted = true;
+  DeviceGuard guard(s->device);
+  auto decline = [&](const char* why) {
+    s->failed = true;
+    char buf[200];
+    snprintf(buf, sizeof buf, "single gzip member not decoded on the device: %s", why);
+    return set_error(SGC_ERR_GZIP, buf);
+  };
+  size_t header = 0;
+  if (inflate::gzip_header(gz, (size_t)n_bytes, &header) != inflate::kOk) return decline("not a gzip member");
+  // Nominal piece size: 32 KiB of compressed input (more pieces than larger ones would give keep more
+  // threads busy; each piece is a serial decode).  SGC_MEMBER_PIECE overrides it and SGC_MEMBER_SKEW=1
+  // moves every other candidate start one bit on (tests: many pieces on small files, absorbed pieces);
+  // SGC_MEMBER_WAVE_TEXT bounds the text of a wave (tests: many waves).
+  uint64_t piece = 32u << 10;
+  if (const char* e = getenv("SGC_MEMBER_PIECE"); e && atoll(e) >= 64) piece = (uint64_t)atoll(e);
+  const char* skew_env = getenv("SGC_MEMBER_SKEW");
+  const bool skew = skew_env && atoi(skew_env) != 0;
+  uint64_t wave_text = s->read_len ? (4ull << 30) : (3ull << 30);
+  if (const char* e = getenv("SGC_MEMBER_WAVE_TEXT"); e && atoll(e) > 0) wave_text = std::min<uint64_t>(wave_text, (uint64_t)atoll(e));
+
+  // 1. candidate starts near every nominal boundary; the member's first block is piece 0
+  const uint32_t n_bounds = (uint32_t)((n_bytes + piece - 1) / piece);
+  int rc = grow(&s->d_gz, &s->gz_cap, (size_t)n_bytes + 64, s->pool, s->stream);  // (the reader's slack)
+  if (rc == SGC_OK) rc = grow(&s->d_cand, &s->cand_cap, (size_t)n_bounds + 1, s->pool, s->stream);
+  if (rc) return rc;
+  SGC_CUDA_TRY(cudaMemcpyAsync(s->d_gz, gz, n_bytes, cudaMemcpyHostToDevice, s->stream));
+  constexpr uint32_t kWarps = kInflateThreads / 32;
+  if (n_bounds > 1)
+    member_find_kernel<<<(n_bounds - 1 + kWarps - 1) / kWarps, kInflateThreads, kInflateSmem, s->stream>>>(s->d_gz, n_bytes, piece,
+                                                                                                          n_bounds, s->d_cand);
+  SGC_CUDA_TRY(cudaGetLastError());
+  std::vector<uint64_t> cand((size_t)n_bounds + 1, ~0ull);
+  if (n_bounds > 1) SGC_CUDA_TRY(cudaMemcpyAsync(cand.data() + 1, s->d_cand + 1, (n_bounds - 1) * 8ull, cudaMemcpyDeviceToHost, s->stream));
+  SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+  std::vector<uint64_t> starts{(uint64_t)header * 8};
+  for (uint32_t j = 1; j < n_bounds; ++j) {
+    if (cand[j] == ~0ull) continue;
+    const uint64_t c = cand[j] + (skew && (starts.size() & 1) ? 1 : 0);
+    if (c > starts.back()) starts.push_back(c);
+  }
+  const uint32_t n = (uint32_t)starts.size();
+
+  // 2. every piece to its first block end at or beyond the next candidate
+  rc = grow(&s->d_meta, &s->meta_cap, (size_t)n, s->pool, s->stream);
+  if (rc) return rc;
+  SGC_CUDA_TRY(cudaMemcpyAsync(s->d_cand, starts.data(), n * 8ull, cudaMemcpyHostToDevice, s->stream));
+  member_boundary_kernel<<<(n + kInflateThreads - 1) / kInflateThreads, kInflateThreads, kInflateSmem, s->stream>>>(
+      s->d_gz, n_bytes, s->d_cand, n, s->d_meta);
+  SGC_CUDA_TRY(cudaGetLastError());
+  std::vector<PieceMeta> meta(n);
+  SGC_CUDA_TRY(cudaMemcpyAsync(meta.data(), s->d_meta, n * sizeof(PieceMeta), cudaMemcpyDeviceToHost, s->stream));
+  SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+
+  // 3. the chain from the first block; its last piece ends the member, whose trailer must end the file
+  std::vector<uint32_t> next(n), chain(n);
+  std::vector<int> status(n);
+  for (uint32_t j = 0; j < n; ++j) next[j] = meta[j].next, status[j] = meta[j].status;
+  uint64_t absorbed = 0;
+  const uint32_t n_chain = inflate::piece_chain(next.data(), status.data(), n, chain.data(), &absorbed);
+  if (n_chain == 0) return decline("its blocks could not be followed from piece to piece");
+  const uint64_t trailer = (meta[chain[n_chain - 1]].end_bit + 7) / 8;
+  if (trailer + 8 != n_bytes) return decline("the member's trailer does not end the file");
+  uint64_t total = 0;
+  for (uint32_t i = 0; i < n_chain; ++i) total += meta[chain[i]].out_len;
+  const uint32_t want_crc = (uint32_t)gz[trailer] | ((uint32_t)gz[trailer + 1] << 8) | ((uint32_t)gz[trailer + 2] << 16) |
+                            ((uint32_t)gz[trailer + 3] << 24);
+  const uint32_t isize = (uint32_t)gz[trailer + 4] | ((uint32_t)gz[trailer + 5] << 8) | ((uint32_t)gz[trailer + 6] << 16) |
+                         ((uint32_t)gz[trailer + 7] << 24);
+  if (isize != (uint32_t)total) return decline("ISIZE differs from the length of the inflated text");
+  s->member_pieces = n;
+  s->member_chain = n_chain;
+  s->member_absorbed = absorbed;
+
+  // 4-7. waves of chain pieces: symbols, windows, text, CRC-32, framing and counting
+  for (int w = 0; w < 2; ++w)
+    if (!s->d_window[w]) {
+      if ((rc = scratch_alloc(reinterpret_cast<void**>(&s->d_window[w]), inflate::kWindow, s->pool, s->stream))) return rc;
+    }
+  SGC_CUDA_TRY(cudaMemsetAsync(s->d_window[0], 0, inflate::kWindow, s->stream));
+  int cur = 0;
+  uint32_t crc = 0;
+  uint64_t done = 0;  // text of the waves before
+  std::vector<WavePiece> h_wave;
+  std::vector<uint32_t> h_crc;
+  for (uint32_t a = 0; a < n_chain;) {
+    uint32_t b = a;
+    uint64_t text = 0;
+    while (b < n_chain && (b == a || text + meta[chain[b]].out_len <= wave_text)) text += meta[chain[b++]].out_len;
+    const uint32_t nw = b - a;
+    if (s->read_len == 0 && text >= (1ull << 32) - 2 * kHeadroom) return decline("a piece inflates to 4 GiB or more");
+    h_wave.resize((size_t)nw + 1);
+    uint64_t off = 0;
+    for (uint32_t i = 0; i < nw; ++i) {
+      const PieceMeta& m = meta[chain[a + i]];
+      const uint64_t global = done + off;
+      h_wave[i] = WavePiece{starts[chain[a + i]], m.end_bit, off, global < inflate::kWindow ? global : inflate::kWindow};
+      off += m.out_len;
+    }
+    h_wave[nw] = WavePiece{0, 0, text, 0};
+    rc = grow(&s->d_wave, &s->wave_cap, (size_t)nw + 1, s->pool, s->stream);
+    if (rc == SGC_OK) rc = grow(&s->d_sym, &s->sym_cap, (size_t)text + 1, s->pool, s->stream);
+    if (rc == SGC_OK) rc = grow(&s->d_text, &s->text_cap, (size_t)kHeadroom + text + 64, s->pool, s->stream);
+    if (rc == SGC_OK) rc = grow(&s->d_crc, &s->crc_cap, (size_t)nw, s->pool, s->stream);
+    if (rc) return rc;
+    SGC_CUDA_TRY(cudaMemcpyAsync(s->d_wave, h_wave.data(), h_wave.size() * sizeof(WavePiece), cudaMemcpyHostToDevice, s->stream));
+    uint8_t* wave_text_ptr = s->d_text + kHeadroom;
+    member_decode_kernel<<<(nw + kInflateThreads - 1) / kInflateThreads, kInflateThreads, kInflateSmem, s->stream>>>(
+        s->d_gz, n_bytes, s->d_wave, nw, s->d_sym, s->d_state);
+    member_window_kernel<<<1, kWindowThreads, 0, s->stream>>>(s->d_sym, s->d_wave, nw, wave_text_ptr, s->d_window[cur]);
+    member_resolve_kernel<<<nw, 256, 0, s->stream>>>(s->d_sym, s->d_wave, wave_text_ptr, s->d_window[cur]);
+    member_crc_kernel<<<(nw + kCrcWarps - 1) / kCrcWarps, kCrcWarps * 32, 0, s->stream>>>(s->d_wave, nw, wave_text_ptr, s->d_crc);
+    member_window_save_kernel<<<32, 256, 0, s->stream>>>(wave_text_ptr, text, s->d_window[cur], s->d_window[cur ^ 1]);
+    cur ^= 1;
+    SGC_CUDA_TRY(cudaGetLastError());
+    wave_begin_kernel<<<1, 1, 0, s->stream>>>(s->d_state, 0, 0);
+    rc = frame_and_count(s, text, a);  // (synchronises: a piece that did not decode is reported there)
+    if (rc) return rc;
+    h_crc.resize(nw);
+    SGC_CUDA_TRY(cudaMemcpyAsync(h_crc.data(), s->d_crc, nw * 4ull, cudaMemcpyDeviceToHost, s->stream));
+    SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+    for (uint32_t i = 0; i < nw; ++i) crc = inflate::crc_combine(crc, h_crc[i], h_wave[i + 1].off - h_wave[i].off);
+    done += text;
+    a = b;
+  }
+  if (crc != want_crc) {
+    s->failed = true;
+    return set_error(SGC_ERR_GZIP, "gzip member: CRC-32 of the inflated bytes differs from the member's trailer");
+  }
+  return SGC_OK;
+}
+
+int sgc_fastq_stream_member_stats(const sgc_fastq_stream* s, uint64_t* pieces, uint64_t* chain, uint64_t* absorbed) {
+  if (!s || !pieces || !chain || !absorbed) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
+  *pieces = s->member_pieces;
+  *chain = s->member_chain;
+  *absorbed = s->member_absorbed;
   return SGC_OK;
 }
 

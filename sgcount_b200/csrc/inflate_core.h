@@ -33,6 +33,7 @@ enum Status : int {
   kBadCode = 4,        // a bit pattern that is no code, or an invalid length / distance symbol
   kBadDistance = 5,    // a match reaching before the start of the member's output
   kOutputFull = 6,     // more output than the caller's capacity
+  kNoEnd = 7,          // a piece of a member: no block end where the next piece starts (see inflate_piece)
 };
 
 constexpr int kMaxBits = 15;
@@ -162,6 +163,12 @@ struct BitReader {
   // bytes of input consumed so far, counting whole bytes still in the buffer as unread
   SGC_HD size_t consumed() const { return next - (size_t)(cnt >> 3); }
   SGC_HD void align_to_byte() { drop(cnt & 7); }
+  // the same reader started at bit `bit` of the range, and the bit it has reached
+  SGC_HD void init_bit(const uint8_t* in, size_t n, uint64_t bit) {
+    init(in, n, (size_t)(bit >> 3));
+    drop((int)(bit & 7));  // (init leaves at least 8 bits in the buffer)
+  }
+  SGC_HD uint64_t bit_pos() const { return (uint64_t)next * 8 - (uint64_t)cnt; }
 };
 
 // Output of one member, written in ALIGNED 64-bit words: the bytes of the word in progress collect
@@ -597,6 +604,236 @@ SGC_HD int gunzip_member(const uint8_t* in, size_t in_len, uint8_t* out, size_t 
   return kOk;
 }
 
+// ---- ONE member in pieces ---------------------------------------------------------------------
+// A single gzip member (what gzip and pigz write) is one DEFLATE stream; it is decoded in parallel
+// by speculation (gzip.cu member_* kernels; host/member_core_test.cpp runs the same steps serially):
+//   1. near every C-th byte, the first bit where a dynamic-Huffman block header parses and a short
+//      trial decode behind it succeeds (probe_block_start) is a candidate piece start;
+//   2. every piece is decoded without output up to the first block end at or beyond the next
+//      candidate (piece_boundary); ending exactly on one links the two, overshooting absorbs it;
+//   3. the links followed from the member's first block give the true block boundaries;
+//   4. each piece on that chain is decoded into 16-bit symbols: 0-255 bytes, 256 + i byte i of the
+//      32 KiB window in front of the piece, still unknown (MarkSink);
+//   5. the windows are resolved piece after piece, then everything else in parallel.
+// These functions are written for that use, separately from gunzip_member, whose symbol loop is the
+// BGZF decoder's hot path and stays as it is.
+constexpr uint32_t kWindow = 32768;
+constexpr uint32_t kPieceFinal = 0xFFFFFFFFu;  // `next` of a piece that ends with the member's last block
+constexpr int kProbeTrial = 64;                // symbols a candidate block start must decode
+constexpr uint32_t kMaxAbsorb = 8;             // candidates a piece may run past before it gives up
+
+// The RFC 1952 header (FEXTRA, FNAME, FCOMMENT, FHCRC): kOk and *pos = where the DEFLATE stream starts.
+SGC_HD int gzip_header(const uint8_t* in, size_t in_len, size_t* pos_out) {
+  if (in_len < 18) return in_len < 4 || (in[0] == 0x1f && in[1] == 0x8b) ? kTruncated : kBadHeader;
+  if (in[0] != 0x1f || in[1] != 0x8b || in[2] != 8 || (in[3] & 0xE0)) return kBadHeader;
+  const uint8_t flg = in[3];
+  size_t pos = 10;
+  if (flg & 4) {
+    if (pos + 2 > in_len) return kTruncated;
+    pos += 2 + ((size_t)in[pos] | ((size_t)in[pos + 1] << 8));
+  }
+  for (int field = 0; field < 2; ++field)
+    if (flg & (field ? 16 : 8)) {
+      while (pos < in_len && in[pos]) ++pos;
+      ++pos;
+    }
+  if (flg & 2) pos += 2;
+  if (pos >= in_len) return kTruncated;
+  *pos_out = pos;
+  return kOk;
+}
+
+// one literal/length or distance symbol (-1: no code)
+template <typename Tables>
+SGC_HD int decode_litlen(BitReader& br, Tables t) {
+  br.refill();
+  const uint16_t e = t.get_lfast((int)br.peek(kFastBits));
+  if (e) {
+    br.drop(e & 15);
+    return e >> 4;
+  }
+  return decode_slow(br, [&](int l) { return (int)t.get_lcount(l); }, [&](int k) { return (int)t.get_lsym(k); });
+}
+template <typename Tables>
+SGC_HD int decode_dist(BitReader& br, Tables t) {
+  br.refill();
+  const uint16_t e = t.get_dfast((int)br.peek(kDistFastBits));
+  if (e) {
+    br.drop(e & 15);
+    return e >> 4;
+  }
+  return decode_slow(br, [&](int l) { return (int)t.get_dcount(l); }, [&](int k) { return (int)t.get_dsym(k); });
+}
+
+// Where a piece's output goes.  `reach`: how far before the piece's first byte a match may copy
+// from (0 for the member's first piece; a match reaching further is kBadDistance).
+struct CountSink {  // nothing: only the length
+  uint64_t op, reach;
+  SGC_HD int literal(uint32_t) {
+    ++op;
+    return kOk;
+  }
+  SGC_HD int match(uint32_t len, uint32_t dist) {
+    if (dist > op + reach) return kBadDistance;
+    op += len;
+    return kOk;
+  }
+  SGC_HD int stored(const uint8_t*, uint32_t n) {
+    op += n;
+    return kOk;
+  }
+};
+struct MarkSink {  // 16-bit symbols: a byte, or 256 + i for byte i of the window in front of the piece
+  uint16_t* out;
+  uint64_t op, cap, reach;
+  SGC_HD int literal(uint32_t b) {
+    if (op >= cap) return kOutputFull;
+    out[op++] = (uint16_t)b;
+    return kOk;
+  }
+  SGC_HD int match(uint32_t len, uint32_t dist) {
+    if (dist > op + reach) return kBadDistance;
+    if (op + len > cap) return kOutputFull;
+    for (uint32_t i = 0; i < len; ++i, ++op) {
+      // a source before the piece is a window marker; a source that is a marker copies the marker
+      const int64_t s = (int64_t)op - (int64_t)dist;
+      out[op] = s >= 0 ? out[s] : (uint16_t)(256 + (int64_t)kWindow + s);
+    }
+    return kOk;
+  }
+  SGC_HD int stored(const uint8_t* p, uint32_t n) {
+    if (op + n > cap) return kOutputFull;
+    for (uint32_t i = 0; i < n; ++i) out[op++] = p[i];
+    return kOk;
+  }
+};
+
+// Decodes blocks of the DEFLATE stream in[0 .. in_len) from bit `start` (a block header) until the
+// end of the member's last block or a block end `stop(end_bit)` accepts; *end_bit, *final_block say
+// which.  A reader position beyond `limit_bit` is kNoEnd.  Reads stay inside the BitReader's range
+// and slack (garbage input included); the sink is the only thing written.
+template <typename Tables, typename Sink, typename Stop>
+SGC_HD int inflate_piece(const uint8_t* in, size_t in_len, uint64_t start, uint64_t limit_bit, Tables t, Sink& out, Stop stop,
+                         uint64_t* end_bit, bool* final_block) {
+  if (start >= (uint64_t)in_len * 8) return kTruncated;
+  BitReader br;
+  br.init_bit(in, in_len, start);
+  for (;;) {
+    br.refill();
+    const uint32_t last = br.take(1);
+    const uint32_t type = br.take(2);
+    if (type == 0) {
+      br.align_to_byte();
+      br.refill();
+      const uint32_t n = br.take(16);
+      br.refill();
+      const uint32_t nn = br.take(16);
+      const size_t at = br.consumed();
+      if ((n ^ nn) != 0xFFFFu) return br.overrun ? kTruncated : kBadBlock;
+      if (at + n > in_len) return kTruncated;
+      if ((uint64_t)(at + n) * 8 > limit_bit) return kNoEnd;
+      if (int rc = out.stored(in + at, n)) return rc;
+      br.init(in, in_len, at + n);
+    } else if (type == 3) {
+      return br.overrun ? kTruncated : kBadBlock;
+    } else {
+      BitReader header_reader = br;  // (a copy, as in gunzip_member: `br` stays in registers)
+      const int rc = read_codes(header_reader, t, type);
+      br = header_reader;
+      if (rc != kOk) return rc;
+      for (;;) {
+        if (br.bit_pos() > limit_bit) return kNoEnd;
+        int sym = decode_litlen(br, t);
+        if (sym < 0 || sym > 285) return br.overrun ? kTruncated : kBadCode;
+        if (sym == 256) break;
+        if (sym < 256) {
+          if (int rc = out.literal((uint32_t)sym)) return rc;
+          continue;
+        }
+        sym -= 257;
+        const uint32_t len = len_base(sym) + br.take((int)len_extra_bits(sym));
+        const int ds = decode_dist(br, t);
+        if (ds < 0 || ds >= 30) return br.overrun ? kTruncated : kBadCode;
+        const uint32_t dist = dist_base(ds) + br.take((int)dist_extra_bits(ds));
+        if (int rc = out.match(len, dist)) return rc;
+      }
+    }
+    if (br.overrun) return kTruncated;
+    const uint64_t e = br.bit_pos();
+    if (e > limit_bit) return kNoEnd;
+    if (last || stop(e)) {
+      *end_bit = e;
+      *final_block = last != 0;
+      return kOk;
+    }
+  }
+}
+
+// Does a dynamic-Huffman block that is not the member's last start at bit `bit`?  Its header must
+// parse (read_codes: HLIT, HDIST <= 29, a complete code-length code, lengths that form valid codes
+// with an end-of-block code) and `trial` symbols after it, or up to its end, must decode.
+template <typename Tables>
+SGC_HD bool probe_block_start(const uint8_t* in, size_t in_len, uint64_t bit, Tables t, int trial) {
+  BitReader br;
+  br.init_bit(in, in_len, bit);
+  br.refill();
+  if (br.peek(3) != 4u) return false;  // BFINAL = 0, BTYPE = 10
+  if ((br.peek(8) >> 3) > 29u || (br.peek(13) >> 8) > 29u) return false;
+  br.drop(3);
+  if (read_codes(br, t, 2) != kOk || br.overrun) return false;
+  for (int i = 0; i < trial; ++i) {
+    int sym = decode_litlen(br, t);
+    if (sym < 0 || sym > 285) return false;
+    if (sym == 256) break;
+    if (sym > 256) {
+      br.take((int)len_extra_bits(sym - 257));
+      const int ds = decode_dist(br, t);
+      if (ds < 0 || ds >= 30) return false;
+      br.take((int)dist_extra_bits(ds));
+    }
+  }
+  return !br.overrun;
+}
+
+// Step 2 for piece j of `n` whose candidate starts (bits, increasing) are starts[0 .. n): decodes it
+// without output to the first block end at or beyond starts[j + 1].  kOk: *next = the piece that
+// starts exactly there (j + 1, or up to j + 1 + max_absorb when candidates in between were false or
+// skipped), or kPieceFinal when the member's last block ended first; *end_bit and *out_len describe
+// the piece.  Anything else means the piece does not lie on the chain.
+template <typename Tables>
+SGC_HD int piece_boundary(const uint8_t* in, size_t in_len, const uint64_t* starts, uint32_t n, uint32_t j,
+                          uint32_t max_absorb, Tables t, uint32_t* next, uint64_t* end_bit, uint64_t* out_len) {
+  CountSink sink{0, j == 0 ? 0u : kWindow};
+  const uint32_t last_ok = j + 1 + max_absorb < n ? j + 1 + max_absorb : n - 1;
+  const uint64_t limit = j + 1 + max_absorb < n ? starts[j + 1 + max_absorb] : (uint64_t)in_len * 8;
+  uint32_t m = j + 1;
+  auto stop = [&](uint64_t e) {
+    while (m < n && starts[m] < e) ++m;
+    return m < n && starts[m] == e;
+  };
+  bool fin = false;
+  const int rc = inflate_piece(in, in_len, starts[j], limit, t, sink, stop, end_bit, &fin);
+  if (rc != kOk) return rc;
+  if (!fin && m > last_ok) return kNoEnd;
+  *next = fin ? kPieceFinal : m;
+  *out_len = sink.op;
+  return kOk;
+}
+
+// Step 3 (host): the pieces linked from piece 0 into chain[]; returns their number, or 0 when the
+// links reach a piece whose step 2 failed (status != kOk).  *absorbed: candidates run past.
+inline uint32_t piece_chain(const uint32_t* next, const int* status, uint32_t n, uint32_t* chain, uint64_t* absorbed) {
+  uint32_t len = 0, j = 0;
+  *absorbed = 0;
+  for (;;) {
+    if (j >= n || status[j] != kOk) return 0;
+    chain[len++] = j;
+    if (next[j] == kPieceFinal) return len;
+    *absorbed += next[j] - j - 1;
+    j = next[j];
+  }
+}
+
 }  // namespace inflate
 }  // namespace sgc
 
@@ -642,6 +879,9 @@ SGC_HD uint32_t crc_x8n(uint64_t n) {
   }
   return p;
 }
+
+// CRC-32 of A || B from crc(A), crc(B) and |B|
+SGC_HD uint32_t crc_combine(uint32_t crc_a, uint32_t crc_b, uint64_t len_b) { return crc_multmodp(crc_x8n(len_b), crc_a) ^ crc_b; }
 
 // standard CRC-32 of bytes [0, n) given a 256-entry table accessor
 template <typename Table>

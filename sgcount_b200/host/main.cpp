@@ -15,6 +15,7 @@
 #include <sys/mman.h>
 #include <sys/stat.h>
 #include <unistd.h>
+#include <zlib.h>
 
 #include <atomic>
 #include <chrono>
@@ -94,7 +95,7 @@ const char* kUsage =
     "      --ingest-threads <N>               Threads inflating the gzip members of one sample [default: cores / samples in flight]\n"
     "      --rc-keep-n                        Reverse complement keeps N (default: the fxread bit trick, N -> J)\n"
     "      --whole-lines                      Copy whole sequence lines to the device (default: for fixed-length reads, only the guide window and one byte either side)\n"
-    "      --host-inflate                     Inflate and frame records on the host even for BGZF input (default: BGZF files of fixed-length FASTQ are inflated, framed and counted on the device)\n"
+    "      --host-inflate                     Inflate and frame records on the host even for BGZF or single-member gzip input (default: BGZF files of FASTQ, and gzip files of FASTQ that are one member, are inflated, framed and counted on the device)\n"
     "      --timing                           Print a JSON line with the phase times to stderr\n"
     "  -h, --help                             Print help\n";
 
@@ -381,6 +382,7 @@ struct SampleResult {
   double dev_index_s = 0, dev_create_s = 0, dev_waves_s = 0, dev_finish_s = 0;  // phases of the device ingest
   bool device_ingest = false;               // inflate and record framing ran on the device (BGZF input)
   uint64_t device_blocks = 0;
+  uint64_t member_pieces = 0, member_chain = 0, member_absorbed = 0;  // one gzip member in pieces on the device
   std::string host_because;                 // why the device ingest was not used
 };
 
@@ -466,16 +468,84 @@ bool plan_waves(const uint8_t* file, const std::vector<uint64_t>& begin, const s
   return true;
 }
 
+// Is the file one gzip member?  Every later position that looks like a member start (the host
+// reader's signature scan: 1f 8b 08, reserved flags clear) is tried with zlib; in compressed data such
+// a position is a coincidence (one in a few MB) that zlib rejects within a few bytes.  The device
+// confirms it: the member's trailer must end the file.
+bool is_single_member(const uint8_t* d, size_t n) {
+  for (const uint8_t* p = d + 1; p + 4 <= d + n; ++p) {
+    p = static_cast<const uint8_t*>(memchr(p, 0x1f, (size_t)(d + n - p)));
+    if (!p || p + 4 > d + n) break;
+    if (p[1] != 0x8b || p[2] != 0x08 || (p[3] & 0xE0) != 0) continue;
+    z_stream zs{};
+    if (inflateInit2(&zs, 15 + 16) != Z_OK) return false;
+    uint8_t out[4096];
+    zs.next_in = const_cast<uint8_t*>(p);
+    zs.avail_in = (uInt)std::min<size_t>((size_t)(d + n - p), 1u << 20);
+    zs.next_out = out;
+    zs.avail_out = sizeof out;
+    const int rc = inflate(&zs, Z_NO_FLUSH);
+    const bool member = (rc == Z_OK || rc == Z_STREAM_END) && (zs.avail_out == 0 || rc == Z_STREAM_END);
+    inflateEnd(&zs);
+    if (member) return false;
+  }
+  return true;
+}
+
+// A single-member (not BGZF) gzip FASTQ through sgc_fastq_stream_submit_member on one device.
+bool count_member_on_device(const sgc_library* lib, uint32_t n_guides, const MappedFile& file, OffsetValue offset, uint32_t span_offset,
+                            uint32_t read_len, uint32_t span_start, uint32_t span_len, bool variable, bool recursion, int rc_mode,
+                            SampleResult& r, std::string& why_not) {
+  const auto t0 = std::chrono::steady_clock::now();
+  struct Guard {
+    sgc_counter* c = nullptr;
+    sgc_fastq_stream* s = nullptr;
+    ~Guard() {
+      sgc_fastq_stream_destroy(s);
+      sgc_counter_destroy(c);
+    }
+  } g;
+  check(sgc_counter_create(lib, offset.reverse, span_offset, recursion, rc_mode, nullptr, nullptr, &g.c));
+  check(sgc_fastq_stream_create(g.c, variable ? 0 : read_len, span_start, span_len, &g.s));
+  const auto t1 = std::chrono::steady_clock::now();
+  uint64_t n_records = 0;
+  int rc = sgc_fastq_stream_submit_member(g.s, file.data, file.size);
+  const auto t2 = std::chrono::steady_clock::now();
+  if (rc == SGC_OK) rc = sgc_fastq_stream_finish(g.s, &n_records);
+  if (rc == SGC_ERR_GZIP || rc == SGC_ERR_FASTQ_FORMAT) {
+    why_not = sgc_last_error();
+    return false;
+  }
+  if (rc != SGC_OK) fail("%s", sgc_last_error());
+  check(sgc_fastq_stream_member_stats(g.s, &r.member_pieces, &r.member_chain, &r.member_absorbed));
+  r.counts.resize(n_guides);
+  check(sgc_counter_finish(g.c, r.counts.data(), &r.total, &r.matched));
+  const auto t3 = std::chrono::steady_clock::now();
+  auto seconds = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
+    return std::chrono::duration<double>(b - a).count();
+  };
+  r.span_reads = variable ? 0 : n_records;
+  r.line_reads = variable ? n_records : 0;
+  r.device_ingest = true;
+  r.shards = 1;
+  r.submit_s = seconds(t0, t3);
+  r.dev_create_s = seconds(t0, t1);
+  r.dev_waves_s = seconds(t1, t2);
+  r.dev_finish_s = seconds(t2, t3);
+  return true;
+}
+
 // One sample through the device ingest, on one device or — `libs.size()` > 1 — with its waves
 // dealt to several, one host thread each, the devices' count vectors summed at the end
-// (sgc_reduce_counts).  Returns false when the file is not BGZF or the device reports input it
+// (sgc_reduce_counts).  A single gzip member that is not BGZF goes to the first device
+// (count_member_on_device) when `member_ok`.  Returns false when the file is neither or the device reports input it
 // does not take — a read of another length (span mode), FASTA, a damaged block — so that the
 // caller can try the other mode or the host path.
 // `variable`: reads of any length (the sequence lines are counted where they lie in the inflated
 // text); otherwise every read has read_len bytes and only its guide-window span is kept.
 bool count_sample_on_device(const std::vector<const sgc_library*>& libs, uint32_t n_guides, uint32_t k, const std::string& path,
-                            OffsetValue offset, uint32_t read_len, bool variable, bool recursion, int rc_mode, SampleResult& r,
-                            std::string& why_not) {
+                            OffsetValue offset, uint32_t read_len, bool variable, bool recursion, int rc_mode, bool member_ok,
+                            SampleResult& r, std::string& why_not) {
   uint32_t span_start = 0, span_len = 0, span_offset = offset.index;
   if (!variable && sgc_span_geometry(k, read_len, offset.reverse, offset.index, recursion, &span_start, &span_len,
                                      &span_offset) != SGC_OK) {
@@ -494,8 +564,16 @@ bool count_sample_on_device(const std::vector<const sgc_library*>& libs, uint32_
   std::vector<uint64_t> begin;
   std::vector<uint32_t> isize;
   if (!bgzf_index(file.data, file.size, begin, isize, std::min(8u, std::max(1u, std::thread::hardware_concurrency())))) {
-    why_not = "not BGZF";
-    return false;
+    if (!member_ok) {
+      why_not = "not BGZF, and read shards asked for";
+      return false;
+    }
+    if (!is_single_member(file.data, file.size)) {
+      why_not = "not BGZF, and more than one gzip member";
+      return false;
+    }
+    return count_member_on_device(libs[0], n_guides, file, offset, span_offset, read_len, span_start, span_len, variable, recursion,
+                                  rc_mode, r, why_not);
   }
   const auto t_indexed = std::chrono::steady_clock::now();
   const size_t n_blocks = isize.size(), n_dev = libs.size();
@@ -860,6 +938,7 @@ int main(int argc, char** argv) {
     std::vector<uint32_t> first_len(n_samples);
     std::vector<char> head_uniform(n_samples, 0), head_fastq(n_samples, 0);  // 4-line FASTQ? head reads of one length?
     bool all_for_the_device = !args.host_inflate;
+    const bool member_ok = args.read_shards <= 1;  // (read shards asked for: one member keeps the host path)
     for (size_t i = 0; i < n_samples; ++i) {
       first_len[i] = (uint32_t)heads[i].first_len;
       head_fastq[i] = heads[i].fastq;
@@ -894,11 +973,11 @@ int main(int argc, char** argv) {
             // reported by the device deeper in the file) with their sequence lines in place
             bool variable = !head_uniform[s] || args.whole_lines;
             on_device = count_sample_on_device(sample_libs, hlib.n, hlib.k, args.input_paths[s], offsets[s], first_len[s],
-                                               variable, !args.no_position_recursion, args.rc_mode, results[s], why_not);
+                                               variable, !args.no_position_recursion, args.rc_mode, member_ok, results[s], why_not);
             if (!on_device && !variable && why_not.find("FASTQ") != std::string::npos) {
               results[s] = SampleResult();
               on_device = count_sample_on_device(sample_libs, hlib.n, hlib.k, args.input_paths[s], offsets[s], first_len[s],
-                                                 true, !args.no_position_recursion, args.rc_mode, results[s], why_not);
+                                                 true, !args.no_position_recursion, args.rc_mode, member_ok, results[s], why_not);
             }
           } else if (!head_fastq[s]) {
             why_not = "not FASTQ";
@@ -937,7 +1016,7 @@ int main(int argc, char** argv) {
       unsigned long long reads = 0;
       double wait_s = 0, copy_s = 0, submit_s = 0;
       unsigned max_shards = 1;
-      unsigned long long span_reads = 0, device_blocks = 0, adopted = 0, reframed = 0;
+      unsigned long long span_reads = 0, device_blocks = 0, adopted = 0, reframed = 0, pieces = 0, chain = 0, absorbed = 0;
       unsigned device_samples = 0;
       std::string host_because;
       double dev_index_s = 0, dev_create_s = 0, dev_waves_s = 0, dev_finish_s = 0;
@@ -948,6 +1027,7 @@ int main(int argc, char** argv) {
         adopted += r.members_adopted, reframed += r.members_reframed;
         device_samples += r.device_ingest;
         device_blocks += r.device_blocks;
+        pieces += r.member_pieces, chain += r.member_chain, absorbed += r.member_absorbed;
         if (!r.device_ingest && host_because.empty()) host_because = r.host_because;
         max_shards = std::max(max_shards, r.shards);
       }
@@ -955,10 +1035,10 @@ int main(int argc, char** argv) {
               "\"ingest_threads\": %u, \"gpus\": %d, \"read_shards_per_sample\": %u, \"span_reads\": %llu, \"device_ingest_samples\": %u, "
               "\"device_blocks\": %llu, \"device_phases_s\": [%.4f, %.4f, %.4f, %.4f], \"host_ingest_because\": \"%s\", \"members_adopted\": %llu, \"members_reframed\": %llu, \"wait_inflate_s\": %.6f, "
               "\"copy_to_pinned_s\": %.6f, \"submit_sync_s\": %.6f, \"read_inputs_s\": %.3f, "
-              "\"device_tables_s\": %.3f, \"offsets_s\": %.3f}\n",
+              "\"device_tables_s\": %.3f, \"offsets_s\": %.3f, \"member_pieces\": %llu, \"member_chain\": %llu, \"member_absorbed\": %llu}\n",
               count_s, reads, n_samples, workers, ingest_threads, gpus, max_shards, span_reads, device_samples, device_blocks,
               dev_index_s, dev_create_s, dev_waves_s, dev_finish_s, host_because.c_str(), adopted, reframed, wait_s, copy_s, submit_s, t_inputs,
-              t_tables - t_inputs, t_offsets - t_tables);
+              t_tables - t_inputs, t_offsets - t_tables, pieces, chain, absorbed);
     }
 
     // write_results (results.rs:71-99).  Counts are keyed by alias (counter.rs:232-235):

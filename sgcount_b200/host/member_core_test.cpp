@@ -1,0 +1,125 @@
+// member_core_test <file.gz> <piece_bytes> <skew 0|1> — decodes a single-member gzip file the way the
+// device does (gzip.cu member_* kernels), serially, from the same csrc/inflate_core.h code: candidate
+// block starts every piece_bytes of compressed input (with skew, every other candidate moved one bit on),
+// the boundary pass, the chain, 16-bit symbols with window markers, the window resolution piece after
+// piece and then the rest, CRC-32 in pieces joined, the trailer.  Prints
+// "<bytes> <fnv1a> <pieces> <chain> <absorbed>" (exit 0), "decline ..." when the chain does not reach
+// the member's end (exit 3: the device would hand the file to the host), or the error (exit 4).
+// Test helper for tests/test_member_inflate_core.py; zlib is the comparison.
+#include <cstdio>
+#include <cstdlib>
+#include <vector>
+
+#include "../csrc/inflate_core.h"
+
+using namespace sgc::inflate;
+
+int main(int argc, char** argv) {
+  if (argc < 4) return 2;
+  FILE* f = fopen(argv[1], "rb");
+  if (!f) return 2;
+  std::vector<unsigned char> data;
+  unsigned char buf[1 << 16];
+  for (size_t got; (got = fread(buf, 1, sizeof buf, f)) > 0;) data.insert(data.end(), buf, buf + got);
+  fclose(f);
+  const size_t n = data.size();
+  const uint64_t piece = (uint64_t)atoll(argv[2]);
+  const bool skew = atoi(argv[3]) != 0;
+  if (piece < 16) return 2;
+  data.resize(n + 64);  // the reader's slack
+  const uint8_t* in = data.data();
+  PlainTableStorage storage;
+  PlainTables t{&storage};
+
+  // 1. candidate starts: the member's first block, then one per piece of input
+  size_t pos = 0;
+  if (int rc = gzip_header(in, n, &pos)) {
+    printf("error: header status %d\n", rc);
+    return 4;
+  }
+  std::vector<uint64_t> starts{(uint64_t)pos * 8};
+  for (uint64_t j = 1; j * piece < n; ++j) {
+    const uint64_t hi = (j + 1) * piece < n ? (j + 1) * piece : n;
+    for (uint64_t bit = j * piece * 8; bit < hi * 8; ++bit)
+      if (probe_block_start(in, n, bit, t, kProbeTrial)) {
+        // (skew: every other candidate one bit late, so that the piece in front of it runs past it)
+        const uint64_t s = bit + (skew && (starts.size() & 1) ? 1 : 0);
+        if (s > starts.back()) starts.push_back(s);
+        break;
+      }
+  }
+  const uint32_t n_pieces = (uint32_t)starts.size();
+
+  // 2. every piece to its first block end at or beyond the next candidate
+  std::vector<uint32_t> next(n_pieces);
+  std::vector<int> status(n_pieces);
+  std::vector<uint64_t> end_bit(n_pieces), out_len(n_pieces);
+  for (uint32_t j = 0; j < n_pieces; ++j)
+    status[j] = piece_boundary(in, n, starts.data(), n_pieces, j, kMaxAbsorb, t, &next[j], &end_bit[j], &out_len[j]);
+
+  // 3. the chain from the first piece
+  std::vector<uint32_t> chain(n_pieces);
+  uint64_t absorbed = 0;
+  const uint32_t n_chain = piece_chain(next.data(), status.data(), n_pieces, chain.data(), &absorbed);
+  if (n_chain == 0) {
+    printf("decline: the chain of pieces does not reach the member's end\n");
+    return 3;
+  }
+  std::vector<uint64_t> off(n_chain + 1, 0);
+  for (uint32_t i = 0; i < n_chain; ++i) off[i + 1] = off[i] + out_len[chain[i]];
+  const uint64_t total = off[n_chain];
+
+  // 4. symbols of every piece on the chain
+  std::vector<uint16_t> sym(total + 1);
+  for (uint32_t i = 0; i < n_chain; ++i) {
+    const uint32_t j = chain[i];
+    MarkSink sink{sym.data() + off[i], 0, out_len[j], off[i] < kWindow ? off[i] : kWindow};
+    uint64_t e = 0;
+    bool fin = false;
+    const uint64_t want_end = end_bit[j];
+    const int rc = inflate_piece(in, n, starts[j], want_end, t, sink, [&](uint64_t b) { return b >= want_end; }, &e, &fin);
+    if (rc != kOk || e != want_end || sink.op != out_len[j]) {
+      printf("error: piece %u decodes differently the second time (status %d)\n", j, rc);
+      return 4;
+    }
+  }
+
+  // 5. the window in front of every piece, in order; then the rest
+  std::vector<uint8_t> text(total + 1);
+  auto resolve = [&](uint32_t i, uint64_t x) {
+    const uint16_t s = sym[x];
+    text[x] = s < 256 ? (uint8_t)s : text[off[i] - kWindow + (s - 256)];
+  };
+  for (uint32_t i = 0; i < n_chain; ++i)
+    for (uint64_t x = off[i + 1] - off[i] > kWindow ? off[i + 1] - kWindow : off[i]; x < off[i + 1]; ++x) resolve(i, x);
+  for (uint32_t i = 0; i < n_chain; ++i)
+    for (uint64_t x = off[i]; x + kWindow < off[i + 1]; ++x) resolve(i, x);
+
+  // 6. CRC-32 in pieces, joined; the trailer must end the file
+  uint32_t table[256];
+  for (uint32_t i = 0; i < 256; ++i) table[i] = crc_table_entry(i);
+  uint32_t crc = 0;
+  for (uint32_t i = 0; i < n_chain; ++i) {
+    const uint64_t len = off[i + 1] - off[i];
+    crc = crc_combine(crc, crc_bytes(text.data() + off[i], len, [&](uint32_t k) { return table[k]; }), len);
+  }
+  const uint64_t at = (end_bit[chain[n_chain - 1]] + 7) / 8;
+  if (at + 8 != n) {
+    printf("error: the member's trailer does not end the file\n");
+    return 4;
+  }
+  const uint32_t want_crc = (uint32_t)in[at] | ((uint32_t)in[at + 1] << 8) | ((uint32_t)in[at + 2] << 16) | ((uint32_t)in[at + 3] << 24);
+  const uint32_t isize = (uint32_t)in[at + 4] | ((uint32_t)in[at + 5] << 8) | ((uint32_t)in[at + 6] << 16) | ((uint32_t)in[at + 7] << 24);
+  if (crc != want_crc) {
+    printf("error: CRC-32 of the inflated bytes differs from the trailer\n");
+    return 4;
+  }
+  if (isize != (uint32_t)total) {
+    printf("error: ISIZE differs from the inflated length\n");
+    return 4;
+  }
+  unsigned long long h = 1469598103934665603ull;
+  for (uint64_t i = 0; i < total; ++i) h = (h ^ text[i]) * 1099511628211ull;
+  printf("%llu %llx %u %u %llu\n", (unsigned long long)total, h, n_pieces, n_chain, (unsigned long long)absorbed);
+  return 0;
+}
