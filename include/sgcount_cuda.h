@@ -274,6 +274,19 @@ int sgc_fastq_stream_submit_member(sgc_fastq_stream*, const uint8_t* gz, uint64_
 /* After sgc_fastq_stream_submit_member: candidate pieces, pieces on the chain of true block
  * boundaries, candidates the chain ran past. */
 int sgc_fastq_stream_member_stats(const sgc_fastq_stream*, uint64_t* pieces, uint64_t* chain, uint64_t* absorbed);
+/* ANY sequence of gzip members — one, several (`cat a.gz b.gz`, appending writers), or BGZF blocks —
+ * the whole file, gz[0 .. n_bytes) in host memory, inflated, framed and counted on the device, once
+ * per stream, then sgc_fastq_stream_finish.  As sgc_fastq_stream_submit_member, with every gzip header
+ * in the file a further candidate piece start where a member begins: the chain of pieces steps from a
+ * member's last block over its trailer and the next header.  The members' texts are one byte stream,
+ * as gzip -d writes it (a record may straddle two members); CRC-32 and ISIZE are checked member by
+ * member.  Fails with SGC_ERR_GZIP when the chain cannot be followed, anything but a whole member
+ * follows a trailer (zero padding included), a member's CRC-32 or ISIZE disagrees, or the file holds
+ * more gzip headers than one per 256 bytes; with SGC_ERR_FASTQ_FORMAT as sgc_fastq_stream_submit
+ * does.  sgc_fastq_stream_member_stats sums over the members. */
+int sgc_fastq_stream_submit_gzip(sgc_fastq_stream*, const uint8_t* gz, uint64_t n_bytes);
+/* Members decoded by sgc_fastq_stream_submit_gzip (1 after sgc_fastq_stream_submit_member, else 0). */
+int sgc_fastq_stream_gzip_members(const sgc_fastq_stream*, uint64_t* members);
 int sgc_fastq_stream_finish(sgc_fastq_stream*, uint64_t* n_records);
 
 /* Statistics of the last sgc_counter_submit_device call, for benchmarking. */

@@ -425,8 +425,23 @@ class FastqStream:
         check(_cabi.load().sgc_fastq_stream_submit_member(self._ptr, blob.ctypes.data, len(blob)))
         self._counter._result = None
 
+    def submit_gzip(self, blob: np.ndarray) -> None:
+        """a whole gzip file (uint8) of one or more members, BGZF included, decoded in parallel pieces on
+        the device; call once, then finish().  SgcError(ERR_GZIP) when the device declines it (count it
+        on the host instead)"""
+        blob = np.ascontiguousarray(blob, dtype=np.uint8)
+        check(_cabi.load().sgc_fastq_stream_submit_gzip(self._ptr, blob.ctypes.data, len(blob)))
+        self._counter._result = None
+
+    def gzip_members(self) -> int:
+        """members decoded by submit_gzip (1 after submit_member)"""
+        v = C.c_uint64()
+        check(_cabi.load().sgc_fastq_stream_gzip_members(self._ptr, C.byref(v)))
+        return int(v.value)
+
     def member_stats(self) -> tuple:
-        """(candidate pieces, pieces on the chain of block boundaries, candidates run past) of submit_member"""
+        """(candidate pieces, pieces on the chain of block boundaries, candidates run past) of submit_member
+        or submit_gzip, summed over the members"""
         v = [C.c_uint64() for _ in range(3)]
         check(_cabi.load().sgc_fastq_stream_member_stats(self._ptr, *[C.byref(x) for x in v]))
         return tuple(int(x.value) for x in v)

@@ -300,8 +300,10 @@ struct PieceMeta {
   uint32_t next;
   int32_t status;
 };
+// is_member[j]: piece j starts a gzip member, so none of its matches may reach in front of it
 __global__ void __launch_bounds__(kInflateThreads) member_boundary_kernel(const uint8_t* __restrict__ gz, uint64_t n_gz,
-                                                                         const uint64_t* __restrict__ starts, uint32_t n,
+                                                                         const uint64_t* __restrict__ starts,
+                                                                         const uint8_t* __restrict__ is_member, uint32_t n,
                                                                          PieceMeta* __restrict__ meta) {
   extern __shared__ uint16_t sm[];
   const uint32_t j = blockIdx.x * kInflateThreads + threadIdx.x;
@@ -309,8 +311,39 @@ __global__ void __launch_bounds__(kInflateThreads) member_boundary_kernel(const 
   DeviceSymbols symbols;
   const DeviceTables t{sm + threadIdx.x, &symbols};
   PieceMeta m{0, 0, 0, 0};
-  m.status = inflate::piece_boundary(gz, (size_t)n_gz, starts, n, j, inflate::kMaxAbsorb, t, &m.next, &m.end_bit, &m.out_len);
+  m.status = inflate::piece_boundary(gz, (size_t)n_gz, starts, n, j, inflate::kMaxAbsorb, t, &m.next, &m.end_bit, &m.out_len,
+                                     is_member[j] ? 0u : inflate::kWindow);
   meta[j] = m;
+}
+
+// Member-start candidates of several members: one thread per 4 KiB of input finds every gzip header in
+// it (inflate::member_start_at) and appends the bit its DEFLATE stream starts at to heads[] (unordered;
+// heads[cap], as a 64-bit counter, ends up holding the number found, which may exceed cap).
+constexpr uint32_t kSignatureBytes = 4096;
+__global__ void __launch_bounds__(256) member_signature_kernel(const uint8_t* __restrict__ gz, uint64_t n_gz,
+                                                              uint64_t* __restrict__ heads, uint64_t cap) {
+  const uint64_t lo = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) * kSignatureBytes;
+  if (lo >= n_gz) return;
+  const uint64_t hi = min(lo + kSignatureBytes, n_gz);
+  unsigned long long* found = reinterpret_cast<unsigned long long*>(heads + cap);
+  for (uint64_t at = lo; at < hi; at += 16) {  // (the buffer has 64 bytes of slack behind the input)
+    const uint4 v = *reinterpret_cast<const uint4*>(gz + at);
+    const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const uint32_t x = w[i] ^ 0x1F1F1F1Fu;                                  // zero byte where a 0x1f is
+      uint32_t z = ~(((x & 0x7F7F7F7Fu) + 0x7F7F7F7Fu) | x) & 0x80808080u;  // bit 7 of every zero byte
+      while (z) {
+        const uint64_t pos = at + 4 * i + ((__ffs((int)z) - 1) >> 3);
+        z &= z - 1;
+        uint64_t bit = 0;
+        if (pos < hi && inflate::member_start_at(gz, (size_t)n_gz, (size_t)pos, &bit)) {
+          const unsigned long long k = atomicAdd(found, 1ull);
+          if (k < cap) heads[k] = bit;
+        }
+      }
+    }
+  }
 }
 
 // a piece of the chain in the current wave: where its bits start and end, where its text goes
@@ -504,6 +537,11 @@ struct sgc_fastq_stream {
   size_t sym_cap = 0, cand_cap = 0, meta_cap = 0, wave_cap = 0, crc_cap = 0;
   uint64_t member_pieces = 0, member_chain = 0, member_absorbed = 0;
   bool member_submitted = false;
+  // several members (sgc_fastq_stream_submit_gzip)
+  uint64_t* d_heads = nullptr;  // member-start candidates, then their count
+  uint8_t* d_is_member = nullptr;
+  size_t heads_cap = 0, is_member_cap = 0;
+  uint64_t gzip_members = 0;
 };
 
 namespace {
@@ -577,6 +615,161 @@ int frame_and_count(sgc_fastq_stream* s, uint64_t n_text, uint64_t first_block) 
   return SGC_OK;
 }
 
+// ---- gzip members in pieces: the host side of sgc_fastq_stream_submit_member / _submit_gzip ----
+// Nominal piece size: 32 KiB of compressed input (more pieces than larger ones would give keep more
+// threads busy; each piece is a serial decode).  SGC_MEMBER_PIECE overrides it and SGC_MEMBER_SKEW=1
+// moves every other candidate start one bit on (tests: many pieces on small files, absorbed pieces);
+// SGC_MEMBER_WAVE_TEXT bounds the text of a wave (tests: many waves).
+struct MemberParams {
+  uint64_t piece, wave_text;
+  bool skew;
+};
+MemberParams member_params(const sgc_fastq_stream* s) {
+  MemberParams p{32u << 10, s->read_len ? (4ull << 30) : (3ull << 30), false};
+  if (const char* e = getenv("SGC_MEMBER_PIECE"); e && atoll(e) >= 64) p.piece = (uint64_t)atoll(e);
+  const char* skew_env = getenv("SGC_MEMBER_SKEW");
+  p.skew = skew_env && atoi(skew_env) != 0;
+  if (const char* e = getenv("SGC_MEMBER_WAVE_TEXT"); e && atoll(e) > 0) p.wave_text = std::min<uint64_t>(p.wave_text, (uint64_t)atoll(e));
+  return p;
+}
+
+// the caller counts the file on the host instead
+int member_decline(sgc_fastq_stream* s, const char* what, const char* why) {
+  s->failed = true;
+  char buf[240];
+  snprintf(buf, sizeof buf, "%s not decoded on the device: %s", what, why);
+  return set_error(SGC_ERR_GZIP, buf);
+}
+
+// 1-2. the compressed bytes to the device; candidate piece starts near every nominal boundary (the first
+// member's first block is piece 0) and, with `members`, at every gzip header; every piece to its first
+// block end at or beyond the next candidate.
+int member_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, size_t header, const MemberParams& p, bool members,
+                  const char* what, std::vector<uint64_t>& starts, std::vector<uint8_t>& is_member, std::vector<PieceMeta>& meta) {
+  const uint32_t n_bounds = (uint32_t)((n_bytes + p.piece - 1) / p.piece);
+  // member-start candidates: up to one per 256 bytes of input (fewer, larger members go to the host)
+  const uint64_t heads_cap = members ? n_bytes / 256 + 4096 : 0;
+  int rc = grow(&s->d_gz, &s->gz_cap, (size_t)n_bytes + 64, s->pool, s->stream);  // (the reader's slack)
+  if (rc == SGC_OK) rc = grow(&s->d_cand, &s->cand_cap, (size_t)n_bounds + 1, s->pool, s->stream);
+  if (rc == SGC_OK && members) rc = grow(&s->d_heads, &s->heads_cap, (size_t)heads_cap + 1, s->pool, s->stream);
+  if (rc) return rc;
+  SGC_CUDA_TRY(cudaMemcpyAsync(s->d_gz, gz, n_bytes, cudaMemcpyHostToDevice, s->stream));
+  constexpr uint32_t kWarps = kInflateThreads / 32;
+  if (n_bounds > 1)
+    member_find_kernel<<<(n_bounds - 1 + kWarps - 1) / kWarps, kInflateThreads, kInflateSmem, s->stream>>>(s->d_gz, n_bytes, p.piece,
+                                                                                                          n_bounds, s->d_cand);
+  uint64_t n_heads = 0;
+  if (members) {
+    SGC_CUDA_TRY(cudaMemsetAsync(s->d_heads + heads_cap, 0, sizeof(uint64_t), s->stream));
+    const uint64_t threads = (n_bytes + kSignatureBytes - 1) / kSignatureBytes;
+    member_signature_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, s->stream>>>(s->d_gz, n_bytes, s->d_heads, heads_cap);
+    SGC_CUDA_TRY(cudaMemcpyAsync(&n_heads, s->d_heads + heads_cap, sizeof n_heads, cudaMemcpyDeviceToHost, s->stream));
+  }
+  SGC_CUDA_TRY(cudaGetLastError());
+  std::vector<uint64_t> cand((size_t)n_bounds + 1, ~0ull);
+  if (n_bounds > 1) SGC_CUDA_TRY(cudaMemcpyAsync(cand.data() + 1, s->d_cand + 1, (n_bounds - 1) * 8ull, cudaMemcpyDeviceToHost, s->stream));
+  SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+  std::vector<uint64_t> probe{(uint64_t)header * 8};
+  for (uint32_t j = 1; j < n_bounds; ++j) {
+    if (cand[j] == ~0ull) continue;
+    const uint64_t c = cand[j] + (p.skew && (probe.size() & 1) ? 1 : 0);
+    if (c > probe.back()) probe.push_back(c);
+  }
+  if (n_heads > heads_cap) return member_decline(s, what, "more gzip headers than one per 256 bytes");
+  std::vector<uint64_t> heads(n_heads);
+  if (n_heads) {
+    SGC_CUDA_TRY(cudaMemcpyAsync(heads.data(), s->d_heads, n_heads * 8, cudaMemcpyDeviceToHost, s->stream));
+    SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+    std::sort(heads.begin(), heads.end());
+  }
+  starts.resize(probe.size() + heads.size());
+  is_member.resize(starts.size());
+  starts.resize(inflate::merge_starts(probe.data(), (uint32_t)probe.size(), heads.data(), (uint32_t)heads.size(), starts.data(),
+                                      is_member.data()));
+  is_member.resize(starts.size());
+  is_member[0] = 1;  // (the first member's start, found by both scans)
+  const uint32_t n = (uint32_t)starts.size();
+
+  rc = grow(&s->d_meta, &s->meta_cap, (size_t)n, s->pool, s->stream);
+  if (rc == SGC_OK) rc = grow(&s->d_cand, &s->cand_cap, (size_t)n, s->pool, s->stream);
+  if (rc == SGC_OK) rc = grow(&s->d_is_member, &s->is_member_cap, (size_t)n, s->pool, s->stream);
+  if (rc) return rc;
+  SGC_CUDA_TRY(cudaMemcpyAsync(s->d_cand, starts.data(), n * 8ull, cudaMemcpyHostToDevice, s->stream));
+  SGC_CUDA_TRY(cudaMemcpyAsync(s->d_is_member, is_member.data(), n, cudaMemcpyHostToDevice, s->stream));
+  member_boundary_kernel<<<(n + kInflateThreads - 1) / kInflateThreads, kInflateThreads, kInflateSmem, s->stream>>>(
+      s->d_gz, n_bytes, s->d_cand, s->d_is_member, n, s->d_meta);
+  SGC_CUDA_TRY(cudaGetLastError());
+  meta.resize(n);
+  SGC_CUDA_TRY(cudaMemcpyAsync(meta.data(), s->d_meta, n * sizeof(PieceMeta), cudaMemcpyDeviceToHost, s->stream));
+  SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+  return SGC_OK;
+}
+
+// 4-7. waves of chain pieces: symbols, windows, text, CRC-32, framing and counting.  member_of[i] is the
+// member of chain piece i: a piece may copy from its member's text only (from none of it when it starts
+// the member).  crc[m] (zero on entry) becomes the CRC-32 of member m's text.
+int member_waves(sgc_fastq_stream* s, uint64_t n_bytes, const MemberParams& p, const char* what, const std::vector<uint64_t>& starts,
+                 const std::vector<PieceMeta>& meta, const uint32_t* chain, const uint32_t* member_of, uint32_t n_chain,
+                 std::vector<uint32_t>& crc) {
+  int rc = SGC_OK;
+  for (int w = 0; w < 2; ++w)
+    if (!s->d_window[w]) {
+      if ((rc = scratch_alloc(reinterpret_cast<void**>(&s->d_window[w]), inflate::kWindow, s->pool, s->stream))) return rc;
+    }
+  SGC_CUDA_TRY(cudaMemsetAsync(s->d_window[0], 0, inflate::kWindow, s->stream));
+  int cur = 0;
+  uint64_t done = 0;          // text of the waves before
+  uint64_t member_begin = 0;  // where the current member's text starts
+  std::vector<WavePiece> h_wave;
+  std::vector<uint32_t> h_crc;
+  for (uint32_t a = 0; a < n_chain;) {
+    uint32_t b = a;
+    uint64_t text = 0;
+    while (b < n_chain && (b == a || text + meta[chain[b]].out_len <= p.wave_text)) text += meta[chain[b++]].out_len;
+    const uint32_t nw = b - a;
+    if (s->read_len == 0 && text >= (1ull << 32) - 2 * kHeadroom) return member_decline(s, what, "a piece inflates to 4 GiB or more");
+    h_wave.resize((size_t)nw + 1);
+    uint64_t off = 0;
+    for (uint32_t i = 0; i < nw; ++i) {
+      const PieceMeta& m = meta[chain[a + i]];
+      const uint64_t global = done + off;
+      if (a + i > 0 && member_of[a + i] != member_of[a + i - 1]) member_begin = global;
+      const uint64_t reach = global - member_begin;
+      h_wave[i] = WavePiece{starts[chain[a + i]], m.end_bit, off, reach < inflate::kWindow ? reach : inflate::kWindow};
+      off += m.out_len;
+    }
+    h_wave[nw] = WavePiece{0, 0, text, 0};
+    rc = grow(&s->d_wave, &s->wave_cap, (size_t)nw + 1, s->pool, s->stream);
+    if (rc == SGC_OK) rc = grow(&s->d_sym, &s->sym_cap, (size_t)text + 1, s->pool, s->stream);
+    if (rc == SGC_OK) rc = grow(&s->d_text, &s->text_cap, (size_t)kHeadroom + text + 64, s->pool, s->stream);
+    if (rc == SGC_OK) rc = grow(&s->d_crc, &s->crc_cap, (size_t)nw, s->pool, s->stream);
+    if (rc) return rc;
+    SGC_CUDA_TRY(cudaMemcpyAsync(s->d_wave, h_wave.data(), h_wave.size() * sizeof(WavePiece), cudaMemcpyHostToDevice, s->stream));
+    uint8_t* wave_text_ptr = s->d_text + kHeadroom;
+    member_decode_kernel<<<(nw + kInflateThreads - 1) / kInflateThreads, kInflateThreads, kInflateSmem, s->stream>>>(
+        s->d_gz, n_bytes, s->d_wave, nw, s->d_sym, s->d_state);
+    member_window_kernel<<<1, kWindowThreads, 0, s->stream>>>(s->d_sym, s->d_wave, nw, wave_text_ptr, s->d_window[cur]);
+    member_resolve_kernel<<<nw, 256, 0, s->stream>>>(s->d_sym, s->d_wave, wave_text_ptr, s->d_window[cur]);
+    member_crc_kernel<<<(nw + kCrcWarps - 1) / kCrcWarps, kCrcWarps * 32, 0, s->stream>>>(s->d_wave, nw, wave_text_ptr, s->d_crc);
+    member_window_save_kernel<<<32, 256, 0, s->stream>>>(wave_text_ptr, text, s->d_window[cur], s->d_window[cur ^ 1]);
+    cur ^= 1;
+    SGC_CUDA_TRY(cudaGetLastError());
+    wave_begin_kernel<<<1, 1, 0, s->stream>>>(s->d_state, 0, 0);
+    rc = frame_and_count(s, text, a);  // (synchronises: a piece that did not decode is reported there)
+    if (rc) return rc;
+    h_crc.resize(nw);
+    SGC_CUDA_TRY(cudaMemcpyAsync(h_crc.data(), s->d_crc, nw * 4ull, cudaMemcpyDeviceToHost, s->stream));
+    SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+    for (uint32_t i = 0; i < nw; ++i) {
+      uint32_t& c = crc[member_of[a + i]];
+      c = inflate::crc_combine(c, h_crc[i], h_wave[i + 1].off - h_wave[i].off);
+    }
+    done += text;
+    a = b;
+  }
+  return SGC_OK;
+}
+
 }  // namespace
 
 // Frees the device side and detaches the stream from its counter; the handle itself stays valid.
@@ -591,8 +784,10 @@ void sgc::fastq_stream_release(sgc_fastq_stream* s) {
   for (void* p : {(void*)s->d_state, (void*)s->d_gz, (void*)s->d_text, (void*)s->d_spans, (void*)s->d_tail, (void*)s->d_seq_start,
                   (void*)s->d_seq_end, (void*)s->d_begin, (void*)s->d_outoff, (void*)s->d_counts, (void*)s->d_first, (void*)s->d_sums,
                   (void*)s->d_sym, (void*)s->d_window[0], (void*)s->d_window[1], (void*)s->d_cand, (void*)s->d_meta,
-                  (void*)s->d_wave, (void*)s->d_crc})
+                  (void*)s->d_wave, (void*)s->d_crc, (void*)s->d_heads, (void*)s->d_is_member})
     scratch_free(p, s->pool, s->stream);
+  s->d_heads = nullptr;
+  s->d_is_member = nullptr;
   s->d_sym = nullptr;
   s->d_window[0] = s->d_window[1] = nullptr;
   s->d_cand = nullptr;
@@ -729,133 +924,107 @@ int sgc_fastq_stream_submit_member(sgc_fastq_stream* s, const uint8_t* gz, uint6
     return set_error(SGC_ERR_INVALID_ARG, "a gzip member goes to a fresh stream, once");
   s->member_submitted = true;
   DeviceGuard guard(s->device);
-  auto decline = [&](const char* why) {
-    s->failed = true;
-    char buf[200];
-    snprintf(buf, sizeof buf, "single gzip member not decoded on the device: %s", why);
-    return set_error(SGC_ERR_GZIP, buf);
-  };
+  const char* what = "single gzip member";
   size_t header = 0;
-  if (inflate::gzip_header(gz, (size_t)n_bytes, &header) != inflate::kOk) return decline("not a gzip member");
-  // Nominal piece size: 32 KiB of compressed input (more pieces than larger ones would give keep more
-  // threads busy; each piece is a serial decode).  SGC_MEMBER_PIECE overrides it and SGC_MEMBER_SKEW=1
-  // moves every other candidate start one bit on (tests: many pieces on small files, absorbed pieces);
-  // SGC_MEMBER_WAVE_TEXT bounds the text of a wave (tests: many waves).
-  uint64_t piece = 32u << 10;
-  if (const char* e = getenv("SGC_MEMBER_PIECE"); e && atoll(e) >= 64) piece = (uint64_t)atoll(e);
-  const char* skew_env = getenv("SGC_MEMBER_SKEW");
-  const bool skew = skew_env && atoi(skew_env) != 0;
-  uint64_t wave_text = s->read_len ? (4ull << 30) : (3ull << 30);
-  if (const char* e = getenv("SGC_MEMBER_WAVE_TEXT"); e && atoll(e) > 0) wave_text = std::min<uint64_t>(wave_text, (uint64_t)atoll(e));
+  if (inflate::gzip_header(gz, (size_t)n_bytes, &header) != inflate::kOk) return member_decline(s, what, "not a gzip member");
+  const MemberParams params = member_params(s);
 
-  // 1. candidate starts near every nominal boundary; the member's first block is piece 0
-  const uint32_t n_bounds = (uint32_t)((n_bytes + piece - 1) / piece);
-  int rc = grow(&s->d_gz, &s->gz_cap, (size_t)n_bytes + 64, s->pool, s->stream);  // (the reader's slack)
-  if (rc == SGC_OK) rc = grow(&s->d_cand, &s->cand_cap, (size_t)n_bounds + 1, s->pool, s->stream);
+  // 1-2. candidate starts near every nominal boundary, the boundary pass
+  std::vector<uint64_t> starts;
+  std::vector<uint8_t> is_member;
+  std::vector<PieceMeta> meta;
+  int rc = member_pieces(s, gz, n_bytes, header, params, false, what, starts, is_member, meta);
   if (rc) return rc;
-  SGC_CUDA_TRY(cudaMemcpyAsync(s->d_gz, gz, n_bytes, cudaMemcpyHostToDevice, s->stream));
-  constexpr uint32_t kWarps = kInflateThreads / 32;
-  if (n_bounds > 1)
-    member_find_kernel<<<(n_bounds - 1 + kWarps - 1) / kWarps, kInflateThreads, kInflateSmem, s->stream>>>(s->d_gz, n_bytes, piece,
-                                                                                                          n_bounds, s->d_cand);
-  SGC_CUDA_TRY(cudaGetLastError());
-  std::vector<uint64_t> cand((size_t)n_bounds + 1, ~0ull);
-  if (n_bounds > 1) SGC_CUDA_TRY(cudaMemcpyAsync(cand.data() + 1, s->d_cand + 1, (n_bounds - 1) * 8ull, cudaMemcpyDeviceToHost, s->stream));
-  SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
-  std::vector<uint64_t> starts{(uint64_t)header * 8};
-  for (uint32_t j = 1; j < n_bounds; ++j) {
-    if (cand[j] == ~0ull) continue;
-    const uint64_t c = cand[j] + (skew && (starts.size() & 1) ? 1 : 0);
-    if (c > starts.back()) starts.push_back(c);
-  }
   const uint32_t n = (uint32_t)starts.size();
 
-  // 2. every piece to its first block end at or beyond the next candidate
-  rc = grow(&s->d_meta, &s->meta_cap, (size_t)n, s->pool, s->stream);
-  if (rc) return rc;
-  SGC_CUDA_TRY(cudaMemcpyAsync(s->d_cand, starts.data(), n * 8ull, cudaMemcpyHostToDevice, s->stream));
-  member_boundary_kernel<<<(n + kInflateThreads - 1) / kInflateThreads, kInflateThreads, kInflateSmem, s->stream>>>(
-      s->d_gz, n_bytes, s->d_cand, n, s->d_meta);
-  SGC_CUDA_TRY(cudaGetLastError());
-  std::vector<PieceMeta> meta(n);
-  SGC_CUDA_TRY(cudaMemcpyAsync(meta.data(), s->d_meta, n * sizeof(PieceMeta), cudaMemcpyDeviceToHost, s->stream));
-  SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
-
   // 3. the chain from the first block; its last piece ends the member, whose trailer must end the file
-  std::vector<uint32_t> next(n), chain(n);
+  std::vector<uint32_t> next(n), chain(n), member_of(n, 0);
   std::vector<int> status(n);
   for (uint32_t j = 0; j < n; ++j) next[j] = meta[j].next, status[j] = meta[j].status;
   uint64_t absorbed = 0;
   const uint32_t n_chain = inflate::piece_chain(next.data(), status.data(), n, chain.data(), &absorbed);
-  if (n_chain == 0) return decline("its blocks could not be followed from piece to piece");
+  if (n_chain == 0) return member_decline(s, what, "its blocks could not be followed from piece to piece");
   const uint64_t trailer = (meta[chain[n_chain - 1]].end_bit + 7) / 8;
-  if (trailer + 8 != n_bytes) return decline("the member's trailer does not end the file");
+  if (trailer + 8 != n_bytes) return member_decline(s, what, "the member's trailer does not end the file");
   uint64_t total = 0;
   for (uint32_t i = 0; i < n_chain; ++i) total += meta[chain[i]].out_len;
-  const uint32_t want_crc = (uint32_t)gz[trailer] | ((uint32_t)gz[trailer + 1] << 8) | ((uint32_t)gz[trailer + 2] << 16) |
-                            ((uint32_t)gz[trailer + 3] << 24);
-  const uint32_t isize = (uint32_t)gz[trailer + 4] | ((uint32_t)gz[trailer + 5] << 8) | ((uint32_t)gz[trailer + 6] << 16) |
-                         ((uint32_t)gz[trailer + 7] << 24);
-  if (isize != (uint32_t)total) return decline("ISIZE differs from the length of the inflated text");
+  const uint32_t want_crc = inflate::le32(gz + trailer), isize = inflate::le32(gz + trailer + 4);
+  if (isize != (uint32_t)total) return member_decline(s, what, "ISIZE differs from the length of the inflated text");
   s->member_pieces = n;
   s->member_chain = n_chain;
   s->member_absorbed = absorbed;
 
-  // 4-7. waves of chain pieces: symbols, windows, text, CRC-32, framing and counting
-  for (int w = 0; w < 2; ++w)
-    if (!s->d_window[w]) {
-      if ((rc = scratch_alloc(reinterpret_cast<void**>(&s->d_window[w]), inflate::kWindow, s->pool, s->stream))) return rc;
-    }
-  SGC_CUDA_TRY(cudaMemsetAsync(s->d_window[0], 0, inflate::kWindow, s->stream));
-  int cur = 0;
-  uint32_t crc = 0;
-  uint64_t done = 0;  // text of the waves before
-  std::vector<WavePiece> h_wave;
-  std::vector<uint32_t> h_crc;
-  for (uint32_t a = 0; a < n_chain;) {
-    uint32_t b = a;
-    uint64_t text = 0;
-    while (b < n_chain && (b == a || text + meta[chain[b]].out_len <= wave_text)) text += meta[chain[b++]].out_len;
-    const uint32_t nw = b - a;
-    if (s->read_len == 0 && text >= (1ull << 32) - 2 * kHeadroom) return decline("a piece inflates to 4 GiB or more");
-    h_wave.resize((size_t)nw + 1);
-    uint64_t off = 0;
-    for (uint32_t i = 0; i < nw; ++i) {
-      const PieceMeta& m = meta[chain[a + i]];
-      const uint64_t global = done + off;
-      h_wave[i] = WavePiece{starts[chain[a + i]], m.end_bit, off, global < inflate::kWindow ? global : inflate::kWindow};
-      off += m.out_len;
-    }
-    h_wave[nw] = WavePiece{0, 0, text, 0};
-    rc = grow(&s->d_wave, &s->wave_cap, (size_t)nw + 1, s->pool, s->stream);
-    if (rc == SGC_OK) rc = grow(&s->d_sym, &s->sym_cap, (size_t)text + 1, s->pool, s->stream);
-    if (rc == SGC_OK) rc = grow(&s->d_text, &s->text_cap, (size_t)kHeadroom + text + 64, s->pool, s->stream);
-    if (rc == SGC_OK) rc = grow(&s->d_crc, &s->crc_cap, (size_t)nw, s->pool, s->stream);
-    if (rc) return rc;
-    SGC_CUDA_TRY(cudaMemcpyAsync(s->d_wave, h_wave.data(), h_wave.size() * sizeof(WavePiece), cudaMemcpyHostToDevice, s->stream));
-    uint8_t* wave_text_ptr = s->d_text + kHeadroom;
-    member_decode_kernel<<<(nw + kInflateThreads - 1) / kInflateThreads, kInflateThreads, kInflateSmem, s->stream>>>(
-        s->d_gz, n_bytes, s->d_wave, nw, s->d_sym, s->d_state);
-    member_window_kernel<<<1, kWindowThreads, 0, s->stream>>>(s->d_sym, s->d_wave, nw, wave_text_ptr, s->d_window[cur]);
-    member_resolve_kernel<<<nw, 256, 0, s->stream>>>(s->d_sym, s->d_wave, wave_text_ptr, s->d_window[cur]);
-    member_crc_kernel<<<(nw + kCrcWarps - 1) / kCrcWarps, kCrcWarps * 32, 0, s->stream>>>(s->d_wave, nw, wave_text_ptr, s->d_crc);
-    member_window_save_kernel<<<32, 256, 0, s->stream>>>(wave_text_ptr, text, s->d_window[cur], s->d_window[cur ^ 1]);
-    cur ^= 1;
-    SGC_CUDA_TRY(cudaGetLastError());
-    wave_begin_kernel<<<1, 1, 0, s->stream>>>(s->d_state, 0, 0);
-    rc = frame_and_count(s, text, a);  // (synchronises: a piece that did not decode is reported there)
-    if (rc) return rc;
-    h_crc.resize(nw);
-    SGC_CUDA_TRY(cudaMemcpyAsync(h_crc.data(), s->d_crc, nw * 4ull, cudaMemcpyDeviceToHost, s->stream));
-    SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
-    for (uint32_t i = 0; i < nw; ++i) crc = inflate::crc_combine(crc, h_crc[i], h_wave[i + 1].off - h_wave[i].off);
-    done += text;
-    a = b;
-  }
-  if (crc != want_crc) {
+  // 4-7. waves of chain pieces
+  std::vector<uint32_t> crc(1, 0);
+  rc = member_waves(s, n_bytes, params, what, starts, meta, chain.data(), member_of.data(), n_chain, crc);
+  if (rc) return rc;
+  if (crc[0] != want_crc) {
     s->failed = true;
     return set_error(SGC_ERR_GZIP, "gzip member: CRC-32 of the inflated bytes differs from the member's trailer");
   }
+  s->gzip_members = 1;
+  return SGC_OK;
+}
+
+int sgc_fastq_stream_submit_gzip(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes) {
+  if (!s || !gz) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
+  if (s->failed || !s->counter) return set_error(SGC_ERR_INVALID_ARG, "the stream has failed or its counter is gone");
+  if (s->member_submitted || s->blocks_total)
+    return set_error(SGC_ERR_INVALID_ARG, "a gzip file goes to a fresh stream, once");
+  s->member_submitted = true;
+  DeviceGuard guard(s->device);
+  const char* what = "gzip members";
+  size_t header = 0;
+  if (inflate::gzip_header(gz, (size_t)n_bytes, &header) != inflate::kOk) return member_decline(s, what, "not a gzip member");
+  const MemberParams params = member_params(s);
+
+  // 1-2. candidate starts near every nominal boundary and at every gzip header, the boundary pass
+  std::vector<uint64_t> starts;
+  std::vector<uint8_t> is_member;
+  std::vector<PieceMeta> meta;
+  int rc = member_pieces(s, gz, n_bytes, header, params, true, what, starts, is_member, meta);
+  if (rc) return rc;
+  const uint32_t n = (uint32_t)starts.size();
+
+  // 3. the chain from the first block, over every trailer and header to the last trailer, which must end the file
+  std::vector<uint32_t> next(n), chain(n), member_of(n);
+  std::vector<int> status(n);
+  std::vector<uint64_t> end_bit(n);
+  for (uint32_t j = 0; j < n; ++j) next[j] = meta[j].next, status[j] = meta[j].status, end_bit[j] = meta[j].end_bit;
+  std::vector<inflate::MemberTrailer> trailers(n);
+  uint32_t n_members = 0;
+  uint64_t absorbed = 0;
+  const uint32_t n_chain = inflate::members_chain(gz, (size_t)n_bytes, starts.data(), is_member.data(), next.data(), status.data(),
+                                                  end_bit.data(), n, chain.data(), member_of.data(), trailers.data(), &n_members,
+                                                  &absorbed);
+  if (n_chain == 0)
+    return member_decline(s, what, "their blocks could not be followed from piece to piece, or a trailer is followed by no gzip member");
+  std::vector<uint64_t> text(n_members, 0);
+  for (uint32_t i = 0; i < n_chain; ++i) text[member_of[i]] += meta[chain[i]].out_len;
+  for (uint32_t m = 0; m < n_members; ++m)
+    if (trailers[m].isize != (uint32_t)text[m]) return member_decline(s, what, "ISIZE of a member differs from the length of its text");
+  s->member_pieces = n;
+  s->member_chain = n_chain;
+  s->member_absorbed = absorbed;
+
+  // 4-7. waves of chain pieces; CRC-32 member by member
+  std::vector<uint32_t> crc(n_members, 0);
+  rc = member_waves(s, n_bytes, params, what, starts, meta, chain.data(), member_of.data(), n_chain, crc);
+  if (rc) return rc;
+  for (uint32_t m = 0; m < n_members; ++m)
+    if (crc[m] != trailers[m].crc) {
+      s->failed = true;
+      char buf[160];
+      snprintf(buf, sizeof buf, "gzip member %u: CRC-32 of the inflated bytes differs from the member's trailer", m);
+      return set_error(SGC_ERR_GZIP, buf);
+    }
+  s->gzip_members = n_members;
+  return SGC_OK;
+}
+
+int sgc_fastq_stream_gzip_members(const sgc_fastq_stream* s, uint64_t* members) {
+  if (!s || !members) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
+  *members = s->gzip_members;
   return SGC_OK;
 }
 

@@ -800,10 +800,11 @@ SGC_HD bool probe_block_start(const uint8_t* in, size_t in_len, uint64_t bit, Ta
 // starts exactly there (j + 1, or up to j + 1 + max_absorb when candidates in between were false or
 // skipped), or kPieceFinal when the member's last block ended first; *end_bit and *out_len describe
 // the piece.  Anything else means the piece does not lie on the chain.
+// `reach`: how far before the piece a match may copy from; 0 for a piece that starts a member.
 template <typename Tables>
 SGC_HD int piece_boundary(const uint8_t* in, size_t in_len, const uint64_t* starts, uint32_t n, uint32_t j,
-                          uint32_t max_absorb, Tables t, uint32_t* next, uint64_t* end_bit, uint64_t* out_len) {
-  CountSink sink{0, j == 0 ? 0u : kWindow};
+                          uint32_t max_absorb, Tables t, uint32_t* next, uint64_t* end_bit, uint64_t* out_len, uint64_t reach) {
+  CountSink sink{0, reach};
   const uint32_t last_ok = j + 1 + max_absorb < n ? j + 1 + max_absorb : n - 1;
   const uint64_t limit = j + 1 + max_absorb < n ? starts[j + 1 + max_absorb] : (uint64_t)in_len * 8;
   uint32_t m = j + 1;
@@ -819,6 +820,12 @@ SGC_HD int piece_boundary(const uint8_t* in, size_t in_len, const uint64_t* star
   *out_len = sink.op;
   return kOk;
 }
+// one member: piece 0 starts it, every other piece may copy from the 32 KiB in front of it
+template <typename Tables>
+SGC_HD int piece_boundary(const uint8_t* in, size_t in_len, const uint64_t* starts, uint32_t n, uint32_t j,
+                          uint32_t max_absorb, Tables t, uint32_t* next, uint64_t* end_bit, uint64_t* out_len) {
+  return piece_boundary(in, in_len, starts, n, j, max_absorb, t, next, end_bit, out_len, j == 0 ? 0u : kWindow);
+}
 
 // Step 3 (host): the pieces linked from piece 0 into chain[]; returns their number, or 0 when the
 // links reach a piece whose step 2 failed (status != kOk).  *absorbed: candidates run past.
@@ -831,6 +838,94 @@ inline uint32_t piece_chain(const uint32_t* next, const int* status, uint32_t n,
     if (next[j] == kPieceFinal) return len;
     *absorbed += next[j] - j - 1;
     j = next[j];
+  }
+}
+
+// ---- SEVERAL members in pieces ----------------------------------------------------------------
+// Concatenated members (`cat a.gz b.gz`, appending writers, BGZF) are one text, decoded by the same
+// steps with two additions: every gzip header in the input is a further candidate, flagged as a
+// member start (its first block may be of any kind, so it is not probed, and its piece may copy
+// from nothing in front of it), and the chain steps from a member's last block over its trailer
+// and the next header to exactly the candidate that follows them.  A false signature costs one
+// piece that fails or is never linked.
+
+// Does a gzip member header start at byte `pos`?  true and *bit = the first bit of its DEFLATE stream.
+SGC_HD bool member_start_at(const uint8_t* in, size_t in_len, size_t pos, uint64_t* bit) {
+  if (pos + 4 > in_len || in[pos] != 0x1f || in[pos + 1] != 0x8b || in[pos + 2] != 8 || (in[pos + 3] & 0xE0)) return false;
+  size_t h = 0;
+  if (gzip_header(in + pos, in_len - pos, &h) != kOk) return false;
+  *bit = (uint64_t)(pos + h) * 8;
+  return true;
+}
+
+SGC_HD uint32_t le32(const uint8_t* p) {
+  return (uint32_t)p[0] | ((uint32_t)p[1] << 8) | ((uint32_t)p[2] << 16) | ((uint32_t)p[3] << 24);
+}
+
+// Step 1 (host): the block-start candidates probe[0 .. np) and the member starts member[0 .. nm), each
+// sorted, into one sorted starts[] without duplicates; is_member[i] = 1 where a member starts (that
+// flag wins over a block-start candidate at the same bit).  Returns the number of starts.
+inline uint32_t merge_starts(const uint64_t* probe, uint32_t np, const uint64_t* member, uint32_t nm, uint64_t* starts,
+                             uint8_t* is_member) {
+  uint32_t i = 0, k = 0, n = 0;
+  while (i < np || k < nm) {
+    const bool m = k < nm && (i >= np || member[k] <= probe[i]);
+    const uint64_t v = m ? member[k++] : probe[i++];
+    if (n && starts[n - 1] == v) {
+      is_member[n - 1] |= (uint8_t)m;
+    } else {
+      starts[n] = v;
+      is_member[n++] = (uint8_t)m;
+    }
+  }
+  return n;
+}
+
+// A member's trailer (RFC 1952): where it starts, the CRC-32 and ISIZE it holds.
+struct MemberTrailer {
+  uint64_t at;
+  uint32_t crc, isize;
+};
+
+// Step 3 across members (host): from piece 0 (the first member's start) along the links; where a
+// piece ends a member's last block, the member's 8-byte trailer follows at the next byte, and unless
+// it ends the input, a gzip header and the member-start candidate right behind it.  Fills chain[],
+// member_of[] (the member of each chain piece) and trailers[] (one per member, *n_members of them);
+// returns the chain's length, or 0 (decline) when a link is missing, a piece on the way failed, or
+// anything but a whole member follows a trailer (zero padding included).
+inline uint32_t members_chain(const uint8_t* in, size_t in_len, const uint64_t* starts, const uint8_t* is_member,
+                              const uint32_t* next, const int* status, const uint64_t* end_bit, uint32_t n, uint32_t* chain,
+                              uint32_t* member_of, MemberTrailer* trailers, uint32_t* n_members, uint64_t* absorbed) {
+  uint32_t len = 0, j = 0, m = 0;
+  *absorbed = 0;
+  *n_members = 0;
+  if (n == 0 || !is_member[0]) return 0;
+  for (;;) {
+    if (j >= n || status[j] != kOk) return 0;
+    chain[len] = j;
+    member_of[len++] = m;
+    if (next[j] != kPieceFinal) {
+      *absorbed += next[j] - j - 1;
+      j = next[j];
+      continue;
+    }
+    const uint64_t at = (end_bit[j] + 7) / 8;
+    if (at + 8 > in_len) return 0;
+    trailers[m++] = MemberTrailer{at, le32(in + at), le32(in + at + 4)};
+    if (at + 8 == in_len) {
+      *n_members = m;
+      return len;
+    }
+    uint64_t bit = 0;
+    if (!member_start_at(in, in_len, (size_t)(at + 8), &bit)) return 0;
+    uint32_t lo = j + 1, hi = n;  // the first start at or beyond `bit`
+    while (lo < hi) {
+      const uint32_t mid = lo + (hi - lo) / 2;
+      if (starts[mid] < bit) lo = mid + 1;
+      else hi = mid;
+    }
+    if (lo >= n || starts[lo] != bit || !is_member[lo]) return 0;
+    j = lo;
   }
 }
 

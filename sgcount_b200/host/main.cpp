@@ -95,7 +95,7 @@ const char* kUsage =
     "      --ingest-threads <N>               Threads inflating the gzip members of one sample [default: cores / samples in flight]\n"
     "      --rc-keep-n                        Reverse complement keeps N (default: the fxread bit trick, N -> J)\n"
     "      --whole-lines                      Copy whole sequence lines to the device (default: for fixed-length reads, only the guide window and one byte either side)\n"
-    "      --host-inflate                     Inflate and frame records on the host even for BGZF or single-member gzip input (default: BGZF files of FASTQ, and gzip files of FASTQ that are one member, are inflated, framed and counted on the device)\n"
+    "      --host-inflate                     Inflate and frame records on the host even for BGZF, single-member or multi-member gzip input (default: BGZF files of FASTQ, and gzip files of FASTQ that are one member, are inflated, framed and counted on the device; so are multi-member gzip files large enough and with too few members or ingest threads for the host to decode them faster side by side)\n"
     "      --timing                           Print a JSON line with the phase times to stderr\n"
     "  -h, --help                             Print help\n";
 
@@ -382,7 +382,8 @@ struct SampleResult {
   double dev_index_s = 0, dev_create_s = 0, dev_waves_s = 0, dev_finish_s = 0;  // phases of the device ingest
   bool device_ingest = false;               // inflate and record framing ran on the device (BGZF input)
   uint64_t device_blocks = 0;
-  uint64_t member_pieces = 0, member_chain = 0, member_absorbed = 0;  // one gzip member in pieces on the device
+  uint64_t member_pieces = 0, member_chain = 0, member_absorbed = 0;  // gzip members in pieces on the device
+  uint64_t gzip_members = 0;                                          // how many (not BGZF), as the device confirmed them
   std::string host_because;                 // why the device ingest was not used
 };
 
@@ -468,17 +469,18 @@ bool plan_waves(const uint8_t* file, const std::vector<uint64_t>& begin, const s
   return true;
 }
 
-// Is the file one gzip member?  Every later position that looks like a member start (the host
-// reader's signature scan: 1f 8b 08, reserved flags clear) is tried with zlib; in compressed data such
-// a position is a coincidence (one in a few MB) that zlib rejects within a few bytes.  The device
-// confirms it: the member's trailer must end the file.
-bool is_single_member(const uint8_t* d, size_t n) {
-  for (const uint8_t* p = d + 1; p + 4 <= d + n; ++p) {
+// How many gzip members does the file hold, counting up to `cap`?  Every later position that looks like
+// a member start (the host reader's signature scan: 1f 8b 08, reserved flags clear) is tried with zlib;
+// in compressed data such a position is a coincidence (one in a few MB) that zlib rejects within a few
+// bytes.  The device confirms the count: each member's trailer must be followed by the next header.
+size_t gzip_members(const uint8_t* d, size_t n, size_t cap) {
+  size_t members = 1;
+  for (const uint8_t* p = d + 1; p + 4 <= d + n && members < cap; ++p) {
     p = static_cast<const uint8_t*>(memchr(p, 0x1f, (size_t)(d + n - p)));
     if (!p || p + 4 > d + n) break;
     if (p[1] != 0x8b || p[2] != 0x08 || (p[3] & 0xE0) != 0) continue;
     z_stream zs{};
-    if (inflateInit2(&zs, 15 + 16) != Z_OK) return false;
+    if (inflateInit2(&zs, 15 + 16) != Z_OK) return cap;
     uint8_t out[4096];
     zs.next_in = const_cast<uint8_t*>(p);
     zs.avail_in = (uInt)std::min<size_t>((size_t)(d + n - p), 1u << 20);
@@ -487,15 +489,25 @@ bool is_single_member(const uint8_t* d, size_t n) {
     const int rc = inflate(&zs, Z_NO_FLUSH);
     const bool member = (rc == Z_OK || rc == Z_STREAM_END) && (zs.avail_out == 0 || rc == Z_STREAM_END);
     inflateEnd(&zs);
-    if (member) return false;
+    members += member;
   }
-  return true;
+  return members;
 }
 
-// A single-member (not BGZF) gzip FASTQ through sgc_fastq_stream_submit_member on one device.
+// Where a gzip file of several members (not BGZF) is counted.  The host decodes members side by side,
+// one ingest thread each, at about one core's speed per member; the device decodes the whole file in
+// pieces, but serially twice per piece, so it has a latency floor.  Both constants are measured with
+// tools/multi_member_time.py (profiles/r4_multi_member_time.txt, one B200): below kMinDeviceGzipBytes of
+// compressed input the host's cores finish first, and once min(members, ingest threads) exceeds
+// kHostCoresPerDevice the host's threads side by side are as quick as the device.
+constexpr size_t kMinDeviceGzipBytes = 64ull << 20;
+constexpr size_t kHostCoresPerDevice = 3;
+
+// A gzip FASTQ that is not BGZF on one device: one member through sgc_fastq_stream_submit_member,
+// several (`several`) through sgc_fastq_stream_submit_gzip.
 bool count_member_on_device(const sgc_library* lib, uint32_t n_guides, const MappedFile& file, OffsetValue offset, uint32_t span_offset,
                             uint32_t read_len, uint32_t span_start, uint32_t span_len, bool variable, bool recursion, int rc_mode,
-                            SampleResult& r, std::string& why_not) {
+                            bool several, SampleResult& r, std::string& why_not) {
   const auto t0 = std::chrono::steady_clock::now();
   struct Guard {
     sgc_counter* c = nullptr;
@@ -509,7 +521,7 @@ bool count_member_on_device(const sgc_library* lib, uint32_t n_guides, const Map
   check(sgc_fastq_stream_create(g.c, variable ? 0 : read_len, span_start, span_len, &g.s));
   const auto t1 = std::chrono::steady_clock::now();
   uint64_t n_records = 0;
-  int rc = sgc_fastq_stream_submit_member(g.s, file.data, file.size);
+  int rc = several ? sgc_fastq_stream_submit_gzip(g.s, file.data, file.size) : sgc_fastq_stream_submit_member(g.s, file.data, file.size);
   const auto t2 = std::chrono::steady_clock::now();
   if (rc == SGC_OK) rc = sgc_fastq_stream_finish(g.s, &n_records);
   if (rc == SGC_ERR_GZIP || rc == SGC_ERR_FASTQ_FORMAT) {
@@ -518,6 +530,7 @@ bool count_member_on_device(const sgc_library* lib, uint32_t n_guides, const Map
   }
   if (rc != SGC_OK) fail("%s", sgc_last_error());
   check(sgc_fastq_stream_member_stats(g.s, &r.member_pieces, &r.member_chain, &r.member_absorbed));
+  check(sgc_fastq_stream_gzip_members(g.s, &r.gzip_members));
   r.counts.resize(n_guides);
   check(sgc_counter_finish(g.c, r.counts.data(), &r.total, &r.matched));
   const auto t3 = std::chrono::steady_clock::now();
@@ -537,15 +550,16 @@ bool count_member_on_device(const sgc_library* lib, uint32_t n_guides, const Map
 
 // One sample through the device ingest, on one device or — `libs.size()` > 1 — with its waves
 // dealt to several, one host thread each, the devices' count vectors summed at the end
-// (sgc_reduce_counts).  A single gzip member that is not BGZF goes to the first device
-// (count_member_on_device) when `member_ok`.  Returns false when the file is neither or the device reports input it
+// (sgc_reduce_counts).  A gzip file that is not BGZF goes to the first device (count_member_on_device)
+// when `member_ok` and it is one member, or several where the device is the quicker (kMinDeviceGzipBytes,
+// kHostCoresPerDevice; `ingest_threads`: the host's threads for the sample).  Returns false when the file is neither or the device reports input it
 // does not take — a read of another length (span mode), FASTA, a damaged block — so that the
 // caller can try the other mode or the host path.
 // `variable`: reads of any length (the sequence lines are counted where they lie in the inflated
 // text); otherwise every read has read_len bytes and only its guide-window span is kept.
 bool count_sample_on_device(const std::vector<const sgc_library*>& libs, uint32_t n_guides, uint32_t k, const std::string& path,
                             OffsetValue offset, uint32_t read_len, bool variable, bool recursion, int rc_mode, bool member_ok,
-                            SampleResult& r, std::string& why_not) {
+                            unsigned ingest_threads, SampleResult& r, std::string& why_not) {
   uint32_t span_start = 0, span_len = 0, span_offset = offset.index;
   if (!variable && sgc_span_geometry(k, read_len, offset.reverse, offset.index, recursion, &span_start, &span_len,
                                      &span_offset) != SGC_OK) {
@@ -568,12 +582,23 @@ bool count_sample_on_device(const std::vector<const sgc_library*>& libs, uint32_
       why_not = "not BGZF, and read shards asked for";
       return false;
     }
-    if (!is_single_member(file.data, file.size)) {
-      why_not = "not BGZF, and more than one gzip member";
+    const size_t members = gzip_members(file.data, file.size, kHostCoresPerDevice + 1);
+    // (SGC_MULTI_MEMBER_DEVICE=1: every multi-member file to the device, for measurements of both paths)
+    const char* force_env = getenv("SGC_MULTI_MEMBER_DEVICE");
+    const bool force = force_env && atoi(force_env) != 0;
+    if (members > 1 && !force && file.size < kMinDeviceGzipBytes) {
+      why_not = "not BGZF, and several gzip members in a file under " + std::to_string(kMinDeviceGzipBytes >> 20) +
+                " MB: the host's cores decode them sooner";
+      return false;
+    }
+    if (members > 1 && !force && std::min<size_t>(members, ingest_threads) > kHostCoresPerDevice) {
+      why_not = "not BGZF, and " + std::string(members > kHostCoresPerDevice ? "more than " + std::to_string(kHostCoresPerDevice)
+                                                                              : std::to_string(members)) +
+                " gzip members: the host decodes them side by side";
       return false;
     }
     return count_member_on_device(libs[0], n_guides, file, offset, span_offset, read_len, span_start, span_len, variable, recursion,
-                                  rc_mode, r, why_not);
+                                  rc_mode, members > 1, r, why_not);
   }
   const auto t_indexed = std::chrono::steady_clock::now();
   const size_t n_blocks = isize.size(), n_dev = libs.size();
@@ -938,7 +963,7 @@ int main(int argc, char** argv) {
     std::vector<uint32_t> first_len(n_samples);
     std::vector<char> head_uniform(n_samples, 0), head_fastq(n_samples, 0);  // 4-line FASTQ? head reads of one length?
     bool all_for_the_device = !args.host_inflate;
-    const bool member_ok = args.read_shards <= 1;  // (read shards asked for: one member keeps the host path)
+    const bool member_ok = args.read_shards <= 1;  // (read shards asked for: gzip that is not BGZF keeps the host path)
     for (size_t i = 0; i < n_samples; ++i) {
       first_len[i] = (uint32_t)heads[i].first_len;
       head_fastq[i] = heads[i].fastq;
@@ -973,11 +998,11 @@ int main(int argc, char** argv) {
             // reported by the device deeper in the file) with their sequence lines in place
             bool variable = !head_uniform[s] || args.whole_lines;
             on_device = count_sample_on_device(sample_libs, hlib.n, hlib.k, args.input_paths[s], offsets[s], first_len[s],
-                                               variable, !args.no_position_recursion, args.rc_mode, member_ok, results[s], why_not);
+                                               variable, !args.no_position_recursion, args.rc_mode, member_ok, ingest_threads, results[s], why_not);
             if (!on_device && !variable && why_not.find("FASTQ") != std::string::npos) {
               results[s] = SampleResult();
               on_device = count_sample_on_device(sample_libs, hlib.n, hlib.k, args.input_paths[s], offsets[s], first_len[s],
-                                                 true, !args.no_position_recursion, args.rc_mode, member_ok, results[s], why_not);
+                                                 true, !args.no_position_recursion, args.rc_mode, member_ok, ingest_threads, results[s], why_not);
             }
           } else if (!head_fastq[s]) {
             why_not = "not FASTQ";
@@ -1016,7 +1041,7 @@ int main(int argc, char** argv) {
       unsigned long long reads = 0;
       double wait_s = 0, copy_s = 0, submit_s = 0;
       unsigned max_shards = 1;
-      unsigned long long span_reads = 0, device_blocks = 0, adopted = 0, reframed = 0, pieces = 0, chain = 0, absorbed = 0;
+      unsigned long long span_reads = 0, device_blocks = 0, adopted = 0, reframed = 0, pieces = 0, chain = 0, absorbed = 0, members = 0;
       unsigned device_samples = 0;
       std::string host_because;
       double dev_index_s = 0, dev_create_s = 0, dev_waves_s = 0, dev_finish_s = 0;
@@ -1027,7 +1052,7 @@ int main(int argc, char** argv) {
         adopted += r.members_adopted, reframed += r.members_reframed;
         device_samples += r.device_ingest;
         device_blocks += r.device_blocks;
-        pieces += r.member_pieces, chain += r.member_chain, absorbed += r.member_absorbed;
+        pieces += r.member_pieces, chain += r.member_chain, absorbed += r.member_absorbed, members += r.gzip_members;
         if (!r.device_ingest && host_because.empty()) host_because = r.host_because;
         max_shards = std::max(max_shards, r.shards);
       }
@@ -1035,10 +1060,10 @@ int main(int argc, char** argv) {
               "\"ingest_threads\": %u, \"gpus\": %d, \"read_shards_per_sample\": %u, \"span_reads\": %llu, \"device_ingest_samples\": %u, "
               "\"device_blocks\": %llu, \"device_phases_s\": [%.4f, %.4f, %.4f, %.4f], \"host_ingest_because\": \"%s\", \"members_adopted\": %llu, \"members_reframed\": %llu, \"wait_inflate_s\": %.6f, "
               "\"copy_to_pinned_s\": %.6f, \"submit_sync_s\": %.6f, \"read_inputs_s\": %.3f, "
-              "\"device_tables_s\": %.3f, \"offsets_s\": %.3f, \"member_pieces\": %llu, \"member_chain\": %llu, \"member_absorbed\": %llu}\n",
+              "\"device_tables_s\": %.3f, \"offsets_s\": %.3f, \"member_pieces\": %llu, \"member_chain\": %llu, \"member_absorbed\": %llu, \"gzip_members\": %llu}\n",
               count_s, reads, n_samples, workers, ingest_threads, gpus, max_shards, span_reads, device_samples, device_blocks,
               dev_index_s, dev_create_s, dev_waves_s, dev_finish_s, host_because.c_str(), adopted, reframed, wait_s, copy_s, submit_s, t_inputs,
-              t_tables - t_inputs, t_offsets - t_tables, pieces, chain, absorbed);
+              t_tables - t_inputs, t_offsets - t_tables, pieces, chain, absorbed, members);
     }
 
     // write_results (results.rs:71-99).  Counts are keyed by alias (counter.rs:232-235):

@@ -1,11 +1,14 @@
-// member_core_test <file.gz> <piece_bytes> <skew 0|1> — decodes a single-member gzip file the way the
-// device does (gzip.cu member_* kernels), serially, from the same csrc/inflate_core.h code: candidate
-// block starts every piece_bytes of compressed input (with skew, every other candidate moved one bit on),
-// the boundary pass, the chain, 16-bit symbols with window markers, the window resolution piece after
-// piece and then the rest, CRC-32 in pieces joined, the trailer.  Prints
-// "<bytes> <fnv1a> <pieces> <chain> <absorbed>" (exit 0), "decline ..." when the chain does not reach
-// the member's end (exit 3: the device would hand the file to the host), or the error (exit 4).
-// Test helper for tests/test_member_inflate_core.py; zlib is the comparison.
+// member_core_test <file.gz> <piece_bytes> <skew 0|1> [members 0|1] — decodes a single-member gzip file
+// the way the device does (gzip.cu member_* kernels), serially, from the same csrc/inflate_core.h code:
+// candidate block starts every piece_bytes of compressed input (with skew, every other candidate moved one
+// bit on), the boundary pass, the chain, 16-bit symbols with window markers, the window resolution piece
+// after piece and then the rest, CRC-32 in pieces joined, the trailer.  With members = 1 the file may hold
+// any number of members (sgc_fastq_stream_submit_gzip): every gzip header is a member-start candidate too,
+// the chain steps over trailers (members_chain), and CRC-32 and ISIZE are checked member by member.
+// Prints "<bytes> <fnv1a> <pieces> <chain> <absorbed>" (with members = 1, then "<members>"; exit 0),
+// "decline ..." when the chain does not reach the end (exit 3: the device would hand the file to the
+// host), or the error (exit 4).  Test helper for tests/test_member_inflate_core.py and
+// tests/test_multi_member_inflate_core.py; zlib is the comparison.
 #include <cstdio>
 #include <cstdlib>
 #include <vector>
@@ -25,6 +28,7 @@ int main(int argc, char** argv) {
   const size_t n = data.size();
   const uint64_t piece = (uint64_t)atoll(argv[2]);
   const bool skew = atoi(argv[3]) != 0;
+  const bool members = argc > 4 && atoi(argv[4]) != 0;
   if (piece < 16) return 2;
   data.resize(n + 64);  // the reader's slack
   const uint8_t* in = data.data();
@@ -48,6 +52,20 @@ int main(int argc, char** argv) {
         break;
       }
   }
+  std::vector<uint8_t> is_member(starts.size(), 0);
+  is_member[0] = 1;
+  if (members) {  // and every gzip header
+    std::vector<uint64_t> heads;
+    for (size_t p = 0; p < n; ++p) {
+      uint64_t bit = 0;
+      if (member_start_at(in, n, p, &bit)) heads.push_back(bit);
+    }
+    std::vector<uint64_t> probe = starts;
+    starts.resize(probe.size() + heads.size());
+    is_member.resize(starts.size());
+    starts.resize(merge_starts(probe.data(), (uint32_t)probe.size(), heads.data(), (uint32_t)heads.size(), starts.data(),
+                               is_member.data()));
+  }
   const uint32_t n_pieces = (uint32_t)starts.size();
 
   // 2. every piece to its first block end at or beyond the next candidate
@@ -55,25 +73,36 @@ int main(int argc, char** argv) {
   std::vector<int> status(n_pieces);
   std::vector<uint64_t> end_bit(n_pieces), out_len(n_pieces);
   for (uint32_t j = 0; j < n_pieces; ++j)
-    status[j] = piece_boundary(in, n, starts.data(), n_pieces, j, kMaxAbsorb, t, &next[j], &end_bit[j], &out_len[j]);
+    status[j] = members ? piece_boundary(in, n, starts.data(), n_pieces, j, kMaxAbsorb, t, &next[j], &end_bit[j], &out_len[j],
+                                         is_member[j] ? 0u : kWindow)
+                        : piece_boundary(in, n, starts.data(), n_pieces, j, kMaxAbsorb, t, &next[j], &end_bit[j], &out_len[j]);
 
   // 3. the chain from the first piece
-  std::vector<uint32_t> chain(n_pieces);
+  std::vector<uint32_t> chain(n_pieces), member_of(n_pieces, 0);
+  std::vector<MemberTrailer> trailers(n_pieces);
+  uint32_t n_members = 1;
   uint64_t absorbed = 0;
-  const uint32_t n_chain = piece_chain(next.data(), status.data(), n_pieces, chain.data(), &absorbed);
+  const uint32_t n_chain = members ? members_chain(in, n, starts.data(), is_member.data(), next.data(), status.data(), end_bit.data(),
+                                                   n_pieces, chain.data(), member_of.data(), trailers.data(), &n_members, &absorbed)
+                                   : piece_chain(next.data(), status.data(), n_pieces, chain.data(), &absorbed);
   if (n_chain == 0) {
     printf("decline: the chain of pieces does not reach the member's end\n");
     return 3;
   }
-  std::vector<uint64_t> off(n_chain + 1, 0);
-  for (uint32_t i = 0; i < n_chain; ++i) off[i + 1] = off[i] + out_len[chain[i]];
+  std::vector<uint64_t> off(n_chain + 1, 0), member_begin(n_members + 1, 0);
+  for (uint32_t i = 0; i < n_chain; ++i) {
+    if (i > 0 && member_of[i] != member_of[i - 1]) member_begin[member_of[i]] = off[i];
+    off[i + 1] = off[i] + out_len[chain[i]];
+  }
   const uint64_t total = off[n_chain];
+  member_begin[n_members] = total;
 
-  // 4. symbols of every piece on the chain
+  // 4. symbols of every piece on the chain; a match may reach back to its member's first byte
   std::vector<uint16_t> sym(total + 1);
   for (uint32_t i = 0; i < n_chain; ++i) {
     const uint32_t j = chain[i];
-    MarkSink sink{sym.data() + off[i], 0, out_len[j], off[i] < kWindow ? off[i] : kWindow};
+    const uint64_t in_member = off[i] - member_begin[member_of[i]];
+    MarkSink sink{sym.data() + off[i], 0, out_len[j], in_member < kWindow ? in_member : kWindow};
     uint64_t e = 0;
     bool fin = false;
     const uint64_t want_end = end_bit[j];
@@ -95,31 +124,35 @@ int main(int argc, char** argv) {
   for (uint32_t i = 0; i < n_chain; ++i)
     for (uint64_t x = off[i]; x + kWindow < off[i + 1]; ++x) resolve(i, x);
 
-  // 6. CRC-32 in pieces, joined; the trailer must end the file
+  // 6. CRC-32 in pieces, joined per member; the last trailer must end the file
   uint32_t table[256];
   for (uint32_t i = 0; i < 256; ++i) table[i] = crc_table_entry(i);
-  uint32_t crc = 0;
+  std::vector<uint32_t> crc(n_members, 0);
   for (uint32_t i = 0; i < n_chain; ++i) {
     const uint64_t len = off[i + 1] - off[i];
-    crc = crc_combine(crc, crc_bytes(text.data() + off[i], len, [&](uint32_t k) { return table[k]; }), len);
+    crc[member_of[i]] = crc_combine(crc[member_of[i]], crc_bytes(text.data() + off[i], len, [&](uint32_t k) { return table[k]; }), len);
   }
-  const uint64_t at = (end_bit[chain[n_chain - 1]] + 7) / 8;
+  if (!members) trailers[0] = MemberTrailer{(end_bit[chain[n_chain - 1]] + 7) / 8, 0, 0};
+  const uint64_t at = trailers[n_members - 1].at;
   if (at + 8 != n) {
     printf("error: the member's trailer does not end the file\n");
     return 4;
   }
-  const uint32_t want_crc = (uint32_t)in[at] | ((uint32_t)in[at + 1] << 8) | ((uint32_t)in[at + 2] << 16) | ((uint32_t)in[at + 3] << 24);
-  const uint32_t isize = (uint32_t)in[at + 4] | ((uint32_t)in[at + 5] << 8) | ((uint32_t)in[at + 6] << 16) | ((uint32_t)in[at + 7] << 24);
-  if (crc != want_crc) {
-    printf("error: CRC-32 of the inflated bytes differs from the trailer\n");
-    return 4;
-  }
-  if (isize != (uint32_t)total) {
-    printf("error: ISIZE differs from the inflated length\n");
-    return 4;
+  if (!members) trailers[0] = MemberTrailer{at, le32(in + at), le32(in + at + 4)};
+  for (uint32_t m = 0; m < n_members; ++m) {
+    if (crc[m] != trailers[m].crc) {
+      printf("error: CRC-32 of the inflated bytes differs from the trailer of member %u\n", m);
+      return 4;
+    }
+    if (trailers[m].isize != (uint32_t)(member_begin[m + 1] - member_begin[m])) {
+      printf("error: ISIZE differs from the inflated length of member %u\n", m);
+      return 4;
+    }
   }
   unsigned long long h = 1469598103934665603ull;
   for (uint64_t i = 0; i < total; ++i) h = (h ^ text[i]) * 1099511628211ull;
-  printf("%llu %llx %u %u %llu\n", (unsigned long long)total, h, n_pieces, n_chain, (unsigned long long)absorbed);
+  printf("%llu %llx %u %u %llu", (unsigned long long)total, h, n_pieces, n_chain, (unsigned long long)absorbed);
+  if (members) printf(" %u", n_members);
+  printf("\n");
   return 0;
 }
