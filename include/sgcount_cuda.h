@@ -258,32 +258,29 @@ int sgc_fastq_stream_submit(sgc_fastq_stream*, const uint8_t* gz, const uint64_t
 int sgc_fastq_stream_submit_range(sgc_fastq_stream*, const uint8_t* gz, const uint64_t* block_begin,
                                   const uint32_t* block_isize, uint32_t n_blocks, uint32_t head_skip,
                                   uint32_t tail_skip, int self_contained);
-/* ONE gzip member that is not BGZF (what gzip and pigz write): the whole file, gz[0 .. n_bytes) in
- * host memory, inflated, framed and counted on the device, once per stream, then
- * sgc_fastq_stream_finish.  One DEFLATE stream is decoded in parallel by speculation: candidate
- * dynamic-Huffman block starts every 32 KiB of compressed input, a decode without output from each
- * to the next that links the true block boundaries from the member's first block on, then every
- * linked piece decoded into 16-bit symbols whose references to the unknown 32 KiB in front of it
- * are resolved afterwards.  The compressed member stays on the device; the text goes in waves (the
- * limits of the BGZF waves), about 3 bytes of device memory per byte of text in a wave.  When the
- * boundaries cannot be followed to the member's end (blocks other than dynamic Huffman codes over
- * long stretches, damage), the trailer does not end the file (a second member) or ISIZE / CRC-32
- * disagree, it fails with SGC_ERR_GZIP, and with SGC_ERR_FASTQ_FORMAT as sgc_fastq_stream_submit
- * does; the caller then counts the file on the host. */
+/* ONE gzip member that is not BGZF (what gzip and pigz write): as sgc_fastq_stream_submit_gzip,
+ * except that no gzip header inside the file becomes a candidate, so a file of more than one member
+ * fails with SGC_ERR_GZIP. */
 int sgc_fastq_stream_submit_member(sgc_fastq_stream*, const uint8_t* gz, uint64_t n_bytes);
-/* After sgc_fastq_stream_submit_member: candidate pieces, pieces on the chain of true block
- * boundaries, candidates the chain ran past. */
+/* After sgc_fastq_stream_submit_member or sgc_fastq_stream_submit_gzip: candidate pieces, pieces on
+ * the chain of true block boundaries, candidates the chain ran past, summed over the members. */
 int sgc_fastq_stream_member_stats(const sgc_fastq_stream*, uint64_t* pieces, uint64_t* chain, uint64_t* absorbed);
 /* ANY sequence of gzip members — one, several (`cat a.gz b.gz`, appending writers), or BGZF blocks —
  * the whole file, gz[0 .. n_bytes) in host memory, inflated, framed and counted on the device, once
- * per stream, then sgc_fastq_stream_finish.  As sgc_fastq_stream_submit_member, with every gzip header
- * in the file a further candidate piece start where a member begins: the chain of pieces steps from a
- * member's last block over its trailer and the next header.  The members' texts are one byte stream,
- * as gzip -d writes it (a record may straddle two members); CRC-32 and ISIZE are checked member by
- * member.  Fails with SGC_ERR_GZIP when the chain cannot be followed, anything but a whole member
+ * per stream, then sgc_fastq_stream_finish.  The DEFLATE streams are decoded in parallel by
+ * speculation: candidate dynamic-Huffman block starts every 32 KiB of compressed input, and behind
+ * every gzip header in the file a candidate where a member begins; a decode without output from each
+ * to the next that links the true block boundaries from the first member's first block on, stepping
+ * from a member's last block over its trailer and the next header; then every linked piece decoded
+ * into 16-bit symbols whose references to the unknown 32 KiB in front of it are resolved afterwards.
+ * The compressed file stays on the device; the text goes in waves (the limits of the BGZF waves),
+ * about 3 bytes of device memory per byte of text in a wave.  The members' texts are one byte
+ * stream, as gzip -d writes it (a record may straddle two members); CRC-32 and ISIZE are checked
+ * member by member.  Fails with SGC_ERR_GZIP when the boundaries cannot be followed to the end
+ * (blocks other than dynamic Huffman codes over long stretches, damage), anything but a whole member
  * follows a trailer (zero padding included), a member's CRC-32 or ISIZE disagrees, or the file holds
  * more gzip headers than one per 256 bytes; with SGC_ERR_FASTQ_FORMAT as sgc_fastq_stream_submit
- * does.  sgc_fastq_stream_member_stats sums over the members. */
+ * does; the caller then counts the file on the host. */
 int sgc_fastq_stream_submit_gzip(sgc_fastq_stream*, const uint8_t* gz, uint64_t n_bytes);
 /* Members decoded by sgc_fastq_stream_submit_gzip (1 after sgc_fastq_stream_submit_member, else 0). */
 int sgc_fastq_stream_gzip_members(const sgc_fastq_stream*, uint64_t* members);

@@ -104,20 +104,10 @@ __global__ void __launch_bounds__(kInflateThreads) inflate_blocks_kernel(const u
   }
 }
 
-// CRC-32 of every block's text against the trailer of its member (RFC 1952; flate2 checks it for
-// the reference): one warp per block, 32 pieces joined as inflate_core.h describes.
-constexpr int kCrcWarps = 8;
-__global__ void __launch_bounds__(kCrcWarps * 32) crc_blocks_kernel(const uint8_t* __restrict__ gz,
-                                                                   const uint64_t* __restrict__ begin,
-                                                                   const uint64_t* __restrict__ out_off, uint32_t n,
-                                                                   const uint8_t* __restrict__ text, StreamState* st) {
-  __shared__ uint32_t table[256];
-  table[threadIdx.x] = inflate::crc_table_entry(threadIdx.x);
-  __syncthreads();
-  const uint32_t m = blockIdx.x * kCrcWarps + (threadIdx.x >> 5), lane = threadIdx.x & 31;
-  if (m >= n) return;
-  const uint8_t* d = text + out_off[m];
-  const size_t len = (size_t)(out_off[m + 1] - out_off[m]);
+// CRC-32 of d[0 .. len) by the 32 lanes of a warp (the same d and len in every lane): 32 pieces joined
+// as inflate_core.h describes, the result in lane 0.  `table`: the byte table, in shared memory.
+__device__ __forceinline__ uint32_t warp_crc32(const uint8_t* d, size_t len, const uint32_t* table) {
+  const uint32_t lane = threadIdx.x & 31;
   const size_t c = inflate::crc_piece_len(len), first = len - 31 * c;
   const size_t at = lane == 0 ? 0 : first + (lane - 1) * c;
   uint32_t crc = inflate::crc_bytes(d + at, lane == 0 ? first : c, [&](uint32_t i) { return table[i]; });
@@ -128,6 +118,22 @@ __global__ void __launch_bounds__(kCrcWarps * 32) crc_blocks_kernel(const uint8_
     if ((lane & (2 * s - 1)) == 0) crc = inflate::crc_multmodp(p, crc) ^ other;
     p = inflate::crc_multmodp(p, p);
   }
+  return crc;
+}
+
+// CRC-32 of every block's text against the trailer of its member (RFC 1952; flate2 checks it for
+// the reference): one warp per block.
+constexpr int kCrcWarps = 8;
+__global__ void __launch_bounds__(kCrcWarps * 32) crc_blocks_kernel(const uint8_t* __restrict__ gz,
+                                                                   const uint64_t* __restrict__ begin,
+                                                                   const uint64_t* __restrict__ out_off, uint32_t n,
+                                                                   const uint8_t* __restrict__ text, StreamState* st) {
+  __shared__ uint32_t table[256];
+  table[threadIdx.x] = inflate::crc_table_entry(threadIdx.x);
+  __syncthreads();
+  const uint32_t m = blockIdx.x * kCrcWarps + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (m >= n) return;
+  const uint32_t crc = warp_crc32(text + out_off[m], (size_t)(out_off[m + 1] - out_off[m]), table);
   if (lane == 0) {
     const uint8_t* t = gz + (begin[m + 1] - begin[0]) - 8;
     const uint32_t stored = (uint32_t)t[0] | ((uint32_t)t[1] << 8) | ((uint32_t)t[2] << 16) | ((uint32_t)t[3] << 24);
@@ -270,7 +276,7 @@ __global__ void tail_restore_kernel(uint8_t* __restrict__ text, const StreamStat
     text[kHeadroom - tail + i] = tail_buf[i];
 }
 
-// ---- one gzip member (not BGZF) decoded in pieces: the steps of inflate_core.h "ONE member in pieces" ----
+// ---- gzip members (not BGZF) decoded in pieces: the steps of inflate_core.h "gzip members in pieces" ----
 // Candidate piece starts: one warp per nominal boundary c_j = j * piece bytes (j >= 1), its lanes probing
 // consecutive bit offsets; the first that passes wins (or ~0: none before c_{j+1}).
 __global__ void __launch_bounds__(kInflateThreads) member_find_kernel(const uint8_t* __restrict__ gz, uint64_t n_gz,
@@ -294,23 +300,17 @@ __global__ void __launch_bounds__(kInflateThreads) member_find_kernel(const uint
   if (lane == 0) cand[j] = found;
 }
 
-// what the boundary pass learns about a piece (inflate::piece_boundary)
-struct PieceMeta {
-  uint64_t end_bit, out_len;
-  uint32_t next;
-  int32_t status;
-};
 // is_member[j]: piece j starts a gzip member, so none of its matches may reach in front of it
 __global__ void __launch_bounds__(kInflateThreads) member_boundary_kernel(const uint8_t* __restrict__ gz, uint64_t n_gz,
                                                                          const uint64_t* __restrict__ starts,
                                                                          const uint8_t* __restrict__ is_member, uint32_t n,
-                                                                         PieceMeta* __restrict__ meta) {
+                                                                         inflate::PieceMeta* __restrict__ meta) {
   extern __shared__ uint16_t sm[];
   const uint32_t j = blockIdx.x * kInflateThreads + threadIdx.x;
   if (j >= n) return;
   DeviceSymbols symbols;
   const DeviceTables t{sm + threadIdx.x, &symbols};
-  PieceMeta m{0, 0, 0, 0};
+  inflate::PieceMeta m{0, 0, 0, 0};
   m.status = inflate::piece_boundary(gz, (size_t)n_gz, starts, n, j, inflate::kMaxAbsorb, t, &m.next, &m.end_bit, &m.out_len,
                                      is_member[j] ? 0u : inflate::kWindow);
   meta[j] = m;
@@ -421,18 +421,7 @@ __global__ void __launch_bounds__(kCrcWarps * 32) member_crc_kernel(const WavePi
   __syncthreads();
   const uint32_t i = blockIdx.x * kCrcWarps + (threadIdx.x >> 5), lane = threadIdx.x & 31;
   if (i >= n) return;
-  const uint8_t* d = text + wp[i].off;
-  const size_t len = (size_t)(wp[i + 1].off - wp[i].off);
-  const size_t c = inflate::crc_piece_len(len), first = len - 31 * c;
-  const size_t at = lane == 0 ? 0 : first + (lane - 1) * c;
-  uint32_t crc = inflate::crc_bytes(d + at, lane == 0 ? first : c, [&](uint32_t k) { return table[k]; });
-  uint32_t p = inflate::crc_x8n(c);
-#pragma unroll
-  for (int s = 1; s < 32; s *= 2) {
-    const uint32_t other = __shfl_down_sync(0xffffffffu, crc, s);
-    if ((lane & (2 * s - 1)) == 0) crc = inflate::crc_multmodp(p, crc) ^ other;
-    p = inflate::crc_multmodp(p, p);
-  }
+  const uint32_t crc = warp_crc32(text + wp[i].off, (size_t)(wp[i + 1].off - wp[i].off), table);
   if (lane == 0) crc_out[i] = crc;
 }
 
@@ -531,7 +520,7 @@ struct sgc_fastq_stream {
   uint16_t* d_sym = nullptr;
   uint8_t* d_window[2] = {nullptr, nullptr};
   uint64_t* d_cand = nullptr;
-  PieceMeta* d_meta = nullptr;
+  inflate::PieceMeta* d_meta = nullptr;
   WavePiece* d_wave = nullptr;
   uint32_t* d_crc = nullptr;
   size_t sym_cap = 0, cand_cap = 0, meta_cap = 0, wave_cap = 0, crc_cap = 0;
@@ -634,24 +623,24 @@ MemberParams member_params(const sgc_fastq_stream* s) {
 }
 
 // the caller counts the file on the host instead
-int member_decline(sgc_fastq_stream* s, const char* what, const char* why) {
+int member_decline(sgc_fastq_stream* s, const char* why) {
   s->failed = true;
   char buf[240];
-  snprintf(buf, sizeof buf, "%s not decoded on the device: %s", what, why);
+  snprintf(buf, sizeof buf, "gzip file not decoded on the device: %s", why);
   return set_error(SGC_ERR_GZIP, buf);
 }
 
 // 1-2. the compressed bytes to the device; candidate piece starts near every nominal boundary (the first
-// member's first block is piece 0) and, with `members`, at every gzip header; every piece to its first
-// block end at or beyond the next candidate.
-int member_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, size_t header, const MemberParams& p, bool members,
-                  const char* what, std::vector<uint64_t>& starts, std::vector<uint8_t>& is_member, std::vector<PieceMeta>& meta) {
+// member's first block is piece 0) and, with `find_headers`, at every gzip header; every piece to its
+// first block end at or beyond the next candidate.
+int member_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, size_t header, const MemberParams& p, bool find_headers,
+                  std::vector<uint64_t>& starts, std::vector<uint8_t>& is_member, std::vector<inflate::PieceMeta>& meta) {
   const uint32_t n_bounds = (uint32_t)((n_bytes + p.piece - 1) / p.piece);
   // member-start candidates: up to one per 256 bytes of input (fewer, larger members go to the host)
-  const uint64_t heads_cap = members ? n_bytes / 256 + 4096 : 0;
+  const uint64_t heads_cap = find_headers ? n_bytes / 256 + 4096 : 0;
   int rc = grow(&s->d_gz, &s->gz_cap, (size_t)n_bytes + 64, s->pool, s->stream);  // (the reader's slack)
   if (rc == SGC_OK) rc = grow(&s->d_cand, &s->cand_cap, (size_t)n_bounds + 1, s->pool, s->stream);
-  if (rc == SGC_OK && members) rc = grow(&s->d_heads, &s->heads_cap, (size_t)heads_cap + 1, s->pool, s->stream);
+  if (rc == SGC_OK && find_headers) rc = grow(&s->d_heads, &s->heads_cap, (size_t)heads_cap + 1, s->pool, s->stream);
   if (rc) return rc;
   SGC_CUDA_TRY(cudaMemcpyAsync(s->d_gz, gz, n_bytes, cudaMemcpyHostToDevice, s->stream));
   constexpr uint32_t kWarps = kInflateThreads / 32;
@@ -659,7 +648,7 @@ int member_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, size
     member_find_kernel<<<(n_bounds - 1 + kWarps - 1) / kWarps, kInflateThreads, kInflateSmem, s->stream>>>(s->d_gz, n_bytes, p.piece,
                                                                                                           n_bounds, s->d_cand);
   uint64_t n_heads = 0;
-  if (members) {
+  if (find_headers) {
     SGC_CUDA_TRY(cudaMemsetAsync(s->d_heads + heads_cap, 0, sizeof(uint64_t), s->stream));
     const uint64_t threads = (n_bytes + kSignatureBytes - 1) / kSignatureBytes;
     member_signature_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, s->stream>>>(s->d_gz, n_bytes, s->d_heads, heads_cap);
@@ -675,7 +664,7 @@ int member_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, size
     const uint64_t c = cand[j] + (p.skew && (probe.size() & 1) ? 1 : 0);
     if (c > probe.back()) probe.push_back(c);
   }
-  if (n_heads > heads_cap) return member_decline(s, what, "more gzip headers than one per 256 bytes");
+  if (n_heads > heads_cap) return member_decline(s, "more gzip headers than one per 256 bytes");
   std::vector<uint64_t> heads(n_heads);
   if (n_heads) {
     SGC_CUDA_TRY(cudaMemcpyAsync(heads.data(), s->d_heads, n_heads * 8, cudaMemcpyDeviceToHost, s->stream));
@@ -700,7 +689,7 @@ int member_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, size
       s->d_gz, n_bytes, s->d_cand, s->d_is_member, n, s->d_meta);
   SGC_CUDA_TRY(cudaGetLastError());
   meta.resize(n);
-  SGC_CUDA_TRY(cudaMemcpyAsync(meta.data(), s->d_meta, n * sizeof(PieceMeta), cudaMemcpyDeviceToHost, s->stream));
+  SGC_CUDA_TRY(cudaMemcpyAsync(meta.data(), s->d_meta, n * sizeof(inflate::PieceMeta), cudaMemcpyDeviceToHost, s->stream));
   SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
   return SGC_OK;
 }
@@ -708,8 +697,8 @@ int member_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, size
 // 4-7. waves of chain pieces: symbols, windows, text, CRC-32, framing and counting.  member_of[i] is the
 // member of chain piece i: a piece may copy from its member's text only (from none of it when it starts
 // the member).  crc[m] (zero on entry) becomes the CRC-32 of member m's text.
-int member_waves(sgc_fastq_stream* s, uint64_t n_bytes, const MemberParams& p, const char* what, const std::vector<uint64_t>& starts,
-                 const std::vector<PieceMeta>& meta, const uint32_t* chain, const uint32_t* member_of, uint32_t n_chain,
+int member_waves(sgc_fastq_stream* s, uint64_t n_bytes, const MemberParams& p, const std::vector<uint64_t>& starts,
+                 const std::vector<inflate::PieceMeta>& meta, const uint32_t* chain, const uint32_t* member_of, uint32_t n_chain,
                  std::vector<uint32_t>& crc) {
   int rc = SGC_OK;
   for (int w = 0; w < 2; ++w)
@@ -727,11 +716,11 @@ int member_waves(sgc_fastq_stream* s, uint64_t n_bytes, const MemberParams& p, c
     uint64_t text = 0;
     while (b < n_chain && (b == a || text + meta[chain[b]].out_len <= p.wave_text)) text += meta[chain[b++]].out_len;
     const uint32_t nw = b - a;
-    if (s->read_len == 0 && text >= (1ull << 32) - 2 * kHeadroom) return member_decline(s, what, "a piece inflates to 4 GiB or more");
+    if (s->read_len == 0 && text >= (1ull << 32) - 2 * kHeadroom) return member_decline(s, "a piece inflates to 4 GiB or more");
     h_wave.resize((size_t)nw + 1);
     uint64_t off = 0;
     for (uint32_t i = 0; i < nw; ++i) {
-      const PieceMeta& m = meta[chain[a + i]];
+      const inflate::PieceMeta& m = meta[chain[a + i]];
       const uint64_t global = done + off;
       if (a + i > 0 && member_of[a + i] != member_of[a + i - 1]) member_begin = global;
       const uint64_t reach = global - member_begin;
@@ -770,6 +759,58 @@ int member_waves(sgc_fastq_stream* s, uint64_t n_bytes, const MemberParams& p, c
   return SGC_OK;
 }
 
+// sgc_fastq_stream_submit_member (`find_headers` false: no gzip header inside the file is a candidate, so
+// the chain must end at the first trailer) and sgc_fastq_stream_submit_gzip.
+int submit_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, bool find_headers) {
+  if (!s || !gz) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
+  if (s->failed || !s->counter) return set_error(SGC_ERR_INVALID_ARG, "the stream has failed or its counter is gone");
+  if (s->member_submitted || s->blocks_total)
+    return set_error(SGC_ERR_INVALID_ARG, "a gzip file goes to a fresh stream, once");
+  s->member_submitted = true;
+  DeviceGuard guard(s->device);
+  size_t header = 0;
+  if (inflate::gzip_header(gz, (size_t)n_bytes, &header) != inflate::kOk) return member_decline(s, "not a gzip member");
+  const MemberParams params = member_params(s);
+
+  // 1-2. candidate starts near every nominal boundary (and at every gzip header), the boundary pass
+  std::vector<uint64_t> starts;
+  std::vector<uint8_t> is_member;
+  std::vector<inflate::PieceMeta> meta;
+  int rc = member_pieces(s, gz, n_bytes, header, params, find_headers, starts, is_member, meta);
+  if (rc) return rc;
+  const uint32_t n = (uint32_t)starts.size();
+
+  // 3. the chain from the first block, over every trailer and header to the last trailer, which must end the file
+  std::vector<uint32_t> chain(n), member_of(n);
+  std::vector<inflate::MemberTrailer> trailers(n);
+  uint32_t n_members = 0;
+  uint64_t absorbed = 0;
+  const uint32_t n_chain = inflate::members_chain(gz, (size_t)n_bytes, starts.data(), is_member.data(), meta.data(), n, chain.data(),
+                                                  member_of.data(), trailers.data(), &n_members, &absorbed);
+  if (n_chain == 0) return member_decline(s, "the blocks could not be followed from piece to piece to a trailer that ends the file");
+  std::vector<uint64_t> text(n_members, 0);
+  for (uint32_t i = 0; i < n_chain; ++i) text[member_of[i]] += meta[chain[i]].out_len;
+  for (uint32_t m = 0; m < n_members; ++m)
+    if (trailers[m].isize != (uint32_t)text[m]) return member_decline(s, "ISIZE of a member differs from the length of its text");
+  s->member_pieces = n;
+  s->member_chain = n_chain;
+  s->member_absorbed = absorbed;
+
+  // 4-7. waves of chain pieces; CRC-32 member by member
+  std::vector<uint32_t> crc(n_members, 0);
+  rc = member_waves(s, n_bytes, params, starts, meta, chain.data(), member_of.data(), n_chain, crc);
+  if (rc) return rc;
+  for (uint32_t m = 0; m < n_members; ++m)
+    if (crc[m] != trailers[m].crc) {
+      s->failed = true;
+      char buf[160];
+      snprintf(buf, sizeof buf, "gzip member %u: CRC-32 of the inflated bytes differs from the member's trailer", m);
+      return set_error(SGC_ERR_GZIP, buf);
+    }
+  s->gzip_members = n_members;
+  return SGC_OK;
+}
+
 }  // namespace
 
 // Frees the device side and detaches the stream from its counter; the handle itself stays valid.
@@ -786,19 +827,6 @@ void sgc::fastq_stream_release(sgc_fastq_stream* s) {
                   (void*)s->d_sym, (void*)s->d_window[0], (void*)s->d_window[1], (void*)s->d_cand, (void*)s->d_meta,
                   (void*)s->d_wave, (void*)s->d_crc, (void*)s->d_heads, (void*)s->d_is_member})
     scratch_free(p, s->pool, s->stream);
-  s->d_heads = nullptr;
-  s->d_is_member = nullptr;
-  s->d_sym = nullptr;
-  s->d_window[0] = s->d_window[1] = nullptr;
-  s->d_cand = nullptr;
-  s->d_meta = nullptr;
-  s->d_wave = nullptr;
-  s->d_crc = nullptr;
-  s->d_state = nullptr;
-  s->d_gz = s->d_text = s->d_spans = s->d_tail = nullptr;
-  s->d_seq_start = s->d_seq_end = nullptr;
-  s->d_begin = s->d_outoff = nullptr;
-  s->d_counts = s->d_first = s->d_sums = nullptr;
 }
 
 extern "C" {
@@ -917,110 +945,9 @@ int sgc_fastq_stream_finish(sgc_fastq_stream* s, uint64_t* n_records) {
   return SGC_OK;
 }
 
-int sgc_fastq_stream_submit_member(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes) {
-  if (!s || !gz) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
-  if (s->failed || !s->counter) return set_error(SGC_ERR_INVALID_ARG, "the stream has failed or its counter is gone");
-  if (s->member_submitted || s->blocks_total)
-    return set_error(SGC_ERR_INVALID_ARG, "a gzip member goes to a fresh stream, once");
-  s->member_submitted = true;
-  DeviceGuard guard(s->device);
-  const char* what = "single gzip member";
-  size_t header = 0;
-  if (inflate::gzip_header(gz, (size_t)n_bytes, &header) != inflate::kOk) return member_decline(s, what, "not a gzip member");
-  const MemberParams params = member_params(s);
+int sgc_fastq_stream_submit_member(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes) { return submit_pieces(s, gz, n_bytes, false); }
 
-  // 1-2. candidate starts near every nominal boundary, the boundary pass
-  std::vector<uint64_t> starts;
-  std::vector<uint8_t> is_member;
-  std::vector<PieceMeta> meta;
-  int rc = member_pieces(s, gz, n_bytes, header, params, false, what, starts, is_member, meta);
-  if (rc) return rc;
-  const uint32_t n = (uint32_t)starts.size();
-
-  // 3. the chain from the first block; its last piece ends the member, whose trailer must end the file
-  std::vector<uint32_t> next(n), chain(n), member_of(n, 0);
-  std::vector<int> status(n);
-  for (uint32_t j = 0; j < n; ++j) next[j] = meta[j].next, status[j] = meta[j].status;
-  uint64_t absorbed = 0;
-  const uint32_t n_chain = inflate::piece_chain(next.data(), status.data(), n, chain.data(), &absorbed);
-  if (n_chain == 0) return member_decline(s, what, "its blocks could not be followed from piece to piece");
-  const uint64_t trailer = (meta[chain[n_chain - 1]].end_bit + 7) / 8;
-  if (trailer + 8 != n_bytes) return member_decline(s, what, "the member's trailer does not end the file");
-  uint64_t total = 0;
-  for (uint32_t i = 0; i < n_chain; ++i) total += meta[chain[i]].out_len;
-  const uint32_t want_crc = inflate::le32(gz + trailer), isize = inflate::le32(gz + trailer + 4);
-  if (isize != (uint32_t)total) return member_decline(s, what, "ISIZE differs from the length of the inflated text");
-  s->member_pieces = n;
-  s->member_chain = n_chain;
-  s->member_absorbed = absorbed;
-
-  // 4-7. waves of chain pieces
-  std::vector<uint32_t> crc(1, 0);
-  rc = member_waves(s, n_bytes, params, what, starts, meta, chain.data(), member_of.data(), n_chain, crc);
-  if (rc) return rc;
-  if (crc[0] != want_crc) {
-    s->failed = true;
-    return set_error(SGC_ERR_GZIP, "gzip member: CRC-32 of the inflated bytes differs from the member's trailer");
-  }
-  s->gzip_members = 1;
-  return SGC_OK;
-}
-
-int sgc_fastq_stream_submit_gzip(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes) {
-  if (!s || !gz) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
-  if (s->failed || !s->counter) return set_error(SGC_ERR_INVALID_ARG, "the stream has failed or its counter is gone");
-  if (s->member_submitted || s->blocks_total)
-    return set_error(SGC_ERR_INVALID_ARG, "a gzip file goes to a fresh stream, once");
-  s->member_submitted = true;
-  DeviceGuard guard(s->device);
-  const char* what = "gzip members";
-  size_t header = 0;
-  if (inflate::gzip_header(gz, (size_t)n_bytes, &header) != inflate::kOk) return member_decline(s, what, "not a gzip member");
-  const MemberParams params = member_params(s);
-
-  // 1-2. candidate starts near every nominal boundary and at every gzip header, the boundary pass
-  std::vector<uint64_t> starts;
-  std::vector<uint8_t> is_member;
-  std::vector<PieceMeta> meta;
-  int rc = member_pieces(s, gz, n_bytes, header, params, true, what, starts, is_member, meta);
-  if (rc) return rc;
-  const uint32_t n = (uint32_t)starts.size();
-
-  // 3. the chain from the first block, over every trailer and header to the last trailer, which must end the file
-  std::vector<uint32_t> next(n), chain(n), member_of(n);
-  std::vector<int> status(n);
-  std::vector<uint64_t> end_bit(n);
-  for (uint32_t j = 0; j < n; ++j) next[j] = meta[j].next, status[j] = meta[j].status, end_bit[j] = meta[j].end_bit;
-  std::vector<inflate::MemberTrailer> trailers(n);
-  uint32_t n_members = 0;
-  uint64_t absorbed = 0;
-  const uint32_t n_chain = inflate::members_chain(gz, (size_t)n_bytes, starts.data(), is_member.data(), next.data(), status.data(),
-                                                  end_bit.data(), n, chain.data(), member_of.data(), trailers.data(), &n_members,
-                                                  &absorbed);
-  if (n_chain == 0)
-    return member_decline(s, what, "their blocks could not be followed from piece to piece, or a trailer is followed by no gzip member");
-  std::vector<uint64_t> text(n_members, 0);
-  for (uint32_t i = 0; i < n_chain; ++i) text[member_of[i]] += meta[chain[i]].out_len;
-  for (uint32_t m = 0; m < n_members; ++m)
-    if (trailers[m].isize != (uint32_t)text[m]) return member_decline(s, what, "ISIZE of a member differs from the length of its text");
-  s->member_pieces = n;
-  s->member_chain = n_chain;
-  s->member_absorbed = absorbed;
-
-  // 4-7. waves of chain pieces; CRC-32 member by member
-  std::vector<uint32_t> crc(n_members, 0);
-  rc = member_waves(s, n_bytes, params, what, starts, meta, chain.data(), member_of.data(), n_chain, crc);
-  if (rc) return rc;
-  for (uint32_t m = 0; m < n_members; ++m)
-    if (crc[m] != trailers[m].crc) {
-      s->failed = true;
-      char buf[160];
-      snprintf(buf, sizeof buf, "gzip member %u: CRC-32 of the inflated bytes differs from the member's trailer", m);
-      return set_error(SGC_ERR_GZIP, buf);
-    }
-  s->gzip_members = n_members;
-  return SGC_OK;
-}
+int sgc_fastq_stream_submit_gzip(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes) { return submit_pieces(s, gz, n_bytes, true); }
 
 int sgc_fastq_stream_gzip_members(const sgc_fastq_stream* s, uint64_t* members) {
   if (!s || !members) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");

@@ -604,17 +604,26 @@ SGC_HD int gunzip_member(const uint8_t* in, size_t in_len, uint8_t* out, size_t 
   return kOk;
 }
 
-// ---- ONE member in pieces ---------------------------------------------------------------------
-// A single gzip member (what gzip and pigz write) is one DEFLATE stream; it is decoded in parallel
-// by speculation (gzip.cu member_* kernels; host/member_core_test.cpp runs the same steps serially):
+// ---- gzip members in pieces --------------------------------------------------------------------
+// A gzip file, one member (what gzip and pigz write) or several concatenated (`cat a.gz b.gz`,
+// appending writers, BGZF), is one text; it is decoded in parallel by speculation (gzip.cu member_*
+// kernels; host/member_core_test.cpp runs the same steps serially):
 //   1. near every C-th byte, the first bit where a dynamic-Huffman block header parses and a short
-//      trial decode behind it succeeds (probe_block_start) is a candidate piece start;
+//      trial decode behind it succeeds (probe_block_start) is a candidate piece start; so is the bit
+//      after every gzip header that is listed (member_start_at), flagged as a member start (its first
+//      block may be of any kind, so it is not probed);
 //   2. every piece is decoded without output up to the first block end at or beyond the next
-//      candidate (piece_boundary); ending exactly on one links the two, overshooting absorbs it;
-//   3. the links followed from the member's first block give the true block boundaries;
+//      candidate (piece_boundary); ending exactly on one links the two, overshooting absorbs it.  A
+//      piece that starts a member may copy from nothing in front of it;
+//   3. the links followed from the first member's first block give the true block boundaries; from a
+//      member's last block the chain steps over its trailer and the next header to exactly the
+//      candidate that follows them (members_chain).  A false signature costs one piece that fails or
+//      is never linked;
 //   4. each piece on that chain is decoded into 16-bit symbols: 0-255 bytes, 256 + i byte i of the
 //      32 KiB window in front of the piece, still unknown (MarkSink);
 //   5. the windows are resolved piece after piece, then everything else in parallel.
+// A single member is the case where no gzip header inside the file is listed: the first trailer must
+// then end the file, and a file of several members is declined.
 // These functions are written for that use, separately from gunzip_member, whose symbol loop is the
 // BGZF decoder's hot path and stays as it is.
 constexpr uint32_t kWindow = 32768;
@@ -820,34 +829,13 @@ SGC_HD int piece_boundary(const uint8_t* in, size_t in_len, const uint64_t* star
   *out_len = sink.op;
   return kOk;
 }
-// one member: piece 0 starts it, every other piece may copy from the 32 KiB in front of it
-template <typename Tables>
-SGC_HD int piece_boundary(const uint8_t* in, size_t in_len, const uint64_t* starts, uint32_t n, uint32_t j,
-                          uint32_t max_absorb, Tables t, uint32_t* next, uint64_t* end_bit, uint64_t* out_len) {
-  return piece_boundary(in, in_len, starts, n, j, max_absorb, t, next, end_bit, out_len, j == 0 ? 0u : kWindow);
-}
 
-// Step 3 (host): the pieces linked from piece 0 into chain[]; returns their number, or 0 when the
-// links reach a piece whose step 2 failed (status != kOk).  *absorbed: candidates run past.
-inline uint32_t piece_chain(const uint32_t* next, const int* status, uint32_t n, uint32_t* chain, uint64_t* absorbed) {
-  uint32_t len = 0, j = 0;
-  *absorbed = 0;
-  for (;;) {
-    if (j >= n || status[j] != kOk) return 0;
-    chain[len++] = j;
-    if (next[j] == kPieceFinal) return len;
-    *absorbed += next[j] - j - 1;
-    j = next[j];
-  }
-}
-
-// ---- SEVERAL members in pieces ----------------------------------------------------------------
-// Concatenated members (`cat a.gz b.gz`, appending writers, BGZF) are one text, decoded by the same
-// steps with two additions: every gzip header in the input is a further candidate, flagged as a
-// member start (its first block may be of any kind, so it is not probed, and its piece may copy
-// from nothing in front of it), and the chain steps from a member's last block over its trailer
-// and the next header to exactly the candidate that follows them.  A false signature costs one
-// piece that fails or is never linked.
+// what step 2 learns about a piece (piece_boundary)
+struct PieceMeta {
+  uint64_t end_bit, out_len;
+  uint32_t next;
+  int32_t status;
+};
 
 // Does a gzip member header start at byte `pos`?  true and *bit = the first bit of its DEFLATE stream.
 SGC_HD bool member_start_at(const uint8_t* in, size_t in_len, size_t pos, uint64_t* bit) {
@@ -887,29 +875,29 @@ struct MemberTrailer {
   uint32_t crc, isize;
 };
 
-// Step 3 across members (host): from piece 0 (the first member's start) along the links; where a
-// piece ends a member's last block, the member's 8-byte trailer follows at the next byte, and unless
-// it ends the input, a gzip header and the member-start candidate right behind it.  Fills chain[],
-// member_of[] (the member of each chain piece) and trailers[] (one per member, *n_members of them);
-// returns the chain's length, or 0 (decline) when a link is missing, a piece on the way failed, or
-// anything but a whole member follows a trailer (zero padding included).
+// Step 3 (host): from piece 0 (the first member's start) along the links of meta[]; where a piece ends
+// a member's last block, the member's 8-byte trailer follows at the next byte, and unless it ends the
+// input, a gzip header and the member-start candidate right behind it.  Fills chain[], member_of[]
+// (the member of each chain piece) and trailers[] (one per member, *n_members of them); returns the
+// chain's length, or 0 (decline) when a link is missing, a piece on the way failed, or anything but a
+// whole member follows a trailer (zero padding included).
 inline uint32_t members_chain(const uint8_t* in, size_t in_len, const uint64_t* starts, const uint8_t* is_member,
-                              const uint32_t* next, const int* status, const uint64_t* end_bit, uint32_t n, uint32_t* chain,
-                              uint32_t* member_of, MemberTrailer* trailers, uint32_t* n_members, uint64_t* absorbed) {
+                              const PieceMeta* meta, uint32_t n, uint32_t* chain, uint32_t* member_of, MemberTrailer* trailers,
+                              uint32_t* n_members, uint64_t* absorbed) {
   uint32_t len = 0, j = 0, m = 0;
   *absorbed = 0;
   *n_members = 0;
   if (n == 0 || !is_member[0]) return 0;
   for (;;) {
-    if (j >= n || status[j] != kOk) return 0;
+    if (j >= n || meta[j].status != kOk) return 0;
     chain[len] = j;
     member_of[len++] = m;
-    if (next[j] != kPieceFinal) {
-      *absorbed += next[j] - j - 1;
-      j = next[j];
+    if (meta[j].next != kPieceFinal) {
+      *absorbed += meta[j].next - j - 1;
+      j = meta[j].next;
       continue;
     }
-    const uint64_t at = (end_bit[j] + 7) / 8;
+    const uint64_t at = (meta[j].end_bit + 7) / 8;
     if (at + 8 > in_len) return 0;
     trailers[m++] = MemberTrailer{at, le32(in + at), le32(in + at + 4)};
     if (at + 8 == in_len) {

@@ -1,10 +1,10 @@
-// member_core_test <file.gz> <piece_bytes> <skew 0|1> [members 0|1] — decodes a single-member gzip file
-// the way the device does (gzip.cu member_* kernels), serially, from the same csrc/inflate_core.h code:
-// candidate block starts every piece_bytes of compressed input (with skew, every other candidate moved one
-// bit on), the boundary pass, the chain, 16-bit symbols with window markers, the window resolution piece
-// after piece and then the rest, CRC-32 in pieces joined, the trailer.  With members = 1 the file may hold
-// any number of members (sgc_fastq_stream_submit_gzip): every gzip header is a member-start candidate too,
-// the chain steps over trailers (members_chain), and CRC-32 and ISIZE are checked member by member.
+// member_core_test <file.gz> <piece_bytes> <skew 0|1> [members 0|1] — decodes a gzip file the way the
+// device does (gzip.cu member_* kernels), serially, from the same csrc/inflate_core.h code: candidate
+// block starts every piece_bytes of compressed input (with skew, every other candidate moved one bit on),
+// the boundary pass, the chain (members_chain), 16-bit symbols with window markers, the window resolution
+// piece after piece and then the rest, CRC-32 in pieces joined and ISIZE, member by member.  With
+// members = 1 every gzip header is a member-start candidate too, so the file may hold any number of
+// members (sgc_fastq_stream_submit_gzip); without, it must be one (sgc_fastq_stream_submit_member).
 // Prints "<bytes> <fnv1a> <pieces> <chain> <absorbed>" (with members = 1, then "<members>"; exit 0),
 // "decline ..." when the chain does not reach the end (exit 3: the device would hand the file to the
 // host), or the error (exit 4).  Test helper for tests/test_member_inflate_core.py and
@@ -69,22 +69,20 @@ int main(int argc, char** argv) {
   const uint32_t n_pieces = (uint32_t)starts.size();
 
   // 2. every piece to its first block end at or beyond the next candidate
-  std::vector<uint32_t> next(n_pieces);
-  std::vector<int> status(n_pieces);
-  std::vector<uint64_t> end_bit(n_pieces), out_len(n_pieces);
-  for (uint32_t j = 0; j < n_pieces; ++j)
-    status[j] = members ? piece_boundary(in, n, starts.data(), n_pieces, j, kMaxAbsorb, t, &next[j], &end_bit[j], &out_len[j],
-                                         is_member[j] ? 0u : kWindow)
-                        : piece_boundary(in, n, starts.data(), n_pieces, j, kMaxAbsorb, t, &next[j], &end_bit[j], &out_len[j]);
+  std::vector<PieceMeta> meta(n_pieces);
+  for (uint32_t j = 0; j < n_pieces; ++j) {
+    PieceMeta& m = meta[j];
+    m.status = piece_boundary(in, n, starts.data(), n_pieces, j, kMaxAbsorb, t, &m.next, &m.end_bit, &m.out_len,
+                              is_member[j] ? 0u : kWindow);
+  }
 
-  // 3. the chain from the first piece
-  std::vector<uint32_t> chain(n_pieces), member_of(n_pieces, 0);
+  // 3. the chain from the first piece to the last trailer, which ends the file
+  std::vector<uint32_t> chain(n_pieces), member_of(n_pieces);
   std::vector<MemberTrailer> trailers(n_pieces);
-  uint32_t n_members = 1;
+  uint32_t n_members = 0;
   uint64_t absorbed = 0;
-  const uint32_t n_chain = members ? members_chain(in, n, starts.data(), is_member.data(), next.data(), status.data(), end_bit.data(),
-                                                   n_pieces, chain.data(), member_of.data(), trailers.data(), &n_members, &absorbed)
-                                   : piece_chain(next.data(), status.data(), n_pieces, chain.data(), &absorbed);
+  const uint32_t n_chain = members_chain(in, n, starts.data(), is_member.data(), meta.data(), n_pieces, chain.data(), member_of.data(),
+                                         trailers.data(), &n_members, &absorbed);
   if (n_chain == 0) {
     printf("decline: the chain of pieces does not reach the member's end\n");
     return 3;
@@ -92,7 +90,7 @@ int main(int argc, char** argv) {
   std::vector<uint64_t> off(n_chain + 1, 0), member_begin(n_members + 1, 0);
   for (uint32_t i = 0; i < n_chain; ++i) {
     if (i > 0 && member_of[i] != member_of[i - 1]) member_begin[member_of[i]] = off[i];
-    off[i + 1] = off[i] + out_len[chain[i]];
+    off[i + 1] = off[i] + meta[chain[i]].out_len;
   }
   const uint64_t total = off[n_chain];
   member_begin[n_members] = total;
@@ -102,12 +100,12 @@ int main(int argc, char** argv) {
   for (uint32_t i = 0; i < n_chain; ++i) {
     const uint32_t j = chain[i];
     const uint64_t in_member = off[i] - member_begin[member_of[i]];
-    MarkSink sink{sym.data() + off[i], 0, out_len[j], in_member < kWindow ? in_member : kWindow};
+    MarkSink sink{sym.data() + off[i], 0, meta[j].out_len, in_member < kWindow ? in_member : kWindow};
     uint64_t e = 0;
     bool fin = false;
-    const uint64_t want_end = end_bit[j];
+    const uint64_t want_end = meta[j].end_bit;
     const int rc = inflate_piece(in, n, starts[j], want_end, t, sink, [&](uint64_t b) { return b >= want_end; }, &e, &fin);
-    if (rc != kOk || e != want_end || sink.op != out_len[j]) {
+    if (rc != kOk || e != want_end || sink.op != meta[j].out_len) {
       printf("error: piece %u decodes differently the second time (status %d)\n", j, rc);
       return 4;
     }
@@ -124,7 +122,7 @@ int main(int argc, char** argv) {
   for (uint32_t i = 0; i < n_chain; ++i)
     for (uint64_t x = off[i]; x + kWindow < off[i + 1]; ++x) resolve(i, x);
 
-  // 6. CRC-32 in pieces, joined per member; the last trailer must end the file
+  // 6. CRC-32 in pieces, joined per member
   uint32_t table[256];
   for (uint32_t i = 0; i < 256; ++i) table[i] = crc_table_entry(i);
   std::vector<uint32_t> crc(n_members, 0);
@@ -132,13 +130,6 @@ int main(int argc, char** argv) {
     const uint64_t len = off[i + 1] - off[i];
     crc[member_of[i]] = crc_combine(crc[member_of[i]], crc_bytes(text.data() + off[i], len, [&](uint32_t k) { return table[k]; }), len);
   }
-  if (!members) trailers[0] = MemberTrailer{(end_bit[chain[n_chain - 1]] + 7) / 8, 0, 0};
-  const uint64_t at = trailers[n_members - 1].at;
-  if (at + 8 != n) {
-    printf("error: the member's trailer does not end the file\n");
-    return 4;
-  }
-  if (!members) trailers[0] = MemberTrailer{at, le32(in + at), le32(in + at + 4)};
   for (uint32_t m = 0; m < n_members; ++m) {
     if (crc[m] != trailers[m].crc) {
       printf("error: CRC-32 of the inflated bytes differs from the trailer of member %u\n", m);
