@@ -282,6 +282,20 @@ int sgc_fastq_stream_member_stats(const sgc_fastq_stream*, uint64_t* pieces, uin
  * more gzip headers than one per 256 bytes; with SGC_ERR_FASTQ_FORMAT as sgc_fastq_stream_submit
  * does; the caller then counts the file on the host. */
 int sgc_fastq_stream_submit_gzip(sgc_fastq_stream*, const uint8_t* gz, uint64_t n_bytes);
+/* One gzip file (one or several members, as sgc_fastq_stream_submit_gzip) inflated, framed and counted by
+ * n_streams fresh streams together, on one device or several (streams may share a device).  Every
+ * stream copies the file to its device; the candidate search and the boundary pass are split by input
+ * range; the text goes in waves of about min(the one-stream wave, text / n_streams), wave k to stream
+ * k mod n_streams, whose windows are relayed through the host so that no wave waits for another to
+ * decode; records are framed wave after wave, the bytes after a wave's last complete record handed to
+ * the next wave's stream.  The streams must share read_len / span_start / span_len, and their counters
+ * must come from libraries of the same guides (else SGC_ERR_INVALID_ARG).  Each stream counts the records
+ * of its own waves into its own counter: sum the counters with sgc_reduce_counts and call
+ * sgc_fastq_stream_finish on every stream; the records they return add up to the file's.
+ * sgc_fastq_stream_member_stats and sgc_fastq_stream_gzip_members report the whole file on every stream.
+ * A file is declined as by sgc_fastq_stream_submit_gzip, and then every stream has failed.  One host
+ * thread per stream, all joined before the call returns.  n_streams == 1 is sgc_fastq_stream_submit_gzip. */
+int sgc_fastq_stream_submit_gzip_split(sgc_fastq_stream* const* streams, uint32_t n_streams, const uint8_t* gz, uint64_t n_bytes);
 /* Members decoded by sgc_fastq_stream_submit_gzip (1 after sgc_fastq_stream_submit_member, else 0). */
 int sgc_fastq_stream_gzip_members(const sgc_fastq_stream*, uint64_t* members);
 int sgc_fastq_stream_finish(sgc_fastq_stream*, uint64_t* n_records);

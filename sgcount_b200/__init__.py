@@ -5,4 +5,5 @@ sgcount_b200/host.  This package is the thin ctypes mirror the tests and bench.p
 """
 from ._cabi import SgcError  # noqa: F401
 from .api import (Counter, FastqStream, bgzf_blocks, Library, Offset, Permuter, ReadBatch, entropy_offset,  # noqa: F401
-                  entropy_offset_group, position_counts, read_fastx, reduce_counts, reduce_prepare, span_batch, span_geometry)
+                  entropy_offset_group, position_counts, read_fastx, reduce_counts, reduce_prepare, span_batch, span_geometry,
+                  submit_gzip_split)

@@ -100,6 +100,7 @@ SIGNATURES = {
     "sgc_fastq_stream_submit_member": (_int, [_vp, _vp, _u64]),
     "sgc_fastq_stream_member_stats": (_int, [_vp, C.POINTER(_u64), C.POINTER(_u64), C.POINTER(_u64)]),
     "sgc_fastq_stream_submit_gzip": (_int, [_vp, _vp, _u64]),
+    "sgc_fastq_stream_submit_gzip_split": (_int, [C.POINTER(_vp), _u32, _vp, _u64]),
     "sgc_fastq_stream_gzip_members": (_int, [_vp, C.POINTER(_u64)]),
     "sgc_fastq_stream_finish": (_int, [_vp, C.POINTER(_u64)]),
     "sgc_counter_launch_info": (_int, [_vp, C.POINTER(LaunchInfo)]),

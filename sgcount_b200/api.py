@@ -451,3 +451,16 @@ class FastqStream:
         check(_cabi.load().sgc_fastq_stream_finish(self._ptr, C.byref(n)))
         self._counter._result = None
         return int(n.value)
+
+
+def submit_gzip_split(streams: Sequence[FastqStream], blob: np.ndarray) -> None:
+    """one whole gzip file (uint8), as FastqStream.submit_gzip, decoded by several fresh streams together
+    (sgc_fastq_stream_submit_gzip_split), on one device or several; wave k of the text goes to
+    streams[k % len(streams)].  Then sum the streams' counters with reduce_counts and call finish() on
+    every stream: their records add up to the file's.  SgcError(ERR_GZIP) when the device declines it
+    (every stream has then failed: count the file on the host instead)"""
+    blob = np.ascontiguousarray(blob, dtype=np.uint8)
+    arr = (C.c_void_p * len(streams))(*[s._ptr for s in streams])
+    check(_cabi.load().sgc_fastq_stream_submit_gzip_split(arr, len(streams), blob.ctypes.data, len(blob)))
+    for s in streams:
+        s._counter._result = None

@@ -26,8 +26,12 @@
 #include <stdlib.h>
 
 #include <algorithm>
+#include <condition_variable>
+#include <cstddef>
 #include <map>
 #include <mutex>
+#include <string>
+#include <thread>
 #include <vector>
 
 #include "inflate_core.h"
@@ -434,6 +438,35 @@ __global__ void member_window_save_kernel(const uint8_t* __restrict__ text, uint
   }
 }
 
+// ---- one file over several streams (sgc_fastq_stream_submit_gzip_split): inflate_core.h "waves on
+// several streams".  The walk of member_window_kernel, in place on the symbols of the last 32 KiB (or
+// all) of every piece: a marker that names a byte of this wave takes the symbol relayed there, one that
+// names a byte in front of the wave becomes a marker of the wave's entering window.  It needs nothing
+// from another wave.
+__global__ void __launch_bounds__(kWindowThreads) member_window_sym_kernel(uint16_t* sym, const WavePiece* __restrict__ wp,
+                                                                          uint32_t n) {
+  for (uint32_t i = 0; i < n; ++i) {
+    const uint64_t a = wp[i].off, b = wp[i + 1].off;
+    const uint64_t lo = b - a > inflate::kWindow ? b - inflate::kWindow : a;
+    const uint64_t x0 = lo + (uint64_t)threadIdx.x * 32;
+    uint16_t v[32];
+#pragma unroll
+    for (int k = 0; k < 32; ++k) v[k] = x0 + k < b ? inflate::relay_symbol(sym[x0 + k], a, sym) : 0;
+#pragma unroll
+    for (int k = 0; k < 32; ++k)
+      if (x0 + k < b) sym[x0 + k] = v[k];
+    __syncthreads();  // (the next piece reads these symbols)
+  }
+}
+
+// with the entering window known: the relayed last 32 KiB (or all) of every piece, side by side
+__global__ void __launch_bounds__(256) member_settle_kernel(const uint16_t* __restrict__ sym, const WavePiece* __restrict__ wp,
+                                                           uint8_t* __restrict__ text, const uint8_t* __restrict__ window) {
+  const uint64_t a = wp[blockIdx.x].off, b = wp[blockIdx.x + 1].off;
+  const uint64_t lo = b - a > inflate::kWindow ? b - inflate::kWindow : a;
+  for (uint64_t x = lo + threadIdx.x; x < b; x += blockDim.x) text[x] = inflate::settle_symbol(sym[x], window);
+}
+
 // Device scratch of the ingest streams comes from one memory pool per device whose unused memory stays
 // cached, through the stream-ordered allocator.  cudaFree waits for ALL work on the device and cudaMalloc
 // queues up behind it: with several samples in flight on one device (the CLI runs four) every sample that
@@ -630,6 +663,27 @@ int member_decline(sgc_fastq_stream* s, const char* why) {
   return set_error(SGC_ERR_GZIP, buf);
 }
 
+constexpr const char* kTooManyHeaders = "more gzip headers than one per 256 bytes";
+
+// step 1 on the host: the candidates near the nominal boundaries, cand[1 .. n_bounds) (~0: none), after
+// the first member's first block, merged with the member starts heads[] (sorted here)
+void merge_candidates(const MemberParams& p, size_t header, const std::vector<uint64_t>& cand, uint32_t n_bounds,
+                      std::vector<uint64_t>& heads, std::vector<uint64_t>& starts, std::vector<uint8_t>& is_member) {
+  std::vector<uint64_t> probe{(uint64_t)header * 8};
+  for (uint32_t j = 1; j < n_bounds; ++j) {
+    if (cand[j] == ~0ull) continue;
+    const uint64_t c = cand[j] + (p.skew && (probe.size() & 1) ? 1 : 0);
+    if (c > probe.back()) probe.push_back(c);
+  }
+  std::sort(heads.begin(), heads.end());
+  starts.resize(probe.size() + heads.size());
+  is_member.resize(starts.size());
+  starts.resize(inflate::merge_starts(probe.data(), (uint32_t)probe.size(), heads.data(), (uint32_t)heads.size(), starts.data(),
+                                      is_member.data()));
+  is_member.resize(starts.size());
+  is_member[0] = 1;  // (the first member's start, found by both scans)
+}
+
 // 1-2. the compressed bytes to the device; candidate piece starts near every nominal boundary (the first
 // member's first block is piece 0) and, with `find_headers`, at every gzip header; every piece to its
 // first block end at or beyond the next candidate.
@@ -658,25 +712,13 @@ int member_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, size
   std::vector<uint64_t> cand((size_t)n_bounds + 1, ~0ull);
   if (n_bounds > 1) SGC_CUDA_TRY(cudaMemcpyAsync(cand.data() + 1, s->d_cand + 1, (n_bounds - 1) * 8ull, cudaMemcpyDeviceToHost, s->stream));
   SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
-  std::vector<uint64_t> probe{(uint64_t)header * 8};
-  for (uint32_t j = 1; j < n_bounds; ++j) {
-    if (cand[j] == ~0ull) continue;
-    const uint64_t c = cand[j] + (p.skew && (probe.size() & 1) ? 1 : 0);
-    if (c > probe.back()) probe.push_back(c);
-  }
-  if (n_heads > heads_cap) return member_decline(s, "more gzip headers than one per 256 bytes");
+  if (n_heads > heads_cap) return member_decline(s, kTooManyHeaders);
   std::vector<uint64_t> heads(n_heads);
   if (n_heads) {
     SGC_CUDA_TRY(cudaMemcpyAsync(heads.data(), s->d_heads, n_heads * 8, cudaMemcpyDeviceToHost, s->stream));
     SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
-    std::sort(heads.begin(), heads.end());
   }
-  starts.resize(probe.size() + heads.size());
-  is_member.resize(starts.size());
-  starts.resize(inflate::merge_starts(probe.data(), (uint32_t)probe.size(), heads.data(), (uint32_t)heads.size(), starts.data(),
-                                      is_member.data()));
-  is_member.resize(starts.size());
-  is_member[0] = 1;  // (the first member's start, found by both scans)
+  merge_candidates(p, header, cand, n_bounds, heads, starts, is_member);
   const uint32_t n = (uint32_t)starts.size();
 
   rc = grow(&s->d_meta, &s->meta_cap, (size_t)n, s->pool, s->stream);
@@ -759,6 +801,41 @@ int member_waves(sgc_fastq_stream* s, uint64_t n_bytes, const MemberParams& p, c
   return SGC_OK;
 }
 
+// step 3: the chain of pieces, the member of each, the trailers
+struct MemberChain {
+  std::vector<uint32_t> chain, member_of;
+  std::vector<inflate::MemberTrailer> trailers;
+  uint32_t n_chain = 0, n_members = 0;
+  uint64_t absorbed = 0;
+};
+// nullptr, or why the file is declined
+const char* follow_chain(const uint8_t* gz, uint64_t n_bytes, const std::vector<uint64_t>& starts, const std::vector<uint8_t>& is_member,
+                         const std::vector<inflate::PieceMeta>& meta, MemberChain& c) {
+  const uint32_t n = (uint32_t)starts.size();
+  c.chain.resize(n);
+  c.member_of.resize(n);
+  c.trailers.resize(n);
+  c.n_chain = inflate::members_chain(gz, (size_t)n_bytes, starts.data(), is_member.data(), meta.data(), n, c.chain.data(),
+                                     c.member_of.data(), c.trailers.data(), &c.n_members, &c.absorbed);
+  if (c.n_chain == 0) return "the blocks could not be followed from piece to piece to a trailer that ends the file";
+  std::vector<uint64_t> text(c.n_members, 0);
+  for (uint32_t i = 0; i < c.n_chain; ++i) text[c.member_of[i]] += meta[c.chain[i]].out_len;
+  for (uint32_t m = 0; m < c.n_members; ++m)
+    if (c.trailers[m].isize != (uint32_t)text[m]) return "ISIZE of a member differs from the length of its text";
+  return nullptr;
+}
+// the first member whose CRC-32 differs from its trailer's, or n_members
+uint32_t crc_mismatch(const MemberChain& c, const std::vector<uint32_t>& crc) {
+  for (uint32_t m = 0; m < c.n_members; ++m)
+    if (crc[m] != c.trailers[m].crc) return m;
+  return c.n_members;
+}
+int crc_error(uint32_t m) {
+  char buf[160];
+  snprintf(buf, sizeof buf, "gzip member %u: CRC-32 of the inflated bytes differs from the member's trailer", m);
+  return set_error(SGC_ERR_GZIP, buf);
+}
+
 // sgc_fastq_stream_submit_member (`find_headers` false: no gzip header inside the file is a candidate, so
 // the chain must end at the first trailer) and sgc_fastq_stream_submit_gzip.
 int submit_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, bool find_headers) {
@@ -781,33 +858,316 @@ int submit_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, bool
   const uint32_t n = (uint32_t)starts.size();
 
   // 3. the chain from the first block, over every trailer and header to the last trailer, which must end the file
-  std::vector<uint32_t> chain(n), member_of(n);
-  std::vector<inflate::MemberTrailer> trailers(n);
-  uint32_t n_members = 0;
-  uint64_t absorbed = 0;
-  const uint32_t n_chain = inflate::members_chain(gz, (size_t)n_bytes, starts.data(), is_member.data(), meta.data(), n, chain.data(),
-                                                  member_of.data(), trailers.data(), &n_members, &absorbed);
-  if (n_chain == 0) return member_decline(s, "the blocks could not be followed from piece to piece to a trailer that ends the file");
-  std::vector<uint64_t> text(n_members, 0);
-  for (uint32_t i = 0; i < n_chain; ++i) text[member_of[i]] += meta[chain[i]].out_len;
-  for (uint32_t m = 0; m < n_members; ++m)
-    if (trailers[m].isize != (uint32_t)text[m]) return member_decline(s, "ISIZE of a member differs from the length of its text");
+  MemberChain c;
+  if (const char* why = follow_chain(gz, n_bytes, starts, is_member, meta, c)) return member_decline(s, why);
   s->member_pieces = n;
-  s->member_chain = n_chain;
-  s->member_absorbed = absorbed;
+  s->member_chain = c.n_chain;
+  s->member_absorbed = c.absorbed;
 
   // 4-7. waves of chain pieces; CRC-32 member by member
-  std::vector<uint32_t> crc(n_members, 0);
-  rc = member_waves(s, n_bytes, params, starts, meta, chain.data(), member_of.data(), n_chain, crc);
+  std::vector<uint32_t> crc(c.n_members, 0);
+  rc = member_waves(s, n_bytes, params, starts, meta, c.chain.data(), c.member_of.data(), c.n_chain, crc);
   if (rc) return rc;
-  for (uint32_t m = 0; m < n_members; ++m)
-    if (crc[m] != trailers[m].crc) {
-      s->failed = true;
-      char buf[160];
-      snprintf(buf, sizeof buf, "gzip member %u: CRC-32 of the inflated bytes differs from the member's trailer", m);
-      return set_error(SGC_ERR_GZIP, buf);
+  if (const uint32_t m = crc_mismatch(c, crc); m < c.n_members) {
+    s->failed = true;
+    return crc_error(m);
+  }
+  s->gzip_members = c.n_members;
+  return SGC_OK;
+}
+
+// ---- one gzip file over several streams: the host side of sgc_fastq_stream_submit_gzip_split ----
+// Runs fn(i) for every stream i on a thread of its own, with the stream's device current, and joins
+// them all.  Returns the first failure by stream index, its message set on the calling thread.
+template <typename Fn>
+int on_each_stream(sgc_fastq_stream* const* ss, uint32_t n, Fn fn) {
+  std::vector<int> rc(n, SGC_OK);
+  std::vector<std::string> msg(n);
+  std::vector<std::thread> threads;
+  threads.reserve(n);
+  for (uint32_t i = 0; i < n; ++i)
+    threads.emplace_back([&, i] {
+      DeviceGuard guard(ss[i]->device);
+      rc[i] = fn(i);
+      if (rc[i]) msg[i] = sgc_last_error();
+    });
+  for (auto& t : threads) t.join();
+  for (uint32_t i = 0; i < n; ++i)
+    if (rc[i]) return set_error(rc[i], msg[i]);
+  return SGC_OK;
+}
+
+// where part i of n_items cut into `parts` starts: equal parts, rounded up to a multiple of `grain`
+uint64_t part_begin(uint64_t n_items, uint32_t parts, uint32_t i, uint64_t grain) {
+  const uint64_t per = (n_items + parts - 1) / parts;
+  return std::min(n_items, (per + grain - 1) / grain * grain * i);
+}
+
+int split_fail(sgc_fastq_stream* const* ss, uint32_t n, int rc) {
+  for (uint32_t i = 0; i < n; ++i) ss[i]->failed = true;
+  return rc;
+}
+
+// 1-2 of member_pieces with find_headers, each kernel over one contiguous part per stream.  The kernels
+// are those of one stream, given shifted pointers: member_find_kernel's boundary 1 is boundary j0, its
+// bits count from byte (j0 - 1) * piece; member_signature_kernel starts at byte b0 (whole blocks of it
+// per part); member_boundary_kernel's piece 0 is piece c0 (so `next` counts from c0).
+int split_pieces(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* gz, uint64_t n_bytes, size_t header, const MemberParams& p,
+                 std::vector<uint64_t>& starts, std::vector<uint8_t>& is_member, std::vector<inflate::PieceMeta>& meta) {
+  const uint32_t n_bounds = (uint32_t)((n_bytes + p.piece - 1) / p.piece);
+  const uint64_t heads_cap = n_bytes / 256 + 4096;
+  constexpr uint32_t kWarps = kInflateThreads / 32;
+  constexpr uint64_t kSignatureSpan = 256ull * kSignatureBytes;  // the input of one block of member_signature_kernel
+  std::vector<uint64_t> cand((size_t)n_bounds + 1, ~0ull), found(ns, 0);
+  std::vector<std::vector<uint64_t>> heads(ns);
+  int rc = on_each_stream(ss, ns, [&](uint32_t i) {
+    sgc_fastq_stream* s = ss[i];
+    int rc = grow(&s->d_gz, &s->gz_cap, (size_t)n_bytes + 64, s->pool, s->stream);  // (the reader's slack)
+    if (rc == SGC_OK) rc = grow(&s->d_cand, &s->cand_cap, (size_t)n_bounds + 1, s->pool, s->stream);
+    if (rc == SGC_OK) rc = grow(&s->d_heads, &s->heads_cap, (size_t)heads_cap + 1, s->pool, s->stream);
+    if (rc) return rc;
+    SGC_CUDA_TRY(cudaMemcpyAsync(s->d_gz, gz, n_bytes, cudaMemcpyHostToDevice, s->stream));
+    const uint64_t j0 = 1 + part_begin(n_bounds - 1, ns, i, kWarps), j1 = 1 + part_begin(n_bounds - 1, ns, i + 1, kWarps);
+    const uint64_t shift = (j0 - 1) * p.piece;
+    if (j1 > j0)
+      member_find_kernel<<<(unsigned)((j1 - j0 + kWarps - 1) / kWarps), kInflateThreads, kInflateSmem, s->stream>>>(
+          s->d_gz + shift, n_bytes - shift, p.piece, (uint32_t)(j1 - j0 + 1), s->d_cand + (j0 - 1));
+    const uint64_t b0 = part_begin(n_bytes, ns, i, kSignatureSpan), b1 = part_begin(n_bytes, ns, i + 1, kSignatureSpan);
+    SGC_CUDA_TRY(cudaMemsetAsync(s->d_heads + heads_cap, 0, sizeof(uint64_t), s->stream));
+    if (b1 > b0)
+      member_signature_kernel<<<(unsigned)((b1 - b0 + kSignatureSpan - 1) / kSignatureSpan), 256, 0, s->stream>>>(
+          s->d_gz + b0, n_bytes - b0, s->d_heads, heads_cap);
+    SGC_CUDA_TRY(cudaGetLastError());
+    SGC_CUDA_TRY(cudaMemcpyAsync(&found[i], s->d_heads + heads_cap, sizeof(uint64_t), cudaMemcpyDeviceToHost, s->stream));
+    if (j1 > j0) SGC_CUDA_TRY(cudaMemcpyAsync(cand.data() + j0, s->d_cand + j0, (j1 - j0) * 8, cudaMemcpyDeviceToHost, s->stream));
+    SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+    for (uint64_t j = j0; j < j1; ++j)
+      if (cand[j] != ~0ull) cand[j] += shift * 8;
+    heads[i].resize(std::min(found[i], heads_cap));
+    if (!heads[i].empty()) {
+      SGC_CUDA_TRY(cudaMemcpyAsync(heads[i].data(), s->d_heads, heads[i].size() * 8, cudaMemcpyDeviceToHost, s->stream));
+      SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
     }
-  s->gzip_members = n_members;
+    for (uint64_t& h : heads[i]) h += b0 * 8;
+    return SGC_OK;
+  });
+  if (rc) return rc;
+  uint64_t n_heads = 0;
+  for (uint32_t i = 0; i < ns; ++i) n_heads += found[i];
+  if (n_heads > heads_cap) return member_decline(ss[0], kTooManyHeaders);
+  std::vector<uint64_t> all_heads;
+  all_heads.reserve(n_heads);
+  for (auto& h : heads) all_heads.insert(all_heads.end(), h.begin(), h.end());
+  merge_candidates(p, header, cand, n_bounds, all_heads, starts, is_member);
+
+  const uint32_t n = (uint32_t)starts.size();
+  meta.resize(n);
+  return on_each_stream(ss, ns, [&](uint32_t i) {
+    sgc_fastq_stream* s = ss[i];
+    const uint32_t c0 = (uint32_t)part_begin(n, ns, i, kInflateThreads), c1 = (uint32_t)part_begin(n, ns, i + 1, kInflateThreads);
+    if (c1 <= c0) return SGC_OK;
+    int rc = grow(&s->d_meta, &s->meta_cap, (size_t)n, s->pool, s->stream);
+    if (rc == SGC_OK) rc = grow(&s->d_cand, &s->cand_cap, (size_t)n, s->pool, s->stream);
+    if (rc == SGC_OK) rc = grow(&s->d_is_member, &s->is_member_cap, (size_t)n, s->pool, s->stream);
+    if (rc) return rc;
+    SGC_CUDA_TRY(cudaMemcpyAsync(s->d_cand, starts.data(), n * 8ull, cudaMemcpyHostToDevice, s->stream));
+    SGC_CUDA_TRY(cudaMemcpyAsync(s->d_is_member, is_member.data(), n, cudaMemcpyHostToDevice, s->stream));
+    member_boundary_kernel<<<(c1 - c0 + kInflateThreads - 1) / kInflateThreads, kInflateThreads, kInflateSmem, s->stream>>>(
+        s->d_gz, n_bytes, s->d_cand + c0, s->d_is_member + c0, n - c0, s->d_meta + c0);
+    SGC_CUDA_TRY(cudaGetLastError());
+    SGC_CUDA_TRY(cudaMemcpyAsync(meta.data() + c0, s->d_meta + c0, (c1 - c0) * sizeof(inflate::PieceMeta), cudaMemcpyDeviceToHost,
+                                 s->stream));
+    SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+    for (uint32_t j = c0; j < c1; ++j)
+      if (meta[j].status == inflate::kOk && meta[j].next != inflate::kPieceFinal) meta[j].next += c0;
+    return SGC_OK;
+  });
+}
+
+// a wave of the chain: pieces [a, b), their text and where it goes
+struct SplitWave {
+  uint32_t a, b;
+  uint64_t text;
+  std::vector<WavePiece> wp;
+};
+
+// What the streams of one split call hand each other: the entering window of every wave, composed on
+// the host as the waves in front publish F_k, and the bytes after the last complete record of the wave
+// framed last (framing goes wave after wave).
+struct WindowRelay {
+  std::mutex mu;
+  std::condition_variable cv;
+  bool stop = false;                         // a stream failed: the others give up
+  std::vector<std::vector<uint16_t>> front;  // F_k, empty until wave k published it
+  std::vector<std::vector<uint8_t>> window;  // W_k, known for k < composed
+  uint32_t composed = 1;
+  uint32_t framed = 0;  // waves framed and counted
+  std::vector<uint8_t> tail;
+};
+
+// 4-7 for the waves k = i, i + ns, ... dealt to stream i; crc[x] (x: chain position) the CRC-32 of piece x.
+// Returns SGC_OK without finishing when another stream failed (relay.stop; the caller sets it on a failure).
+int split_stream_waves(sgc_fastq_stream* s, uint32_t i, uint32_t ns, uint64_t n_bytes, const std::vector<SplitWave>& waves,
+                       WindowRelay& relay, std::vector<uint32_t>& crc) {
+  const uint32_t n_waves = (uint32_t)waves.size();
+  auto wait_for = [&](auto ready) {  // false: another stream failed
+    std::unique_lock<std::mutex> lk(relay.mu);
+    relay.cv.wait(lk, [&] { return relay.stop || ready(); });
+    return !relay.stop;
+  };
+  const size_t tail_at = offsetof(StreamState, tail);
+  int rc = SGC_OK;
+  if (!s->d_window[0] && (rc = scratch_alloc(reinterpret_cast<void**>(&s->d_window[0]), inflate::kWindow, s->pool, s->stream)))
+    return rc;
+  for (uint32_t k = i; k < n_waves; k += ns) {
+    const SplitWave& w = waves[k];
+    const uint32_t nw = w.b - w.a;
+    rc = grow(&s->d_wave, &s->wave_cap, (size_t)nw + 1, s->pool, s->stream);
+    if (rc == SGC_OK) rc = grow(&s->d_sym, &s->sym_cap, (size_t)w.text + 1, s->pool, s->stream);
+    if (rc == SGC_OK) rc = grow(&s->d_text, &s->text_cap, (size_t)kHeadroom + w.text + 64, s->pool, s->stream);
+    if (rc == SGC_OK) rc = grow(&s->d_crc, &s->crc_cap, (size_t)nw, s->pool, s->stream);
+    if (rc) return rc;
+    SGC_CUDA_TRY(cudaMemcpyAsync(s->d_wave, w.wp.data(), w.wp.size() * sizeof(WavePiece), cudaMemcpyHostToDevice, s->stream));
+    // symbols, relayed windows, F_k
+    member_decode_kernel<<<(nw + kInflateThreads - 1) / kInflateThreads, kInflateThreads, kInflateSmem, s->stream>>>(
+        s->d_gz, n_bytes, s->d_wave, nw, s->d_sym, s->d_state);
+    member_window_sym_kernel<<<1, kWindowThreads, 0, s->stream>>>(s->d_sym, s->d_wave, nw);
+    SGC_CUDA_TRY(cudaGetLastError());
+    std::vector<uint16_t> f(inflate::kWindow);
+    const uint64_t m = std::min<uint64_t>(w.text, inflate::kWindow);
+    StreamState st;
+    SGC_CUDA_TRY(cudaMemcpyAsync(f.data() + (inflate::kWindow - m), s->d_sym + (w.text - m), m * 2, cudaMemcpyDeviceToHost, s->stream));
+    SGC_CUDA_TRY(cudaMemcpyAsync(&st, s->d_state, sizeof st, cudaMemcpyDeviceToHost, s->stream));
+    SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+    if (st.bad_block != 0xFFFFFFFFu) return stream_error(s, st, w.a);
+    inflate::wave_front(f.data(), w.text);
+    {
+      std::lock_guard<std::mutex> lk(relay.mu);
+      relay.front[k] = std::move(f);
+      for (; relay.composed < n_waves && !relay.front[relay.composed - 1].empty(); ++relay.composed)
+        inflate::compose_window(relay.front[relay.composed - 1].data(), relay.window[relay.composed - 1].data(),
+                                relay.window[relay.composed].data());
+      relay.cv.notify_all();
+    }
+    // the text, once W_k is known
+    if (!wait_for([&] { return relay.composed > k; })) return SGC_OK;
+    SGC_CUDA_TRY(cudaMemcpyAsync(s->d_window[0], relay.window[k].data(), inflate::kWindow, cudaMemcpyHostToDevice, s->stream));
+    uint8_t* text = s->d_text + kHeadroom;
+    member_settle_kernel<<<nw, 256, 0, s->stream>>>(s->d_sym, s->d_wave, text, s->d_window[0]);
+    member_resolve_kernel<<<nw, 256, 0, s->stream>>>(s->d_sym, s->d_wave, text, s->d_window[0]);
+    member_crc_kernel<<<(nw + kCrcWarps - 1) / kCrcWarps, kCrcWarps * 32, 0, s->stream>>>(s->d_wave, nw, text, s->d_crc);
+    SGC_CUDA_TRY(cudaGetLastError());
+    // framing, behind the wave in front: its carried bytes come first
+    if (!wait_for([&] { return relay.framed == k; })) return SGC_OK;
+    const uint32_t carried = (uint32_t)relay.tail.size();
+    if (carried) SGC_CUDA_TRY(cudaMemcpyAsync(s->d_tail, relay.tail.data(), carried, cudaMemcpyHostToDevice, s->stream));
+    SGC_CUDA_TRY(cudaMemcpyAsync(reinterpret_cast<uint8_t*>(s->d_state) + tail_at, &carried, 4, cudaMemcpyHostToDevice, s->stream));
+    wave_begin_kernel<<<1, 1, 0, s->stream>>>(s->d_state, 0, 0);
+    if ((rc = frame_and_count(s, w.text, w.a))) return rc;  // (synchronises)
+    SGC_CUDA_TRY(cudaMemcpyAsync(crc.data() + w.a, s->d_crc, nw * 4ull, cudaMemcpyDeviceToHost, s->stream));
+    SGC_CUDA_TRY(cudaMemcpyAsync(&st, s->d_state, sizeof st, cudaMemcpyDeviceToHost, s->stream));
+    SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+    std::vector<uint8_t> tail;
+    if (k + 1 < n_waves) {  // the wave's tail goes on to the next wave's stream (the last wave's stays: finish() counts it)
+      tail.resize(st.tail);
+      const uint32_t zero = 0;
+      if (st.tail) SGC_CUDA_TRY(cudaMemcpyAsync(tail.data(), s->d_tail, st.tail, cudaMemcpyDeviceToHost, s->stream));
+      SGC_CUDA_TRY(cudaMemcpyAsync(reinterpret_cast<uint8_t*>(s->d_state) + tail_at, &zero, 4, cudaMemcpyHostToDevice, s->stream));
+      SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+    }
+    std::lock_guard<std::mutex> lk(relay.mu);
+    relay.tail = std::move(tail);
+    relay.framed = k + 1;
+    relay.cv.notify_all();
+  }
+  return SGC_OK;
+}
+
+int submit_split(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* gz, uint64_t n_bytes) {
+  if (!ss || !gz || ns == 0) return set_error(SGC_ERR_INVALID_ARG, "NULL argument or no stream");
+  for (uint32_t i = 0; i < ns; ++i)
+    if (!ss[i]) return set_error(SGC_ERR_INVALID_ARG, "NULL stream");
+  if (ns == 1) return submit_pieces(ss[0], gz, n_bytes, true);
+  for (uint32_t i = 0; i < ns; ++i) {
+    const sgc_fastq_stream* s = ss[i];
+    if (s->failed || !s->counter) return set_error(SGC_ERR_INVALID_ARG, "a stream has failed or its counter is gone");
+    if (s->member_submitted || s->blocks_total) return set_error(SGC_ERR_INVALID_ARG, "a gzip file goes to fresh streams, once");
+    for (uint32_t j = 0; j < i; ++j)
+      if (ss[j] == s) return set_error(SGC_ERR_INVALID_ARG, "a stream is given twice");
+    const sgc_fastq_stream* s0 = ss[0];
+    if (s->read_len != s0->read_len || s->span_start != s0->span_start || s->span_len != s0->span_len)
+      return set_error(SGC_ERR_INVALID_ARG, "the streams differ in read length or span");
+    const sgc_library *l = s->counter->lib, *l0 = s0->counter->lib;
+    if (l->n != l0->n || l->k != l0->k || l->with_perm != l0->with_perm)
+      return set_error(SGC_ERR_INVALID_ARG, "the streams' counters come from different libraries");
+  }
+  for (uint32_t i = 0; i < ns; ++i) ss[i]->member_submitted = true;
+  size_t header = 0;
+  if (inflate::gzip_header(gz, (size_t)n_bytes, &header) != inflate::kOk)
+    return split_fail(ss, ns, member_decline(ss[0], "not a gzip member"));
+  const MemberParams params = member_params(ss[0]);
+
+  // 1-2. split by input range
+  std::vector<uint64_t> starts;
+  std::vector<uint8_t> is_member;
+  std::vector<inflate::PieceMeta> meta;
+  int rc = split_pieces(ss, ns, gz, n_bytes, header, params, starts, is_member, meta);
+  if (rc) return split_fail(ss, ns, rc);
+
+  // 3. the chain, as for one stream
+  MemberChain c;
+  if (const char* why = follow_chain(gz, n_bytes, starts, is_member, meta, c)) return split_fail(ss, ns, member_decline(ss[0], why));
+
+  // 4-7. waves of about min(wave_text, text / streams), dealt round robin
+  uint64_t total = 0;
+  for (uint32_t i = 0; i < c.n_chain; ++i) total += meta[c.chain[i]].out_len;
+  const uint64_t cap = std::min(params.wave_text, std::max<uint64_t>(1, (total + ns - 1) / ns));
+  std::vector<SplitWave> waves;
+  uint64_t done = 0, member_begin = 0;
+  for (uint32_t a = 0; a < c.n_chain;) {
+    SplitWave w{a, a, 0, {}};
+    while (w.b < c.n_chain && (w.b == a || w.text + meta[c.chain[w.b]].out_len <= cap)) w.text += meta[c.chain[w.b++]].out_len;
+    if (ss[0]->read_len == 0 && w.text >= (1ull << 32) - 2 * kHeadroom)
+      return split_fail(ss, ns, member_decline(ss[0], "a piece inflates to 4 GiB or more"));
+    uint64_t off = 0;
+    for (uint32_t x = a; x < w.b; ++x) {
+      if (x > 0 && c.member_of[x] != c.member_of[x - 1]) member_begin = done + off;
+      const uint64_t reach = done + off - member_begin;
+      w.wp.push_back(WavePiece{starts[c.chain[x]], meta[c.chain[x]].end_bit, off, std::min<uint64_t>(reach, inflate::kWindow)});
+      off += meta[c.chain[x]].out_len;
+    }
+    w.wp.push_back(WavePiece{0, 0, w.text, 0});
+    done += w.text;
+    a = w.b;
+    waves.push_back(std::move(w));
+  }
+  WindowRelay relay;
+  relay.front.resize(waves.size());
+  relay.window.assign(waves.size(), std::vector<uint8_t>(inflate::kWindow, 0));  // W_0: zeros
+  std::vector<uint32_t> piece_crc(c.n_chain, 0);
+  rc = on_each_stream(ss, ns, [&](uint32_t i) {
+    const int rc = split_stream_waves(ss[i], i, ns, n_bytes, waves, relay, piece_crc);
+    if (rc) {
+      std::lock_guard<std::mutex> lk(relay.mu);
+      relay.stop = true;
+      relay.cv.notify_all();
+    }
+    return rc;
+  });
+  if (rc) return split_fail(ss, ns, rc);
+  std::vector<uint32_t> crc(c.n_members, 0);
+  for (const SplitWave& w : waves)
+    for (uint32_t x = w.a; x < w.b; ++x) {
+      uint32_t& m = crc[c.member_of[x]];
+      m = inflate::crc_combine(m, piece_crc[x], w.wp[x - w.a + 1].off - w.wp[x - w.a].off);
+    }
+  if (const uint32_t m = crc_mismatch(c, crc); m < c.n_members) return split_fail(ss, ns, crc_error(m));
+  for (uint32_t i = 0; i < ns; ++i) {
+    ss[i]->member_pieces = starts.size();
+    ss[i]->member_chain = c.n_chain;
+    ss[i]->member_absorbed = c.absorbed;
+    ss[i]->gzip_members = c.n_members;
+  }
   return SGC_OK;
 }
 
@@ -948,6 +1308,10 @@ int sgc_fastq_stream_finish(sgc_fastq_stream* s, uint64_t* n_records) {
 int sgc_fastq_stream_submit_member(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes) { return submit_pieces(s, gz, n_bytes, false); }
 
 int sgc_fastq_stream_submit_gzip(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes) { return submit_pieces(s, gz, n_bytes, true); }
+
+int sgc_fastq_stream_submit_gzip_split(sgc_fastq_stream* const* streams, uint32_t n_streams, const uint8_t* gz, uint64_t n_bytes) {
+  return submit_split(streams, n_streams, gz, n_bytes);
+}
 
 int sgc_fastq_stream_gzip_members(const sgc_fastq_stream* s, uint64_t* members) {
   if (!s || !members) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");

@@ -917,6 +917,37 @@ inline uint32_t members_chain(const uint8_t* in, size_t in_len, const uint64_t* 
   }
 }
 
+// ---- waves on several streams: the window relay ------------------------------------------------
+// The chain's text, cut into waves k = 0, 1, ..., may be decoded by several streams at once
+// (sgc_fastq_stream_submit_gzip_split; member_core_test with <waves>).  Wave k's first pieces refer,
+// through their markers, to W_k, the 32 KiB of text in front of the wave, which earlier waves make.
+// So that no wave waits for another while it decodes:
+//   a. the last 32 KiB (or all) of every piece, piece after piece, are relayed in place
+//      (relay_symbol): a marker that names a byte of the wave takes the symbol already relayed
+//      there, one that names a byte in front of the wave becomes 256 + j, byte j of W_k;
+//   b. F_k, the wave's last 32 KiB as such symbols (wave_front), composes the next window:
+//      W_0 is zeros and W_{k+1} = compose_window(F_k, W_k), one wave after another;
+//   c. with W_k known every relayed symbol settles (settle_symbol), all pieces side by side.
+// A symbol of a piece that did not decode may be anything: the window index is masked so that it
+// stays inside the window (that wave is reported as bad).
+SGC_HD uint16_t relay_symbol(uint16_t s, uint64_t piece_off, const uint16_t* wave_sym) {
+  if (s < 256) return s;
+  const int64_t g = (int64_t)piece_off - (int64_t)kWindow + (int64_t)((s - 256) & (kWindow - 1));
+  return g >= 0 ? wave_sym[g] : (uint16_t)(256 + (int64_t)kWindow + g);
+}
+SGC_HD uint8_t settle_symbol(uint16_t s, const uint8_t* window) {
+  return s < 256 ? (uint8_t)s : window[(s - 256) & (kWindow - 1)];
+}
+// F_k of a wave of n_text bytes: the caller put its last min(n_text, kWindow) relayed symbols at the
+// end of f[kWindow]; in front of them, when the wave is shorter than the window, the bytes in front
+// of the wave: f[j] names byte n_text + j of W_k.
+SGC_HD void wave_front(uint16_t* f, uint64_t n_text) {
+  for (uint64_t j = 0; j + n_text < kWindow; ++j) f[j] = (uint16_t)(256 + n_text + j);
+}
+SGC_HD void compose_window(const uint16_t* f, const uint8_t* w_in, uint8_t* w_out) {
+  for (uint32_t j = 0; j < kWindow; ++j) w_out[j] = settle_symbol(f[j], w_in);
+}
+
 }  // namespace inflate
 }  // namespace sgc
 

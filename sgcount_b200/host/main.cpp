@@ -384,6 +384,7 @@ struct SampleResult {
   uint64_t device_blocks = 0;
   uint64_t member_pieces = 0, member_chain = 0, member_absorbed = 0;  // gzip members in pieces on the device
   uint64_t gzip_members = 0;                                          // how many (not BGZF), as the device confirmed them
+  unsigned member_lanes = 0;                                          // streams that decoded them together
   std::string host_because;                 // why the device ingest was not used
 };
 
@@ -503,36 +504,49 @@ size_t gzip_members(const uint8_t* d, size_t n, size_t cap) {
 constexpr size_t kMinDeviceGzipBytes = 64ull << 20;
 constexpr size_t kHostCoresPerDevice = 3;
 
-// A gzip FASTQ that is not BGZF on one device: one member through sgc_fastq_stream_submit_member,
-// several (`several`) through sgc_fastq_stream_submit_gzip.
-bool count_member_on_device(const sgc_library* lib, uint32_t n_guides, const MappedFile& file, OffsetValue offset, uint32_t span_offset,
-                            uint32_t read_len, uint32_t span_start, uint32_t span_len, bool variable, bool recursion, int rc_mode,
-                            bool several, SampleResult& r, std::string& why_not) {
+// A gzip FASTQ that is not BGZF: one member through sgc_fastq_stream_submit_member, several (`several`)
+// through sgc_fastq_stream_submit_gzip, on the first device; or, with lanes > 1, the file through
+// sgc_fastq_stream_submit_gzip_split by `lanes` streams dealt over the sample's devices (lane d on
+// libs[d % libs.size()]), their counters summed with sgc_reduce_counts.
+bool count_member_on_device(const std::vector<const sgc_library*>& libs, size_t lanes, uint32_t n_guides, const MappedFile& file,
+                            OffsetValue offset, uint32_t span_offset, uint32_t read_len, uint32_t span_start, uint32_t span_len,
+                            bool variable, bool recursion, int rc_mode, bool several, SampleResult& r, std::string& why_not) {
   const auto t0 = std::chrono::steady_clock::now();
   struct Guard {
-    sgc_counter* c = nullptr;
-    sgc_fastq_stream* s = nullptr;
+    std::vector<sgc_counter*> c;
+    std::vector<sgc_fastq_stream*> s;
     ~Guard() {
-      sgc_fastq_stream_destroy(s);
-      sgc_counter_destroy(c);
+      for (auto* x : s) sgc_fastq_stream_destroy(x);
+      for (auto* x : c) sgc_counter_destroy(x);
     }
   } g;
-  check(sgc_counter_create(lib, offset.reverse, span_offset, recursion, rc_mode, nullptr, nullptr, &g.c));
-  check(sgc_fastq_stream_create(g.c, variable ? 0 : read_len, span_start, span_len, &g.s));
+  g.c.assign(lanes, nullptr);
+  g.s.assign(lanes, nullptr);
+  for (size_t d = 0; d < lanes; ++d) {
+    check(sgc_counter_create(libs[d % libs.size()], offset.reverse, span_offset, recursion, rc_mode, nullptr, nullptr, &g.c[d]));
+    check(sgc_fastq_stream_create(g.c[d], variable ? 0 : read_len, span_start, span_len, &g.s[d]));
+  }
   const auto t1 = std::chrono::steady_clock::now();
   uint64_t n_records = 0;
-  int rc = several ? sgc_fastq_stream_submit_gzip(g.s, file.data, file.size) : sgc_fastq_stream_submit_member(g.s, file.data, file.size);
+  int rc = lanes > 1 ? sgc_fastq_stream_submit_gzip_split(g.s.data(), (uint32_t)lanes, file.data, file.size)
+           : several ? sgc_fastq_stream_submit_gzip(g.s[0], file.data, file.size)
+                     : sgc_fastq_stream_submit_member(g.s[0], file.data, file.size);
   const auto t2 = std::chrono::steady_clock::now();
-  if (rc == SGC_OK) rc = sgc_fastq_stream_finish(g.s, &n_records);
+  for (size_t d = 0; d < lanes && rc == SGC_OK; ++d) {
+    uint64_t records = 0;
+    rc = sgc_fastq_stream_finish(g.s[d], &records);
+    n_records += records;
+  }
   if (rc == SGC_ERR_GZIP || rc == SGC_ERR_FASTQ_FORMAT) {
     why_not = sgc_last_error();
     return false;
   }
   if (rc != SGC_OK) fail("%s", sgc_last_error());
-  check(sgc_fastq_stream_member_stats(g.s, &r.member_pieces, &r.member_chain, &r.member_absorbed));
-  check(sgc_fastq_stream_gzip_members(g.s, &r.gzip_members));
+  check(sgc_fastq_stream_member_stats(g.s[0], &r.member_pieces, &r.member_chain, &r.member_absorbed));
+  check(sgc_fastq_stream_gzip_members(g.s[0], &r.gzip_members));
+  if (lanes > 1) check(sgc_reduce_counts(g.c.data(), (int)lanes, 0));
   r.counts.resize(n_guides);
-  check(sgc_counter_finish(g.c, r.counts.data(), &r.total, &r.matched));
+  check(sgc_counter_finish(g.c[0], r.counts.data(), &r.total, &r.matched));
   const auto t3 = std::chrono::steady_clock::now();
   auto seconds = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
     return std::chrono::duration<double>(b - a).count();
@@ -540,7 +554,8 @@ bool count_member_on_device(const sgc_library* lib, uint32_t n_guides, const Map
   r.span_reads = variable ? 0 : n_records;
   r.line_reads = variable ? n_records : 0;
   r.device_ingest = true;
-  r.shards = 1;
+  r.shards = (unsigned)std::min(lanes, libs.size());
+  r.member_lanes = (unsigned)lanes;
   r.submit_s = seconds(t0, t3);
   r.dev_create_s = seconds(t0, t1);
   r.dev_waves_s = seconds(t1, t2);
@@ -597,7 +612,11 @@ bool count_sample_on_device(const std::vector<const sgc_library*>& libs, uint32_
                 " gzip members: the host decodes them side by side";
       return false;
     }
-    return count_member_on_device(libs[0], n_guides, file, offset, span_offset, read_len, span_start, span_len, variable, recursion,
+    // SGC_MEMBER_LANES=n: n streams dealt over the sample's devices decode the file together (n on the
+    // one device when the sample has one).  Without it the file goes to the first device alone.
+    size_t lanes = 1;
+    if (const char* e = getenv("SGC_MEMBER_LANES"); e && atoi(e) > 0) lanes = (size_t)atoi(e);
+    return count_member_on_device(libs, lanes, n_guides, file, offset, span_offset, read_len, span_start, span_len, variable, recursion,
                                   rc_mode, members > 1, r, why_not);
   }
   const auto t_indexed = std::chrono::steady_clock::now();
@@ -1042,7 +1061,7 @@ int main(int argc, char** argv) {
       double wait_s = 0, copy_s = 0, submit_s = 0;
       unsigned max_shards = 1;
       unsigned long long span_reads = 0, device_blocks = 0, adopted = 0, reframed = 0, pieces = 0, chain = 0, absorbed = 0, members = 0;
-      unsigned device_samples = 0;
+      unsigned device_samples = 0, member_lanes = 0;
       std::string host_because;
       double dev_index_s = 0, dev_create_s = 0, dev_waves_s = 0, dev_finish_s = 0;
       for (const auto& r : results) {
@@ -1055,15 +1074,17 @@ int main(int argc, char** argv) {
         pieces += r.member_pieces, chain += r.member_chain, absorbed += r.member_absorbed, members += r.gzip_members;
         if (!r.device_ingest && host_because.empty()) host_because = r.host_because;
         max_shards = std::max(max_shards, r.shards);
+        member_lanes = std::max(member_lanes, r.member_lanes);
       }
       fprintf(stderr, "{\"count_s\": %.6f, \"reads\": %llu, \"samples\": %zu, \"sample_workers\": %u, "
               "\"ingest_threads\": %u, \"gpus\": %d, \"read_shards_per_sample\": %u, \"span_reads\": %llu, \"device_ingest_samples\": %u, "
               "\"device_blocks\": %llu, \"device_phases_s\": [%.4f, %.4f, %.4f, %.4f], \"host_ingest_because\": \"%s\", \"members_adopted\": %llu, \"members_reframed\": %llu, \"wait_inflate_s\": %.6f, "
               "\"copy_to_pinned_s\": %.6f, \"submit_sync_s\": %.6f, \"read_inputs_s\": %.3f, "
-              "\"device_tables_s\": %.3f, \"offsets_s\": %.3f, \"member_pieces\": %llu, \"member_chain\": %llu, \"member_absorbed\": %llu, \"gzip_members\": %llu}\n",
+              "\"device_tables_s\": %.3f, \"offsets_s\": %.3f, \"member_pieces\": %llu, \"member_chain\": %llu, \"member_absorbed\": %llu, \"gzip_members\": %llu, "
+              "\"member_lanes\": %u}\n",
               count_s, reads, n_samples, workers, ingest_threads, gpus, max_shards, span_reads, device_samples, device_blocks,
               dev_index_s, dev_create_s, dev_waves_s, dev_finish_s, host_because.c_str(), adopted, reframed, wait_s, copy_s, submit_s, t_inputs,
-              t_tables - t_inputs, t_offsets - t_tables, pieces, chain, absorbed, members);
+              t_tables - t_inputs, t_offsets - t_tables, pieces, chain, absorbed, members, member_lanes);
     }
 
     // write_results (results.rs:71-99).  Counts are keyed by alias (counter.rs:232-235):

@@ -1,7 +1,7 @@
 #!/bin/bash
 # usage: bash tools/sanitize_host.sh — the host-side test helpers (fastx_dump: host reader + whole-member
 # inflate; inflate_core_test: the device's gzip decoder compiled for the host; member_core_test: one member,
-# or with its fourth argument several, decoded in pieces as the device does it) rebuilt with
+# or with its fourth argument several, decoded in pieces as the device does it, with its fifth in waves) rebuilt with
 # -fsanitize=address,undefined, their test files run against them, the ordinary builds put back.
 # Needs a g++ that ships libasan (CXX_SAN, default /usr/bin/g++).
 set -e
@@ -16,4 +16,4 @@ trap 'cp /tmp/sgc_san/fastx_dump /tmp/sgc_san/inflate_core_test /tmp/sgc_san/mem
   $CXX_SAN $SAN -o ../lib/member_core_test member_core_test.cpp)
 ASAN_OPTIONS=detect_leaks=0 UBSAN_OPTIONS=print_stacktrace=1:halt_on_error=1 \
   python -m pytest tests/test_host_reader.py tests/test_host_inflate.py tests/test_device_inflate_core.py tests/test_member_inflate_core.py \
-  tests/test_multi_member_inflate_core.py -x -q
+  tests/test_multi_member_inflate_core.py tests/test_member_waves_core.py -x -q
