@@ -61,6 +61,8 @@ typedef struct sgc_counter sgc_counter;
 const char* sgc_last_error(void);
 int sgc_abi_version(void);
 int sgc_device_count(int* n);
+/* Free and total memory of a device (cudaMemGetInfo), in bytes. */
+int sgc_device_memory(int device, uint64_t* free_bytes, uint64_t* total_bytes);
 
 /* Pinned host memory for the caller's read batches (the ingest ring buffers). */
 int sgc_host_alloc(void** ptr, size_t bytes);
@@ -296,6 +298,18 @@ int sgc_fastq_stream_submit_gzip(sgc_fastq_stream*, const uint8_t* gz, uint64_t 
  * A file is declined as by sgc_fastq_stream_submit_gzip, and then every stream has failed.  One host
  * thread per stream, all joined before the call returns.  n_streams == 1 is sgc_fastq_stream_submit_gzip. */
 int sgc_fastq_stream_submit_gzip_split(sgc_fastq_stream* const* streams, uint32_t n_streams, const uint8_t* gz, uint64_t n_bytes);
+/* An upper bound of the device scratch ONE stream allocates (compressed bytes, 16-bit symbols, text,
+ * span or line-offset buffers, piece tables), so that a caller running several samples on a device at
+ * once can keep their sum within its memory.  bgzf != 0: sgc_fastq_stream_submit / _submit_range with
+ * waves of at most gz_bytes compressed and text_bytes inflated bytes.  bgzf == 0: a gzip file of gz_bytes
+ * through sgc_fastq_stream_submit_member, _submit_gzip or (per stream) _submit_gzip_split; text_bytes is
+ * its text when known, else 0 (then every byte is taken to inflate to the most DEFLATE allows, up to the
+ * wave limit).  It does not cover a single 32 KiB piece of input that inflates to more than a whole wave
+ * (4 GiB), which no FASTQ does.  read_len / span_len: as sgc_fastq_stream_create.  Streams on several
+ * threads: each stream is used by one thread at a time; distinct streams, on one device or several, may
+ * submit at the same time. */
+int sgc_fastq_stream_scratch_bound(int bgzf, uint64_t gz_bytes, uint64_t text_bytes, uint32_t read_len, uint32_t span_len,
+                                   uint64_t* bytes);
 /* Members decoded by sgc_fastq_stream_submit_gzip (1 after sgc_fastq_stream_submit_member, else 0). */
 int sgc_fastq_stream_gzip_members(const sgc_fastq_stream*, uint64_t* members);
 int sgc_fastq_stream_finish(sgc_fastq_stream*, uint64_t* n_records);

@@ -72,6 +72,7 @@ SIGNATURES = {
     "sgc_last_error": (C.c_char_p, []),
     "sgc_abi_version": (_int, []),
     "sgc_device_count": (_int, [C.POINTER(_int)]),
+    "sgc_device_memory": (_int, [_int, C.POINTER(_u64), C.POINTER(_u64)]),
     "sgc_host_alloc": (_int, [C.POINTER(_vp), C.c_size_t]),
     "sgc_host_free": (_int, [_vp]),
     "sgc_library_create": (_int, [_int, _vp, _u32, _u32, _int, C.POINTER(_vp)]),
@@ -101,6 +102,7 @@ SIGNATURES = {
     "sgc_fastq_stream_member_stats": (_int, [_vp, C.POINTER(_u64), C.POINTER(_u64), C.POINTER(_u64)]),
     "sgc_fastq_stream_submit_gzip": (_int, [_vp, _vp, _u64]),
     "sgc_fastq_stream_submit_gzip_split": (_int, [C.POINTER(_vp), _u32, _vp, _u64]),
+    "sgc_fastq_stream_scratch_bound": (_int, [_int, _u64, _u64, _u32, _u32, C.POINTER(_u64)]),
     "sgc_fastq_stream_gzip_members": (_int, [_vp, C.POINTER(_u64)]),
     "sgc_fastq_stream_finish": (_int, [_vp, C.POINTER(_u64)]),
     "sgc_counter_launch_info": (_int, [_vp, C.POINTER(LaunchInfo)]),

@@ -464,3 +464,19 @@ def submit_gzip_split(streams: Sequence[FastqStream], blob: np.ndarray) -> None:
     check(_cabi.load().sgc_fastq_stream_submit_gzip_split(arr, len(streams), blob.ctypes.data, len(blob)))
     for s in streams:
         s._counter._result = None
+
+
+def device_memory(device: int = 0):
+    """(free, total) bytes of a device's memory"""
+    free, total = C.c_uint64(), C.c_uint64()
+    check(_cabi.load().sgc_device_memory(int(device), C.byref(free), C.byref(total)))
+    return int(free.value), int(total.value)
+
+
+def fastq_stream_scratch_bound(bgzf: bool, gz_bytes: int, text_bytes: int, read_len: int, span_len: int) -> int:
+    """the most device scratch one FastqStream allocates (sgc_fastq_stream_scratch_bound): BGZF waves of at most
+    gz_bytes / text_bytes, or a gzip file of gz_bytes whose text is text_bytes (0: unknown)"""
+    out = C.c_uint64()
+    check(_cabi.load().sgc_fastq_stream_scratch_bound(1 if bgzf else 0, int(gz_bytes), int(text_bytes), int(read_len),
+                                                      int(span_len), C.byref(out)))
+    return int(out.value)

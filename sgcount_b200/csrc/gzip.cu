@@ -646,8 +646,8 @@ struct MemberParams {
   uint64_t piece, wave_text;
   bool skew;
 };
-MemberParams member_params(const sgc_fastq_stream* s) {
-  MemberParams p{32u << 10, s->read_len ? (4ull << 30) : (3ull << 30), false};
+MemberParams member_params(uint32_t read_len) {
+  MemberParams p{32u << 10, read_len ? (4ull << 30) : (3ull << 30), false};
   if (const char* e = getenv("SGC_MEMBER_PIECE"); e && atoll(e) >= 64) p.piece = (uint64_t)atoll(e);
   const char* skew_env = getenv("SGC_MEMBER_SKEW");
   p.skew = skew_env && atoi(skew_env) != 0;
@@ -847,7 +847,7 @@ int submit_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, bool
   DeviceGuard guard(s->device);
   size_t header = 0;
   if (inflate::gzip_header(gz, (size_t)n_bytes, &header) != inflate::kOk) return member_decline(s, "not a gzip member");
-  const MemberParams params = member_params(s);
+  const MemberParams params = member_params(s->read_len);
 
   // 1-2. candidate starts near every nominal boundary (and at every gzip header), the boundary pass
   std::vector<uint64_t> starts;
@@ -1105,7 +1105,7 @@ int submit_split(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* gz, ui
   size_t header = 0;
   if (inflate::gzip_header(gz, (size_t)n_bytes, &header) != inflate::kOk)
     return split_fail(ss, ns, member_decline(ss[0], "not a gzip member"));
-  const MemberParams params = member_params(ss[0]);
+  const MemberParams params = member_params(ss[0]->read_len);
 
   // 1-2. split by input range
   std::vector<uint64_t> starts;
@@ -1219,6 +1219,8 @@ int sgc_fastq_stream_create(sgc_counter* counter, uint32_t read_len, uint32_t sp
   st0.bad_block = 0xFFFFFFFFu;
   SGC_CUDA_TRY(cudaMemcpyAsync(s->d_state, &st0, sizeof st0, cudaMemcpyHostToDevice, s->stream));
   SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+  // (every create sets the same kInflateSmem, so streams created on several threads at once cannot
+  // lower the opt-in under each other's launches, as count.cu's ensure_smem_optin guards against)
   SGC_CUDA_TRY(cudaFuncSetAttribute(inflate_blocks_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kInflateSmem));
   SGC_CUDA_TRY(cudaFuncSetAttribute(member_find_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kInflateSmem));
   SGC_CUDA_TRY(cudaFuncSetAttribute(member_boundary_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kInflateSmem));
@@ -1311,6 +1313,40 @@ int sgc_fastq_stream_submit_gzip(sgc_fastq_stream* s, const uint8_t* gz, uint64_
 
 int sgc_fastq_stream_submit_gzip_split(sgc_fastq_stream* const* streams, uint32_t n_streams, const uint8_t* gz, uint64_t n_bytes) {
   return submit_split(streams, n_streams, gz, n_bytes);
+}
+
+// Every buffer a stream keeps is sized by `grow` (need + need / 4 when it grows), so none ever holds
+// more than 1.25 times the most the stream needed of it; the needs follow from the wave's text.
+int sgc_fastq_stream_scratch_bound(int bgzf, uint64_t gz_bytes, uint64_t text_bytes, uint32_t read_len, uint32_t span_len,
+                                   uint64_t* bytes) {
+  if (!bytes) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
+  if (read_len != 0 && (span_len == 0 || span_len > read_len)) return set_error(SGC_ERR_INVALID_ARG, "the span does not fit the read");
+  auto grown = [](uint64_t need) { return need + need / 4; };
+  const MemberParams p = member_params(read_len);
+  // the text of one wave: a member wave stops before it passes p.wave_text, and DEFLATE inflates no byte
+  // to more than 1032
+  const uint64_t text = bgzf ? text_bytes : std::min(text_bytes ? text_bytes : gz_bytes * 1032, p.wave_text);
+  const uint64_t region = kHeadroom + text;  // with the bytes carried in front of it
+  const uint64_t chunks = region / kChunk + 2;
+  uint64_t b = sizeof(StreamState) + kHeadroom;                             // d_state, d_tail
+  b += grown(region + 64);                                                  // d_text
+  b += 2 * grown((chunks + 1) * 4) + grown((chunks / 2048 + 2) * 4);        // d_counts, d_first, d_sums
+  const uint64_t records = region / ((uint64_t)read_len + 6) + 2;           // a record takes its read and 6 more bytes
+  b += read_len ? grown(records * ((span_len + 7u) & ~7u) + 256) : 2 * grown(records * 4);  // d_spans / d_seq_start, d_seq_end
+  if (bgzf) {
+    const uint64_t blocks = gz_bytes / 28 + 2;  // a BGZF block takes 28 bytes at least
+    b += grown(gz_bytes + 64) + 2 * grown(blocks * 8);  // d_gz, d_begin, d_outoff
+  } else {
+    const uint64_t heads = gz_bytes / 256 + 4096 + 1;
+    const uint64_t pieces = (gz_bytes + p.piece - 1) / p.piece + 1 + heads;  // candidates near the boundaries and behind headers
+    b += grown(gz_bytes + 64) + grown(pieces * 8) + grown(heads * 8);                      // d_gz, d_cand, d_heads
+    b += grown(pieces * sizeof(inflate::PieceMeta)) + grown(pieces);                       // d_meta, d_is_member
+    b += grown((text + 1) * 2) + grown((pieces + 1) * sizeof(WavePiece)) + grown(pieces * 4);  // d_sym, d_wave, d_crc
+    b += 2 * inflate::kWindow;                                                             // d_window
+  }
+  // the pool's rounding of some twenty buffers, and the counter's skew replicas (at most 64 MB)
+  *bytes = b + (128ull << 20);
+  return SGC_OK;
 }
 
 int sgc_fastq_stream_gzip_members(const sgc_fastq_stream* s, uint64_t* members) {

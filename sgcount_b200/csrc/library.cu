@@ -369,6 +369,17 @@ int sgc_device_count(int* n) {
   return SGC_OK;
 }
 
+int sgc_device_memory(int device, uint64_t* free_bytes, uint64_t* total_bytes) {
+  if (!free_bytes || !total_bytes) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
+  DeviceGuard guard(device);
+  if (!guard.ok()) return set_error(SGC_ERR_CUDA, "no such device");
+  size_t f = 0, t = 0;
+  SGC_CUDA_TRY(cudaMemGetInfo(&f, &t));
+  *free_bytes = f;
+  *total_bytes = t;
+  return SGC_OK;
+}
+
 int sgc_host_alloc(void** ptr, size_t bytes) {
   if (!ptr) return set_error(SGC_ERR_INVALID_ARG, "ptr is NULL");
   SGC_CUDA_TRY(cudaHostAlloc(ptr, bytes, cudaHostAllocPortable));

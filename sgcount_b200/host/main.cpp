@@ -17,13 +17,18 @@
 #include <unistd.h>
 #include <zlib.h>
 
+#include <algorithm>
 #include <atomic>
 #include <chrono>
+#include <condition_variable>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <exception>
 #include <fstream>
+#include <map>
+#include <memory>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -86,7 +91,7 @@ const char* kUsage =
     "  -r, --reverse                          Read Direction (reverse complement reads)\n"
     "  -x, --exact                            Disallow One Off Mismatch\n"
     "  -s, --subsample <SUBSAMPLE>            Number of Reads to Subsample in Determining Offset [default: 5000]\n"
-    "  -t, --threads <THREADS>                Number of Threads to Use for Parallel Jobs [default: 1]\n"
+    "  -t, --threads <THREADS>                Number of Threads to Use for Parallel Jobs [default: 1]; samples counted at once (at least one per device, and four per device when every input is inflated on the device, within each device's free memory)\n"
     "  -q, --quiet                            Does not show progress\n"
     "  -z, --include-zero                     Include zero count sgRNAs in output table\n"
     "      --gpus <N>                         Spread the samples (and, with fewer samples than devices, read shards of each sample) over N devices [default: 1]\n"
@@ -504,13 +509,82 @@ size_t gzip_members(const uint8_t* d, size_t n, size_t cap) {
 constexpr size_t kMinDeviceGzipBytes = 64ull << 20;
 constexpr size_t kHostCoresPerDevice = 3;
 
+// Does a gzip file that is not BGZF, of `members` members (counted up to kHostCoresPerDevice + 1), go to the
+// device?  `why_not`: the reason when it does not.
+bool gzip_file_to_device(size_t members, uint64_t bytes, unsigned ingest_threads, std::string& why_not) {
+  // (SGC_MULTI_MEMBER_DEVICE=1: every multi-member file to the device, for measurements of both paths)
+  const char* force_env = getenv("SGC_MULTI_MEMBER_DEVICE");
+  const bool force = force_env && atoi(force_env) != 0;
+  if (members > 1 && !force && bytes < kMinDeviceGzipBytes) {
+    why_not = "not BGZF, and several gzip members in a file under " + std::to_string(kMinDeviceGzipBytes >> 20) +
+              " MB: the host's cores decode them sooner";
+    return false;
+  }
+  if (members > 1 && !force && std::min<size_t>(members, ingest_threads) > kHostCoresPerDevice) {
+    why_not = "not BGZF, and " + std::string(members > kHostCoresPerDevice ? "more than " + std::to_string(kHostCoresPerDevice)
+                                                                            : std::to_string(members)) +
+              " gzip members: the host decodes them side by side";
+    return false;
+  }
+  return true;
+}
+
+// Device-memory admission of the device ingest.  Before a sample creates its streams on a device it
+// reserves the library's bound of their scratch (sgc_fastq_stream_scratch_bound) from the device's
+// budget, waiting while other samples hold too much of it, and gives it back once its streams are
+// destroyed.  A sample whose bound exceeds the whole budget runs alone on its device.
+struct DeviceBudget {
+  std::mutex mu;
+  std::condition_variable cv;
+  uint64_t budget = 0, used = 0;
+  unsigned running = 0, most = 0;  // samples holding a reservation now / at most
+  void acquire(uint64_t bytes) {
+    std::unique_lock<std::mutex> lk(mu);
+    cv.wait(lk, [&] { return running == 0 || used + bytes <= budget; });
+    used += bytes;
+    most = std::max(most, ++running);
+  }
+  void release(uint64_t bytes) {
+    {
+      std::lock_guard<std::mutex> lk(mu);
+      used -= bytes;
+      --running;
+    }
+    cv.notify_all();
+  }
+};
+// One sample's reservations, taken in device order (so that no two samples hold one device each and
+// wait for the other's) and released when the guard goes.
+struct Reservation {
+  std::map<DeviceBudget*, uint64_t> held;  // (the budgets are one array: pointer order is device order)
+  explicit Reservation(const std::map<DeviceBudget*, uint64_t>& want) {
+    for (const auto& [b, bytes] : want) {
+      b->acquire(bytes);
+      held.emplace(b, bytes);
+    }
+  }
+  ~Reservation() {
+    for (const auto& [b, bytes] : held) b->release(bytes);
+  }
+};
+// `lanes` streams of `bound` bytes each, stream d on the device of budgets[d % budgets.size()]
+std::map<DeviceBudget*, uint64_t> lane_bytes(const std::vector<DeviceBudget*>& budgets, size_t lanes, uint64_t bound) {
+  std::map<DeviceBudget*, uint64_t> want;
+  for (size_t d = 0; d < lanes; ++d) want[budgets[d % budgets.size()]] += bound;
+  return want;
+}
+
 // A gzip FASTQ that is not BGZF: one member through sgc_fastq_stream_submit_member, several (`several`)
 // through sgc_fastq_stream_submit_gzip, on the first device; or, with lanes > 1, the file through
 // sgc_fastq_stream_submit_gzip_split by `lanes` streams dealt over the sample's devices (lane d on
 // libs[d % libs.size()]), their counters summed with sgc_reduce_counts.
-bool count_member_on_device(const std::vector<const sgc_library*>& libs, size_t lanes, uint32_t n_guides, const MappedFile& file,
-                            OffsetValue offset, uint32_t span_offset, uint32_t read_len, uint32_t span_start, uint32_t span_len,
-                            bool variable, bool recursion, int rc_mode, bool several, SampleResult& r, std::string& why_not) {
+bool count_member_on_device(const std::vector<const sgc_library*>& libs, const std::vector<DeviceBudget*>& budgets, size_t lanes,
+                            uint32_t n_guides, const MappedFile& file, OffsetValue offset, uint32_t span_offset, uint32_t read_len,
+                            uint32_t span_start, uint32_t span_len, bool variable, bool recursion, int rc_mode, bool several,
+                            SampleResult& r, std::string& why_not) {
+  uint64_t bound = 0;
+  check(sgc_fastq_stream_scratch_bound(0, file.size, 0, variable ? 0 : read_len, span_len, &bound));
+  Reservation reserved(lane_bytes(budgets, lanes, bound));  // (declared before the streams: released after them)
   const auto t0 = std::chrono::steady_clock::now();
   struct Guard {
     std::vector<sgc_counter*> c;
@@ -572,9 +646,9 @@ bool count_member_on_device(const std::vector<const sgc_library*>& libs, size_t 
 // caller can try the other mode or the host path.
 // `variable`: reads of any length (the sequence lines are counted where they lie in the inflated
 // text); otherwise every read has read_len bytes and only its guide-window span is kept.
-bool count_sample_on_device(const std::vector<const sgc_library*>& libs, uint32_t n_guides, uint32_t k, const std::string& path,
-                            OffsetValue offset, uint32_t read_len, bool variable, bool recursion, int rc_mode, bool member_ok,
-                            unsigned ingest_threads, SampleResult& r, std::string& why_not) {
+bool count_sample_on_device(const std::vector<const sgc_library*>& libs, const std::vector<DeviceBudget*>& budgets, uint32_t n_guides,
+                            uint32_t k, const std::string& path, OffsetValue offset, uint32_t read_len, bool variable, bool recursion,
+                            int rc_mode, bool member_ok, size_t members, unsigned ingest_threads, SampleResult& r, std::string& why_not) {
   uint32_t span_start = 0, span_len = 0, span_offset = offset.index;
   if (!variable && sgc_span_geometry(k, read_len, offset.reverse, offset.index, recursion, &span_start, &span_len,
                                      &span_offset) != SGC_OK) {
@@ -597,26 +671,12 @@ bool count_sample_on_device(const std::vector<const sgc_library*>& libs, uint32_
       why_not = "not BGZF, and read shards asked for";
       return false;
     }
-    const size_t members = gzip_members(file.data, file.size, kHostCoresPerDevice + 1);
-    // (SGC_MULTI_MEMBER_DEVICE=1: every multi-member file to the device, for measurements of both paths)
-    const char* force_env = getenv("SGC_MULTI_MEMBER_DEVICE");
-    const bool force = force_env && atoi(force_env) != 0;
-    if (members > 1 && !force && file.size < kMinDeviceGzipBytes) {
-      why_not = "not BGZF, and several gzip members in a file under " + std::to_string(kMinDeviceGzipBytes >> 20) +
-                " MB: the host's cores decode them sooner";
-      return false;
-    }
-    if (members > 1 && !force && std::min<size_t>(members, ingest_threads) > kHostCoresPerDevice) {
-      why_not = "not BGZF, and " + std::string(members > kHostCoresPerDevice ? "more than " + std::to_string(kHostCoresPerDevice)
-                                                                              : std::to_string(members)) +
-                " gzip members: the host decodes them side by side";
-      return false;
-    }
+    if (!gzip_file_to_device(members, file.size, ingest_threads, why_not)) return false;
     // SGC_MEMBER_LANES=n: n streams dealt over the sample's devices decode the file together (n on the
     // one device when the sample has one).  Without it the file goes to the first device alone.
     size_t lanes = 1;
     if (const char* e = getenv("SGC_MEMBER_LANES"); e && atoi(e) > 0) lanes = (size_t)atoi(e);
-    return count_member_on_device(libs, lanes, n_guides, file, offset, span_offset, read_len, span_start, span_len, variable, recursion,
+    return count_member_on_device(libs, budgets, lanes, n_guides, file, offset, span_offset, read_len, span_start, span_len, variable, recursion,
                                   rc_mode, members > 1, r, why_not);
   }
   const auto t_indexed = std::chrono::steady_clock::now();
@@ -653,6 +713,15 @@ bool count_sample_on_device(const std::vector<const sgc_library*>& libs, uint32_
     }
   }
   const size_t n_lanes = independent ? std::min(lanes_wanted, waves.size()) : 1;
+  uint64_t wave_gz = 0, wave_text_most = 0, bound = 0;
+  for (const Wave& w : waves) {
+    uint64_t text = 0;
+    for (size_t b = w.first; b < w.first + w.n; ++b) text += isize[b];
+    wave_gz = std::max<uint64_t>(wave_gz, begin[w.first + w.n] - begin[w.first]);
+    wave_text_most = std::max(wave_text_most, text);
+  }
+  check(sgc_fastq_stream_scratch_bound(1, wave_gz, wave_text_most, variable ? 0 : read_len, span_len, &bound));
+  Reservation reserved(lane_bytes(budgets, n_lanes, bound));  // (declared before the streams: released after them)
   struct Lane {
     sgc_counter* c = nullptr;
     sgc_fastq_stream* stream = nullptr;
@@ -891,15 +960,44 @@ int main(int argc, char** argv) {
       for (const auto& alias : hlib.aliases)  // count.rs:90-95
         if (!genemap.count(alias)) fail("Missing sgRNA aliases in gene map: \"%s\"", alias.c_str());
     }
-    // validate_library_size (count.rs:62-71); the same records feed the offset detector below
+    // validate_library_size (count.rs:62-71); the same records feed the offset detector below.  The heads
+    // are read side by side, and so are the members of every gzip FASTQ the device ingest may take
+    // counted (once: count_sample_on_device is given the count).
     std::vector<SampleHead> heads(n_samples);
-    for (size_t i = 0; i < n_samples; ++i) {
-      heads[i] = read_head(args.input_paths[i], args.have_offset ? 0 : args.subsample);
-      if (!heads[i].any) fail("empty reader: %s", args.input_paths[i].c_str());
-      if (hlib.k > heads[i].first_len)
-        fail("Sequences in reference library are larger than the sequences in input.\n\nConsider reducing the length of "
-             "your reference sequences (i.e. extracting the variable region of the sgRNA or reducing the length of the "
-             "adapters.)");
+    std::vector<size_t> members(n_samples, 0);
+    auto device_candidate = [&](size_t i) {
+      const std::string& p = args.input_paths[i];
+      return !args.host_inflate && heads[i].fastq && p.size() > 3 && p.compare(p.size() - 3, 3, ".gz") == 0;
+    };
+    {
+      std::vector<std::exception_ptr> errors(n_samples);
+      std::atomic<size_t> next_head{0};
+      auto read_heads = [&] {
+        for (size_t i; (i = next_head.fetch_add(1)) < n_samples;) {
+          try {
+            heads[i] = read_head(args.input_paths[i], args.have_offset ? 0 : args.subsample);
+            if (device_candidate(i) && args.read_shards <= 1) {  // (with read shards only BGZF goes to the device)
+              MappedFile file(args.input_paths[i]);
+              if (file.data) members[i] = gzip_members(file.data, file.size, kHostCoresPerDevice + 1);
+            }
+          } catch (...) {
+            errors[i] = std::current_exception();
+          }
+        }
+      };
+      std::vector<std::thread> readers;
+      const size_t n_readers = std::min<size_t>(n_samples, std::max(1u, std::thread::hardware_concurrency()));
+      for (size_t t = 1; t < n_readers; ++t) readers.emplace_back(read_heads);
+      read_heads();
+      for (auto& t : readers) t.join();
+      for (size_t i = 0; i < n_samples; ++i) {
+        if (errors[i]) std::rethrow_exception(errors[i]);
+        if (!heads[i].any) fail("empty reader: %s", args.input_paths[i].c_str());
+        if (hlib.k > heads[i].first_len)
+          fail("Sequences in reference library are larger than the sequences in input.\n\nConsider reducing the length of "
+               "your reference sequences (i.e. extracting the variable region of the sgRNA or reducing the length of the "
+               "adapters.)");
+      }
     }
 
     t_inputs = seconds_since_start();
@@ -958,6 +1056,16 @@ int main(int argc, char** argv) {
         if (!e.empty()) fail("%s", e.c_str());
     }
 
+    // the budget of the device ingest on every device: its free memory now, less an eighth for the
+    // counters' own buffers (SGC_DEVICE_BUDGET=bytes sets it, for tests of the admission)
+    std::unique_ptr<DeviceBudget[]> budgets(new DeviceBudget[gpus]);
+    for (int d = 0; d < gpus; ++d) {
+      uint64_t free_bytes = 0, total_bytes = 0;
+      check(sgc_device_memory(args.device + d, &free_bytes, &total_bytes));
+      budgets[d].budget = free_bytes - free_bytes / 8;
+      if (const char* e = getenv("SGC_DEVICE_BUDGET"); e && *e) budgets[d].budget = strtoull(e, nullptr, 10);
+    }
+
     t_tables = seconds_since_start();
     std::vector<OffsetValue> offsets(n_samples);
     if (args.have_offset) {
@@ -981,47 +1089,70 @@ int main(int argc, char** argv) {
     size_t next_to_print = 0;
     std::vector<uint32_t> first_len(n_samples);
     std::vector<char> head_uniform(n_samples, 0), head_fastq(n_samples, 0);  // 4-line FASTQ? head reads of one length?
-    bool all_for_the_device = !args.host_inflate;
     const bool member_ok = args.read_shards <= 1;  // (read shards asked for: gzip that is not BGZF keeps the host path)
+    std::vector<char> candidate(n_samples, 0);
+    std::vector<uint64_t> input_bytes(n_samples, 0);
     for (size_t i = 0; i < n_samples; ++i) {
       first_len[i] = (uint32_t)heads[i].first_len;
       head_fastq[i] = heads[i].fastq;
       head_uniform[i] = heads[i].fastq && heads[i].uniform;
-      all_for_the_device &= heads[i].fastq && heads[i].bgzf;
+      candidate[i] = device_candidate(i);
+      struct stat st;
+      if (stat(args.input_paths[i].c_str(), &st) == 0) input_bytes[i] = (uint64_t)st.st_size;
+    }
+    // Samples in flight: the reference's -t (count.rs:117-136), at least one per device — and, when
+    // every sample is inflated, framed and counted on its device (BGZF, and gzip files that
+    // count_sample_on_device takes), four per device whatever -t says.  A sample's host thread only
+    // hands work over, and the device's inflate of one sample is bound by latency, not by throughput:
+    // of its longest BGZF block, or of the serial passes over a plain gzip file's pieces, whose decodes
+    // fill a fraction of the SMs (profiles/r7_member_samples_time.txt).  Samples side by side fill the
+    // rest; the device budgets above keep their scratch within the devices' memory.
+    // (SGC_DEVICE_SAMPLES_IN_FLIGHT=n replaces the four, for measurements)
+    constexpr unsigned kDeviceSamplesInFlight = 4;
+    unsigned device_in_flight = kDeviceSamplesInFlight;
+    if (const char* e = getenv("SGC_DEVICE_SAMPLES_IN_FLIGHT"); e && atoi(e) > 0) device_in_flight = (unsigned)atoi(e);
+    auto ingest_for = [&](unsigned workers) {
+      return args.ingest_threads ? args.ingest_threads : std::max(1u, std::thread::hardware_concurrency() / workers);
+    };
+    const unsigned device_workers =
+        (unsigned)std::min<size_t>(std::max(args.threads, (unsigned)gpus * device_in_flight), n_samples);
+    bool all_for_the_device = per_sample == 1;
+    for (size_t i = 0; i < n_samples && all_for_the_device; ++i) {
+      std::string why_not;
+      all_for_the_device = (!args.host_inflate && heads[i].fastq && heads[i].bgzf) ||
+                           (candidate[i] && member_ok && gzip_file_to_device(members[i], input_bytes[i], ingest_for(device_workers), why_not));
     }
     heads.clear();
-    // Samples in flight: the reference's -t (count.rs:117-136), at least one per device — and, when
-    // every sample is BGZF and so inflated, framed and counted on its device, four per device
-    // whatever -t says: a sample's host thread only hands blocks over, and the device's inflate of
-    // one sample is bound by the latency of its longest block, not by throughput (a wave takes about
-    // as long with 10 000 blocks as with 60 000), so samples side by side cost next to nothing.
-    constexpr unsigned kDeviceSamplesInFlight = 4;
-    const unsigned wanted = std::max(args.threads, (unsigned)gpus * (all_for_the_device && per_sample == 1 ? kDeviceSamplesInFlight : 1u));
-    const unsigned workers = (unsigned)std::min<size_t>(wanted, n_samples);
-    const unsigned ingest_threads =
-        args.ingest_threads ? args.ingest_threads : std::max(1u, std::thread::hardware_concurrency() / workers);
+    const unsigned workers =
+        all_for_the_device ? device_workers : (unsigned)std::min<size_t>(std::max(args.threads, (unsigned)gpus), n_samples);
+    const unsigned ingest_threads = ingest_for(workers);
     auto work = [&]() {
       for (;;) {
         const size_t s = next.fetch_add(1);
         if (s >= n_samples) return;
         try {
           std::vector<const sgc_library*> sample_libs;
-          for (size_t j = 0; j < per_sample; ++j) sample_libs.push_back(libs[(s * per_sample + j) % gpus]);
+          std::vector<DeviceBudget*> sample_budgets;
+          for (size_t j = 0; j < per_sample; ++j) {
+            sample_libs.push_back(libs[(s * per_sample + j) % gpus]);
+            sample_budgets.push_back(&budgets[(s * per_sample + j) % gpus]);
+          }
           // BGZF input of fixed-length FASTQ: the whole ingest on the device (one device per sample);
           // anything else, or anything the device declines, through the host's inflate threads
           bool on_device = false;
           std::string why_not = "switched off";
-          if (!args.host_inflate && head_fastq[s] && args.input_paths[s].size() > 3 &&
-              args.input_paths[s].compare(args.input_paths[s].size() - 3, 3, ".gz") == 0) {
+          if (candidate[s]) {
             // fixed-length reads as span records; reads of several lengths (seen in the head, or
             // reported by the device deeper in the file) with their sequence lines in place
             bool variable = !head_uniform[s] || args.whole_lines;
-            on_device = count_sample_on_device(sample_libs, hlib.n, hlib.k, args.input_paths[s], offsets[s], first_len[s],
-                                               variable, !args.no_position_recursion, args.rc_mode, member_ok, ingest_threads, results[s], why_not);
+            on_device = count_sample_on_device(sample_libs, sample_budgets, hlib.n, hlib.k, args.input_paths[s], offsets[s], first_len[s],
+                                               variable, !args.no_position_recursion, args.rc_mode, member_ok, members[s], ingest_threads,
+                                               results[s], why_not);
             if (!on_device && !variable && why_not.find("FASTQ") != std::string::npos) {
               results[s] = SampleResult();
-              on_device = count_sample_on_device(sample_libs, hlib.n, hlib.k, args.input_paths[s], offsets[s], first_len[s],
-                                                 true, !args.no_position_recursion, args.rc_mode, member_ok, ingest_threads, results[s], why_not);
+              on_device = count_sample_on_device(sample_libs, sample_budgets, hlib.n, hlib.k, args.input_paths[s], offsets[s],
+                                                 first_len[s], true, !args.no_position_recursion, args.rc_mode, member_ok, members[s],
+                                                 ingest_threads, results[s], why_not);
             }
           } else if (!head_fastq[s]) {
             why_not = "not FASTQ";
@@ -1060,8 +1191,9 @@ int main(int argc, char** argv) {
       unsigned long long reads = 0;
       double wait_s = 0, copy_s = 0, submit_s = 0;
       unsigned max_shards = 1;
-      unsigned long long span_reads = 0, device_blocks = 0, adopted = 0, reframed = 0, pieces = 0, chain = 0, absorbed = 0, members = 0;
-      unsigned device_samples = 0, member_lanes = 0;
+      unsigned long long span_reads = 0, device_blocks = 0, adopted = 0, reframed = 0, pieces = 0, chain = 0, absorbed = 0, gzip_member_count = 0;
+      unsigned device_samples = 0, member_lanes = 0, in_flight = 0;
+      for (int d = 0; d < gpus; ++d) in_flight = std::max(in_flight, budgets[d].most);
       std::string host_because;
       double dev_index_s = 0, dev_create_s = 0, dev_waves_s = 0, dev_finish_s = 0;
       for (const auto& r : results) {
@@ -1071,7 +1203,7 @@ int main(int argc, char** argv) {
         adopted += r.members_adopted, reframed += r.members_reframed;
         device_samples += r.device_ingest;
         device_blocks += r.device_blocks;
-        pieces += r.member_pieces, chain += r.member_chain, absorbed += r.member_absorbed, members += r.gzip_members;
+        pieces += r.member_pieces, chain += r.member_chain, absorbed += r.member_absorbed, gzip_member_count += r.gzip_members;
         if (!r.device_ingest && host_because.empty()) host_because = r.host_because;
         max_shards = std::max(max_shards, r.shards);
         member_lanes = std::max(member_lanes, r.member_lanes);
@@ -1081,10 +1213,10 @@ int main(int argc, char** argv) {
               "\"device_blocks\": %llu, \"device_phases_s\": [%.4f, %.4f, %.4f, %.4f], \"host_ingest_because\": \"%s\", \"members_adopted\": %llu, \"members_reframed\": %llu, \"wait_inflate_s\": %.6f, "
               "\"copy_to_pinned_s\": %.6f, \"submit_sync_s\": %.6f, \"read_inputs_s\": %.3f, "
               "\"device_tables_s\": %.3f, \"offsets_s\": %.3f, \"member_pieces\": %llu, \"member_chain\": %llu, \"member_absorbed\": %llu, \"gzip_members\": %llu, "
-              "\"member_lanes\": %u}\n",
+              "\"member_lanes\": %u, \"device_samples_in_flight\": %u}\n",
               count_s, reads, n_samples, workers, ingest_threads, gpus, max_shards, span_reads, device_samples, device_blocks,
               dev_index_s, dev_create_s, dev_waves_s, dev_finish_s, host_because.c_str(), adopted, reframed, wait_s, copy_s, submit_s, t_inputs,
-              t_tables - t_inputs, t_offsets - t_tables, pieces, chain, absorbed, members, member_lanes);
+              t_tables - t_inputs, t_offsets - t_tables, pieces, chain, absorbed, gzip_member_count, member_lanes, in_flight);
     }
 
     // write_results (results.rs:71-99).  Counts are keyed by alias (counter.rs:232-235):
