@@ -385,29 +385,6 @@ __device__ __forceinline__ uint8_t member_resolve(uint16_t s, uint64_t piece_off
   return g >= 0 ? text[g] : window[inflate::kWindow + g];
 }
 
-// The last 32 KiB (or all) of every piece, piece after piece: each depends on the 32 KiB in front of
-// its piece, which the pieces before resolved.  The only sequential step: one block, 32 bytes a thread.
-constexpr int kWindowThreads = 1024;
-__global__ void __launch_bounds__(kWindowThreads) member_window_kernel(const uint16_t* __restrict__ sym,
-                                                                      const WavePiece* __restrict__ wp, uint32_t n,
-                                                                      uint8_t* text, const uint8_t* __restrict__ window) {
-  for (uint32_t i = 0; i < n; ++i) {
-    const uint64_t a = wp[i].off, b = wp[i + 1].off;
-    const uint64_t lo = b - a > inflate::kWindow ? b - inflate::kWindow : a;
-    const uint64_t x0 = lo + (uint64_t)threadIdx.x * 32;
-    uint16_t s[32];
-#pragma unroll
-    for (int k = 0; k < 32; ++k) s[k] = x0 + k < b ? sym[x0 + k] : 0;
-    uint8_t v[32];
-#pragma unroll
-    for (int k = 0; k < 32; ++k) v[k] = x0 + k < b ? member_resolve(s[k], a, text, window) : 0;
-#pragma unroll
-    for (int k = 0; k < 32; ++k)
-      if (x0 + k < b) text[x0 + k] = v[k];
-    __syncthreads();  // (the next piece reads these bytes)
-  }
-}
-
 // everything else, every piece side by side (its window is resolved)
 __global__ void __launch_bounds__(256) member_resolve_kernel(const uint16_t* __restrict__ sym, const WavePiece* __restrict__ wp,
                                                             uint8_t* text, const uint8_t* __restrict__ window) {
@@ -429,20 +406,12 @@ __global__ void __launch_bounds__(kCrcWarps * 32) member_crc_kernel(const WavePi
   if (lane == 0) crc_out[i] = crc;
 }
 
-// the 32 KiB in front of the next wave: the end of this wave's text, preceded by the old window
-__global__ void member_window_save_kernel(const uint8_t* __restrict__ text, uint64_t n_text, const uint8_t* __restrict__ old_window,
-                                          uint8_t* __restrict__ new_window) {
-  for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < inflate::kWindow; k += gridDim.x * blockDim.x) {
-    const int64_t p = (int64_t)n_text - (int64_t)inflate::kWindow + k;
-    new_window[k] = p >= 0 ? text[p] : old_window[inflate::kWindow + p];
-  }
-}
-
-// ---- one file over several streams (sgc_fastq_stream_submit_gzip_split): inflate_core.h "waves on
-// several streams".  The walk of member_window_kernel, in place on the symbols of the last 32 KiB (or
-// all) of every piece: a marker that names a byte of this wave takes the symbol relayed there, one that
-// names a byte in front of the wave becomes a marker of the wave's entering window.  It needs nothing
-// from another wave.
+// Step 5 of inflate_core.h, the window relay ("waves: the window relay"), in place on the symbols of the
+// last 32 KiB (or all) of every piece, piece after piece: a marker that names a byte of this wave takes
+// the symbol relayed there, one that names a byte in front of the wave becomes a marker of the wave's
+// entering window.  It needs nothing from another wave.  The only sequential step: one block, 32
+// symbols a thread.
+constexpr int kWindowThreads = 1024;
 __global__ void __launch_bounds__(kWindowThreads) member_window_sym_kernel(uint16_t* sym, const WavePiece* __restrict__ wp,
                                                                           uint32_t n) {
   for (uint32_t i = 0; i < n; ++i) {
@@ -549,9 +518,9 @@ struct sgc_fastq_stream {
   std::vector<uint64_t> h_begin, h_outoff;
   uint64_t blocks_total = 0, records_total = 0;
   bool failed = false;
-  // one member in pieces (sgc_fastq_stream_submit_member)
+  // plain gzip in pieces (sgc_fastq_stream_submit_member, _submit_gzip, _submit_gzip_split)
   uint16_t* d_sym = nullptr;
-  uint8_t* d_window[2] = {nullptr, nullptr};
+  uint8_t* d_window = nullptr;  // W_k, the 32 KiB in front of the current wave
   uint64_t* d_cand = nullptr;
   inflate::PieceMeta* d_meta = nullptr;
   WavePiece* d_wave = nullptr;
@@ -559,7 +528,7 @@ struct sgc_fastq_stream {
   size_t sym_cap = 0, cand_cap = 0, meta_cap = 0, wave_cap = 0, crc_cap = 0;
   uint64_t member_pieces = 0, member_chain = 0, member_absorbed = 0;
   bool member_submitted = false;
-  // several members (sgc_fastq_stream_submit_gzip)
+  // gzip headers inside the file as member starts (all but sgc_fastq_stream_submit_member)
   uint64_t* d_heads = nullptr;  // member-start candidates, then their count
   uint8_t* d_is_member = nullptr;
   size_t heads_cap = 0, is_member_cap = 0;
@@ -637,7 +606,7 @@ int frame_and_count(sgc_fastq_stream* s, uint64_t n_text, uint64_t first_block) 
   return SGC_OK;
 }
 
-// ---- gzip members in pieces: the host side of sgc_fastq_stream_submit_member / _submit_gzip ----
+// ---- gzip members in pieces: the host side of sgc_fastq_stream_submit_member / _submit_gzip / _submit_gzip_split ----
 // Nominal piece size: 32 KiB of compressed input (more pieces than larger ones would give keep more
 // threads busy; each piece is a serial decode).  SGC_MEMBER_PIECE overrides it and SGC_MEMBER_SKEW=1
 // moves every other candidate start one bit on (tests: many pieces on small files, absorbed pieces);
@@ -684,123 +653,6 @@ void merge_candidates(const MemberParams& p, size_t header, const std::vector<ui
   is_member[0] = 1;  // (the first member's start, found by both scans)
 }
 
-// 1-2. the compressed bytes to the device; candidate piece starts near every nominal boundary (the first
-// member's first block is piece 0) and, with `find_headers`, at every gzip header; every piece to its
-// first block end at or beyond the next candidate.
-int member_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, size_t header, const MemberParams& p, bool find_headers,
-                  std::vector<uint64_t>& starts, std::vector<uint8_t>& is_member, std::vector<inflate::PieceMeta>& meta) {
-  const uint32_t n_bounds = (uint32_t)((n_bytes + p.piece - 1) / p.piece);
-  // member-start candidates: up to one per 256 bytes of input (fewer, larger members go to the host)
-  const uint64_t heads_cap = find_headers ? n_bytes / 256 + 4096 : 0;
-  int rc = grow(&s->d_gz, &s->gz_cap, (size_t)n_bytes + 64, s->pool, s->stream);  // (the reader's slack)
-  if (rc == SGC_OK) rc = grow(&s->d_cand, &s->cand_cap, (size_t)n_bounds + 1, s->pool, s->stream);
-  if (rc == SGC_OK && find_headers) rc = grow(&s->d_heads, &s->heads_cap, (size_t)heads_cap + 1, s->pool, s->stream);
-  if (rc) return rc;
-  SGC_CUDA_TRY(cudaMemcpyAsync(s->d_gz, gz, n_bytes, cudaMemcpyHostToDevice, s->stream));
-  constexpr uint32_t kWarps = kInflateThreads / 32;
-  if (n_bounds > 1)
-    member_find_kernel<<<(n_bounds - 1 + kWarps - 1) / kWarps, kInflateThreads, kInflateSmem, s->stream>>>(s->d_gz, n_bytes, p.piece,
-                                                                                                          n_bounds, s->d_cand);
-  uint64_t n_heads = 0;
-  if (find_headers) {
-    SGC_CUDA_TRY(cudaMemsetAsync(s->d_heads + heads_cap, 0, sizeof(uint64_t), s->stream));
-    const uint64_t threads = (n_bytes + kSignatureBytes - 1) / kSignatureBytes;
-    member_signature_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, s->stream>>>(s->d_gz, n_bytes, s->d_heads, heads_cap);
-    SGC_CUDA_TRY(cudaMemcpyAsync(&n_heads, s->d_heads + heads_cap, sizeof n_heads, cudaMemcpyDeviceToHost, s->stream));
-  }
-  SGC_CUDA_TRY(cudaGetLastError());
-  std::vector<uint64_t> cand((size_t)n_bounds + 1, ~0ull);
-  if (n_bounds > 1) SGC_CUDA_TRY(cudaMemcpyAsync(cand.data() + 1, s->d_cand + 1, (n_bounds - 1) * 8ull, cudaMemcpyDeviceToHost, s->stream));
-  SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
-  if (n_heads > heads_cap) return member_decline(s, kTooManyHeaders);
-  std::vector<uint64_t> heads(n_heads);
-  if (n_heads) {
-    SGC_CUDA_TRY(cudaMemcpyAsync(heads.data(), s->d_heads, n_heads * 8, cudaMemcpyDeviceToHost, s->stream));
-    SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
-  }
-  merge_candidates(p, header, cand, n_bounds, heads, starts, is_member);
-  const uint32_t n = (uint32_t)starts.size();
-
-  rc = grow(&s->d_meta, &s->meta_cap, (size_t)n, s->pool, s->stream);
-  if (rc == SGC_OK) rc = grow(&s->d_cand, &s->cand_cap, (size_t)n, s->pool, s->stream);
-  if (rc == SGC_OK) rc = grow(&s->d_is_member, &s->is_member_cap, (size_t)n, s->pool, s->stream);
-  if (rc) return rc;
-  SGC_CUDA_TRY(cudaMemcpyAsync(s->d_cand, starts.data(), n * 8ull, cudaMemcpyHostToDevice, s->stream));
-  SGC_CUDA_TRY(cudaMemcpyAsync(s->d_is_member, is_member.data(), n, cudaMemcpyHostToDevice, s->stream));
-  member_boundary_kernel<<<(n + kInflateThreads - 1) / kInflateThreads, kInflateThreads, kInflateSmem, s->stream>>>(
-      s->d_gz, n_bytes, s->d_cand, s->d_is_member, n, s->d_meta);
-  SGC_CUDA_TRY(cudaGetLastError());
-  meta.resize(n);
-  SGC_CUDA_TRY(cudaMemcpyAsync(meta.data(), s->d_meta, n * sizeof(inflate::PieceMeta), cudaMemcpyDeviceToHost, s->stream));
-  SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
-  return SGC_OK;
-}
-
-// 4-7. waves of chain pieces: symbols, windows, text, CRC-32, framing and counting.  member_of[i] is the
-// member of chain piece i: a piece may copy from its member's text only (from none of it when it starts
-// the member).  crc[m] (zero on entry) becomes the CRC-32 of member m's text.
-int member_waves(sgc_fastq_stream* s, uint64_t n_bytes, const MemberParams& p, const std::vector<uint64_t>& starts,
-                 const std::vector<inflate::PieceMeta>& meta, const uint32_t* chain, const uint32_t* member_of, uint32_t n_chain,
-                 std::vector<uint32_t>& crc) {
-  int rc = SGC_OK;
-  for (int w = 0; w < 2; ++w)
-    if (!s->d_window[w]) {
-      if ((rc = scratch_alloc(reinterpret_cast<void**>(&s->d_window[w]), inflate::kWindow, s->pool, s->stream))) return rc;
-    }
-  SGC_CUDA_TRY(cudaMemsetAsync(s->d_window[0], 0, inflate::kWindow, s->stream));
-  int cur = 0;
-  uint64_t done = 0;          // text of the waves before
-  uint64_t member_begin = 0;  // where the current member's text starts
-  std::vector<WavePiece> h_wave;
-  std::vector<uint32_t> h_crc;
-  for (uint32_t a = 0; a < n_chain;) {
-    uint32_t b = a;
-    uint64_t text = 0;
-    while (b < n_chain && (b == a || text + meta[chain[b]].out_len <= p.wave_text)) text += meta[chain[b++]].out_len;
-    const uint32_t nw = b - a;
-    if (s->read_len == 0 && text >= (1ull << 32) - 2 * kHeadroom) return member_decline(s, "a piece inflates to 4 GiB or more");
-    h_wave.resize((size_t)nw + 1);
-    uint64_t off = 0;
-    for (uint32_t i = 0; i < nw; ++i) {
-      const inflate::PieceMeta& m = meta[chain[a + i]];
-      const uint64_t global = done + off;
-      if (a + i > 0 && member_of[a + i] != member_of[a + i - 1]) member_begin = global;
-      const uint64_t reach = global - member_begin;
-      h_wave[i] = WavePiece{starts[chain[a + i]], m.end_bit, off, reach < inflate::kWindow ? reach : inflate::kWindow};
-      off += m.out_len;
-    }
-    h_wave[nw] = WavePiece{0, 0, text, 0};
-    rc = grow(&s->d_wave, &s->wave_cap, (size_t)nw + 1, s->pool, s->stream);
-    if (rc == SGC_OK) rc = grow(&s->d_sym, &s->sym_cap, (size_t)text + 1, s->pool, s->stream);
-    if (rc == SGC_OK) rc = grow(&s->d_text, &s->text_cap, (size_t)kHeadroom + text + 64, s->pool, s->stream);
-    if (rc == SGC_OK) rc = grow(&s->d_crc, &s->crc_cap, (size_t)nw, s->pool, s->stream);
-    if (rc) return rc;
-    SGC_CUDA_TRY(cudaMemcpyAsync(s->d_wave, h_wave.data(), h_wave.size() * sizeof(WavePiece), cudaMemcpyHostToDevice, s->stream));
-    uint8_t* wave_text_ptr = s->d_text + kHeadroom;
-    member_decode_kernel<<<(nw + kInflateThreads - 1) / kInflateThreads, kInflateThreads, kInflateSmem, s->stream>>>(
-        s->d_gz, n_bytes, s->d_wave, nw, s->d_sym, s->d_state);
-    member_window_kernel<<<1, kWindowThreads, 0, s->stream>>>(s->d_sym, s->d_wave, nw, wave_text_ptr, s->d_window[cur]);
-    member_resolve_kernel<<<nw, 256, 0, s->stream>>>(s->d_sym, s->d_wave, wave_text_ptr, s->d_window[cur]);
-    member_crc_kernel<<<(nw + kCrcWarps - 1) / kCrcWarps, kCrcWarps * 32, 0, s->stream>>>(s->d_wave, nw, wave_text_ptr, s->d_crc);
-    member_window_save_kernel<<<32, 256, 0, s->stream>>>(wave_text_ptr, text, s->d_window[cur], s->d_window[cur ^ 1]);
-    cur ^= 1;
-    SGC_CUDA_TRY(cudaGetLastError());
-    wave_begin_kernel<<<1, 1, 0, s->stream>>>(s->d_state, 0, 0);
-    rc = frame_and_count(s, text, a);  // (synchronises: a piece that did not decode is reported there)
-    if (rc) return rc;
-    h_crc.resize(nw);
-    SGC_CUDA_TRY(cudaMemcpyAsync(h_crc.data(), s->d_crc, nw * 4ull, cudaMemcpyDeviceToHost, s->stream));
-    SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
-    for (uint32_t i = 0; i < nw; ++i) {
-      uint32_t& c = crc[member_of[a + i]];
-      c = inflate::crc_combine(c, h_crc[i], h_wave[i + 1].off - h_wave[i].off);
-    }
-    done += text;
-    a = b;
-  }
-  return SGC_OK;
-}
-
 // step 3: the chain of pieces, the member of each, the trailers
 struct MemberChain {
   std::vector<uint32_t> chain, member_of;
@@ -824,59 +676,7 @@ const char* follow_chain(const uint8_t* gz, uint64_t n_bytes, const std::vector<
     if (c.trailers[m].isize != (uint32_t)text[m]) return "ISIZE of a member differs from the length of its text";
   return nullptr;
 }
-// the first member whose CRC-32 differs from its trailer's, or n_members
-uint32_t crc_mismatch(const MemberChain& c, const std::vector<uint32_t>& crc) {
-  for (uint32_t m = 0; m < c.n_members; ++m)
-    if (crc[m] != c.trailers[m].crc) return m;
-  return c.n_members;
-}
-int crc_error(uint32_t m) {
-  char buf[160];
-  snprintf(buf, sizeof buf, "gzip member %u: CRC-32 of the inflated bytes differs from the member's trailer", m);
-  return set_error(SGC_ERR_GZIP, buf);
-}
 
-// sgc_fastq_stream_submit_member (`find_headers` false: no gzip header inside the file is a candidate, so
-// the chain must end at the first trailer) and sgc_fastq_stream_submit_gzip.
-int submit_pieces(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes, bool find_headers) {
-  if (!s || !gz) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
-  if (s->failed || !s->counter) return set_error(SGC_ERR_INVALID_ARG, "the stream has failed or its counter is gone");
-  if (s->member_submitted || s->blocks_total)
-    return set_error(SGC_ERR_INVALID_ARG, "a gzip file goes to a fresh stream, once");
-  s->member_submitted = true;
-  DeviceGuard guard(s->device);
-  size_t header = 0;
-  if (inflate::gzip_header(gz, (size_t)n_bytes, &header) != inflate::kOk) return member_decline(s, "not a gzip member");
-  const MemberParams params = member_params(s->read_len);
-
-  // 1-2. candidate starts near every nominal boundary (and at every gzip header), the boundary pass
-  std::vector<uint64_t> starts;
-  std::vector<uint8_t> is_member;
-  std::vector<inflate::PieceMeta> meta;
-  int rc = member_pieces(s, gz, n_bytes, header, params, find_headers, starts, is_member, meta);
-  if (rc) return rc;
-  const uint32_t n = (uint32_t)starts.size();
-
-  // 3. the chain from the first block, over every trailer and header to the last trailer, which must end the file
-  MemberChain c;
-  if (const char* why = follow_chain(gz, n_bytes, starts, is_member, meta, c)) return member_decline(s, why);
-  s->member_pieces = n;
-  s->member_chain = c.n_chain;
-  s->member_absorbed = c.absorbed;
-
-  // 4-7. waves of chain pieces; CRC-32 member by member
-  std::vector<uint32_t> crc(c.n_members, 0);
-  rc = member_waves(s, n_bytes, params, starts, meta, c.chain.data(), c.member_of.data(), c.n_chain, crc);
-  if (rc) return rc;
-  if (const uint32_t m = crc_mismatch(c, crc); m < c.n_members) {
-    s->failed = true;
-    return crc_error(m);
-  }
-  s->gzip_members = c.n_members;
-  return SGC_OK;
-}
-
-// ---- one gzip file over several streams: the host side of sgc_fastq_stream_submit_gzip_split ----
 // Runs fn(i) for every stream i on a thread of its own, with the stream's device current, and joins
 // them all.  Returns the first failure by stream index, its message set on the calling thread.
 template <typename Fn>
@@ -903,19 +703,23 @@ uint64_t part_begin(uint64_t n_items, uint32_t parts, uint32_t i, uint64_t grain
   return std::min(n_items, (per + grain - 1) / grain * grain * i);
 }
 
-int split_fail(sgc_fastq_stream* const* ss, uint32_t n, int rc) {
+int fail_all(sgc_fastq_stream* const* ss, uint32_t n, int rc) {
   for (uint32_t i = 0; i < n; ++i) ss[i]->failed = true;
   return rc;
 }
 
-// 1-2 of member_pieces with find_headers, each kernel over one contiguous part per stream.  The kernels
-// are those of one stream, given shifted pointers: member_find_kernel's boundary 1 is boundary j0, its
-// bits count from byte (j0 - 1) * piece; member_signature_kernel starts at byte b0 (whole blocks of it
-// per part); member_boundary_kernel's piece 0 is piece c0 (so `next` counts from c0).
-int split_pieces(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* gz, uint64_t n_bytes, size_t header, const MemberParams& p,
-                 std::vector<uint64_t>& starts, std::vector<uint8_t>& is_member, std::vector<inflate::PieceMeta>& meta) {
+// 1-2. the compressed bytes to every stream's device; candidate piece starts near every nominal boundary
+// (the first member's first block is piece 0) and, with `find_headers`, at every gzip header; every
+// piece to its first block end at or beyond the next candidate.  Each kernel runs over one contiguous
+// part per stream, given shifted pointers: member_find_kernel's boundary 1 is boundary j0, its bits
+// count from byte (j0 - 1) * piece; member_signature_kernel starts at byte b0 (whole blocks of it per
+// part); member_boundary_kernel's piece 0 is piece c0 (so `next` counts from c0).
+int find_pieces(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* gz, uint64_t n_bytes, size_t header, const MemberParams& p,
+                bool find_headers, std::vector<uint64_t>& starts, std::vector<uint8_t>& is_member,
+                std::vector<inflate::PieceMeta>& meta) {
   const uint32_t n_bounds = (uint32_t)((n_bytes + p.piece - 1) / p.piece);
-  const uint64_t heads_cap = n_bytes / 256 + 4096;
+  // member-start candidates: up to one per 256 bytes of input (fewer, larger members go to the host)
+  const uint64_t heads_cap = find_headers ? n_bytes / 256 + 4096 : 0;
   constexpr uint32_t kWarps = kInflateThreads / 32;
   constexpr uint64_t kSignatureSpan = 256ull * kSignatureBytes;  // the input of one block of member_signature_kernel
   std::vector<uint64_t> cand((size_t)n_bounds + 1, ~0ull), found(ns, 0);
@@ -924,7 +728,7 @@ int split_pieces(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* gz, ui
     sgc_fastq_stream* s = ss[i];
     int rc = grow(&s->d_gz, &s->gz_cap, (size_t)n_bytes + 64, s->pool, s->stream);  // (the reader's slack)
     if (rc == SGC_OK) rc = grow(&s->d_cand, &s->cand_cap, (size_t)n_bounds + 1, s->pool, s->stream);
-    if (rc == SGC_OK) rc = grow(&s->d_heads, &s->heads_cap, (size_t)heads_cap + 1, s->pool, s->stream);
+    if (rc == SGC_OK && find_headers) rc = grow(&s->d_heads, &s->heads_cap, (size_t)heads_cap + 1, s->pool, s->stream);
     if (rc) return rc;
     SGC_CUDA_TRY(cudaMemcpyAsync(s->d_gz, gz, n_bytes, cudaMemcpyHostToDevice, s->stream));
     const uint64_t j0 = 1 + part_begin(n_bounds - 1, ns, i, kWarps), j1 = 1 + part_begin(n_bounds - 1, ns, i + 1, kWarps);
@@ -933,12 +737,14 @@ int split_pieces(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* gz, ui
       member_find_kernel<<<(unsigned)((j1 - j0 + kWarps - 1) / kWarps), kInflateThreads, kInflateSmem, s->stream>>>(
           s->d_gz + shift, n_bytes - shift, p.piece, (uint32_t)(j1 - j0 + 1), s->d_cand + (j0 - 1));
     const uint64_t b0 = part_begin(n_bytes, ns, i, kSignatureSpan), b1 = part_begin(n_bytes, ns, i + 1, kSignatureSpan);
-    SGC_CUDA_TRY(cudaMemsetAsync(s->d_heads + heads_cap, 0, sizeof(uint64_t), s->stream));
-    if (b1 > b0)
-      member_signature_kernel<<<(unsigned)((b1 - b0 + kSignatureSpan - 1) / kSignatureSpan), 256, 0, s->stream>>>(
-          s->d_gz + b0, n_bytes - b0, s->d_heads, heads_cap);
+    if (find_headers) {
+      SGC_CUDA_TRY(cudaMemsetAsync(s->d_heads + heads_cap, 0, sizeof(uint64_t), s->stream));
+      if (b1 > b0)
+        member_signature_kernel<<<(unsigned)((b1 - b0 + kSignatureSpan - 1) / kSignatureSpan), 256, 0, s->stream>>>(
+            s->d_gz + b0, n_bytes - b0, s->d_heads, heads_cap);
+      SGC_CUDA_TRY(cudaMemcpyAsync(&found[i], s->d_heads + heads_cap, sizeof(uint64_t), cudaMemcpyDeviceToHost, s->stream));
+    }
     SGC_CUDA_TRY(cudaGetLastError());
-    SGC_CUDA_TRY(cudaMemcpyAsync(&found[i], s->d_heads + heads_cap, sizeof(uint64_t), cudaMemcpyDeviceToHost, s->stream));
     if (j1 > j0) SGC_CUDA_TRY(cudaMemcpyAsync(cand.data() + j0, s->d_cand + j0, (j1 - j0) * 8, cudaMemcpyDeviceToHost, s->stream));
     SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
     for (uint64_t j = j0; j < j1; ++j)
@@ -985,15 +791,15 @@ int split_pieces(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* gz, ui
 }
 
 // a wave of the chain: pieces [a, b), their text and where it goes
-struct SplitWave {
+struct Wave {
   uint32_t a, b;
   uint64_t text;
   std::vector<WavePiece> wp;
 };
 
-// What the streams of one split call hand each other: the entering window of every wave, composed on
-// the host as the waves in front publish F_k, and the bytes after the last complete record of the wave
-// framed last (framing goes wave after wave).
+// What the streams of one call hand each other (one stream: itself, from wave to wave): the entering
+// window of every wave, composed on the host as the waves in front publish F_k, and the bytes after the
+// last complete record of the wave framed last (framing goes wave after wave).
 struct WindowRelay {
   std::mutex mu;
   std::condition_variable cv;
@@ -1007,8 +813,8 @@ struct WindowRelay {
 
 // 4-7 for the waves k = i, i + ns, ... dealt to stream i; crc[x] (x: chain position) the CRC-32 of piece x.
 // Returns SGC_OK without finishing when another stream failed (relay.stop; the caller sets it on a failure).
-int split_stream_waves(sgc_fastq_stream* s, uint32_t i, uint32_t ns, uint64_t n_bytes, const std::vector<SplitWave>& waves,
-                       WindowRelay& relay, std::vector<uint32_t>& crc) {
+int stream_waves(sgc_fastq_stream* s, uint32_t i, uint32_t ns, uint64_t n_bytes, const std::vector<Wave>& waves, WindowRelay& relay,
+                 std::vector<uint32_t>& crc) {
   const uint32_t n_waves = (uint32_t)waves.size();
   auto wait_for = [&](auto ready) {  // false: another stream failed
     std::unique_lock<std::mutex> lk(relay.mu);
@@ -1017,10 +823,9 @@ int split_stream_waves(sgc_fastq_stream* s, uint32_t i, uint32_t ns, uint64_t n_
   };
   const size_t tail_at = offsetof(StreamState, tail);
   int rc = SGC_OK;
-  if (!s->d_window[0] && (rc = scratch_alloc(reinterpret_cast<void**>(&s->d_window[0]), inflate::kWindow, s->pool, s->stream)))
-    return rc;
+  if (!s->d_window && (rc = scratch_alloc(reinterpret_cast<void**>(&s->d_window), inflate::kWindow, s->pool, s->stream))) return rc;
   for (uint32_t k = i; k < n_waves; k += ns) {
-    const SplitWave& w = waves[k];
+    const Wave& w = waves[k];
     const uint32_t nw = w.b - w.a;
     rc = grow(&s->d_wave, &s->wave_cap, (size_t)nw + 1, s->pool, s->stream);
     if (rc == SGC_OK) rc = grow(&s->d_sym, &s->sym_cap, (size_t)w.text + 1, s->pool, s->stream);
@@ -1051,10 +856,10 @@ int split_stream_waves(sgc_fastq_stream* s, uint32_t i, uint32_t ns, uint64_t n_
     }
     // the text, once W_k is known
     if (!wait_for([&] { return relay.composed > k; })) return SGC_OK;
-    SGC_CUDA_TRY(cudaMemcpyAsync(s->d_window[0], relay.window[k].data(), inflate::kWindow, cudaMemcpyHostToDevice, s->stream));
+    SGC_CUDA_TRY(cudaMemcpyAsync(s->d_window, relay.window[k].data(), inflate::kWindow, cudaMemcpyHostToDevice, s->stream));
     uint8_t* text = s->d_text + kHeadroom;
-    member_settle_kernel<<<nw, 256, 0, s->stream>>>(s->d_sym, s->d_wave, text, s->d_window[0]);
-    member_resolve_kernel<<<nw, 256, 0, s->stream>>>(s->d_sym, s->d_wave, text, s->d_window[0]);
+    member_settle_kernel<<<nw, 256, 0, s->stream>>>(s->d_sym, s->d_wave, text, s->d_window);
+    member_resolve_kernel<<<nw, 256, 0, s->stream>>>(s->d_sym, s->d_wave, text, s->d_window);
     member_crc_kernel<<<(nw + kCrcWarps - 1) / kCrcWarps, kCrcWarps * 32, 0, s->stream>>>(s->d_wave, nw, text, s->d_crc);
     SGC_CUDA_TRY(cudaGetLastError());
     // framing, behind the wave in front: its carried bytes come first
@@ -1083,11 +888,13 @@ int split_stream_waves(sgc_fastq_stream* s, uint32_t i, uint32_t ns, uint64_t n_
   return SGC_OK;
 }
 
-int submit_split(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* gz, uint64_t n_bytes) {
+// One gzip file decoded by the ns streams ss[] together: sgc_fastq_stream_submit_gzip_split, and with one
+// stream sgc_fastq_stream_submit_gzip and sgc_fastq_stream_submit_member (`find_headers` false: no gzip
+// header inside the file is a candidate, so the chain must end at the first trailer).
+int submit_plain_gzip(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* gz, uint64_t n_bytes, bool find_headers) {
   if (!ss || !gz || ns == 0) return set_error(SGC_ERR_INVALID_ARG, "NULL argument or no stream");
   for (uint32_t i = 0; i < ns; ++i)
     if (!ss[i]) return set_error(SGC_ERR_INVALID_ARG, "NULL stream");
-  if (ns == 1) return submit_pieces(ss[0], gz, n_bytes, true);
   for (uint32_t i = 0; i < ns; ++i) {
     const sgc_fastq_stream* s = ss[i];
     if (s->failed || !s->counter) return set_error(SGC_ERR_INVALID_ARG, "a stream has failed or its counter is gone");
@@ -1104,31 +911,31 @@ int submit_split(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* gz, ui
   for (uint32_t i = 0; i < ns; ++i) ss[i]->member_submitted = true;
   size_t header = 0;
   if (inflate::gzip_header(gz, (size_t)n_bytes, &header) != inflate::kOk)
-    return split_fail(ss, ns, member_decline(ss[0], "not a gzip member"));
+    return fail_all(ss, ns, member_decline(ss[0], "not a gzip member"));
   const MemberParams params = member_params(ss[0]->read_len);
 
-  // 1-2. split by input range
+  // 1-2. candidate starts near every nominal boundary (and at every gzip header), the boundary pass
   std::vector<uint64_t> starts;
   std::vector<uint8_t> is_member;
   std::vector<inflate::PieceMeta> meta;
-  int rc = split_pieces(ss, ns, gz, n_bytes, header, params, starts, is_member, meta);
-  if (rc) return split_fail(ss, ns, rc);
+  int rc = find_pieces(ss, ns, gz, n_bytes, header, params, find_headers, starts, is_member, meta);
+  if (rc) return fail_all(ss, ns, rc);
 
-  // 3. the chain, as for one stream
+  // 3. the chain from the first block, over every trailer and header to the last trailer, which must end the file
   MemberChain c;
-  if (const char* why = follow_chain(gz, n_bytes, starts, is_member, meta, c)) return split_fail(ss, ns, member_decline(ss[0], why));
+  if (const char* why = follow_chain(gz, n_bytes, starts, is_member, meta, c)) return fail_all(ss, ns, member_decline(ss[0], why));
 
   // 4-7. waves of about min(wave_text, text / streams), dealt round robin
   uint64_t total = 0;
   for (uint32_t i = 0; i < c.n_chain; ++i) total += meta[c.chain[i]].out_len;
   const uint64_t cap = std::min(params.wave_text, std::max<uint64_t>(1, (total + ns - 1) / ns));
-  std::vector<SplitWave> waves;
+  std::vector<Wave> waves;
   uint64_t done = 0, member_begin = 0;
   for (uint32_t a = 0; a < c.n_chain;) {
-    SplitWave w{a, a, 0, {}};
+    Wave w{a, a, 0, {}};
     while (w.b < c.n_chain && (w.b == a || w.text + meta[c.chain[w.b]].out_len <= cap)) w.text += meta[c.chain[w.b++]].out_len;
     if (ss[0]->read_len == 0 && w.text >= (1ull << 32) - 2 * kHeadroom)
-      return split_fail(ss, ns, member_decline(ss[0], "a piece inflates to 4 GiB or more"));
+      return fail_all(ss, ns, member_decline(ss[0], "a piece inflates to 4 GiB or more"));
     uint64_t off = 0;
     for (uint32_t x = a; x < w.b; ++x) {
       if (x > 0 && c.member_of[x] != c.member_of[x - 1]) member_begin = done + off;
@@ -1146,7 +953,7 @@ int submit_split(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* gz, ui
   relay.window.assign(waves.size(), std::vector<uint8_t>(inflate::kWindow, 0));  // W_0: zeros
   std::vector<uint32_t> piece_crc(c.n_chain, 0);
   rc = on_each_stream(ss, ns, [&](uint32_t i) {
-    const int rc = split_stream_waves(ss[i], i, ns, n_bytes, waves, relay, piece_crc);
+    const int rc = stream_waves(ss[i], i, ns, n_bytes, waves, relay, piece_crc);
     if (rc) {
       std::lock_guard<std::mutex> lk(relay.mu);
       relay.stop = true;
@@ -1154,14 +961,19 @@ int submit_split(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* gz, ui
     }
     return rc;
   });
-  if (rc) return split_fail(ss, ns, rc);
+  if (rc) return fail_all(ss, ns, rc);
   std::vector<uint32_t> crc(c.n_members, 0);
-  for (const SplitWave& w : waves)
+  for (const Wave& w : waves)
     for (uint32_t x = w.a; x < w.b; ++x) {
       uint32_t& m = crc[c.member_of[x]];
       m = inflate::crc_combine(m, piece_crc[x], w.wp[x - w.a + 1].off - w.wp[x - w.a].off);
     }
-  if (const uint32_t m = crc_mismatch(c, crc); m < c.n_members) return split_fail(ss, ns, crc_error(m));
+  for (uint32_t m = 0; m < c.n_members; ++m)
+    if (crc[m] != c.trailers[m].crc) {
+      char buf[160];
+      snprintf(buf, sizeof buf, "gzip member %u: CRC-32 of the inflated bytes differs from the member's trailer", m);
+      return fail_all(ss, ns, set_error(SGC_ERR_GZIP, buf));
+    }
   for (uint32_t i = 0; i < ns; ++i) {
     ss[i]->member_pieces = starts.size();
     ss[i]->member_chain = c.n_chain;
@@ -1184,7 +996,7 @@ void sgc::fastq_stream_release(sgc_fastq_stream* s) {
   s->failed = true;  // nothing more can be submitted
   for (void* p : {(void*)s->d_state, (void*)s->d_gz, (void*)s->d_text, (void*)s->d_spans, (void*)s->d_tail, (void*)s->d_seq_start,
                   (void*)s->d_seq_end, (void*)s->d_begin, (void*)s->d_outoff, (void*)s->d_counts, (void*)s->d_first, (void*)s->d_sums,
-                  (void*)s->d_sym, (void*)s->d_window[0], (void*)s->d_window[1], (void*)s->d_cand, (void*)s->d_meta,
+                  (void*)s->d_sym, (void*)s->d_window, (void*)s->d_cand, (void*)s->d_meta,
                   (void*)s->d_wave, (void*)s->d_crc, (void*)s->d_heads, (void*)s->d_is_member})
     scratch_free(p, s->pool, s->stream);
 }
@@ -1307,12 +1119,12 @@ int sgc_fastq_stream_finish(sgc_fastq_stream* s, uint64_t* n_records) {
   return SGC_OK;
 }
 
-int sgc_fastq_stream_submit_member(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes) { return submit_pieces(s, gz, n_bytes, false); }
+int sgc_fastq_stream_submit_member(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes) { return submit_plain_gzip(&s, 1, gz, n_bytes, false); }
 
-int sgc_fastq_stream_submit_gzip(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes) { return submit_pieces(s, gz, n_bytes, true); }
+int sgc_fastq_stream_submit_gzip(sgc_fastq_stream* s, const uint8_t* gz, uint64_t n_bytes) { return submit_plain_gzip(&s, 1, gz, n_bytes, true); }
 
 int sgc_fastq_stream_submit_gzip_split(sgc_fastq_stream* const* streams, uint32_t n_streams, const uint8_t* gz, uint64_t n_bytes) {
-  return submit_split(streams, n_streams, gz, n_bytes);
+  return submit_plain_gzip(streams, n_streams, gz, n_bytes, true);
 }
 
 // Every buffer a stream keeps is sized by `grow` (need + need / 4 when it grows), so none ever holds
@@ -1342,7 +1154,7 @@ int sgc_fastq_stream_scratch_bound(int bgzf, uint64_t gz_bytes, uint64_t text_by
     b += grown(gz_bytes + 64) + grown(pieces * 8) + grown(heads * 8);                      // d_gz, d_cand, d_heads
     b += grown(pieces * sizeof(inflate::PieceMeta)) + grown(pieces);                       // d_meta, d_is_member
     b += grown((text + 1) * 2) + grown((pieces + 1) * sizeof(WavePiece)) + grown(pieces * 4);  // d_sym, d_wave, d_crc
-    b += 2 * inflate::kWindow;                                                             // d_window
+    b += inflate::kWindow;                                                                 // d_window
   }
   // the pool's rounding of some twenty buffers, and the counter's skew replicas (at most 64 MB)
   *bytes = b + (128ull << 20);

@@ -621,7 +621,8 @@ SGC_HD int gunzip_member(const uint8_t* in, size_t in_len, uint8_t* out, size_t 
 //      is never linked;
 //   4. each piece on that chain is decoded into 16-bit symbols: 0-255 bytes, 256 + i byte i of the
 //      32 KiB window in front of the piece, still unknown (MarkSink);
-//   5. the windows are resolved piece after piece, then everything else in parallel.
+//   5. the text is cut into waves, and each wave's windows are relayed piece after piece ("waves: the
+//      window relay" below), then everything else is resolved in parallel.
 // A single member is the case where no gzip header inside the file is listed: the first trailer must
 // then end the file, and a file of several members is declined.
 // These functions are written for that use, separately from gunzip_member, whose symbol loop is the
@@ -917,11 +918,12 @@ inline uint32_t members_chain(const uint8_t* in, size_t in_len, const uint64_t* 
   }
 }
 
-// ---- waves on several streams: the window relay ------------------------------------------------
-// The chain's text, cut into waves k = 0, 1, ..., may be decoded by several streams at once
-// (sgc_fastq_stream_submit_gzip_split; member_core_test with <waves>).  Wave k's first pieces refer,
-// through their markers, to W_k, the 32 KiB of text in front of the wave, which earlier waves make.
-// So that no wave waits for another while it decodes:
+// ---- waves: the window relay --------------------------------------------------------------------
+// The chain's text is cut into waves k = 0, 1, ..., which one stream decodes one after another or
+// several streams at once (sgc_fastq_stream_submit_gzip_split; one stream is its n = 1 case;
+// member_core_test with <waves>).  Wave k's first pieces refer, through their markers, to W_k, the
+// 32 KiB of text in front of the wave, which earlier waves make.  So that no wave waits for another
+// while it decodes:
 //   a. the last 32 KiB (or all) of every piece, piece after piece, are relayed in place
 //      (relay_symbol): a marker that names a byte of the wave takes the symbol already relayed
 //      there, one that names a byte in front of the wave becomes 256 + j, byte j of W_k;

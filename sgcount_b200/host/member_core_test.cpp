@@ -1,13 +1,12 @@
 // member_core_test <file.gz> <piece_bytes> <skew 0|1> [members 0|1 [waves]] — decodes a gzip file the way the
 // device does (gzip.cu member_* kernels), serially, from the same csrc/inflate_core.h code: candidate
 // block starts every piece_bytes of compressed input (with skew, every other candidate moved one bit on),
-// the boundary pass, the chain (members_chain), 16-bit symbols with window markers, the window resolution
-// piece after piece and then the rest, CRC-32 in pieces joined and ISIZE, member by member.  With
-// members = 1 every gzip header is a member-start candidate too, so the file may hold any number of
-// members (sgc_fastq_stream_submit_gzip); without, it must be one (sgc_fastq_stream_submit_member).
-// With <waves>, the chain is cut into about that many waves as sgc_fastq_stream_submit_gzip_split cuts
-// it, and each wave's windows are relayed through F_k and W_k (inflate_core.h "waves on several
-// streams") instead of being resolved over the whole text.
+// the boundary pass, the chain (members_chain), 16-bit symbols with window markers, the chain cut into
+// about <waves> waves (default 1) as sgc_fastq_stream_submit_gzip_split cuts it over that many streams,
+// each wave's windows relayed through F_k and W_k (inflate_core.h "waves: the window relay"), CRC-32 in
+// pieces joined and ISIZE, member by member.  With members = 1 every gzip header is a member-start
+// candidate too, so the file may hold any number of members (sgc_fastq_stream_submit_gzip); without, it
+// must be one (sgc_fastq_stream_submit_member).
 // Prints "<bytes> <fnv1a> <pieces> <chain> <absorbed>" (with members = 1, then "<members>"; exit 0),
 // "decline ..." when the chain does not reach the end (exit 3: the device would hand the file to the
 // host), or the error (exit 4).  Test helper for tests/test_member_inflate_core.py and
@@ -32,8 +31,8 @@ int main(int argc, char** argv) {
   const uint64_t piece = (uint64_t)atoll(argv[2]);
   const bool skew = atoi(argv[3]) != 0;
   const bool members = argc > 4 && atoi(argv[4]) != 0;
-  const uint64_t waves = argc > 5 ? (uint64_t)atoll(argv[5]) : 0;
-  if (piece < 16 || (argc > 5 && waves < 1)) return 2;
+  const uint64_t waves = argc > 5 ? (uint64_t)atoll(argv[5]) : 1;
+  if (piece < 16 || waves < 1) return 2;
   data.resize(n + 64);  // the reader's slack
   const uint8_t* in = data.data();
   PlainTableStorage storage;
@@ -115,44 +114,32 @@ int main(int argc, char** argv) {
     }
   }
 
-  // 5. the window in front of every piece, in order; then the rest
+  // 5. waves of about total / waves bytes (at least one piece each); every wave sees only its own
+  // symbols and the window composed from the waves before it
   std::vector<uint8_t> text(total + 1);
-  auto resolve = [&](uint32_t i, uint64_t x) {
-    const uint16_t s = sym[x];
-    text[x] = s < 256 ? (uint8_t)s : text[off[i] - kWindow + (s - 256)];
-  };
-  if (!waves) {
-    for (uint32_t i = 0; i < n_chain; ++i)
-      for (uint64_t x = off[i + 1] - off[i] > kWindow ? off[i + 1] - kWindow : off[i]; x < off[i + 1]; ++x) resolve(i, x);
-    for (uint32_t i = 0; i < n_chain; ++i)
-      for (uint64_t x = off[i]; x + kWindow < off[i + 1]; ++x) resolve(i, x);
-  } else {
-    // waves of about total / waves bytes (at least one piece each); every wave sees only its own
-    // symbols and the window composed from the waves before it
-    const uint64_t cap = (total + waves - 1) / waves;
-    std::vector<uint8_t> window(kWindow, 0), next(kWindow);  // W_0: zeros
-    std::vector<uint16_t> front(kWindow);
-    for (uint32_t a = 0; a < n_chain;) {
-      uint32_t b = a;
-      uint64_t len = 0;
-      while (b < n_chain && (b == a || len + (off[b + 1] - off[b]) <= cap)) len += off[b + 1] - off[b], ++b;
-      uint16_t* ws = sym.data() + off[a];  // the wave's symbols, addressed from its first byte
-      uint8_t* wt = text.data() + off[a];
-      auto region = [&](uint32_t i) { return off[i + 1] - off[i] > kWindow ? off[i + 1] - kWindow : off[i]; };
-      for (uint32_t i = a; i < b; ++i)  // a. piece after piece
-        for (uint64_t x = region(i); x < off[i + 1]; ++x) ws[x - off[a]] = relay_symbol(ws[x - off[a]], off[i] - off[a], ws);
-      const uint64_t m = len < kWindow ? len : kWindow;  // b. F_k and W_{k+1}
-      for (uint64_t j = 0; j < m; ++j) front[kWindow - m + j] = ws[len - m + j];
-      wave_front(front.data(), len);
-      compose_window(front.data(), window.data(), next.data());
-      for (uint32_t i = a; i < b; ++i) {  // c. the relayed symbols, then the rest
-        for (uint64_t x = region(i); x < off[i + 1]; ++x) wt[x - off[a]] = settle_symbol(ws[x - off[a]], window.data());
-        for (uint64_t x = off[i]; x + kWindow < off[i + 1]; ++x)
-          wt[x - off[a]] = settle_symbol(relay_symbol(ws[x - off[a]], off[i] - off[a], ws), window.data());
-      }
-      window.swap(next);
-      a = b;
+  const uint64_t cap = (total + waves - 1) / waves;
+  std::vector<uint8_t> window(kWindow, 0), next(kWindow);  // W_0: zeros
+  std::vector<uint16_t> front(kWindow);
+  for (uint32_t a = 0; a < n_chain;) {
+    uint32_t b = a;
+    uint64_t len = 0;
+    while (b < n_chain && (b == a || len + (off[b + 1] - off[b]) <= cap)) len += off[b + 1] - off[b], ++b;
+    uint16_t* ws = sym.data() + off[a];  // the wave's symbols, addressed from its first byte
+    uint8_t* wt = text.data() + off[a];
+    auto region = [&](uint32_t i) { return off[i + 1] - off[i] > kWindow ? off[i + 1] - kWindow : off[i]; };
+    for (uint32_t i = a; i < b; ++i)  // a. piece after piece
+      for (uint64_t x = region(i); x < off[i + 1]; ++x) ws[x - off[a]] = relay_symbol(ws[x - off[a]], off[i] - off[a], ws);
+    const uint64_t m = len < kWindow ? len : kWindow;  // b. F_k and W_{k+1}
+    for (uint64_t j = 0; j < m; ++j) front[kWindow - m + j] = ws[len - m + j];
+    wave_front(front.data(), len);
+    compose_window(front.data(), window.data(), next.data());
+    for (uint32_t i = a; i < b; ++i) {  // c. the relayed symbols, then the rest
+      for (uint64_t x = region(i); x < off[i + 1]; ++x) wt[x - off[a]] = settle_symbol(ws[x - off[a]], window.data());
+      for (uint64_t x = off[i]; x + kWindow < off[i + 1]; ++x)
+        wt[x - off[a]] = settle_symbol(relay_symbol(ws[x - off[a]], off[i] - off[a], ws), window.data());
     }
+    window.swap(next);
+    a = b;
   }
 
   // 6. CRC-32 in pieces, joined per member

@@ -1,8 +1,9 @@
 #!/bin/bash
 # usage: bash tools/sanitize_host.sh — the host-side test helpers (fastx_dump: host reader + whole-member
 # inflate; inflate_core_test: the device's gzip decoder compiled for the host; member_core_test: one member,
-# or with its fourth argument several, decoded in pieces as the device does it, with its fifth in waves) rebuilt with
-# -fsanitize=address,undefined, their test files run against them, the ordinary builds put back.
+# or with its fourth argument several, decoded in pieces and relayed wave by wave as the device does it, in
+# one wave or as many as its fifth argument asks) rebuilt with -fsanitize=address,undefined, their test
+# files run against them, the ordinary builds put back.
 # Needs a g++ that ships libasan (CXX_SAN, default /usr/bin/g++).
 set -e
 cd "$(dirname "$0")/.."
