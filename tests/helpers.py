@@ -85,6 +85,36 @@ def make_reads(rng, guides, n_reads, read_len, offset, reverse=False, variable=F
     return out
 
 
+def realistic_fastq(rng, seqs):
+    """FASTQ text as an Illumina instrument writes it, around the sequences `seqs`: headers
+    '@A00123:45:HXXXXDSXX:1:1101:<x>:<y> 1:N:0:<index>' of varying length, a '+' line that repeats
+    the name on some records, and Phred+33 qualities over '#'..'J' drawn per position, some of them
+    starting with '@' (Q31) or '+' (Q10), which a framer must not take for a record or separator
+    line.  Such text inflates from literal-heavy DEFLATE with long codes, unlike constant qualities.
+    Returns the text and the (begin, end) of every quality line."""
+    n = len(seqs)
+    width = max(len(s) for s in seqs) if n else 0
+    qual = rng.integers(ord("#"), ord("J") + 1, size=(n, max(width, 1)), dtype=np.uint8)
+    first = rng.random(n)
+    qual[first < 0.05, 0] = ord("@")
+    qual[(first >= 0.05) & (first < 0.08), 0] = ord("+")
+    xs, ys = rng.integers(1000, 10 ** rng.integers(4, 6, n)), rng.integers(1000, 10 ** rng.integers(4, 6, n))
+    lanes, tiles = rng.integers(1, 5, n), rng.integers(1101, 2679, n)
+    index = ACGT[rng.integers(0, 4, (n, 16))]
+    dual = rng.random(n) < 0.5
+    repeat = rng.random(n) < 0.2
+    parts, slots, at = [], [], 0
+    for i, s in enumerate(seqs):
+        name = b"A00123:45:HXXXXDSXX:%d:%d:%d:%d" % (lanes[i], tiles[i], xs[i], ys[i])
+        idx = index[i].tobytes() if dual[i] else index[i, :8].tobytes()
+        rec = b"@%s 1:N:0:%s\n%s\n+%s\n" % (name, idx, s, name if repeat[i] else b"")
+        q = qual[i, :len(s)].tobytes()
+        slots.append((at + len(rec), at + len(rec) + len(q)))
+        parts.append(rec + q + b"\n")
+        at += len(parts[-1])
+    return b"".join(parts), slots
+
+
 def oracle_library(guides, aliases=None):
     aliases = aliases or [b"g%d" % i for i in range(len(guides))]
     recs = orc.Records.from_bytes(b"".join(b">" + a + b"\n" + s + b"\n" for a, s in zip(aliases, guides)))

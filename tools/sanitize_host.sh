@@ -17,4 +17,4 @@ trap 'cp /tmp/sgc_san/fastx_dump /tmp/sgc_san/inflate_core_test /tmp/sgc_san/mem
   $CXX_SAN $SAN -o ../lib/member_core_test member_core_test.cpp)
 ASAN_OPTIONS=detect_leaks=0 UBSAN_OPTIONS=print_stacktrace=1:halt_on_error=1 \
   python -m pytest tests/test_host_reader.py tests/test_host_inflate.py tests/test_device_inflate_core.py tests/test_member_inflate_core.py \
-  tests/test_multi_member_inflate_core.py tests/test_member_waves_core.py -x -q
+  tests/test_multi_member_inflate_core.py tests/test_member_waves_core.py tests/test_deflate_edges.py -x -q
