@@ -310,6 +310,25 @@ int sgc_fastq_stream_submit_gzip_split(sgc_fastq_stream* const* streams, uint32_
  * submit at the same time. */
 int sgc_fastq_stream_scratch_bound(int bgzf, uint64_t gz_bytes, uint64_t text_bytes, uint32_t read_len, uint32_t span_len,
                                    uint64_t* bytes);
+/* Uncompressed FASTQ text, text[0 .. n_bytes) in host memory of any kind (a read-only file mapping,
+ * mostly), framed and counted as the text of a BGZF wave, in the mode sgc_fastq_stream_create fixed.
+ * self_contained == 0: the call continues where the previous one stopped and may end anywhere in a
+ * record (the bytes after its last complete record are carried on).  self_contained != 0: the text
+ * starts and ends on a record boundary and the stream holds no carried bytes (SGC_ERR_FASTQ_FORMAT
+ * otherwise), so that the waves of one file may be dealt to several streams or devices.  Declines as
+ * sgc_fastq_stream_submit does (a record that does not start with '@', a read of another length in the
+ * first mode, a record over 64 KiB, a bad cut); a failed stream refuses later calls; n_bytes == 0 does
+ * nothing.  The stream cuts a call into waves of a fixed size (64 MiB): the next wave's bytes go
+ * through pinned staging (several host threads) and a copy stream of their own into a second device
+ * text buffer while the current wave is framed and counted.  All host threads are joined, and the
+ * caller's memory is no longer read, when the call returns.  Host memory: the stream pins two staging
+ * buffers of one wave (128 MiB in all) at its first text call; a destroyed stream's buffers go to a list of
+ * the process from which later streams take theirs, which keeps at most eight of them. */
+int sgc_fastq_stream_submit_text(sgc_fastq_stream*, const uint8_t* text, uint64_t n_bytes, int self_contained);
+/* An upper bound of the device scratch ONE stream allocates through sgc_fastq_stream_submit_text (both
+ * text buffers, the chunk counts and scan, span records or line offsets of the fullest wave), as
+ * sgc_fastq_stream_scratch_bound; it needs no device.  read_len / span_len: as sgc_fastq_stream_create. */
+int sgc_fastq_stream_text_scratch_bound(uint32_t read_len, uint32_t span_len, uint64_t* bytes);
 /* Members decoded by sgc_fastq_stream_submit_gzip (1 after sgc_fastq_stream_submit_member, else 0). */
 int sgc_fastq_stream_gzip_members(const sgc_fastq_stream*, uint64_t* members);
 int sgc_fastq_stream_finish(sgc_fastq_stream*, uint64_t* n_records);

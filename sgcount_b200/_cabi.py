@@ -103,6 +103,8 @@ SIGNATURES = {
     "sgc_fastq_stream_submit_gzip": (_int, [_vp, _vp, _u64]),
     "sgc_fastq_stream_submit_gzip_split": (_int, [C.POINTER(_vp), _u32, _vp, _u64]),
     "sgc_fastq_stream_scratch_bound": (_int, [_int, _u64, _u64, _u32, _u32, C.POINTER(_u64)]),
+    "sgc_fastq_stream_submit_text": (_int, [_vp, _vp, _u64, _int]),
+    "sgc_fastq_stream_text_scratch_bound": (_int, [_u32, _u32, C.POINTER(_u64)]),
     "sgc_fastq_stream_gzip_members": (_int, [_vp, C.POINTER(_u64)]),
     "sgc_fastq_stream_finish": (_int, [_vp, C.POINTER(_u64)]),
     "sgc_counter_launch_info": (_int, [_vp, C.POINTER(LaunchInfo)]),

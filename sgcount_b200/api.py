@@ -433,6 +433,15 @@ class FastqStream:
         check(_cabi.load().sgc_fastq_stream_submit_gzip(self._ptr, blob.ctypes.data, len(blob)))
         self._counter._result = None
 
+    def submit_text(self, blob: np.ndarray, self_contained: bool = False) -> None:
+        """uncompressed FASTQ text (any uint8 array, an np.memmap included), framed and counted on the device
+        (sgc_fastq_stream_submit_text).  self_contained=False: continues where the previous call stopped and
+        may end anywhere in a record; True: starts and ends on a record boundary with nothing carried in
+        (SgcError(ERR_FASTQ_FORMAT) otherwise)"""
+        blob = np.ascontiguousarray(blob).view(np.uint8).reshape(-1)
+        check(_cabi.load().sgc_fastq_stream_submit_text(self._ptr, blob.ctypes.data, blob.nbytes, 1 if self_contained else 0))
+        self._counter._result = None
+
     def gzip_members(self) -> int:
         """members decoded by submit_gzip (1 after submit_member)"""
         v = C.c_uint64()
@@ -479,4 +488,12 @@ def fastq_stream_scratch_bound(bgzf: bool, gz_bytes: int, text_bytes: int, read_
     out = C.c_uint64()
     check(_cabi.load().sgc_fastq_stream_scratch_bound(1 if bgzf else 0, int(gz_bytes), int(text_bytes), int(read_len),
                                                       int(span_len), C.byref(out)))
+    return int(out.value)
+
+
+def fastq_stream_text_scratch_bound(read_len: int, span_len: int) -> int:
+    """the most device scratch one FastqStream allocates for FastqStream.submit_text
+    (sgc_fastq_stream_text_scratch_bound)"""
+    out = C.c_uint64()
+    check(_cabi.load().sgc_fastq_stream_text_scratch_bound(int(read_len), int(span_len), C.byref(out)))
     return int(out.value)

@@ -22,16 +22,22 @@
 // complete record are carried in front of the next wave's text.  Only fixed-length 4-line FASTQ
 // takes this path (the head of the sample, which the host reads for the offset detector, says so);
 // anything irregular is reported and the caller counts the sample through the host path instead.
+//
+// Uncompressed FASTQ (sgc_fastq_stream_submit_text) skips the inflate: the text of a call goes in waves
+// through pinned staging and a copy stream into one of two device text buffers, the next wave's copy
+// running while the current wave is framed and counted by the same kernels.
 #include <stdio.h>
 #include <stdlib.h>
 
 #include <algorithm>
 #include <condition_variable>
 #include <cstddef>
+#include <cstring>
 #include <map>
 #include <mutex>
 #include <string>
 #include <thread>
+#include <tuple>
 #include <vector>
 
 #include "inflate_core.h"
@@ -484,6 +490,58 @@ void scratch_free(void* p, cudaMemPool_t pool, cudaStream_t stream) {
     cudaFree(p);
 }
 
+// Pinned staging buffers of the text path, shared by the streams of the process: a destroyed stream's
+// buffers go back to a free list instead of to cudaFreeHost, which may wait for the device the way
+// cudaFree does, and pinning anew costs about as much as the copy it serves.  The list keeps at most
+// kStagingKept buffers (the rest are freed, outside the lock); the ones it holds at exit go with the
+// process.  Host footprint: two buffers of one wave (2 x kTextWave) per stream submitting text, plus at
+// most kStagingKept waves on the list.
+constexpr size_t kStagingKept = 8;
+struct StagingPool {
+  std::mutex mu;
+  std::vector<std::pair<uint8_t*, size_t>> free;
+};
+StagingPool& staging_pool() {
+  static StagingPool* pool = new StagingPool();  // (never destroyed: no CUDA call after the runtime's teardown)
+  return *pool;
+}
+// *p, of *cap bytes, holds at least `need` bytes (a kept buffer if one is large enough)
+void staging_give(uint8_t* p, size_t cap);
+int staging_take(uint8_t** p, size_t* cap, size_t need) {
+  if (need <= *cap) return SGC_OK;
+  staging_give(*p, *cap);
+  *p = nullptr;
+  *cap = 0;
+  StagingPool& pool = staging_pool();
+  {
+    std::lock_guard<std::mutex> lk(pool.mu);
+    for (size_t i = 0; i < pool.free.size(); ++i)
+      if (pool.free[i].second >= need) {
+        std::tie(*p, *cap) = pool.free[i];
+        pool.free.erase(pool.free.begin() + i);
+        return SGC_OK;
+      }
+  }
+  SGC_CUDA_TRY(cudaHostAlloc(reinterpret_cast<void**>(p), need, cudaHostAllocPortable));
+  *cap = need;
+  return SGC_OK;
+}
+void staging_give(uint8_t* p, size_t cap) {
+  if (!p) return;
+  StagingPool& pool = staging_pool();
+  uint8_t* drop = nullptr;
+  {
+    std::lock_guard<std::mutex> lk(pool.mu);
+    pool.free.emplace_back(p, cap);
+    if (pool.free.size() > kStagingKept) {
+      auto smallest = std::min_element(pool.free.begin(), pool.free.end(), [](auto& a, auto& b) { return a.second < b.second; });
+      drop = smallest->first;
+      pool.free.erase(smallest);
+    }
+  }
+  if (drop) cudaFreeHost(drop);
+}
+
 template <typename T>
 int grow(T** p, size_t* cap, size_t need, cudaMemPool_t pool, cudaStream_t stream) {
   if (need <= *cap) return SGC_OK;
@@ -533,6 +591,16 @@ struct sgc_fastq_stream {
   uint8_t* d_is_member = nullptr;
   size_t heads_cap = 0, is_member_cap = 0;
   uint64_t gzip_members = 0;
+  // plain text (sgc_fastq_stream_submit_text): the next wave is copied into d_text_next while the wave in
+  // d_text is framed and counted; its bytes pass through pinned staging, on a copy stream of its own
+  uint8_t* d_text_next = nullptr;
+  size_t text_next_cap = 0;
+  uint8_t* h_stage[2] = {nullptr, nullptr};
+  size_t stage_cap[2] = {0, 0};
+  cudaStream_t copy_stream = nullptr;
+  cudaEvent_t copied = nullptr;     // the last host-to-device copy of a wave's text
+  cudaEvent_t text_free = nullptr;  // the stream's work up to the count of the wave before the current one
+  cudaEvent_t stage_free[2] = {nullptr, nullptr};  // the copy out of h_stage[i]
 };
 
 namespace {
@@ -983,6 +1051,109 @@ int submit_plain_gzip(sgc_fastq_stream* const* ss, uint32_t ns, const uint8_t* g
   return SGC_OK;
 }
 
+// ---- plain FASTQ text (sgc_fastq_stream_submit_text) ----
+// A call's text goes in waves of kTextWave bytes (SGC_TEXT_WAVE=bytes sets it, at most 1 GiB: tests run
+// many small waves); the wave bounds both text buffers and the staging, and keeps line mode's text far
+// below its 4 GiB.  Measured with tools/text_ingest_time.py (profiles/r9_text_ingest_time.txt).
+constexpr uint64_t kTextWave = 64ull << 20;
+uint64_t text_wave() {
+  uint64_t w = kTextWave;
+  if (const char* e = getenv("SGC_TEXT_WAVE"); e && atoll(e) > 0) w = std::min<uint64_t>((uint64_t)atoll(e), 1ull << 30);
+  return w;
+}
+
+// Copies from the caller's memory (a file mapping, mostly: its first touch of a page is a page fault) into
+// pinned staging, split over up to kStageThreads threads from kStageThreadBytes a thread.
+constexpr unsigned kStageThreads = 8;
+constexpr size_t kStageThreadBytes = 8u << 20;
+struct Staging {
+  std::vector<std::thread> threads;
+  void start(uint8_t* dst, const uint8_t* src, size_t n) {
+    const size_t parts = std::max<size_t>(1, std::min<size_t>(kStageThreads, n / kStageThreadBytes));
+    const size_t part = (n / parts + 4095) & ~(size_t)4095;
+    for (size_t i = 0; i < parts; ++i) {
+      const size_t at = std::min(n, part * i), len = i + 1 == parts ? n - at : std::min(n - at, part);
+      threads.emplace_back([=] { memcpy(dst + at, src + at, len); });
+    }
+  }
+  void join() {
+    for (auto& t : threads) t.join();
+    threads.clear();
+  }
+  ~Staging() { join(); }
+};
+
+int submit_text(sgc_fastq_stream* s, const uint8_t* text, uint64_t n_bytes, bool self_contained) {
+  const uint64_t wave = text_wave(), n_waves = (n_bytes + wave - 1) / wave;
+  const size_t most = (size_t)std::min(wave, n_bytes);
+  if (!s->copy_stream) {
+    SGC_CUDA_TRY(cudaStreamCreateWithFlags(&s->copy_stream, cudaStreamNonBlocking));
+    for (cudaEvent_t* e : {&s->copied, &s->text_free, &s->stage_free[0], &s->stage_free[1]})
+      SGC_CUDA_TRY(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+  }
+  if (self_contained) {  // nothing may be carried into the call
+    StreamState st;
+    SGC_CUDA_TRY(cudaMemcpyAsync(&st, s->d_state, sizeof st, cudaMemcpyDeviceToHost, s->stream));
+    SGC_CUDA_TRY(cudaStreamSynchronize(s->stream));
+    if (st.tail) {
+      st.format_error = 8;
+      return stream_error(s, st, 0);
+    }
+  }
+  int rc = grow(&s->d_text, &s->text_cap, (size_t)kHeadroom + most + 64, s->pool, s->stream);
+  if (rc == SGC_OK) rc = grow(&s->d_text_next, &s->text_next_cap, (size_t)kHeadroom + most + 64, s->pool, s->stream);
+  for (int i = 0; i < 2 && rc == SGC_OK; ++i) rc = staging_take(&s->h_stage[i], &s->stage_cap[i], most);
+  if (rc) return rc;
+  // (the copy stream writes buffers the pool allocated on s->stream, whose last counts may still read them)
+  SGC_CUDA_TRY(cudaEventRecord(s->text_free, s->stream));
+  Staging staging;
+  auto wave_bytes = [&](uint64_t k) { return (size_t)std::min(wave, n_bytes - k * wave); };
+  auto stage = [&](uint64_t k) -> int {  // wave k's bytes into h_stage[k & 1], once its last copy is done
+    SGC_CUDA_TRY(cudaEventSynchronize(s->stage_free[k & 1]));
+    staging.start(s->h_stage[k & 1], text + k * wave, wave_bytes(k));
+    return SGC_OK;
+  };
+  auto send = [&](uint64_t k) -> int {  // ... and on to d_text_next, once the count that read it is done
+    staging.join();
+    SGC_CUDA_TRY(cudaStreamWaitEvent(s->copy_stream, s->text_free, 0));
+    SGC_CUDA_TRY(cudaMemcpyAsync(s->d_text_next + kHeadroom, s->h_stage[k & 1], wave_bytes(k), cudaMemcpyHostToDevice, s->copy_stream));
+    SGC_CUDA_TRY(cudaEventRecord(s->stage_free[k & 1], s->copy_stream));
+    SGC_CUDA_TRY(cudaEventRecord(s->copied, s->copy_stream));
+    return SGC_OK;
+  };
+  // The bytes a wave carries on must fit kHeadroom.  Of any four consecutive newlines one ends a record, so
+  // four in the last kHeadroom bytes of a wave bound them; a wave smaller than that carries less than itself,
+  // or nothing complete at all, which frame_and_count reports.
+  auto tail_fits = [&](uint64_t k) {
+    const size_t n = wave_bytes(k);
+    if (n < kHeadroom) return true;
+    const uint8_t *lo = text + k * wave + n - kHeadroom, *p = lo + kHeadroom;
+    for (int found = 0; found < 4; ++found) {
+      p = static_cast<const uint8_t*>(memrchr(lo, '\n', (size_t)(p - lo)));
+      if (!p) return false;
+    }
+    return true;
+  };
+  if ((rc = stage(0)) || (rc = send(0))) return rc;
+  for (uint64_t k = 0; k < n_waves; ++k) {
+    if (!tail_fits(k)) {
+      StreamState st{};
+      st.bad_block = 0xFFFFFFFFu;
+      st.format_error = 4;
+      return stream_error(s, st, 0);
+    }
+    std::swap(s->d_text, s->d_text_next);
+    std::swap(s->text_cap, s->text_next_cap);
+    if (k + 1 < n_waves && (rc = stage(k + 1))) return rc;  // (under the framing of wave k)
+    SGC_CUDA_TRY(cudaStreamWaitEvent(s->stream, s->copied, 0));
+    wave_begin_kernel<<<1, 1, 0, s->stream>>>(s->d_state, 0, self_contained && k + 1 == n_waves ? 1u : 0u);
+    if ((rc = frame_and_count(s, wave_bytes(k), 0))) return rc;
+    if (k + 1 < n_waves && (rc = send(k + 1))) return rc;  // (under the count of wave k)
+    SGC_CUDA_TRY(cudaEventRecord(s->text_free, s->stream));
+  }
+  return SGC_OK;
+}
+
 }  // namespace
 
 // Frees the device side and detaches the stream from its counter; the handle itself stays valid.
@@ -990,6 +1161,7 @@ void sgc::fastq_stream_release(sgc_fastq_stream* s) {
   if (!s || !s->counter) return;
   DeviceGuard guard(s->device);
   cudaStreamSynchronize(s->stream);
+  if (s->copy_stream) cudaStreamSynchronize(s->copy_stream);  // (a declined text call may leave a copy in flight)
   auto& list = s->counter->fastq_streams;
   list.erase(std::remove(list.begin(), list.end(), s), list.end());
   s->counter = nullptr;
@@ -997,8 +1169,15 @@ void sgc::fastq_stream_release(sgc_fastq_stream* s) {
   for (void* p : {(void*)s->d_state, (void*)s->d_gz, (void*)s->d_text, (void*)s->d_spans, (void*)s->d_tail, (void*)s->d_seq_start,
                   (void*)s->d_seq_end, (void*)s->d_begin, (void*)s->d_outoff, (void*)s->d_counts, (void*)s->d_first, (void*)s->d_sums,
                   (void*)s->d_sym, (void*)s->d_window, (void*)s->d_cand, (void*)s->d_meta,
-                  (void*)s->d_wave, (void*)s->d_crc, (void*)s->d_heads, (void*)s->d_is_member})
+                  (void*)s->d_wave, (void*)s->d_crc, (void*)s->d_heads, (void*)s->d_is_member, (void*)s->d_text_next})
     scratch_free(p, s->pool, s->stream);
+  if (s->copy_stream) {
+    cudaStreamSynchronize(s->copy_stream);
+    for (int i = 0; i < 2; ++i) staging_give(s->h_stage[i], s->stage_cap[i]);
+    for (cudaEvent_t e : {s->copied, s->text_free, s->stage_free[0], s->stage_free[1]}) cudaEventDestroy(e);
+    cudaStreamDestroy(s->copy_stream);
+    s->copy_stream = nullptr;
+  }
 }
 
 extern "C" {
@@ -1157,6 +1336,36 @@ int sgc_fastq_stream_scratch_bound(int bgzf, uint64_t gz_bytes, uint64_t text_by
     b += inflate::kWindow;                                                                 // d_window
   }
   // the pool's rounding of some twenty buffers, and the counter's skew replicas (at most 64 MB)
+  *bytes = b + (128ull << 20);
+  return SGC_OK;
+}
+
+int sgc_fastq_stream_submit_text(sgc_fastq_stream* s, const uint8_t* text, uint64_t n_bytes, int self_contained) {
+  if (!s || !text) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
+  if (s->failed || !s->counter) return set_error(SGC_ERR_INVALID_ARG, "the stream has failed or its counter is gone");
+  if (n_bytes == 0) return SGC_OK;
+  DeviceGuard guard(s->device);
+  const int rc = submit_text(s, text, n_bytes, self_contained != 0);
+  // a call that fails between a wave's copy and its framing leaves that copy in flight: it must land before
+  // the caller may release the buffers it writes (or the caller's memory)
+  if (rc && s->copy_stream) cudaStreamSynchronize(s->copy_stream);
+  return rc;
+}
+
+// As sgc_fastq_stream_scratch_bound, for the buffers of sgc_fastq_stream_submit_text: two text buffers
+// of one wave each (text_wave()), and what frame_and_count grows for a region of that size.
+int sgc_fastq_stream_text_scratch_bound(uint32_t read_len, uint32_t span_len, uint64_t* bytes) {
+  if (!bytes) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
+  if (read_len != 0 && (span_len == 0 || span_len > read_len)) return set_error(SGC_ERR_INVALID_ARG, "the span does not fit the read");
+  auto grown = [](uint64_t need) { return need + need / 4; };
+  const uint64_t region = kHeadroom + text_wave();
+  const uint64_t chunks = region / kChunk + 2;
+  uint64_t b = sizeof(StreamState) + kHeadroom;                                            // d_state, d_tail
+  b += 2 * grown(region + 64);                                                             // d_text, d_text_next
+  b += 2 * grown((chunks + 1) * 4) + grown((chunks / 2048 + 2) * 4);                       // d_counts, d_first, d_sums
+  const uint64_t records = region / ((uint64_t)read_len + 6) + 2;                          // a record takes its read and 6 more bytes
+  b += read_len ? grown(records * ((span_len + 7u) & ~7u) + 256) : 2 * grown(records * 4);  // d_spans / d_seq_start, d_seq_end
+  // the pool's rounding, and the counter's skew replicas (at most 64 MB), as sgc_fastq_stream_scratch_bound
   *bytes = b + (128ull << 20);
   return SGC_OK;
 }

@@ -100,7 +100,7 @@ const char* kUsage =
     "      --ingest-threads <N>               Threads inflating the gzip members of one sample [default: cores / samples in flight]\n"
     "      --rc-keep-n                        Reverse complement keeps N (default: the fxread bit trick, N -> J)\n"
     "      --whole-lines                      Copy whole sequence lines to the device (default: for fixed-length reads, only the guide window and one byte either side)\n"
-    "      --host-inflate                     Inflate and frame records on the host even for BGZF, single-member or multi-member gzip input (default: BGZF files of FASTQ, and gzip files of FASTQ that are one member, are inflated, framed and counted on the device; so are multi-member gzip files large enough and with too few members or ingest threads for the host to decode them faster side by side)\n"
+    "      --host-inflate                     Inflate and frame records on the host even for BGZF, single-member or multi-member gzip input, and read and frame uncompressed FASTQ there too (default: BGZF files of FASTQ, gzip files of FASTQ that are one member, and uncompressed FASTQ files are inflated or copied, framed and counted on the device; so are multi-member gzip files large enough and with too few members or ingest threads for the host to decode them faster side by side)\n"
     "      --timing                           Print a JSON line with the phase times to stderr\n"
     "  -h, --help                             Print help\n";
 
@@ -330,6 +330,7 @@ struct SampleHead {
   bool fastq = false;    // '@' records (4 lines)
   bool uniform = true;   // every record read so far has first_len bases
   bool bgzf = false;     // the file begins with a BGZF block (a candidate for the device ingest)
+  bool text = false;     // the file begins with '@' or '>': uncompressed, whatever its name
 };
 // Does the file begin with a gzip member that carries a 'BC' extra subfield (BGZF)?
 bool begins_with_bgzf_block(const std::string& path) {
@@ -350,6 +351,11 @@ bool begins_with_bgzf_block(const std::string& path) {
 SampleHead read_head(const std::string& path, unsigned long records) {
   SampleHead h;
   h.bgzf = begins_with_bgzf_block(path);
+  if (FILE* f = fopen(path.c_str(), "rb")) {
+    const int c = fgetc(f);
+    h.text = c == '@' || c == '>';
+    fclose(f);
+  }
   sgh::FastxReader reader(path);
   const char *id, *seq;
   size_t id_len, seq_len;
@@ -387,6 +393,7 @@ struct SampleResult {
   double dev_index_s = 0, dev_create_s = 0, dev_waves_s = 0, dev_finish_s = 0;  // phases of the device ingest
   bool device_ingest = false;               // inflate and record framing ran on the device (BGZF input)
   uint64_t device_blocks = 0;
+  uint64_t device_text_bytes = 0;           // uncompressed FASTQ counted on the device
   uint64_t member_pieces = 0, member_chain = 0, member_absorbed = 0;  // gzip members in pieces on the device
   uint64_t gzip_members = 0;                                          // how many (not BGZF), as the device confirmed them
   unsigned member_lanes = 0;                                          // streams that decoded them together
@@ -634,6 +641,130 @@ bool count_member_on_device(const std::vector<const sgc_library*>& libs, const s
   r.dev_create_s = seconds(t0, t1);
   r.dev_waves_s = seconds(t1, t2);
   r.dev_finish_s = seconds(t2, t3);
+  return true;
+}
+
+// An uncompressed FASTQ through sgc_fastq_stream_submit_text: mapped, and on one device the whole file in
+// one call (the stream carries cut records from wave to wave).  With libs.size() > 1 lanes the text is cut
+// here into parts at record ends, about two per lane (at least kTextPartMin, or SGC_TEXT_WAVE bytes when
+// set: tests), dealt to the lanes as self-contained calls, the counters summed with sgc_reduce_counts.  A
+// cut is the end of the last record that fastq_last_record_end recognises in the 64 KiB before the
+// nominal one; where it finds none the file goes to one lane.  A wrong guess is reported by the device
+// (the part does not start on a record), and the sample then goes to the host.
+constexpr uint64_t kTextPartMin = 64ull << 20;
+bool count_text_on_device(const std::vector<const sgc_library*>& libs, const std::vector<DeviceBudget*>& budgets, uint32_t n_guides,
+                          uint32_t k, const std::string& path, OffsetValue offset, uint32_t read_len, bool variable, bool recursion,
+                          int rc_mode, SampleResult& r, std::string& why_not) {
+  uint32_t span_start = 0, span_len = 0, span_offset = offset.index;
+  if (!variable && sgc_span_geometry(k, read_len, offset.reverse, offset.index, recursion, &span_start, &span_len,
+                                     &span_offset) != SGC_OK) {
+    why_not = "the guide window does not fit the reads";
+    return false;
+  }
+  auto seconds = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) {
+    return std::chrono::duration<double>(b - a).count();
+  };
+  const auto t_start = std::chrono::steady_clock::now();
+  MappedFile file(path);
+  if (!file.data) {
+    why_not = "cannot map the file";
+    return false;
+  }
+  if (file.data[0] != '@') {  // (a compressed file not named .gz: the host reader knows it by its magic)
+    why_not = "not uncompressed text";
+    return false;
+  }
+  // parts [cuts[i], cuts[i + 1]) of the text
+  std::vector<uint64_t> cuts{0};
+  if (libs.size() > 1) {
+    uint64_t part = std::max<uint64_t>(kTextPartMin, file.size / (2 * libs.size()) + 1);
+    if (const char* e = getenv("SGC_TEXT_WAVE"); e && atoll(e) > 0) part = (uint64_t)atoll(e);
+    constexpr uint64_t kWindow = 64u << 10;
+    for (uint64_t c = part; c < file.size; c += part) {
+      const uint64_t lo = std::max(cuts.back(), c > kWindow ? c - kWindow : 0);
+      const size_t end = sgh::fastq_last_record_end(reinterpret_cast<const char*>(file.data) + lo, (size_t)(c - lo));
+      if (end == SIZE_MAX) {
+        cuts.assign(1, 0);
+        break;
+      }
+      if (lo + end > cuts.back()) cuts.push_back(lo + end);
+    }
+  }
+  cuts.push_back(file.size);
+  const size_t n_parts = cuts.size() - 1, n_lanes = std::min(libs.size(), n_parts);
+  const auto t_planned = std::chrono::steady_clock::now();
+  uint64_t bound = 0;
+  check(sgc_fastq_stream_text_scratch_bound(variable ? 0 : read_len, span_len, &bound));
+  Reservation reserved(lane_bytes(budgets, n_lanes, bound));  // (declared before the streams: released after them)
+  struct Lane {
+    sgc_counter* c = nullptr;
+    sgc_fastq_stream* stream = nullptr;
+    uint64_t records = 0;
+    int status = SGC_OK;
+    std::string error;
+  };
+  struct Guard {
+    std::vector<Lane> lanes;
+    ~Guard() {
+      for (auto& l : lanes) {
+        sgc_fastq_stream_destroy(l.stream);
+        sgc_counter_destroy(l.c);
+      }
+    }
+  } g;
+  g.lanes.resize(n_lanes);
+  for (size_t d = 0; d < n_lanes; ++d) {
+    check(sgc_counter_create(libs[d], offset.reverse, span_offset, recursion, rc_mode, nullptr, nullptr, &g.lanes[d].c));
+    check(sgc_fastq_stream_create(g.lanes[d].c, variable ? 0 : read_len, span_start, span_len, &g.lanes[d].stream));
+  }
+  const auto t_created = std::chrono::steady_clock::now();
+  std::atomic<size_t> next_part{0};
+  std::atomic<bool> failed{false};
+  auto run_lane = [&](Lane& l) {
+    for (size_t p; l.status == SGC_OK && !failed.load() && (p = next_part.fetch_add(1)) < n_parts;) {
+      // (the last part may end without a newline or in a cut record: finish() sees to it)
+      l.status = sgc_fastq_stream_submit_text(l.stream, file.data + cuts[p], cuts[p + 1] - cuts[p], n_parts > 1 && p + 1 < n_parts);
+    }
+    if (l.status == SGC_OK && !failed.load()) l.status = sgc_fastq_stream_finish(l.stream, &l.records);
+    if (l.status != SGC_OK) {
+      l.error = sgc_last_error();
+      failed.store(true);
+    }
+  };
+  {
+    std::vector<std::thread> pool;
+    for (size_t d = 1; d < n_lanes; ++d) pool.emplace_back([&, d] { run_lane(g.lanes[d]); });
+    run_lane(g.lanes[0]);
+    for (auto& t : pool) t.join();
+  }
+  const auto t_waved = std::chrono::steady_clock::now();
+  uint64_t n_records = 0;
+  for (auto& l : g.lanes) {
+    if (l.status == SGC_ERR_FASTQ_FORMAT) {
+      why_not = l.error;
+      return false;
+    }
+    if (l.status != SGC_OK) fail("%s", l.error.c_str());
+    n_records += l.records;
+  }
+  if (n_lanes > 1) {
+    std::vector<sgc_counter*> shards;
+    for (auto& l : g.lanes) shards.push_back(l.c);
+    check(sgc_reduce_counts(shards.data(), (int)shards.size(), 0));
+  }
+  r.counts.resize(n_guides);
+  check(sgc_counter_finish(g.lanes[0].c, r.counts.data(), &r.total, &r.matched));
+  r.span_reads = variable ? 0 : n_records;
+  r.line_reads = variable ? n_records : 0;
+  r.device_ingest = true;
+  r.device_text_bytes = file.size;
+  r.shards = (unsigned)n_lanes;
+  const auto t_end = std::chrono::steady_clock::now();
+  r.submit_s = seconds(t_start, t_end);
+  r.dev_index_s = seconds(t_start, t_planned);
+  r.dev_create_s = seconds(t_planned, t_created);
+  r.dev_waves_s = seconds(t_created, t_waved);
+  r.dev_finish_s = seconds(t_waved, t_end);
   return true;
 }
 
@@ -965,10 +1096,12 @@ int main(int argc, char** argv) {
     // counted (once: count_sample_on_device is given the count).
     std::vector<SampleHead> heads(n_samples);
     std::vector<size_t> members(n_samples, 0);
-    auto device_candidate = [&](size_t i) {
+    auto named_gz = [&](size_t i) {
       const std::string& p = args.input_paths[i];
-      return !args.host_inflate && heads[i].fastq && p.size() > 3 && p.compare(p.size() - 3, 3, ".gz") == 0;
+      return p.size() > 3 && p.compare(p.size() - 3, 3, ".gz") == 0;
     };
+    // gzip FASTQ (named .gz) and uncompressed FASTQ (whose first byte says so) go to the device ingest
+    auto device_candidate = [&](size_t i) { return !args.host_inflate && heads[i].fastq && (named_gz(i) || heads[i].text); };
     {
       std::vector<std::exception_ptr> errors(n_samples);
       std::atomic<size_t> next_head{0};
@@ -976,7 +1109,7 @@ int main(int argc, char** argv) {
         for (size_t i; (i = next_head.fetch_add(1)) < n_samples;) {
           try {
             heads[i] = read_head(args.input_paths[i], args.have_offset ? 0 : args.subsample);
-            if (device_candidate(i) && args.read_shards <= 1) {  // (with read shards only BGZF goes to the device)
+            if (device_candidate(i) && named_gz(i) && args.read_shards <= 1) {  // (with read shards only BGZF goes to the device)
               MappedFile file(args.input_paths[i]);
               if (file.data) members[i] = gzip_members(file.data, file.size, kHostCoresPerDevice + 1);
             }
@@ -1090,13 +1223,14 @@ int main(int argc, char** argv) {
     std::vector<uint32_t> first_len(n_samples);
     std::vector<char> head_uniform(n_samples, 0), head_fastq(n_samples, 0);  // 4-line FASTQ? head reads of one length?
     const bool member_ok = args.read_shards <= 1;  // (read shards asked for: gzip that is not BGZF keeps the host path)
-    std::vector<char> candidate(n_samples, 0);
+    std::vector<char> candidate(n_samples, 0), plain(n_samples, 0);
     std::vector<uint64_t> input_bytes(n_samples, 0);
     for (size_t i = 0; i < n_samples; ++i) {
       first_len[i] = (uint32_t)heads[i].first_len;
       head_fastq[i] = heads[i].fastq;
       head_uniform[i] = heads[i].fastq && heads[i].uniform;
       candidate[i] = device_candidate(i);
+      plain[i] = !named_gz(i) && heads[i].text;
       struct stat st;
       if (stat(args.input_paths[i].c_str(), &st) == 0) input_bytes[i] = (uint64_t)st.st_size;
     }
@@ -1119,7 +1253,7 @@ int main(int argc, char** argv) {
     bool all_for_the_device = per_sample == 1;
     for (size_t i = 0; i < n_samples && all_for_the_device; ++i) {
       std::string why_not;
-      all_for_the_device = (!args.host_inflate && heads[i].fastq && heads[i].bgzf) ||
+      all_for_the_device = (!args.host_inflate && heads[i].fastq && heads[i].bgzf) || (candidate[i] && plain[i]) ||
                            (candidate[i] && member_ok && gzip_file_to_device(members[i], input_bytes[i], ingest_for(device_workers), why_not));
     }
     heads.clear();
@@ -1137,22 +1271,25 @@ int main(int argc, char** argv) {
             sample_libs.push_back(libs[(s * per_sample + j) % gpus]);
             sample_budgets.push_back(&budgets[(s * per_sample + j) % gpus]);
           }
-          // BGZF input of fixed-length FASTQ: the whole ingest on the device (one device per sample);
-          // anything else, or anything the device declines, through the host's inflate threads
+          // gzip and uncompressed FASTQ: the whole ingest on the device; anything else, or anything the
+          // device declines, through the host's reader and inflate threads
           bool on_device = false;
           std::string why_not = "switched off";
           if (candidate[s]) {
+            auto to_device = [&](bool variable) {
+              return plain[s] ? count_text_on_device(sample_libs, sample_budgets, hlib.n, hlib.k, args.input_paths[s], offsets[s],
+                                                     first_len[s], variable, !args.no_position_recursion, args.rc_mode, results[s], why_not)
+                              : count_sample_on_device(sample_libs, sample_budgets, hlib.n, hlib.k, args.input_paths[s], offsets[s],
+                                                       first_len[s], variable, !args.no_position_recursion, args.rc_mode, member_ok,
+                                                       members[s], ingest_threads, results[s], why_not);
+            };
             // fixed-length reads as span records; reads of several lengths (seen in the head, or
             // reported by the device deeper in the file) with their sequence lines in place
             bool variable = !head_uniform[s] || args.whole_lines;
-            on_device = count_sample_on_device(sample_libs, sample_budgets, hlib.n, hlib.k, args.input_paths[s], offsets[s], first_len[s],
-                                               variable, !args.no_position_recursion, args.rc_mode, member_ok, members[s], ingest_threads,
-                                               results[s], why_not);
+            on_device = to_device(variable);
             if (!on_device && !variable && why_not.find("FASTQ") != std::string::npos) {
               results[s] = SampleResult();
-              on_device = count_sample_on_device(sample_libs, sample_budgets, hlib.n, hlib.k, args.input_paths[s], offsets[s],
-                                                 first_len[s], true, !args.no_position_recursion, args.rc_mode, member_ok, members[s],
-                                                 ingest_threads, results[s], why_not);
+              on_device = to_device(true);
             }
           } else if (!head_fastq[s]) {
             why_not = "not FASTQ";
@@ -1191,7 +1328,7 @@ int main(int argc, char** argv) {
       unsigned long long reads = 0;
       double wait_s = 0, copy_s = 0, submit_s = 0;
       unsigned max_shards = 1;
-      unsigned long long span_reads = 0, device_blocks = 0, adopted = 0, reframed = 0, pieces = 0, chain = 0, absorbed = 0, gzip_member_count = 0;
+      unsigned long long span_reads = 0, device_blocks = 0, device_text_bytes = 0, adopted = 0, reframed = 0, pieces = 0, chain = 0, absorbed = 0, gzip_member_count = 0;
       unsigned device_samples = 0, member_lanes = 0, in_flight = 0;
       for (int d = 0; d < gpus; ++d) in_flight = std::max(in_flight, budgets[d].most);
       std::string host_because;
@@ -1203,6 +1340,7 @@ int main(int argc, char** argv) {
         adopted += r.members_adopted, reframed += r.members_reframed;
         device_samples += r.device_ingest;
         device_blocks += r.device_blocks;
+        device_text_bytes += r.device_text_bytes;
         pieces += r.member_pieces, chain += r.member_chain, absorbed += r.member_absorbed, gzip_member_count += r.gzip_members;
         if (!r.device_ingest && host_because.empty()) host_because = r.host_because;
         max_shards = std::max(max_shards, r.shards);
@@ -1210,11 +1348,11 @@ int main(int argc, char** argv) {
       }
       fprintf(stderr, "{\"count_s\": %.6f, \"reads\": %llu, \"samples\": %zu, \"sample_workers\": %u, "
               "\"ingest_threads\": %u, \"gpus\": %d, \"read_shards_per_sample\": %u, \"span_reads\": %llu, \"device_ingest_samples\": %u, "
-              "\"device_blocks\": %llu, \"device_phases_s\": [%.4f, %.4f, %.4f, %.4f], \"host_ingest_because\": \"%s\", \"members_adopted\": %llu, \"members_reframed\": %llu, \"wait_inflate_s\": %.6f, "
+              "\"device_blocks\": %llu, \"device_text_bytes\": %llu, \"device_phases_s\": [%.4f, %.4f, %.4f, %.4f], \"host_ingest_because\": \"%s\", \"members_adopted\": %llu, \"members_reframed\": %llu, \"wait_inflate_s\": %.6f, "
               "\"copy_to_pinned_s\": %.6f, \"submit_sync_s\": %.6f, \"read_inputs_s\": %.3f, "
               "\"device_tables_s\": %.3f, \"offsets_s\": %.3f, \"member_pieces\": %llu, \"member_chain\": %llu, \"member_absorbed\": %llu, \"gzip_members\": %llu, "
               "\"member_lanes\": %u, \"device_samples_in_flight\": %u}\n",
-              count_s, reads, n_samples, workers, ingest_threads, gpus, max_shards, span_reads, device_samples, device_blocks,
+              count_s, reads, n_samples, workers, ingest_threads, gpus, max_shards, span_reads, device_samples, device_blocks, device_text_bytes,
               dev_index_s, dev_create_s, dev_waves_s, dev_finish_s, host_because.c_str(), adopted, reframed, wait_s, copy_s, submit_s, t_inputs,
               t_tables - t_inputs, t_offsets - t_tables, pieces, chain, absorbed, gzip_member_count, member_lanes, in_flight);
     }
