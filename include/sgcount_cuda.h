@@ -159,6 +159,15 @@ void sgc_counter_destroy(sgc_counter*);
  * Centered window does not fit the read (offset + k > read_len: every read is unmatched anyway). */
 int sgc_span_geometry(uint32_t k, uint32_t read_len, int is_reverse, uint32_t offset, int position_recursion,
                       uint32_t* span_start, uint32_t* span_len, uint32_t* span_offset);
+/* The span for a counter with max_shift S (sgc_counter_set_max_shift).  S = 1 returns exactly what
+ * sgc_span_geometry(..., position_recursion = 1, ...) returns.  S >= 2: the span is
+ * [max(0, o - S), min(read_len, o + k + S)) in the coordinates of the trimmed read (the reverse
+ * complement of the whole read when is_reverse), mirrored to stored coordinates for reverse reads,
+ * and span_offset = o - max(0, o - S), so the span records hold exactly the windows the read holds.
+ * Fails with SGC_ERR_INVALID_ARG only when no window offset + d, |d| <= S, fits the read, or when S
+ * is outside 1..16. */
+int sgc_span_geometry_shift(uint32_t k, uint32_t read_len, int is_reverse, uint32_t offset, uint32_t max_shift,
+                            uint32_t* span_start, uint32_t* span_len, uint32_t* span_offset);
 
 /* Count a batch held in HOST memory (pinned memory makes the copies asynchronous).  The
  * batch is cut into chunks that are copied and counted on alternating buffers so copy and
@@ -182,6 +191,18 @@ int sgc_counter_submit_device(sgc_counter*, const uint8_t* d_lines, uint64_t n_b
  * overrides the plan: 1 = never, >1 = that many copies (rounded down to a power of two, at most
  * 64 copies / 64 MB), 0 = back to automatic.  The counts never depend on it. */
 int sgc_counter_set_replicas(sgc_counter*, uint32_t replicas);
+
+/* Staggered reads (amplicons sequenced with staggered primers move the guide by a few bases from
+ * read to read).  max_shift = S, 1..16.  S = 1 (the default) is the reference's recursion: Centered,
+ * then Plus, then Minus, returning when a trim fails (counter.rs:96-140).  S >= 2 tries the windows
+ * at offset + d for d = 0, +1, -1, ..., +S, -S in the coordinates of the trimmed read (the reverse
+ * complement of the whole read in Reverse), each looked up as counter.rs:111-117 does (member, then
+ * the Permuter's unique one-mismatch parent); the first that yields a guide wins, and a window that
+ * does not fit the read is skipped instead of ending the search.  total_reads and matched_reads keep
+ * their meaning.  Must be called before the counter's first submit.  SGC_ERR_INVALID_ARG: S outside
+ * 1..16, a counter that has counted, S >= 2 without position recursion or with a byte-keyed library
+ * (sgc_library_info.opaque).  Span records for such a counter: sgc_span_geometry_shift. */
+int sgc_counter_set_max_shift(sgc_counter*, uint32_t max_shift);
 
 int sgc_counter_sync(sgc_counter*);
 /* Wait until all but the last `keep_in_flight` sgc_counter_submit calls have had their host
@@ -336,7 +357,8 @@ int sgc_fastq_stream_finish(sgc_fastq_stream*, uint64_t* n_records);
 /* Statistics of the last sgc_counter_submit_device call, for benchmarking. */
 typedef struct sgc_launch_info {
   uint32_t grid, block, smem_bytes;
-  uint32_t kernel; /* 0 = streaming fixed-stride kernel, 1 = line kernel (any layout), 2 = byte-keyed (opaque library) */
+  uint32_t kernel; /* 0 = streaming fixed-stride kernel, 1 = line kernel (any layout), 2 = byte-keyed (opaque library),
+                      3 = shift kernel (max_shift >= 2, any layout) */
   uint64_t launches_total;
   uint32_t replicas;   /* copies of the count vector in use (1 = none) */
   uint32_t hot_guides; /* guides counted in registers */

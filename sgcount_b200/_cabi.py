@@ -82,11 +82,14 @@ SIGNATURES = {
     "sgc_position_counts": (_int, [_int, _vp, _u64, _vp, _u32, _u32, _u64, _vp, _u32, C.POINTER(_u32)]),
     "sgc_offset_detect": (_int, [_vp, _vp, _u64, _vp, _u32, _u32, _u64, C.POINTER(_int), C.POINTER(_u32)]),
     "sgc_span_geometry": (_int, [_u32, _u32, _int, _u32, _int, C.POINTER(_u32), C.POINTER(_u32), C.POINTER(_u32)]),
+    "sgc_span_geometry_shift": (_int, [_u32, _u32, _int, _u32, _u32, C.POINTER(_u32), C.POINTER(_u32),
+                                        C.POINTER(_u32)]),
     "sgc_counter_create": (_int, [_vp, _int, _u32, _int, _int, _vp, _vp, C.POINTER(_vp)]),
     "sgc_counter_destroy": (None, [_vp]),
     "sgc_counter_submit": (_int, [_vp, _vp, _u64, _vp, _u32, _u32, _u64]),
     "sgc_counter_submit_device": (_int, [_vp, _vp, _u64, _vp, _u32, _u32, _u64, _vp]),
     "sgc_counter_set_replicas": (_int, [_vp, _u32]),
+    "sgc_counter_set_max_shift": (_int, [_vp, _u32]),
     "sgc_counter_sync": (_int, [_vp]),
     "sgc_counter_wait_copies": (_int, [_vp, _u32]),
     "sgc_reduce_counts": (_int, [C.POINTER(_vp), _int, _int]),

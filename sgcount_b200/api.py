@@ -211,21 +211,29 @@ class Permuter:
         return self._handle.info()
 
 
-def span_geometry(k: int, read_len: int, offset: Offset, position_recursion: bool = True):
+def span_geometry(k: int, read_len: int, offset: Offset, position_recursion: bool = True, max_shift: int = 1):
     """sgc_span_geometry: (start, length) of the span of a `read_len`-byte read — the guide window
     and the byte either side that Counter::assign may look at (counter.rs:164-174) — and the Offset
-    under which a counter treats span records as reads with the same outcome."""
+    under which a counter treats span records as reads with the same outcome.  max_shift >= 2: the
+    span of a counter searching offset +- max_shift (sgc_span_geometry_shift)."""
     start, length, idx = C.c_uint32(), C.c_uint32(), C.c_uint32()
-    check(_cabi.load().sgc_span_geometry(k, read_len, int(offset.reverse), offset.index, int(position_recursion),
-                                         C.byref(start), C.byref(length), C.byref(idx)))
+    if max_shift != 1:
+        if not position_recursion:
+            raise SgcError(_cabi.ERR_INVALID_ARG, "max_shift >= 2 needs position recursion")
+        check(_cabi.load().sgc_span_geometry_shift(k, read_len, int(offset.reverse), offset.index, int(max_shift),
+                                                   C.byref(start), C.byref(length), C.byref(idx)))
+    else:
+        check(_cabi.load().sgc_span_geometry(k, read_len, int(offset.reverse), offset.index, int(position_recursion),
+                                             C.byref(start), C.byref(length), C.byref(idx)))
     return start.value, length.value, Offset(offset.reverse, idx.value)
 
 
-def span_batch(reader: ReadBatch, k: int, offset: Offset, position_recursion: bool = True, out: Optional[np.ndarray] = None):
+def span_batch(reader: ReadBatch, k: int, offset: Offset, position_recursion: bool = True, out: Optional[np.ndarray] = None,
+               max_shift: int = 1):
     """Fixed-length reads cut down to span records of stride round_up(length, 8): what a host that
     frames its own records sends instead of whole lines.  Returns (ReadBatch of spans, Offset)."""
     assert reader.line_off is None, "span records need fixed-length reads"
-    start, length, span_offset = span_geometry(k, reader.read_len, offset, position_recursion)
+    start, length, span_offset = span_geometry(k, reader.read_len, offset, position_recursion, max_shift)
     stride = (length + 7) & ~7
     n = reader.n_reads
     rows = reader.lines[:n * reader.stride].reshape(n, reader.stride)
@@ -276,17 +284,20 @@ def entropy_offset_group(library: Library, readers: Sequence[ReadBatch], subsamp
 
 
 class Counter:
-    """counter.rs:17-252"""
+    """counter.rs:17-252.  max_shift: 1 (default) is the reference's +-1 position recursion; 2..16
+    searches offset + 0, +1, -1, ..., +S, -S for staggered reads (sgc_counter_set_max_shift)."""
 
     def __init__(self, library: Library, permuter: Optional[Permuter], offset: Offset,
                  position_recursion: bool = True, rc_mode: int = _cabi.RC_BITTRICK,
-                 stream: Optional[int] = None, d_state: Optional[int] = None):
+                 stream: Optional[int] = None, d_state: Optional[int] = None, max_shift: int = 1):
         self._library = library
         self._handle = permuter._handle if permuter is not None else library._exact
         self._ptr = C.c_void_p()
         check(_cabi.load().sgc_counter_create(self._handle.ptr, int(offset.reverse), offset.index,
                                               int(position_recursion), rc_mode, stream, d_state, C.byref(self._ptr)))
         self._result = None
+        if max_shift != 1:
+            self.set_max_shift(max_shift)
 
     def __del__(self):
         try:
@@ -321,6 +332,10 @@ class Counter:
         """override the skew plan: 0 = automatic (default), 1 = never, >1 = that many copies of the
         count vector"""
         check(_cabi.load().sgc_counter_set_replicas(self._ptr, int(replicas)))
+
+    def set_max_shift(self, max_shift: int) -> None:
+        """sgc_counter_set_max_shift: 1..16, before the first submit"""
+        check(_cabi.load().sgc_counter_set_max_shift(self._ptr, int(max_shift)))
 
     def wait_copies(self, keep_in_flight: int = 0) -> None:
         check(_cabi.load().sgc_counter_wait_copies(self._ptr, int(keep_in_flight)))

@@ -20,6 +20,8 @@
 //   count_lines_kernel   : any layout (variable-length lines via u32 offsets, unaligned
 //                          buffers, tile remainders); one thread per read, the span lifted from
 //                          global memory with 64-bit loads, same window arithmetic and tables.
+//   count_shift_kernel   : staggered reads (max_shift S >= 2): the line kernel's layouts, every
+//                          position offset + d, |d| <= S, through the parked queue.
 // Per-guide counts are 64-bit atomics in the L2-resident state vector; matched reads are
 // accumulated in registers and flushed once per warp.
 #include <algorithm>
@@ -545,6 +547,180 @@ __global__ void __launch_bounds__(kLineWarps * 32) count_lines_kernel(CountParam
   flush_matched<4>(p, matched, hot);
 }
 
+// ------------------------------------------------------------------------------------------
+// shift kernel: staggered reads (sgc_counter_set_max_shift, S = 2..16).  The windows at
+// offset + d, d = 0, +1, -1, ..., +S, -S in the coordinates of the read the reference trims (the
+// reverse complement of the whole read in Reverse), the first that yields a guide wins, and a
+// window that does not fit the read is skipped.  Any layout, like the line kernel: a warp takes
+// 32 consecutive reads, every lane works out its read's positions from the read's length, lifts
+// the span that holds them (k + 2S bytes at most) with 64-bit loads and parks it; the warp-private
+// queue is drained 32 reads at a time, each trying ONE position through the seed index
+// (try_position) and going back on the queue for its next position after a miss.  A position is
+// the NW + 1 parked words around it and a bit shift.
+// ------------------------------------------------------------------------------------------
+constexpr int kMaxShift = 16;
+constexpr uint32_t kShiftIdxBits = 26;  // tag: position index (0 .. 2S) << 26 | read index
+
+template <int NW>
+struct ShiftQueueT {
+  // span words: k + 2S <= 4 NW + 32 bytes; a window starts at most 2S bytes into the span and its
+  // NW + 1 words go up to word 8 + NW
+  uint32_t w[NW + 9][kQueueCap];
+  uint32_t tag[kQueueCap];
+  uint32_t range[kQueueCap];  // the read's positions: (dlo + S) | (dhi + S) << 8
+};
+
+// displacement of position index j (0, +1, -1, +2, -2, ...)
+__device__ __forceinline__ int shift_of(int j) { return (j & 1) ? (j + 1) >> 1 : -(j >> 1); }
+
+template <int NW, bool WIDE>
+__global__ void __launch_bounds__(kLineWarps * 32) count_shift_kernel(CountParams p, int max_shift) {
+  constexpr int SW = NW + 9;
+  __shared__ ShiftQueueT<NW> queues[kLineWarps];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  ShiftQueueT<NW>* q = &queues[warp];
+  uint32_t matched = 0;
+  HotCounts hot{};
+  const uint64_t table_policy = l2_evict_last_policy();
+  const uint64_t line_policy = l2_evict_first_policy();
+  const int k = (int)p.lib.k, S = max_shift, n_pos = 2 * max_shift + 1;
+  const StreamGeom& g = p.geom;  // n_words, last_mask, with_perm, wild_byte: the same for every read
+  const IndexView& ix = p.reverse ? p.lib.rev : p.lib.fwd;
+  const uint32_t gwarp = blockIdx.x * kLineWarps + warp, gwarps = gridDim.x * kLineWarps;
+  unsigned long long* my_counts = p.rep + (size_t)(gwarp & (p.n_rep - 1)) * p.n_guides;
+  constexpr int NL = (4 * SW + 7 + 7) / 8;  // 64-bit loads that cover SW words at any alignment
+  static_assert(2 * NL >= SW + 2, "span words");
+  constexpr uint32_t kIdxMask = (1u << kShiftIdxBits) - 1;
+  uint32_t qn = 0;  // parked reads (warp-uniform)
+
+  auto settle = [&](int32_t hit, uint32_t ridx) {
+    if (p.assign_out) p.assign_out[p.first_read + ridx] = hit;
+    count_hit<4>(p, my_counts, hit, matched, hot);
+  };
+  // the position index after j whose window fits the read, or n_pos
+  auto next_position = [&](int j, int dlo, int dhi) {
+    for (++j; j < n_pos; ++j) {
+      const int d = shift_of(j);
+      if (d >= dlo && d <= dhi) break;
+    }
+    return j;
+  };
+  auto drain = [&](bool all) {
+    while (qn >= 32 || (all && qn > 0)) {
+      const uint32_t cnt = qn < 32 ? qn : 32;
+      qn -= cnt;
+      int next = -1;
+      uint32_t U[SW], tag = 0, range = 0;
+      if ((uint32_t)lane < cnt) {
+        const uint32_t e = qn + lane;
+        tag = q->tag[e];
+        range = q->range[e];
+        const int j = (int)(tag >> kShiftIdxBits);
+        const int dlo = (int)(range & 0xFFu) - S, dhi = (int)(range >> 8) - S, d = shift_of(j);
+        const int b = p.reverse ? dhi - d : d - dlo;  // first window byte in the span (stored order)
+        uint32_t T[NW + 1];
+#pragma unroll
+        for (int i = 0; i < NW + 1; ++i) T[i] = q->w[(b >> 2) + i][e];
+        const int32_t hit = try_position<NW, WIDE>(p.lib, ix, g, T, 8u * (uint32_t)(b & 3), table_policy);
+        if (hit == kMiss) {
+          next = next_position(j, dlo, dhi);
+          if (next >= n_pos) next = -1;
+        }
+        if (next < 0) {
+          settle(hit, tag & kIdxMask);
+        } else {
+#pragma unroll
+          for (int i = 0; i < SW; ++i) U[i] = q->w[i][e];
+        }
+      }
+      __syncwarp();  // every lane has read its entry before any slot is overwritten
+      const uint32_t pm = __ballot_sync(0xffffffffu, next >= 0);
+      if (pm) {
+        if (next >= 0) {
+          const uint32_t e = qn + __popc(pm & ((1u << lane) - 1));
+#pragma unroll
+          for (int i = 0; i < SW; ++i) q->w[i][e] = U[i];
+          q->tag[e] = ((uint32_t)next << kShiftIdxBits) | (tag & kIdxMask);
+          q->range[e] = range;
+        }
+        qn += __popc(pm);
+      }
+      __syncwarp();
+    }
+  };
+
+  const uint64_t n_tiles = (p.n_reads + 31) / 32;
+  for (uint64_t t = gwarp; t < n_tiles; t += gwarps) {
+    const uint64_t i = t * 32 + lane;  // read of this lane, relative to the launch
+    int park = -1;                     // first position index whose window fits, or -1
+    uint32_t span[SW] = {}, range = 0;
+    if (i < p.n_reads) {
+      const uint64_t r = p.first_read + i;
+      uint64_t start;
+      int n;
+      if (p.line_end) {
+        start = p.line_off[r];
+        n = (int)(p.line_end[r] - p.line_off[r]);
+      } else if (p.line_off) {
+        const uint32_t a = p.line_off[r], b = p.line_off[r + 1];
+        start = a - p.off_base;
+        n = (int)(b - a) - 1;
+      } else {
+        start = r * p.stride;
+        n = (int)p.read_len;
+      }
+      // the displacements whose window fits: [dlo, dhi], possibly empty
+      const int dlo = p.offset < S ? -p.offset : -S;
+      const int dhi = min(S, n - k - p.offset);
+      if (dlo <= dhi) {
+        park = dhi >= 0 ? 0 : next_position(0, dlo, dhi);
+        range = (uint32_t)(dlo + S) | ((uint32_t)(dhi + S) << 8);
+        const int span_bytes = k + dhi - dlo;
+        const int first = p.reverse ? n - p.offset - dhi - k : p.offset + dlo;  // stored coordinates
+        const uint8_t* sb = p.lines + start + first;
+        const uint64_t* a8 = reinterpret_cast<const uint64_t*>((uintptr_t)sb & ~(uintptr_t)7);
+        const uint32_t sh = (uint32_t)((uintptr_t)sb & 7u);
+        const int need = ((int)sh + span_bytes + 4 + 7) >> 3;  // loads that reach one word past the span
+        uint32_t R[2 * NL];
+#pragma unroll
+        for (int j = 0; j < NL; ++j) {
+          // never a load that starts at or past the end of the buffer (bytes past the read only
+          // ever reach masked-off positions of a window)
+          const uint64_t v = j < need && reinterpret_cast<const uint8_t*>(a8 + j) < p.lines_end
+                                 ? ldg_stream_u64(a8 + j, line_policy)
+                                 : 0ull;
+          R[2 * j] = (uint32_t)v;
+          R[2 * j + 1] = (uint32_t)(v >> 32);
+        }
+        const bool odd = (sh & 4u) != 0;
+        const uint32_t bits = (sh & 3u) * 8u;
+#pragma unroll
+        for (int j = 0; j < SW; ++j) {
+          const uint32_t w0 = odd ? R[j + 1] : R[j], w1 = odd ? R[j + 2] : R[j + 1];
+          span[j] = __funnelshift_r(w0, w1, bits);
+        }
+      } else {
+        settle(kMiss, (uint32_t)i);  // no window fits the read
+      }
+    }
+    const uint32_t pm = __ballot_sync(0xffffffffu, park >= 0);
+    if (pm) {
+      if (park >= 0) {
+        const uint32_t e = qn + __popc(pm & ((1u << lane) - 1));
+#pragma unroll
+        for (int j = 0; j < SW; ++j) q->w[j][e] = span[j];
+        q->tag[e] = ((uint32_t)park << kShiftIdxBits) | (uint32_t)i;
+        q->range[e] = range;
+      }
+      qn += __popc(pm);
+      __syncwarp();
+    }
+    drain(false);
+  }
+  drain(true);
+  flush_matched<4>(p, matched, hot);
+}
+
 // NW = words that hold the k window bytes: 4 (k <= 16, the number of words in use is read from the
 // geometry), or exactly ceil(k / 4) = 5 (k = 17..20, the common guide lengths), 6, 7 or 8.
 template <int NW, bool WIDE, int MODE>
@@ -1011,11 +1187,13 @@ int launch_count(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const
   c->last.kernel = 1;
   c->last.replicas = c->n_rep;
   for (int j = 0; j < kHotGuides; ++j) c->last.hot_guides += c->hot[j] >= 0;
+  // staggered reads (max_shift >= 2) take the shift kernel whatever the layout
+  const bool shifted = c->max_shift >= 2;
   // streaming kernel: fixed stride, 16-byte aligned base, whole warp tiles, < 2^32 reads per
   // launch, and a Centered window that fits (otherwise every read fails its first trim)
   const uint32_t tile_bytes = kWarpReads * stride;
   const uint32_t stage_bytes = (tile_bytes + 48 + 15) & ~15u;  // +48: span words may run past the tile
-  const bool stageable = d_off == nullptr && ((uintptr_t)d_lines & 15u) == 0 && stride >= read_len &&
+  const bool stageable = !shifted && d_off == nullptr && ((uintptr_t)d_lines & 15u) == 0 && stride >= read_len &&
                          (uint64_t)c->offset + c->lib->k <= read_len;
   // kernel family by the words that hold the k window bytes: narrow keys 4 (k <= 16) or 5
   // (k = 17..20, the common guide lengths); wide keys 6 (k = 21..24), 7 (k = 25..28) or 8 (k = 29, 30)
@@ -1070,9 +1248,14 @@ int launch_count(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const
     c->last.launches_total += 1;
   }
   const bool lines_only = done == first;
+  // the shift kernel's queue tags keep a 26-bit read index; SGC_MAX_LAUNCH_TILES cuts its launches too
+  uint64_t shift_launch_reads = 1ull << kShiftIdxBits;
+  if (const long long cap = env_ll("SGC_MAX_LAUNCH_TILES", 0); cap > 0)
+    shift_launch_reads = std::min<uint64_t>(shift_launch_reads, (uint64_t)cap * kWarpReads);
+  if (shifted) c->last.kernel = 3;
   while (done < n_reads) {  // what the streaming kernel did not take; at most 2^27 reads per launch
     p.first_read = done;
-    p.n_reads = std::min<uint64_t>(n_reads - done, 1ull << kLineIdxBits);
+    p.n_reads = std::min<uint64_t>(n_reads - done, shifted ? shift_launch_reads : 1ull << kLineIdxBits);
     uint64_t blocks = (p.n_reads + 32 * kLineWarps - 1) / (32 * kLineWarps);
     const uint64_t cap = (uint64_t)c->lib->sm_count * 8;
     if (blocks > cap) blocks = cap;
@@ -1080,7 +1263,14 @@ int launch_count(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const
     static const LineKernel line_kernels[5] = {count_lines_kernel<4, false>, count_lines_kernel<5, false>,
                                                count_lines_kernel<6, true>, count_lines_kernel<7, true>,
                                                count_lines_kernel<8, true>};
-    line_kernels[family]<<<(unsigned)blocks, 32 * kLineWarps, 0, stream>>>(p);
+    using ShiftKernel = void (*)(CountParams, int);
+    static const ShiftKernel shift_kernels[5] = {count_shift_kernel<4, false>, count_shift_kernel<5, false>,
+                                                 count_shift_kernel<6, true>, count_shift_kernel<7, true>,
+                                                 count_shift_kernel<8, true>};
+    if (shifted)
+      shift_kernels[family]<<<(unsigned)blocks, 32 * kLineWarps, 0, stream>>>(p, (int)c->max_shift);
+    else
+      line_kernels[family]<<<(unsigned)blocks, 32 * kLineWarps, 0, stream>>>(p);
     SGC_CUDA_TRY(cudaGetLastError());
     if (lines_only) {
       c->last.grid = (uint32_t)blocks;
@@ -1151,6 +1341,7 @@ int plan_skew(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const ui
 int count_batch(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const uint32_t* d_off, uint32_t off_base,
                 uint32_t stride, uint32_t read_len, uint64_t n_reads, int32_t* d_assign, cudaStream_t stream) {
   uint64_t counted = 0;
+  c->submitted = true;
   if (c->auto_skew && !c->skew_planned && !d_assign && n_reads >= kSkewMinBatch && !c->lib->opaque) {
     int rc = plan_skew(c, d_lines, n_bytes, d_off, off_base, stride, read_len, n_reads, stream, &counted);
     if (rc) return rc;
@@ -1205,6 +1396,22 @@ int sgc_span_geometry(uint32_t k, uint32_t read_len, int is_reverse, uint32_t of
   *span_start = (uint32_t)g.win_src - before;
   *span_len = before + k + after;
   *span_offset = is_reverse ? after : before;  // Offset index of the span records
+  return SGC_OK;
+}
+
+int sgc_span_geometry_shift(uint32_t k, uint32_t read_len, int is_reverse, uint32_t offset, uint32_t max_shift,
+                            uint32_t* span_start, uint32_t* span_len, uint32_t* span_offset) {
+  if (max_shift < 1 || max_shift > (uint32_t)kMaxShift) return set_error(SGC_ERR_INVALID_ARG, "max_shift must be 1..16");
+  if (max_shift == 1)
+    return sgc_span_geometry(k, read_len, is_reverse, offset, 1, span_start, span_len, span_offset);
+  if (!span_start || !span_len || !span_offset) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
+  // [lo, hi) in the coordinates of the trimmed read: every window offset + d, |d| <= S, that fits
+  const int64_t o = offset, lo = std::max<int64_t>(0, o - max_shift),
+                hi = std::min<int64_t>(read_len, o + (int64_t)k + max_shift);
+  if (k == 0 || hi - lo < (int64_t)k) return set_error(SGC_ERR_INVALID_ARG, "no shifted window fits the read");
+  *span_start = (uint32_t)(is_reverse ? read_len - hi : lo);
+  *span_len = (uint32_t)(hi - lo);
+  *span_offset = (uint32_t)(o - lo);
   return SGC_OK;
 }
 
@@ -1389,6 +1596,18 @@ int sgc_counter_set_replicas(sgc_counter* c, uint32_t replicas) {
   c->auto_skew = false;
   for (int j = 0; j < kHotGuides; ++j) c->hot[j] = -2;
   return alloc_replicas(c, replicas);
+}
+
+int sgc_counter_set_max_shift(sgc_counter* c, uint32_t max_shift) {
+  if (!c) return set_error(SGC_ERR_INVALID_ARG, "counter is NULL");
+  if (max_shift < 1 || max_shift > (uint32_t)kMaxShift) return set_error(SGC_ERR_INVALID_ARG, "max_shift must be 1..16");
+  if (c->submitted) return set_error(SGC_ERR_INVALID_ARG, "max_shift must be set before the counter's first submit");
+  if (max_shift >= 2 && !c->recursion)
+    return set_error(SGC_ERR_INVALID_ARG, "max_shift >= 2 needs position recursion");
+  if (max_shift >= 2 && c->lib->opaque)
+    return set_error(SGC_ERR_INVALID_ARG, "max_shift >= 2 needs a library of guides of at most 30 bases over A,C,G,T");
+  c->max_shift = max_shift;
+  return SGC_OK;
 }
 
 int sgc_counter_sync(sgc_counter* c) {

@@ -71,6 +71,8 @@ struct sgc_counter {
   uint32_t offset = 0;
   int recursion = 1;
   int rc_mode = SGC_RC_BITTRICK;
+  uint32_t max_shift = 1;  // sgc_counter_set_max_shift: >= 2 takes the shift kernel
+  bool submitted = false;  // a batch has been submitted (max_shift is fixed from then on)
   cudaStream_t stream = nullptr;
   bool own_stream = false;
   unsigned long long* d_state = nullptr;

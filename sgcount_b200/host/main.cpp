@@ -76,6 +76,8 @@ struct Args {
   bool whole_lines = false;  // never frame span records
   bool host_inflate = false; // never inflate on the device
   int rc_mode = SGC_RC_BITTRICK;
+  unsigned long max_shift = 1;  // search offset +- max_shift for staggered reads
+  bool have_max_shift = false;
 };
 
 const char* kUsage =
@@ -101,6 +103,7 @@ const char* kUsage =
     "      --rc-keep-n                        Reverse complement keeps N (default: the fxread bit trick, N -> J)\n"
     "      --whole-lines                      Copy whole sequence lines to the device (default: for fixed-length reads, only the guide window and one byte either side)\n"
     "      --host-inflate                     Inflate and frame records on the host even for BGZF, single-member or multi-member gzip input, and read and frame uncompressed FASTQ there too (default: BGZF files of FASTQ, gzip files of FASTQ that are one member, and uncompressed FASTQ files are inflated or copied, framed and counted on the device; so are multi-member gzip files large enough and with too few members or ingest threads for the host to decode them faster side by side)\n"
+    "      --max-shift <N>                    Search for the guide up to N bases either side of the offset, for staggered reads [default: 1, the reference's +/-1 position recursion]\n"
     "      --timing                           Print a JSON line with the phase times to stderr\n"
     "  -h, --help                             Print help\n";
 
@@ -144,6 +147,7 @@ Args parse_args(int argc, char** argv) {
     else if (f == "--ingest-threads") a.ingest_threads = (unsigned)parse_uint(f, value());
     else if (f == "--rc-keep-n") a.rc_mode = SGC_RC_KEEP_N;
     else if (f == "--timing") a.timing = true;
+    else if (f == "--max-shift") { a.max_shift = parse_uint(f, value()); a.have_max_shift = true; }
     else if (f == "--whole-lines") a.whole_lines = true;
     else if (f == "--host-inflate") a.host_inflate = true;
     else if (f == "-h" || f == "--help") { fputs(kUsage, stdout); exit(0); }
@@ -153,7 +157,27 @@ Args parse_args(int argc, char** argv) {
   if (a.input_paths.empty()) fail("the following required arguments were not provided:\n  --input-paths <INPUT_PATHS>...");
   if (a.threads == 0) a.threads = 1;
   if (a.gpus < 1) a.gpus = 1;
+  if (a.max_shift < 1 || a.max_shift > 16) fail("invalid value '%lu' for '--max-shift': must be 1..16", a.max_shift);
+  if (a.max_shift >= 2 && a.no_position_recursion)
+    fail("'--max-shift %lu' searches positions around the offset and cannot be used with '--no-position-recursion'", a.max_shift);
   return a;
+}
+
+// --max-shift, set once before any counting starts: every counter the program creates searches
+// offset +- g_max_shift, and every span of a read it frames holds those windows
+uint32_t g_max_shift = 1;
+
+int create_counter(const sgc_library* lib, int is_reverse, uint32_t offset, bool recursion, int rc_mode, sgc_counter** out) {
+  int rc = sgc_counter_create(lib, is_reverse, offset, recursion, rc_mode, nullptr, nullptr, out);
+  if (rc == SGC_OK && g_max_shift != 1) rc = sgc_counter_set_max_shift(*out, g_max_shift);
+  return rc;
+}
+
+int span_geometry(uint32_t k, uint32_t read_len, bool is_reverse, uint32_t offset, bool recursion, uint32_t* span_start,
+                  uint32_t* span_len, uint32_t* span_offset) {
+  if (g_max_shift != 1)
+    return sgc_span_geometry_shift(k, read_len, is_reverse, offset, g_max_shift, span_start, span_len, span_offset);
+  return sgc_span_geometry(k, read_len, is_reverse, offset, recursion, span_start, span_len, span_offset);
 }
 
 bool exists(const std::string& p) {
@@ -604,7 +628,7 @@ bool count_member_on_device(const std::vector<const sgc_library*>& libs, const s
   g.c.assign(lanes, nullptr);
   g.s.assign(lanes, nullptr);
   for (size_t d = 0; d < lanes; ++d) {
-    check(sgc_counter_create(libs[d % libs.size()], offset.reverse, span_offset, recursion, rc_mode, nullptr, nullptr, &g.c[d]));
+    check(create_counter(libs[d % libs.size()], offset.reverse, span_offset, recursion, rc_mode, &g.c[d]));
     check(sgc_fastq_stream_create(g.c[d], variable ? 0 : read_len, span_start, span_len, &g.s[d]));
   }
   const auto t1 = std::chrono::steady_clock::now();
@@ -656,8 +680,8 @@ bool count_text_on_device(const std::vector<const sgc_library*>& libs, const std
                           uint32_t k, const std::string& path, OffsetValue offset, uint32_t read_len, bool variable, bool recursion,
                           int rc_mode, SampleResult& r, std::string& why_not) {
   uint32_t span_start = 0, span_len = 0, span_offset = offset.index;
-  if (!variable && sgc_span_geometry(k, read_len, offset.reverse, offset.index, recursion, &span_start, &span_len,
-                                     &span_offset) != SGC_OK) {
+  if (!variable && span_geometry(k, read_len, offset.reverse, offset.index, recursion, &span_start, &span_len,
+                                 &span_offset) != SGC_OK) {
     why_not = "the guide window does not fit the reads";
     return false;
   }
@@ -714,7 +738,7 @@ bool count_text_on_device(const std::vector<const sgc_library*>& libs, const std
   } g;
   g.lanes.resize(n_lanes);
   for (size_t d = 0; d < n_lanes; ++d) {
-    check(sgc_counter_create(libs[d], offset.reverse, span_offset, recursion, rc_mode, nullptr, nullptr, &g.lanes[d].c));
+    check(create_counter(libs[d], offset.reverse, span_offset, recursion, rc_mode, &g.lanes[d].c));
     check(sgc_fastq_stream_create(g.lanes[d].c, variable ? 0 : read_len, span_start, span_len, &g.lanes[d].stream));
   }
   const auto t_created = std::chrono::steady_clock::now();
@@ -781,8 +805,8 @@ bool count_sample_on_device(const std::vector<const sgc_library*>& libs, const s
                             uint32_t k, const std::string& path, OffsetValue offset, uint32_t read_len, bool variable, bool recursion,
                             int rc_mode, bool member_ok, size_t members, unsigned ingest_threads, SampleResult& r, std::string& why_not) {
   uint32_t span_start = 0, span_len = 0, span_offset = offset.index;
-  if (!variable && sgc_span_geometry(k, read_len, offset.reverse, offset.index, recursion, &span_start, &span_len,
-                                     &span_offset) != SGC_OK) {
+  if (!variable && span_geometry(k, read_len, offset.reverse, offset.index, recursion, &span_start, &span_len,
+                                 &span_offset) != SGC_OK) {
     why_not = "the guide window does not fit the reads";
     return false;
   }
@@ -871,7 +895,7 @@ bool count_sample_on_device(const std::vector<const sgc_library*>& libs, const s
   } g;
   g.lanes.resize(n_lanes);
   for (size_t d = 0; d < n_lanes; ++d) {
-    check(sgc_counter_create(libs[d % n_dev], offset.reverse, span_offset, recursion, rc_mode, nullptr, nullptr, &g.lanes[d].c));
+    check(create_counter(libs[d % n_dev], offset.reverse, span_offset, recursion, rc_mode, &g.lanes[d].c));
     check(sgc_fastq_stream_create(g.lanes[d].c, variable ? 0 : read_len, span_start, span_len, &g.lanes[d].stream));
   }
   const auto t_created = std::chrono::steady_clock::now();
@@ -977,8 +1001,8 @@ SampleResult count_sample(const std::vector<const sgc_library*>& libs, uint32_t 
   g.lanes.resize(libs.size());
   sgh::SpanSpec spec;
   uint32_t span_offset = 0;
-  if (use_spans && sgc_span_geometry(k, read_len, offset.reverse, offset.index, recursion, &spec.start, &spec.len,
-                                     &span_offset) == SGC_OK) {
+  if (use_spans && span_geometry(k, read_len, offset.reverse, offset.index, recursion, &spec.start, &spec.len,
+                                 &span_offset) == SGC_OK) {
     spec.read_len = read_len;
     spec.stride = (spec.len + 7u) & ~7u;
     use_spans = spec.stride < read_len + 1;  // only if it sends fewer bytes
@@ -992,8 +1016,7 @@ SampleResult count_sample(const std::vector<const sgc_library*>& libs, uint32_t 
   auto ready = [&](size_t d, int kind) -> Channel& {  // counter and pinned buffers on first use
     Channel& ch = g.lanes[d].ch[kind];
     if (ch.c) return ch;
-    check(sgc_counter_create(libs[d], offset.reverse, kind ? span_offset : offset.index, recursion, rc_mode, nullptr,
-                             nullptr, &ch.c));
+    check(create_counter(libs[d], offset.reverse, kind ? span_offset : offset.index, recursion, rc_mode, &ch.c));
     for (auto& b : ch.b) {
       void* p = nullptr;
       check(sgc_host_alloc(&p, cap));
@@ -1068,6 +1091,7 @@ SampleResult count_sample(const std::vector<const sgc_library*>& libs, uint32_t 
 int main(int argc, char** argv) {
   try {
     Args args = parse_args(argc, argv);
+    g_max_shift = (uint32_t)args.max_shift;
     const auto t_start = std::chrono::steady_clock::now();
     auto seconds_since_start = [&] { return std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count(); };
     double t_inputs = 0, t_tables = 0, t_offsets = 0;
@@ -1187,6 +1211,12 @@ int main(int argc, char** argv) {
       for (auto& t : builders) t.join();
       for (const auto& e : errors)
         if (!e.empty()) fail("%s", e.c_str());
+    }
+    if (g_max_shift >= 2) {
+      sgc_library_info info{};
+      check(sgc_library_get_info(libs[0], &info));
+      if (info.opaque)
+        fail("'--max-shift %u' needs a library of guides of at most %u bases over A, C, G and T", g_max_shift, SGC_MAX_K_PACKED);
     }
 
     // the budget of the device ingest on every device: its free memory now, less an eighth for the
@@ -1351,10 +1381,11 @@ int main(int argc, char** argv) {
               "\"device_blocks\": %llu, \"device_text_bytes\": %llu, \"device_phases_s\": [%.4f, %.4f, %.4f, %.4f], \"host_ingest_because\": \"%s\", \"members_adopted\": %llu, \"members_reframed\": %llu, \"wait_inflate_s\": %.6f, "
               "\"copy_to_pinned_s\": %.6f, \"submit_sync_s\": %.6f, \"read_inputs_s\": %.3f, "
               "\"device_tables_s\": %.3f, \"offsets_s\": %.3f, \"member_pieces\": %llu, \"member_chain\": %llu, \"member_absorbed\": %llu, \"gzip_members\": %llu, "
-              "\"member_lanes\": %u, \"device_samples_in_flight\": %u}\n",
+              "\"member_lanes\": %u, \"device_samples_in_flight\": %u%s}\n",
               count_s, reads, n_samples, workers, ingest_threads, gpus, max_shards, span_reads, device_samples, device_blocks, device_text_bytes,
               dev_index_s, dev_create_s, dev_waves_s, dev_finish_s, host_because.c_str(), adopted, reframed, wait_s, copy_s, submit_s, t_inputs,
-              t_tables - t_inputs, t_offsets - t_tables, pieces, chain, absorbed, gzip_member_count, member_lanes, in_flight);
+              t_tables - t_inputs, t_offsets - t_tables, pieces, chain, absorbed, gzip_member_count, member_lanes, in_flight,
+              args.have_max_shift ? (", \"max_shift\": " + std::to_string(g_max_shift)).c_str() : "");
     }
 
     // write_results (results.rs:71-99).  Counts are keyed by alias (counter.rs:232-235):
