@@ -204,6 +204,38 @@ int sgc_counter_set_replicas(sgc_counter*, uint32_t replicas);
  * (sgc_library_info.opaque).  Span records for such a counter: sgc_span_geometry_shift. */
 int sgc_counter_set_max_shift(sgc_counter*, uint32_t max_shift);
 
+/* Unmatched report: the most frequent guide windows of the reads a counter leaves unmatched (counted in
+ * total_reads, not in matched_reads), to tell a wrong offset or orientation, staggered primers, the wrong
+ * library, adapter dimers or PhiX apart.  A read's window is trimmed[o, o + k): the read, or in Reverse its
+ * reverse complement under the counter's rc_mode, at the counter's Offset index o, whatever the recursion
+ * and max_shift.  Every unmatched read falls into one class: short_reads (o + k > read length: no window),
+ * non_acgt (a window byte outside A, C, G, T, N included), or its window, tallied in library orientation.
+ * So unmatched = short_reads + non_acgt + overflow + the sum of the window counts.
+ * Bounded memory: the report holds at most `capacity` distinct windows.  A window that finds no slot
+ * (the table is full around it) is added to overflow, and slots are never freed, so a window once refused
+ * stays refused: every window the report holds has its exact count, and every other window's count is at
+ * most overflow.  With overflow == 0 the report is exact.
+ * The counter then counts through the line (or shift) kernel and, after each launch of at most 2^24 reads,
+ * tallies the launch's unmatched reads on its stream.  Counts, totals and the skew plan do not change.
+ * Call it before the counter's first submit.  SGC_ERR_INVALID_ARG: a byte-keyed library
+ * (sgc_library_info.opaque), a counter that has counted, capacity 0 or above 2^26.  sgc_counter_reset
+ * clears the report; sgc_reduce_counts does not merge reports (merge them on the host by window). */
+int sgc_counter_set_unmatched_report(sgc_counter*, uint64_t capacity);
+typedef struct sgc_unmatched_info {
+  uint64_t unmatched;   /* reads counted and not matched                                  */
+  uint64_t short_reads; /* of them, reads with no window at the offset                     */
+  uint64_t non_acgt;    /* of them, windows with a byte outside A, C, G, T                 */
+  uint64_t overflow;    /* of them, A/C/G/T windows refused for want of a slot             */
+  uint64_t distinct;    /* windows the report holds                                        */
+} sgc_unmatched_info;
+/* Waits for the counter, then writes the first max_windows windows of the report in report order (count
+ * descending, then window bytes ascending): windows = max_windows x k ASCII bytes, counts = max_windows
+ * words (both may be NULL when max_windows == 0); *n_windows = how many were written.  info is optional. */
+int sgc_counter_unmatched(sgc_counter*, uint64_t max_windows, uint8_t* windows, uint64_t* counts, uint64_t* n_windows,
+                          sgc_unmatched_info* info);
+/* Device memory one counter's report takes (its table and its per-launch assignment scratch of 64 MiB). */
+int sgc_unmatched_report_bytes(uint64_t capacity, uint64_t* bytes);
+
 int sgc_counter_sync(sgc_counter*);
 /* Wait until all but the last `keep_in_flight` sgc_counter_submit calls have had their host
  * buffers copied to the device (those buffers may be refilled), without waiting for the kernels
@@ -224,7 +256,7 @@ int sgc_counter_state(sgc_counter*, uint64_t** d_state, uint64_t* n_words);
  * its per-sample Counters at count.rs:136; a sample cut into read shards needs them summed):
  * state[root] = sum over i of state[i], i.e. counts, total_reads and matched_reads of the whole
  * sample land in shards[root]; the other shards' vectors are left unspecified (reset them before
- * reuse).  Shards that share a device are folded on that device first.  Across devices:
+ * reuse).  Unmatched reports (sgc_counter_set_unmatched_report) are not merged: each shard keeps its own.  Shards that share a device are folded on that device first.  Across devices:
  *   - with NCCL communicators for the device set in place (sgc_reduce_prepare was called, or an
  *     earlier reduce created them): ONE ncclReduce(ncclUint64, ncclSum) of n_guides + 2 words over
  *     NVLink, each rank's call enqueued on its counter's own stream (libnccl.so.2 is loaded on first

@@ -66,6 +66,16 @@ class LaunchInfo(C.Structure):
     ]
 
 
+class UnmatchedInfo(C.Structure):
+    _fields_ = [
+        ("unmatched", C.c_uint64),
+        ("short_reads", C.c_uint64),
+        ("non_acgt", C.c_uint64),
+        ("overflow", C.c_uint64),
+        ("distinct", C.c_uint64),
+    ]
+
+
 # every symbol include/sgcount_cuda.h declares: name -> (restype, argtypes)
 _vp, _u32, _u64, _int = C.c_void_p, C.c_uint32, C.c_uint64, C.c_int
 SIGNATURES = {
@@ -90,6 +100,9 @@ SIGNATURES = {
     "sgc_counter_submit_device": (_int, [_vp, _vp, _u64, _vp, _u32, _u32, _u64, _vp]),
     "sgc_counter_set_replicas": (_int, [_vp, _u32]),
     "sgc_counter_set_max_shift": (_int, [_vp, _u32]),
+    "sgc_counter_set_unmatched_report": (_int, [_vp, _u64]),
+    "sgc_counter_unmatched": (_int, [_vp, _u64, _vp, _vp, C.POINTER(_u64), C.POINTER(UnmatchedInfo)]),
+    "sgc_unmatched_report_bytes": (_int, [_u64, C.POINTER(_u64)]),
     "sgc_counter_sync": (_int, [_vp]),
     "sgc_counter_wait_copies": (_int, [_vp, _u32]),
     "sgc_reduce_counts": (_int, [C.POINTER(_vp), _int, _int]),

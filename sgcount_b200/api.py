@@ -285,11 +285,14 @@ def entropy_offset_group(library: Library, readers: Sequence[ReadBatch], subsamp
 
 class Counter:
     """counter.rs:17-252.  max_shift: 1 (default) is the reference's +-1 position recursion; 2..16
-    searches offset + 0, +1, -1, ..., +S, -S for staggered reads (sgc_counter_set_max_shift)."""
+    searches offset + 0, +1, -1, ..., +S, -S for staggered reads (sgc_counter_set_max_shift).
+    unmatched_capacity: keep a report of the windows of unmatched reads, at most that many distinct
+    windows (sgc_counter_set_unmatched_report; read it with unmatched())."""
 
     def __init__(self, library: Library, permuter: Optional[Permuter], offset: Offset,
                  position_recursion: bool = True, rc_mode: int = _cabi.RC_BITTRICK,
-                 stream: Optional[int] = None, d_state: Optional[int] = None, max_shift: int = 1):
+                 stream: Optional[int] = None, d_state: Optional[int] = None, max_shift: int = 1,
+                 unmatched_capacity: Optional[int] = None):
         self._library = library
         self._handle = permuter._handle if permuter is not None else library._exact
         self._ptr = C.c_void_p()
@@ -298,6 +301,8 @@ class Counter:
         self._result = None
         if max_shift != 1:
             self.set_max_shift(max_shift)
+        if unmatched_capacity is not None:
+            self.set_unmatched_report(unmatched_capacity)
 
     def __del__(self):
         try:
@@ -336,6 +341,27 @@ class Counter:
     def set_max_shift(self, max_shift: int) -> None:
         """sgc_counter_set_max_shift: 1..16, before the first submit"""
         check(_cabi.load().sgc_counter_set_max_shift(self._ptr, int(max_shift)))
+
+    def set_unmatched_report(self, capacity: int) -> None:
+        """sgc_counter_set_unmatched_report: before the first submit; at most `capacity` distinct windows"""
+        check(_cabi.load().sgc_counter_set_unmatched_report(self._ptr, int(capacity)))
+
+    def unmatched(self, max_windows: Optional[int] = None):
+        """The unmatched report: ([(window bytes, count)] by count descending then window ascending, the
+        first max_windows of them or all; {unmatched, short_reads, non_acgt, overflow, distinct})"""
+        lib = _cabi.load()
+        info = _cabi.UnmatchedInfo()
+        n = C.c_uint64()
+        if max_windows is None:
+            check(lib.sgc_counter_unmatched(self._ptr, 0, None, None, C.byref(n), C.byref(info)))
+            max_windows = int(info.distinct)
+        k = self._library.size()
+        windows = np.zeros(max(max_windows, 1) * k, dtype=np.uint8)
+        counts = np.zeros(max(max_windows, 1), dtype=np.uint64)
+        check(lib.sgc_counter_unmatched(self._ptr, int(max_windows), windows.ctypes.data, counts.ctypes.data, C.byref(n),
+                                        C.byref(info)))
+        rows = [(windows[i * k:(i + 1) * k].tobytes(), int(counts[i])) for i in range(int(n.value))]
+        return rows, {name: int(getattr(info, name)) for name, _ in _cabi.UnmatchedInfo._fields_}
 
     def wait_copies(self, keep_in_flight: int = 0) -> None:
         check(_cabi.load().sgc_counter_wait_copies(self._ptr, int(keep_in_flight)))
@@ -503,6 +529,13 @@ def fastq_stream_scratch_bound(bgzf: bool, gz_bytes: int, text_bytes: int, read_
     out = C.c_uint64()
     check(_cabi.load().sgc_fastq_stream_scratch_bound(1 if bgzf else 0, int(gz_bytes), int(text_bytes), int(read_len),
                                                       int(span_len), C.byref(out)))
+    return int(out.value)
+
+
+def unmatched_report_bytes(capacity: int) -> int:
+    """device memory of one counter's unmatched report of `capacity` windows (sgc_unmatched_report_bytes)"""
+    out = C.c_uint64()
+    check(_cabi.load().sgc_unmatched_report_bytes(int(capacity), C.byref(out)))
     return int(out.value)
 
 

@@ -22,6 +22,9 @@
 //                          global memory with 64-bit loads, same window arithmetic and tables.
 //   count_shift_kernel   : staggered reads (max_shift S >= 2): the line kernel's layouts, every
 //                          position offset + d, |d| <= S, through the parked queue.
+//   unmatched_collect_kernel : the unmatched report (sgc_counter_set_unmatched_report): after a line or
+//                          shift launch, the windows at the offset of the reads it left unmatched,
+//                          tallied in an open-addressing table.
 // Per-guide counts are 64-bit atomics in the L2-resident state vector; matched reads are
 // accumulated in registers and flushed once per warp.
 #include <algorithm>
@@ -721,6 +724,146 @@ __global__ void __launch_bounds__(kLineWarps * 32) count_shift_kernel(CountParam
   flush_matched<4>(p, matched, hot);
 }
 
+// ------------------------------------------------------------------------------------------
+// unmatched report (sgc_counter_set_unmatched_report): after a count launch of the line or shift
+// kernel, the reads it left unmatched (assignment -1) are tallied by their window at the offset,
+// trimmed[o, o + k) in library orientation, into an open-addressing table of {key, count} slots.
+// A key is the window packed 2-bit, first base in the highest bits (A 0, C 1, G 2, T 3), so keys of
+// one k sort like the window bytes; the empty key is all ones (no window has bits 60..63 set).
+// A slot is claimed once and never freed: a window that is in the table has every one of its reads
+// counted there, and one that found its probe range full is refused for good (tally[3], overflow).
+// ------------------------------------------------------------------------------------------
+constexpr unsigned long long kEmptyKey = ~0ull;
+constexpr int kUnmatchedProbes = 128;  // linear probes before a window is refused
+constexpr int kUnmatchedWarps = 8;
+enum { kTallyUnmatched, kTallyShort, kTallyNonAcgt, kTallyOverflow, kTallyCompacted, kTallyWords };
+
+__global__ void unmatched_clear_kernel(ulonglong2* __restrict__ table, uint64_t capacity) {
+  for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < capacity; i += (uint64_t)gridDim.x * blockDim.x)
+    table[i] = make_ulonglong2(kEmptyKey, 0ull);
+}
+
+// One warp per 32 consecutive reads of the launch p (the read layouts of the line kernel); the
+// assignment of read i of the launch is p.assign_out[p.first_read + i].
+__global__ void __launch_bounds__(kUnmatchedWarps * 32)
+    unmatched_collect_kernel(CountParams p, ulonglong2* __restrict__ table, uint64_t capacity,
+                             unsigned long long* __restrict__ tally) {
+  const int lane = threadIdx.x & 31;
+  const uint32_t gwarp = blockIdx.x * kUnmatchedWarps + (threadIdx.x >> 5), gwarps = gridDim.x * kUnmatchedWarps;
+  const int k = (int)p.lib.k, o = p.offset;
+  const uint64_t line_policy = l2_evict_first_policy();
+  const int probes = capacity < (uint64_t)kUnmatchedProbes ? (int)capacity : kUnmatchedProbes;
+  uint32_t n_unmatched = 0, n_short = 0, n_bad = 0, n_over = 0;
+  const uint64_t n_tiles = (p.n_reads + 31) / 32;
+  for (uint64_t t = gwarp; t < n_tiles; t += gwarps) {
+    const uint64_t i = t * 32 + lane;
+    bool have_key = false;
+    unsigned long long key = 0;
+    if (i < p.n_reads && p.assign_out[p.first_read + i] < 0) {
+      ++n_unmatched;
+      const uint64_t r = p.first_read + i;
+      uint64_t start;
+      int n;
+      if (p.line_end) {
+        start = p.line_off[r];
+        n = (int)(p.line_end[r] - p.line_off[r]);
+      } else if (p.line_off) {
+        const uint32_t a = p.line_off[r], b = p.line_off[r + 1];
+        start = a - p.off_base;
+        n = (int)(b - a) - 1;
+      } else {
+        start = r * p.stride;
+        n = (int)p.read_len;
+      }
+      if (o + k > n) {
+        ++n_short;  // the Centered trim fails: no window
+      } else {
+        // the stored window: [o, o + k) forward, [n - o - k, n - o) reversed and complemented
+        const uint8_t* sb = p.lines + start + (p.reverse ? n - o - k : o);
+        const uint64_t* a8 = reinterpret_cast<const uint64_t*>((uintptr_t)sb & ~(uintptr_t)7);
+        const uint32_t sh = (uint32_t)((uintptr_t)sb & 7u);
+        const int need = ((int)sh + k + 7) >> 3;
+        uint64_t R[5];
+#pragma unroll
+        for (int j = 0; j < 5; ++j)
+          R[j] = j < need && reinterpret_cast<const uint8_t*>(a8 + j) < p.lines_end ? ldg_stream_u64(a8 + j, line_policy) : 0ull;
+        uint64_t W[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) W[j] = sh ? (R[j] >> (8 * sh)) | (R[j + 1] << (64 - 8 * sh)) : R[j];
+        // stored bytes in order, codes A 0 C 1 G 2 T 3; complement and reversal come after (a byte
+        // outside A, C, G, T stays outside under either rc_mode, and A, C, G, T complement alike)
+        bool bad = false;
+#pragma unroll
+        for (int j = 0; j < (int)kMaxK; ++j) {
+          if (j < k) {
+            const uint32_t b = (uint32_t)(W[j >> 3] >> (8 * (j & 7))) & 0xFFu;
+            bad |= b != 'A' && b != 'C' && b != 'G' && b != 'T';
+            key = (key << 2) | (unsigned long long)((b == 'C') + 2 * (b == 'G') + 3 * (b == 'T'));
+          }
+        }
+        if (bad) {
+          ++n_bad;
+        } else {
+          if (p.reverse) {  // reverse the 2-bit groups, complement every base
+            key = __brevll(key);
+            key = ((key >> 1) & 0x5555555555555555ull) | ((key & 0x5555555555555555ull) << 1);
+            key = (key >> (64 - 2 * k)) ^ ((1ull << (2 * k)) - 1);
+          }
+          have_key = true;
+        }
+      }
+    }
+    // one table update per distinct window of the warp: a window that holds most of the reads
+    // costs one atomic per warp, not one per read
+    const uint32_t want = __ballot_sync(0xffffffffu, have_key);
+    const uint32_t group = have_key ? __match_any_sync(want, key) : 0u;
+    if (have_key && lane == __ffs((int)group) - 1) {
+      const unsigned long long cnt = (unsigned long long)__popc(group);
+      uint64_t slot = __umul64hi(key * 0x9E3779B97F4A7C15ull, capacity);
+      bool done = false;
+      for (int q = 0; q < probes && !done; ++q) {
+        unsigned long long* kp = &table[slot].x;
+        unsigned long long cur = __ldcg(kp);
+        if (cur == kEmptyKey) cur = atomicCAS(kp, kEmptyKey, key);
+        if (cur == kEmptyKey || cur == key) {
+          atomicAdd(&table[slot].y, cnt);
+          done = true;
+        }
+        slot = slot + 1 == capacity ? 0 : slot + 1;
+      }
+      if (!done) n_over += (uint32_t)cnt;
+    }
+  }
+  n_unmatched = __reduce_add_sync(0xffffffffu, n_unmatched);
+  n_short = __reduce_add_sync(0xffffffffu, n_short);
+  n_bad = __reduce_add_sync(0xffffffffu, n_bad);
+  n_over = __reduce_add_sync(0xffffffffu, n_over);
+  if (lane == 0) {
+    if (n_unmatched) atomicAdd(tally + kTallyUnmatched, (unsigned long long)n_unmatched);
+    if (n_short) atomicAdd(tally + kTallyShort, (unsigned long long)n_short);
+    if (n_bad) atomicAdd(tally + kTallyNonAcgt, (unsigned long long)n_bad);
+    if (n_over) atomicAdd(tally + kTallyOverflow, (unsigned long long)n_over);
+  }
+}
+
+// The occupied slots of table[0, n) to out[0, ...), in any order; tally[kTallyCompacted] counts them
+// (zero before the launch).
+__global__ void unmatched_compact_kernel(const ulonglong2* __restrict__ table, uint64_t n, ulonglong2* __restrict__ out,
+                                         unsigned long long* __restrict__ tally) {
+  const int lane = threadIdx.x & 31;
+  for (uint64_t base = (blockIdx.x * (uint64_t)blockDim.x + threadIdx.x) & ~31ull; base < n;
+       base += (uint64_t)gridDim.x * blockDim.x) {
+    const uint64_t i = base + lane;
+    const ulonglong2 s = i < n ? table[i] : make_ulonglong2(kEmptyKey, 0ull);
+    const bool full = s.x != kEmptyKey;
+    const uint32_t m = __ballot_sync(0xffffffffu, full);
+    unsigned long long at = 0;
+    if (lane == 0 && m) at = atomicAdd(tally + kTallyCompacted, (unsigned long long)__popc(m));
+    at = __shfl_sync(0xffffffffu, at, 0);
+    if (full) out[at + __popc(m & ((1u << lane) - 1))] = s;
+  }
+}
+
 // NW = words that hold the k window bytes: 4 (k <= 16, the number of words in use is read from the
 // geometry), or exactly ceil(k / 4) = 5 (k = 17..20, the common guide lengths), 6, 7 or 8.
 template <int NW, bool WIDE, int MODE>
@@ -1052,6 +1195,8 @@ constexpr size_t kChunkBytes = 64ull << 20;
 constexpr uint64_t kChunkAlignReads = 256;  // chunk starts stay 16-byte aligned for any stride
 constexpr uint64_t kSkewSampleReads = 65536;   // reads of the first batch the skew plan looks at
 constexpr uint64_t kSkewMinBatch = 4 * kSkewSampleReads;  // smaller first batches are not worth a plan
+constexpr uint64_t kUnmatchedLaunchReads = 1ull << 24;    // reads per launch with the unmatched report (its scratch)
+constexpr uint64_t kUnmatchedMaxCapacity = 1ull << 26;
 
 // Tuning switches (SGC_DEBUG, SGC_WARPS, SGC_CTAS, SGC_STAGES, SGC_CARVEOUT, SGC_REPLICAS) exist only
 // in the tuning build (make tuning: -DSGC_TUNING -> libsgcount_cuda_tuning.so); the production
@@ -1193,7 +1338,9 @@ int launch_count(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const
   // launch, and a Centered window that fits (otherwise every read fails its first trim)
   const uint32_t tile_bytes = kWarpReads * stride;
   const uint32_t stage_bytes = (tile_bytes + 48 + 15) & ~15u;  // +48: span words may run past the tile
-  const bool stageable = !shifted && d_off == nullptr && ((uintptr_t)d_lines & 15u) == 0 && stride >= read_len &&
+  // a counter with the unmatched report counts through the line or shift kernel, which write assignments
+  const bool report = c->um_capacity != 0;
+  const bool stageable = !shifted && !report && d_off == nullptr && ((uintptr_t)d_lines & 15u) == 0 && stride >= read_len &&
                          (uint64_t)c->offset + c->lib->k <= read_len;
   // kernel family by the words that hold the k window bytes: narrow keys 4 (k <= 16) or 5
   // (k = 17..20, the common guide lengths); wide keys 6 (k = 21..24), 7 (k = 25..28) or 8 (k = 29, 30)
@@ -1252,10 +1399,26 @@ int launch_count(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const
   uint64_t shift_launch_reads = 1ull << kShiftIdxBits;
   if (const long long cap = env_ll("SGC_MAX_LAUNCH_TILES", 0); cap > 0)
     shift_launch_reads = std::min<uint64_t>(shift_launch_reads, (uint64_t)cap * kWarpReads);
+  // with the unmatched report a launch's assignments go to the counter's scratch of kUnmatchedLaunchReads
+  uint64_t report_launch_reads = kUnmatchedLaunchReads;
+  if (const long long cap = env_ll("SGC_MAX_LAUNCH_TILES", 0); cap > 0)
+    report_launch_reads = std::min<uint64_t>(report_launch_reads, (uint64_t)cap * kWarpReads);
   if (shifted) c->last.kernel = 3;
   while (done < n_reads) {  // what the streaming kernel did not take; at most 2^27 reads per launch
     p.first_read = done;
-    p.n_reads = std::min<uint64_t>(n_reads - done, shifted ? shift_launch_reads : 1ull << kLineIdxBits);
+    p.n_reads = std::min<uint64_t>(n_reads - done, report ? report_launch_reads
+                                                          : (shifted ? shift_launch_reads : 1ull << kLineIdxBits));
+    CountParams q = p;
+    if (report && !d_assign) {  // the launch's reads start at index 0 of the scratch
+      q.first_read = 0;
+      if (q.line_off) {
+        q.line_off += done;
+        if (q.line_end) q.line_end += done;
+      } else {
+        q.lines += done * stride;
+      }
+      q.assign_out = c->d_um_assign;
+    }
     uint64_t blocks = (p.n_reads + 32 * kLineWarps - 1) / (32 * kLineWarps);
     const uint64_t cap = (uint64_t)c->lib->sm_count * 8;
     if (blocks > cap) blocks = cap;
@@ -1268,10 +1431,18 @@ int launch_count(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const
                                                  count_shift_kernel<6, true>, count_shift_kernel<7, true>,
                                                  count_shift_kernel<8, true>};
     if (shifted)
-      shift_kernels[family]<<<(unsigned)blocks, 32 * kLineWarps, 0, stream>>>(p, (int)c->max_shift);
+      shift_kernels[family]<<<(unsigned)blocks, 32 * kLineWarps, 0, stream>>>(q, (int)c->max_shift);
     else
-      line_kernels[family]<<<(unsigned)blocks, 32 * kLineWarps, 0, stream>>>(p);
+      line_kernels[family]<<<(unsigned)blocks, 32 * kLineWarps, 0, stream>>>(q);
     SGC_CUDA_TRY(cudaGetLastError());
+    if (report) {
+      uint64_t collect_blocks = (q.n_reads + 32 * kUnmatchedWarps - 1) / (32 * kUnmatchedWarps);
+      collect_blocks = std::min<uint64_t>(collect_blocks, (uint64_t)c->lib->sm_count * 8);
+      unmatched_collect_kernel<<<(unsigned)collect_blocks, 32 * kUnmatchedWarps, 0, stream>>>(
+          q, static_cast<ulonglong2*>(c->d_um_table), c->um_capacity, c->d_um_tally);
+      SGC_CUDA_TRY(cudaGetLastError());
+      c->last.launches_total += 1;
+    }
     if (lines_only) {
       c->last.grid = (uint32_t)blocks;
       c->last.block = 32 * kLineWarps;
@@ -1364,6 +1535,15 @@ int sgc::count_gathered_lines(sgc_counter* c, const uint8_t* d_text, uint64_t n_
 }
 
 namespace {
+
+// an empty unmatched report
+int clear_unmatched(sgc_counter* c) {
+  const uint64_t blocks = std::min<uint64_t>((c->um_capacity + 255) / 256, (uint64_t)c->lib->sm_count * 8);
+  unmatched_clear_kernel<<<(unsigned)blocks, 256, 0, c->stream>>>(static_cast<ulonglong2*>(c->d_um_table), c->um_capacity);
+  SGC_CUDA_TRY(cudaGetLastError());
+  SGC_CUDA_TRY(cudaMemsetAsync(c->d_um_tally, 0, kTallyWords * sizeof(uint64_t), c->stream));
+  return SGC_OK;
+}
 
 int check_batch(const sgc_counter* c, const uint8_t* lines, uint64_t n_bytes, const uint32_t* line_off,
                 uint32_t stride, uint32_t read_len, uint64_t n_reads) {
@@ -1483,6 +1663,9 @@ void sgc_counter_destroy(sgc_counter* c) {
   for (cudaEvent_t e : c->free_tickets) cudaEventDestroy(e);
   cudaFree(c->d_rep);
   cudaFree(c->d_top);
+  cudaFree(c->d_um_table);
+  cudaFree(c->d_um_assign);
+  cudaFree(c->d_um_tally);
   if (c->own_state) cudaFree(c->d_state);
   if (c->own_stream) cudaStreamDestroy(c->stream);
   delete c;
@@ -1633,6 +1816,86 @@ int sgc_counter_reset(sgc_counter* c) {
   if (!c) return set_error(SGC_ERR_INVALID_ARG, "counter is NULL");
   DeviceGuard guard(c->lib->device);
   SGC_CUDA_TRY(cudaMemsetAsync(c->d_state, 0, ((size_t)c->lib->n + 2) * sizeof(uint64_t), c->stream));
+  return c->um_capacity ? clear_unmatched(c) : SGC_OK;
+}
+
+int sgc_unmatched_report_bytes(uint64_t capacity, uint64_t* bytes) {
+  if (!bytes) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
+  if (capacity == 0 || capacity > kUnmatchedMaxCapacity)
+    return set_error(SGC_ERR_INVALID_ARG, "the unmatched report's capacity must be 1..2^26 windows");
+  *bytes = capacity * sizeof(ulonglong2) + kUnmatchedLaunchReads * sizeof(int32_t) + kTallyWords * sizeof(uint64_t);
+  return SGC_OK;
+}
+
+int sgc_counter_set_unmatched_report(sgc_counter* c, uint64_t capacity) {
+  if (!c) return set_error(SGC_ERR_INVALID_ARG, "counter is NULL");
+  uint64_t bytes = 0;
+  if (int rc = sgc_unmatched_report_bytes(capacity, &bytes)) return rc;
+  if (c->submitted) return set_error(SGC_ERR_INVALID_ARG, "the unmatched report must be set before the counter's first submit");
+  if (c->lib->opaque)
+    return set_error(SGC_ERR_INVALID_ARG,
+                     "the unmatched report needs a library of guides of at most 30 bases over A,C,G,T");
+  DeviceGuard guard(c->lib->device);
+  if (capacity != c->um_capacity) {
+    SGC_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    cudaFree(c->d_um_table);
+    c->d_um_table = nullptr;
+    c->um_capacity = 0;
+    SGC_CUDA_TRY(cudaMalloc(&c->d_um_table, capacity * sizeof(ulonglong2)));
+    c->um_capacity = capacity;
+  }
+  if (!c->d_um_assign) SGC_CUDA_TRY(cudaMalloc(&c->d_um_assign, kUnmatchedLaunchReads * sizeof(int32_t)));
+  if (!c->d_um_tally) SGC_CUDA_TRY(cudaMalloc(&c->d_um_tally, kTallyWords * sizeof(uint64_t)));
+  return clear_unmatched(c);
+}
+
+int sgc_counter_unmatched(sgc_counter* c, uint64_t max_windows, uint8_t* windows, uint64_t* counts, uint64_t* n_windows,
+                          sgc_unmatched_info* info) {
+  if (!c) return set_error(SGC_ERR_INVALID_ARG, "counter is NULL");
+  if (!c->um_capacity) return set_error(SGC_ERR_INVALID_ARG, "the counter has no unmatched report");
+  if (max_windows && (!windows || !counts)) return set_error(SGC_ERR_INVALID_ARG, "NULL argument");
+  DeviceGuard guard(c->lib->device);
+  // the compaction goes through the assignment scratch, one piece of the table at a time
+  constexpr uint64_t kPiece = kUnmatchedLaunchReads * sizeof(int32_t) / sizeof(ulonglong2);
+  ulonglong2* buf = reinterpret_cast<ulonglong2*>(c->d_um_assign);
+  std::vector<ulonglong2> held;
+  unsigned long long tally[kTallyWords];
+  uint64_t distinct = 0;
+  for (uint64_t a = 0; a < c->um_capacity; a += kPiece) {
+    const uint64_t n = std::min(kPiece, c->um_capacity - a);
+    SGC_CUDA_TRY(cudaMemsetAsync(c->d_um_tally + kTallyCompacted, 0, sizeof(uint64_t), c->stream));
+    const uint64_t blocks = std::min<uint64_t>((n + 255) / 256, (uint64_t)c->lib->sm_count * 8);
+    unmatched_compact_kernel<<<(unsigned)blocks, 256, 0, c->stream>>>(static_cast<const ulonglong2*>(c->d_um_table) + a, n,
+                                                                       buf, c->d_um_tally);
+    SGC_CUDA_TRY(cudaGetLastError());
+    SGC_CUDA_TRY(cudaMemcpyAsync(tally, c->d_um_tally, sizeof tally, cudaMemcpyDeviceToHost, c->stream));
+    SGC_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    distinct += tally[kTallyCompacted];
+    if (!max_windows) continue;  // the tallies alone
+    const size_t at = held.size();
+    held.resize(at + tally[kTallyCompacted]);
+    SGC_CUDA_TRY(cudaMemcpyAsync(held.data() + at, buf, tally[kTallyCompacted] * sizeof(ulonglong2), cudaMemcpyDeviceToHost,
+                                 c->stream));
+  }
+  SGC_CUDA_TRY(cudaStreamSynchronize(c->stream));
+  // report order: count descending, then window ascending (the key order of one k)
+  const uint64_t n_out = std::min<uint64_t>(max_windows, held.size());
+  auto before = [](const ulonglong2& a, const ulonglong2& b) { return a.y != b.y ? a.y > b.y : a.x < b.x; };
+  std::nth_element(held.begin(), held.begin() + n_out, held.end(), before);
+  std::sort(held.begin(), held.begin() + n_out, before);
+  const uint32_t k = c->lib->k;
+  for (uint64_t i = 0; i < n_out; ++i) {
+    for (uint32_t j = 0; j < k; ++j) windows[i * k + j] = "ACGT"[(held[i].x >> (2 * (k - 1 - j))) & 3];
+    counts[i] = held[i].y;
+  }
+  if (n_windows) *n_windows = n_out;
+  if (info) {
+    info->unmatched = tally[kTallyUnmatched];
+    info->short_reads = tally[kTallyShort];
+    info->non_acgt = tally[kTallyNonAcgt];
+    info->overflow = tally[kTallyOverflow];
+    info->distinct = distinct;
+  }
   return SGC_OK;
 }
 

@@ -94,6 +94,12 @@ struct sgc_counter {
   std::deque<cudaEvent_t> copy_tickets;   // one per sgc_counter_submit call whose copies may still run
   std::vector<cudaEvent_t> free_tickets;
   sgc_launch_info last{};
+  // unmatched report (sgc_counter_set_unmatched_report; count.cu unmatched_collect_kernel): capacity
+  // {key, count} slots, the per-read assignments of one launch (also the compaction buffer), tallies
+  uint64_t um_capacity = 0;  // 0 = off
+  void* d_um_table = nullptr;
+  int32_t* d_um_assign = nullptr;
+  unsigned long long* d_um_tally = nullptr;
   // device-ingest streams that count into this counter (gzip.cu); released with it if still open
   std::vector<struct sgc_fastq_stream*> fastq_streams;
 };

@@ -78,6 +78,7 @@ struct Args {
   int rc_mode = SGC_RC_BITTRICK;
   unsigned long max_shift = 1;  // search offset +- max_shift for staggered reads
   bool have_max_shift = false;
+  std::string unmatched_report;  // TSV of the most frequent windows of unmatched reads, per sample
 };
 
 const char* kUsage =
@@ -104,6 +105,7 @@ const char* kUsage =
     "      --whole-lines                      Copy whole sequence lines to the device (default: for fixed-length reads, only the guide window and one byte either side)\n"
     "      --host-inflate                     Inflate and frame records on the host even for BGZF, single-member or multi-member gzip input, and read and frame uncompressed FASTQ there too (default: BGZF files of FASTQ, gzip files of FASTQ that are one member, and uncompressed FASTQ files are inflated or copied, framed and counted on the device; so are multi-member gzip files large enough and with too few members or ingest threads for the host to decode them faster side by side)\n"
     "      --max-shift <N>                    Search for the guide up to N bases either side of the offset, for staggered reads [default: 1, the reference's +/-1 position recursion]\n"
+    "      --unmatched-report <PATH>          Write the most frequent sequences at the guide position of the unmatched reads of every sample to a TSV\n"
     "      --timing                           Print a JSON line with the phase times to stderr\n"
     "  -h, --help                             Print help\n";
 
@@ -148,6 +150,7 @@ Args parse_args(int argc, char** argv) {
     else if (f == "--rc-keep-n") a.rc_mode = SGC_RC_KEEP_N;
     else if (f == "--timing") a.timing = true;
     else if (f == "--max-shift") { a.max_shift = parse_uint(f, value()); a.have_max_shift = true; }
+    else if (f == "--unmatched-report") a.unmatched_report = value();
     else if (f == "--whole-lines") a.whole_lines = true;
     else if (f == "--host-inflate") a.host_inflate = true;
     else if (f == "-h" || f == "--help") { fputs(kUsage, stdout); exit(0); }
@@ -167,9 +170,18 @@ Args parse_args(int argc, char** argv) {
 // offset +- g_max_shift, and every span of a read it frames holds those windows
 uint32_t g_max_shift = 1;
 
+// --unmatched-report: every counter keeps a report of this many distinct windows (0 = none), which takes
+// g_unmatched_bytes of device memory
+constexpr uint64_t kUnmatchedCapacity = 1ull << 22;
+uint64_t g_unmatched_capacity = 0, g_unmatched_bytes = 0;
+uint32_t g_unmatched_k = 0;  // the guide length: bytes of a window
+// rows of a sample in the report: its most frequent windows, then <other>, <non-ACGT> and <short>
+constexpr size_t kUnmatchedRows = 100;
+
 int create_counter(const sgc_library* lib, int is_reverse, uint32_t offset, bool recursion, int rc_mode, sgc_counter** out) {
   int rc = sgc_counter_create(lib, is_reverse, offset, recursion, rc_mode, nullptr, nullptr, out);
   if (rc == SGC_OK && g_max_shift != 1) rc = sgc_counter_set_max_shift(*out, g_max_shift);
+  if (rc == SGC_OK && g_unmatched_capacity) rc = sgc_counter_set_unmatched_report(*out, g_unmatched_capacity);
   return rc;
 }
 
@@ -178,6 +190,14 @@ int span_geometry(uint32_t k, uint32_t read_len, bool is_reverse, uint32_t offse
   if (g_max_shift != 1)
     return sgc_span_geometry_shift(k, read_len, is_reverse, offset, g_max_shift, span_start, span_len, span_offset);
   return sgc_span_geometry(k, read_len, is_reverse, offset, recursion, span_start, span_len, span_offset);
+}
+
+// the --timing key of the report, only when it was asked for
+std::string unmatched_s_key(bool off, double seconds) {
+  if (off) return "";
+  char buf[64];
+  snprintf(buf, sizeof buf, ", \"unmatched_s\": %.6f", seconds);
+  return buf;
 }
 
 bool exists(const std::string& p) {
@@ -422,7 +442,46 @@ struct SampleResult {
   uint64_t gzip_members = 0;                                          // how many (not BGZF), as the device confirmed them
   unsigned member_lanes = 0;                                          // streams that decoded them together
   std::string host_because;                 // why the device ingest was not used
+  // --unmatched-report: the reports of all the sample's counters merged by window (packed 2-bit, first
+  // base highest: A 0, C 1, G 2, T 3), and their tallies
+  std::unordered_map<uint64_t, uint64_t> unmatched;
+  uint64_t um_short = 0, um_non_acgt = 0, um_overflow = 0;
+  double unmatched_s = 0;
 };
+
+// Merges the unmatched reports of a sample's counters (span and whole-line counters, read shards, lanes)
+// into r; call it before the counters are destroyed.
+void collect_unmatched(const std::vector<sgc_counter*>& counters, SampleResult& r) {
+  if (!g_unmatched_capacity) return;
+  const auto t0 = std::chrono::steady_clock::now();
+  std::vector<uint8_t> windows;
+  std::vector<uint64_t> counts;
+  for (sgc_counter* c : counters) {
+    if (!c) continue;
+    sgc_unmatched_info info{};
+    uint64_t n = 0;
+    check(sgc_counter_unmatched(c, 0, nullptr, nullptr, &n, &info));
+    if (info.distinct) {
+      const size_t k = g_unmatched_k;
+      windows.resize(info.distinct * k);
+      counts.resize(info.distinct);
+      check(sgc_counter_unmatched(c, info.distinct, windows.data(), counts.data(), &n, &info));
+      r.unmatched.reserve(r.unmatched.size() + n);
+      for (uint64_t i = 0; i < n; ++i) {
+        uint64_t key = 0;
+        for (size_t j = 0; j < k; ++j) {
+          const uint8_t b = windows[i * k + j];
+          key = key << 2 | (uint64_t)((b == 'C') + 2 * (b == 'G') + 3 * (b == 'T'));
+        }
+        r.unmatched[key] += counts[i];
+      }
+    }
+    r.um_short += info.short_reads;
+    r.um_non_acgt += info.non_acgt;
+    r.um_overflow += info.overflow;
+  }
+  r.unmatched_s += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+}
 
 // ---- device ingest: BGZF blocks inflated, framed and counted on the GPU (sgc_fastq_stream_*) ----
 // A read-only mapping of a file.
@@ -615,6 +674,7 @@ bool count_member_on_device(const std::vector<const sgc_library*>& libs, const s
                             SampleResult& r, std::string& why_not) {
   uint64_t bound = 0;
   check(sgc_fastq_stream_scratch_bound(0, file.size, 0, variable ? 0 : read_len, span_len, &bound));
+  bound += g_unmatched_bytes;
   Reservation reserved(lane_bytes(budgets, lanes, bound));  // (declared before the streams: released after them)
   const auto t0 = std::chrono::steady_clock::now();
   struct Guard {
@@ -650,6 +710,7 @@ bool count_member_on_device(const std::vector<const sgc_library*>& libs, const s
   check(sgc_fastq_stream_member_stats(g.s[0], &r.member_pieces, &r.member_chain, &r.member_absorbed));
   check(sgc_fastq_stream_gzip_members(g.s[0], &r.gzip_members));
   if (lanes > 1) check(sgc_reduce_counts(g.c.data(), (int)lanes, 0));
+  collect_unmatched(g.c, r);
   r.counts.resize(n_guides);
   check(sgc_counter_finish(g.c[0], r.counts.data(), &r.total, &r.matched));
   const auto t3 = std::chrono::steady_clock::now();
@@ -719,6 +780,7 @@ bool count_text_on_device(const std::vector<const sgc_library*>& libs, const std
   const auto t_planned = std::chrono::steady_clock::now();
   uint64_t bound = 0;
   check(sgc_fastq_stream_text_scratch_bound(variable ? 0 : read_len, span_len, &bound));
+  bound += g_unmatched_bytes;
   Reservation reserved(lane_bytes(budgets, n_lanes, bound));  // (declared before the streams: released after them)
   struct Lane {
     sgc_counter* c = nullptr;
@@ -771,11 +833,10 @@ bool count_text_on_device(const std::vector<const sgc_library*>& libs, const std
     if (l.status != SGC_OK) fail("%s", l.error.c_str());
     n_records += l.records;
   }
-  if (n_lanes > 1) {
-    std::vector<sgc_counter*> shards;
-    for (auto& l : g.lanes) shards.push_back(l.c);
-    check(sgc_reduce_counts(shards.data(), (int)shards.size(), 0));
-  }
+  std::vector<sgc_counter*> shards;
+  for (auto& l : g.lanes) shards.push_back(l.c);
+  if (n_lanes > 1) check(sgc_reduce_counts(shards.data(), (int)shards.size(), 0));
+  collect_unmatched(shards, r);
   r.counts.resize(n_guides);
   check(sgc_counter_finish(g.lanes[0].c, r.counts.data(), &r.total, &r.matched));
   r.span_reads = variable ? 0 : n_records;
@@ -876,6 +937,7 @@ bool count_sample_on_device(const std::vector<const sgc_library*>& libs, const s
     wave_text_most = std::max(wave_text_most, text);
   }
   check(sgc_fastq_stream_scratch_bound(1, wave_gz, wave_text_most, variable ? 0 : read_len, span_len, &bound));
+  bound += g_unmatched_bytes;
   Reservation reserved(lane_bytes(budgets, n_lanes, bound));  // (declared before the streams: released after them)
   struct Lane {
     sgc_counter* c = nullptr;
@@ -942,11 +1004,10 @@ bool count_sample_on_device(const std::vector<const sgc_library*>& libs, const s
     why_not = "a wave failed";
     return false;
   }
-  if (n_lanes > 1) {
-    std::vector<sgc_counter*> shards;
-    for (auto& l : g.lanes) shards.push_back(l.c);
-    check(sgc_reduce_counts(shards.data(), (int)shards.size(), 0));
-  }
+  std::vector<sgc_counter*> shards;
+  for (auto& l : g.lanes) shards.push_back(l.c);
+  if (n_lanes > 1) check(sgc_reduce_counts(shards.data(), (int)shards.size(), 0));
+  collect_unmatched(shards, r);
   r.counts.resize(n_guides);
   check(sgc_counter_finish(g.lanes[0].c, r.counts.data(), &r.total, &r.matched));
   r.span_reads = variable ? 0 : n_records;
@@ -1080,6 +1141,12 @@ SampleResult count_sample(const std::vector<const sgc_library*>& libs, uint32_t 
   }
   r.shards = std::max(devices_used, 1u);
   if (shards.size() > 1) check(sgc_reduce_counts(shards.data(), (int)shards.size(), 0));
+  {
+    std::vector<sgc_counter*> all;
+    for (auto& l : g.lanes)
+      for (auto& ch : l.ch) all.push_back(ch.c);
+    collect_unmatched(all, r);
+  }
   r.counts.resize(n_guides);
   check(sgc_counter_finish(shards[0], r.counts.data(), &r.total, &r.matched));
   r.submit_s += since(t0);
@@ -1218,6 +1285,26 @@ int main(int argc, char** argv) {
       if (info.opaque)
         fail("'--max-shift %u' needs a library of guides of at most %u bases over A, C, G and T", g_max_shift, SGC_MAX_K_PACKED);
     }
+    // --unmatched-report: the library must take the 2-bit index, and the report's file must be writable
+    // before any read is counted
+    FILE* unmatched_out = nullptr;
+    struct FileGuard {
+      FILE*& f;
+      ~FileGuard() {
+        if (f) fclose(f);
+      }
+    } unmatched_guard{unmatched_out};
+    if (!args.unmatched_report.empty()) {
+      sgc_library_info info{};
+      check(sgc_library_get_info(libs[0], &info));
+      if (info.opaque)
+        fail("'--unmatched-report' needs a library of guides of at most %u bases over A, C, G and T", SGC_MAX_K_PACKED);
+      unmatched_out = fopen(args.unmatched_report.c_str(), "wb");
+      if (!unmatched_out) fail("cannot create %s", args.unmatched_report.c_str());
+      g_unmatched_capacity = kUnmatchedCapacity;
+      g_unmatched_k = hlib.k;
+      check(sgc_unmatched_report_bytes(kUnmatchedCapacity, &g_unmatched_bytes));
+    }
 
     // the budget of the device ingest on every device: its free memory now, less an eighth for the
     // counters' own buffers (SGC_DEVICE_BUDGET=bytes sets it, for tests of the admission)
@@ -1353,6 +1440,45 @@ int main(int argc, char** argv) {
     work();
     for (auto& t : pool) t.join();
     if (!first_error.empty()) fail("%s", first_error.c_str());
+    double unmatched_s = 0;
+    if (unmatched_out) {
+      // per sample, in input order: its most frequent windows (count descending, then window ascending),
+      // then the rest; the rows of a sample add up to total - matched of its Finished: line
+      const auto t0 = std::chrono::steady_clock::now();
+      std::string tsv = "Sample\tWindow\tCount\n";
+      for (size_t s = 0; s < n_samples; ++s) {
+        SampleResult& r = results[s];
+        // (keys of one length sort like the window bytes)
+        std::vector<std::pair<uint64_t, uint64_t>> rows(r.unmatched.begin(), r.unmatched.end());
+        auto before = [](const std::pair<uint64_t, uint64_t>& a, const std::pair<uint64_t, uint64_t>& b) {
+          return a.second != b.second ? a.second > b.second : a.first < b.first;
+        };
+        const size_t top = std::min(rows.size(), kUnmatchedRows);
+        std::partial_sort(rows.begin(), rows.begin() + top, rows.end(), before);
+        uint64_t other = r.um_overflow;
+        for (size_t i = top; i < rows.size(); ++i) other += rows[i].second;
+        for (size_t i = 0; i < top; ++i) {
+          std::string window(g_unmatched_k, 'A');
+          for (uint32_t j = 0; j < g_unmatched_k; ++j) window[j] = "ACGT"[(rows[i].first >> (2 * (g_unmatched_k - 1 - j))) & 3];
+          tsv += names[s] + "\t" + window + "\t" + std::to_string(rows[i].second) + "\n";
+        }
+        tsv += names[s] + "\t<other>\t" + std::to_string(other) + "\n";
+        tsv += names[s] + "\t<non-ACGT>\t" + std::to_string(r.um_non_acgt) + "\n";
+        tsv += names[s] + "\t<short>\t" + std::to_string(r.um_short) + "\n";
+        if (r.um_overflow)
+          fprintf(stderr,
+                  "WARNING: unmatched report of %s: %llu reads had a window the report had no room for; its window counts are "
+                  "lower bounds, short by at most %llu\n",
+                  names[s].c_str(), (unsigned long long)r.um_overflow, (unsigned long long)r.um_overflow);
+        unmatched_s += r.unmatched_s;
+      }
+      if (fwrite(tsv.data(), 1, tsv.size(), unmatched_out) != tsv.size() || fclose(unmatched_out) != 0) {
+        unmatched_out = nullptr;
+        fail("cannot write %s", args.unmatched_report.c_str());
+      }
+      unmatched_out = nullptr;
+      unmatched_s += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+    }
     if (args.timing) {
       const double count_s = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_count0).count();
       unsigned long long reads = 0;
@@ -1381,11 +1507,12 @@ int main(int argc, char** argv) {
               "\"device_blocks\": %llu, \"device_text_bytes\": %llu, \"device_phases_s\": [%.4f, %.4f, %.4f, %.4f], \"host_ingest_because\": \"%s\", \"members_adopted\": %llu, \"members_reframed\": %llu, \"wait_inflate_s\": %.6f, "
               "\"copy_to_pinned_s\": %.6f, \"submit_sync_s\": %.6f, \"read_inputs_s\": %.3f, "
               "\"device_tables_s\": %.3f, \"offsets_s\": %.3f, \"member_pieces\": %llu, \"member_chain\": %llu, \"member_absorbed\": %llu, \"gzip_members\": %llu, "
-              "\"member_lanes\": %u, \"device_samples_in_flight\": %u%s}\n",
+              "\"member_lanes\": %u, \"device_samples_in_flight\": %u%s%s}\n",
               count_s, reads, n_samples, workers, ingest_threads, gpus, max_shards, span_reads, device_samples, device_blocks, device_text_bytes,
               dev_index_s, dev_create_s, dev_waves_s, dev_finish_s, host_because.c_str(), adopted, reframed, wait_s, copy_s, submit_s, t_inputs,
               t_tables - t_inputs, t_offsets - t_tables, pieces, chain, absorbed, gzip_member_count, member_lanes, in_flight,
-              args.have_max_shift ? (", \"max_shift\": " + std::to_string(g_max_shift)).c_str() : "");
+              args.have_max_shift ? (", \"max_shift\": " + std::to_string(g_max_shift)).c_str() : "",
+              unmatched_s_key(args.unmatched_report.empty(), unmatched_s).c_str());
     }
 
     // write_results (results.rs:71-99).  Counts are keyed by alias (counter.rs:232-235):
