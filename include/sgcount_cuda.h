@@ -386,6 +386,65 @@ int sgc_fastq_stream_text_scratch_bound(uint32_t read_len, uint32_t span_len, ui
 int sgc_fastq_stream_gzip_members(const sgc_fastq_stream*, uint64_t* members);
 int sgc_fastq_stream_finish(sgc_fastq_stream*, uint64_t* n_records);
 
+/* ---- Dual-guide constructs from paired reads ------------------------------------------------------
+ * Screens with two guides per vector read guide A in R1 and guide B in R2 and count the listed (A, B)
+ * construct.  A pair counter joins two ordinary counters, one per mate, each with its own library,
+ * Offset, position recursion, rc_mode and max_shift: mate m of pair i gets a_m[i], exactly what that
+ * counter assigns to the read alone (guide index or -1).  Construct j is (pair_first[j], pair_second[j]),
+ * guide indices of the two libraries.  Every pair falls into one class:
+ *   listed       both mates matched and (a1, a2) is construct j: counted on j;
+ *   recombined   both mates matched and (a1, a2) is not listed (template switching);
+ *   first_only / second_only   only that mate matched;   neither   no mate matched.
+ * total = listed + recombined + first_only + second_only + neither and listed = the sum of the construct
+ * counts.  The mates' counters keep their usual state (marginal guide counts; total_reads = total), as if
+ * each had counted its file alone.
+ * Recombinant report (recombinant_capacity > 0): the recombined pairs keyed by (a1, a2), at most
+ * `capacity` distinct; slots are never freed and a pair that finds no slot in 128 probes goes to
+ * overflow, so every held count is exact and recombined = overflow + the held counts.
+ * Each mate is counted in chunks of at most 2^24 pairs through the line (shift, byte-keyed) kernel into
+ * pair-owned assignment scratch, then the chunk is combined; all of it runs on the first counter's
+ * stream, and the second counter's stream waits for the end of every submit, so sgc_counter_finish on
+ * either counter sees it.
+ * create refuses (SGC_ERR_INVALID_ARG) counters on different devices, the same counter twice, a counter
+ * that has counted or has an unmatched report, n_pairs outside 1..2^26, capacity above 2^26 and a guide
+ * index outside its library; a (first, second) entry listed twice is SGC_ERR_DUPLICATE_SEQUENCE.  The
+ * pair counter does not own the counters: destroy it first. */
+typedef struct sgc_pair_counter sgc_pair_counter;
+int sgc_pair_counter_create(sgc_counter* first, sgc_counter* second, const uint32_t* pair_first,
+                            const uint32_t* pair_second, uint64_t n_pairs, uint64_t recombinant_capacity,
+                            sgc_pair_counter** out);
+void sgc_pair_counter_destroy(sgc_pair_counter*);
+/* n_pairs pairs: read i of mate 1 and read i of mate 2, each in its own layout (as sgc_counter_submit:
+ * fixed stride at any alignment, or u32 line offsets; span records of each mate's own geometry).  Host
+ * memory, copied and counted chunk by chunk on double buffers; the buffers must stay valid until
+ * sgc_pair_counter_wait_copies or sgc_pair_counter_finish. */
+int sgc_pair_counter_submit(sgc_pair_counter*, const uint8_t* lines1, uint64_t n_bytes1, const uint32_t* line_off1,
+                            uint32_t stride1, uint32_t read_len1, const uint8_t* lines2, uint64_t n_bytes2,
+                            const uint32_t* line_off2, uint32_t stride2, uint32_t read_len2, uint64_t n_pairs);
+/* The same for batches resident in device memory. */
+int sgc_pair_counter_submit_device(sgc_pair_counter*, const uint8_t* d_lines1, uint64_t n_bytes1,
+                                   const uint32_t* d_line_off1, uint32_t stride1, uint32_t read_len1,
+                                   const uint8_t* d_lines2, uint64_t n_bytes2, const uint32_t* d_line_off2,
+                                   uint32_t stride2, uint32_t read_len2, uint64_t n_pairs);
+/* sgc_counter_wait_copies for both mates. */
+int sgc_pair_counter_wait_copies(sgc_pair_counter*, uint32_t keep_in_flight);
+typedef struct sgc_pair_info {
+  uint64_t total, listed, recombined, first_only, second_only, neither;
+  uint64_t overflow; /* recombined pairs the report refused for want of a slot */
+  uint64_t distinct; /* recombinant pairs the report holds                     */
+} sgc_pair_info;
+/* Waits, then copies out construct_counts[n_pairs] (list order; may be NULL) and info (may be NULL). */
+int sgc_pair_counter_finish(sgc_pair_counter*, uint64_t* construct_counts, sgc_pair_info* info);
+/* Waits, then writes the first max_pairs recombinant pairs of the report in report order (count descending,
+ * then (first, second) ascending); *n_out = how many were written.  SGC_ERR_INVALID_ARG without a report. */
+int sgc_pair_counter_recombinants(sgc_pair_counter*, uint64_t max_pairs, uint32_t* first, uint32_t* second,
+                                  uint64_t* counts, uint64_t* n_out);
+/* Zeroes the construct counts, the tallies, the report and both mates' state vectors. */
+int sgc_pair_counter_reset(sgc_pair_counter*);
+/* Device memory one pair counter takes (construct table and counts, both mates' assignment scratch of
+ * 64 MiB each, the report). */
+int sgc_pair_counter_bytes(uint64_t n_pairs, uint64_t recombinant_capacity, uint64_t* bytes);
+
 /* Statistics of the last sgc_counter_submit_device call, for benchmarking. */
 typedef struct sgc_launch_info {
   uint32_t grid, block, smem_bytes;

@@ -76,6 +76,19 @@ class UnmatchedInfo(C.Structure):
     ]
 
 
+class PairInfo(C.Structure):
+    _fields_ = [
+        ("total", C.c_uint64),
+        ("listed", C.c_uint64),
+        ("recombined", C.c_uint64),
+        ("first_only", C.c_uint64),
+        ("second_only", C.c_uint64),
+        ("neither", C.c_uint64),
+        ("overflow", C.c_uint64),
+        ("distinct", C.c_uint64),
+    ]
+
+
 # every symbol include/sgcount_cuda.h declares: name -> (restype, argtypes)
 _vp, _u32, _u64, _int = C.c_void_p, C.c_uint32, C.c_uint64, C.c_int
 SIGNATURES = {
@@ -124,6 +137,15 @@ SIGNATURES = {
     "sgc_fastq_stream_gzip_members": (_int, [_vp, C.POINTER(_u64)]),
     "sgc_fastq_stream_finish": (_int, [_vp, C.POINTER(_u64)]),
     "sgc_counter_launch_info": (_int, [_vp, C.POINTER(LaunchInfo)]),
+    "sgc_pair_counter_create": (_int, [_vp, _vp, _vp, _vp, _u64, _u64, C.POINTER(_vp)]),
+    "sgc_pair_counter_destroy": (None, [_vp]),
+    "sgc_pair_counter_submit": (_int, [_vp, _vp, _u64, _vp, _u32, _u32, _vp, _u64, _vp, _u32, _u32, _u64]),
+    "sgc_pair_counter_submit_device": (_int, [_vp, _vp, _u64, _vp, _u32, _u32, _vp, _u64, _vp, _u32, _u32, _u64]),
+    "sgc_pair_counter_wait_copies": (_int, [_vp, _u32]),
+    "sgc_pair_counter_finish": (_int, [_vp, _vp, C.POINTER(PairInfo)]),
+    "sgc_pair_counter_recombinants": (_int, [_vp, _u64, _vp, _vp, _vp, C.POINTER(_u64)]),
+    "sgc_pair_counter_reset": (_int, [_vp]),
+    "sgc_pair_counter_bytes": (_int, [_u64, _u64, C.POINTER(_u64)]),
 }
 
 _lib = None

@@ -410,6 +410,90 @@ class Counter:
         return self.matched_reads() / self.total_reads()
 
 
+class PairCounter:
+    """Dual-guide constructs from paired reads (sgc_pair_counter): mate 1 counted by `first`, mate 2 by
+    `second` (ordinary counters that have not counted yet, on one device), and every pair classified as
+    listed (counted on its construct), recombined, first_only, second_only or neither.  `pairs`: the
+    constructs, (first guide index, second guide index) in list order.  recombinant_capacity > 0 keeps a
+    report of the recombined pairs (recombinants()).  The counters keep their own marginal results; keep
+    them alive as long as this object."""
+
+    def __init__(self, first: Counter, second: Counter, pairs, recombinant_capacity: int = 0):
+        pairs = np.asarray(pairs, dtype=np.int64).reshape(-1, 2)
+        if pairs.size and (pairs.min() < 0 or pairs.max() >= 2**32):
+            raise SgcError(_cabi.ERR_INVALID_ARG, "a pair names a guide outside its library")
+        a = np.ascontiguousarray(pairs[:, 0], dtype=np.uint32)
+        b = np.ascontiguousarray(pairs[:, 1], dtype=np.uint32)
+        self._mates = (first, second)
+        self.n_pairs = len(a)
+        self._ptr = C.c_void_p()
+        check(_cabi.load().sgc_pair_counter_create(first._ptr, second._ptr, a.ctypes.data, b.ctypes.data, len(a),
+                                                   int(recombinant_capacity), C.byref(self._ptr)))
+
+    def __del__(self):
+        try:
+            if getattr(self, "_ptr", None):
+                _cabi.load().sgc_pair_counter_destroy(self._ptr)
+                self._ptr = None
+        except Exception:  # interpreter shutdown
+            pass
+
+    def _touched(self):
+        for c in self._mates:
+            c._result = None
+
+    def submit(self, batch1: ReadBatch, batch2: ReadBatch) -> None:
+        """host batches of the same number of reads, read i of each forming pair i"""
+        if batch1.n_reads != batch2.n_reads:
+            raise SgcError(_cabi.ERR_INVALID_ARG, "the mates' batches hold different numbers of reads")
+        a, b = batch1._args(), batch2._args()
+        check(_cabi.load().sgc_pair_counter_submit(self._ptr, *a[:5], *b[:5], batch1.n_reads))
+        self._touched()
+
+    def submit_device(self, n_pairs: int, d_lines1: int, n_bytes1: int, d_lines2: int, n_bytes2: int,
+                      stride1: int = 0, read_len1: int = 0, d_line_off1: Optional[int] = None,
+                      stride2: int = 0, read_len2: int = 0, d_line_off2: Optional[int] = None) -> None:
+        check(_cabi.load().sgc_pair_counter_submit_device(self._ptr, d_lines1, n_bytes1, d_line_off1, stride1, read_len1,
+                                                          d_lines2, n_bytes2, d_line_off2, stride2, read_len2, n_pairs))
+        self._touched()
+
+    def wait_copies(self, keep_in_flight: int = 0) -> None:
+        check(_cabi.load().sgc_pair_counter_wait_copies(self._ptr, int(keep_in_flight)))
+
+    def finish(self):
+        """(construct counts uint64[n_pairs] in list order, {total, listed, recombined, first_only, second_only,
+        neither, overflow, distinct})"""
+        counts = np.zeros(self.n_pairs, dtype=np.uint64)
+        info = _cabi.PairInfo()
+        check(_cabi.load().sgc_pair_counter_finish(self._ptr, counts.ctypes.data, C.byref(info)))
+        return counts, {name: int(getattr(info, name)) for name, _ in _cabi.PairInfo._fields_}
+
+    def recombinants(self, max_pairs: Optional[int] = None):
+        """[(first index, second index, count)] of the recombinant report, by count descending then pair
+        ascending: the first max_pairs of them or all"""
+        lib = _cabi.load()
+        if max_pairs is None:
+            max_pairs = self.finish()[1]["distinct"]
+        m = max(int(max_pairs), 1)
+        a, b, n = np.zeros(m, np.uint32), np.zeros(m, np.uint32), np.zeros(m, np.uint64)
+        got = C.c_uint64()
+        check(lib.sgc_pair_counter_recombinants(self._ptr, int(max_pairs), a.ctypes.data, b.ctypes.data, n.ctypes.data,
+                                                C.byref(got)))
+        return [(int(a[i]), int(b[i]), int(n[i])) for i in range(int(got.value))]
+
+    def reset(self) -> None:
+        """zero the constructs, tallies, report and both mates' state"""
+        check(_cabi.load().sgc_pair_counter_reset(self._ptr))
+        self._touched()
+
+
+def pair_counter_bytes(n_pairs: int, capacity: int = 0) -> int:
+    """device memory of one PairCounter of n_pairs constructs and a report of `capacity` pairs (sgc_pair_counter_bytes)"""
+    out = C.c_uint64()
+    check(_cabi.load().sgc_pair_counter_bytes(int(n_pairs), int(capacity), C.byref(out)))
+    return int(out.value)
+
+
 def bgzf_blocks(blob: bytes):
     """(begin offsets [n + 1], ISIZE [n]) of the blocks of a BGZF file (the 'BC' extra subfield
     holds the block size - 1), or None when the bytes are not BGZF."""

@@ -1195,7 +1195,7 @@ constexpr size_t kChunkBytes = 64ull << 20;
 constexpr uint64_t kChunkAlignReads = 256;  // chunk starts stay 16-byte aligned for any stride
 constexpr uint64_t kSkewSampleReads = 65536;   // reads of the first batch the skew plan looks at
 constexpr uint64_t kSkewMinBatch = 4 * kSkewSampleReads;  // smaller first batches are not worth a plan
-constexpr uint64_t kUnmatchedLaunchReads = 1ull << 24;    // reads per launch with the unmatched report (its scratch)
+constexpr uint64_t kUnmatchedLaunchReads = kAssignScratchReads;  // reads per launch with the unmatched report (its scratch)
 constexpr uint64_t kUnmatchedMaxCapacity = 1ull << 26;
 
 // Tuning switches (SGC_DEBUG, SGC_WARPS, SGC_CTAS, SGC_STAGES, SGC_CARVEOUT, SGC_REPLICAS) exist only
@@ -1319,7 +1319,8 @@ int launch_count(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const
     c->last.replicas = 1;
     c->last.hot_guides = 0;
     c->last.launches_total += 1;
-    return opaque_count(c, d_lines, d_off, off_base, stride, read_len, first, n_reads, d_assign, stream, &c->last.grid);
+    return opaque_count(c, d_lines, d_off, off_base, stride, read_len, first, n_reads, d_assign ? d_assign : c->pair_assign,
+                        stream, &c->last.grid);
   }
   CountParams p = make_params(c, d_lines, d_off, stride, read_len, d_assign);
   p.off_base = off_base;
@@ -1338,9 +1339,11 @@ int launch_count(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const
   // launch, and a Centered window that fits (otherwise every read fails its first trim)
   const uint32_t tile_bytes = kWarpReads * stride;
   const uint32_t stage_bytes = (tile_bytes + 48 + 15) & ~15u;  // +48: span words may run past the tile
-  // a counter with the unmatched report counts through the line or shift kernel, which write assignments
+  // a counter with the unmatched report, or one mate of a pair counter, counts through the line or shift
+  // kernel, which write assignments
   const bool report = c->um_capacity != 0;
-  const bool stageable = !shifted && !report && d_off == nullptr && ((uintptr_t)d_lines & 15u) == 0 && stride >= read_len &&
+  const bool to_scratch = report || c->pair_assign;
+  const bool stageable = !shifted && !to_scratch && d_off == nullptr && ((uintptr_t)d_lines & 15u) == 0 && stride >= read_len &&
                          (uint64_t)c->offset + c->lib->k <= read_len;
   // kernel family by the words that hold the k window bytes: narrow keys 4 (k <= 16) or 5
   // (k = 17..20, the common guide lengths); wide keys 6 (k = 21..24), 7 (k = 25..28) or 8 (k = 29, 30)
@@ -1400,15 +1403,15 @@ int launch_count(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const
   if (const long long cap = env_ll("SGC_MAX_LAUNCH_TILES", 0); cap > 0)
     shift_launch_reads = std::min<uint64_t>(shift_launch_reads, (uint64_t)cap * kWarpReads);
   // with the unmatched report a launch's assignments go to the counter's scratch of kUnmatchedLaunchReads
-  uint64_t report_launch_reads = kUnmatchedLaunchReads;
-  if (const long long cap = env_ll("SGC_MAX_LAUNCH_TILES", 0); cap > 0)
-    report_launch_reads = std::min<uint64_t>(report_launch_reads, (uint64_t)cap * kWarpReads);
+  const uint64_t report_launch_reads = assign_scratch_reads();
   if (shifted) c->last.kernel = 3;
   while (done < n_reads) {  // what the streaming kernel did not take; at most 2^27 reads per launch
     p.first_read = done;
-    p.n_reads = std::min<uint64_t>(n_reads - done, report ? report_launch_reads
-                                                          : (shifted ? shift_launch_reads : 1ull << kLineIdxBits));
+    p.n_reads = std::min<uint64_t>(n_reads - done, to_scratch ? report_launch_reads
+                                                              : (shifted ? shift_launch_reads : 1ull << kLineIdxBits));
     CountParams q = p;
+    // a pair counter's batch is one chunk of its scratch: read r's assignment goes to pair_assign[r]
+    if (c->pair_assign && !d_assign) q.assign_out = c->pair_assign;
     if (report && !d_assign) {  // the launch's reads start at index 0 of the scratch
       q.first_read = 0;
       if (q.line_off) {
@@ -1458,19 +1461,20 @@ int launch_count(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const
   return SGC_OK;
 }
 
-int alloc_replicas(sgc_counter* c, uint32_t replicas) {
+// stream: the stream the counter's kernels run on (a pair counter runs both mates on the first mate's)
+int alloc_replicas(sgc_counter* c, uint32_t replicas, cudaStream_t stream) {
   // a power of two, at most 64 copies and 64 MB
   uint32_t n_rep = 1;
   while (n_rep * 2 <= replicas && n_rep < 64 && (size_t)n_rep * 2 * c->lib->n * sizeof(uint64_t) <= (64u << 20))
     n_rep *= 2;
   if (n_rep == c->n_rep) return SGC_OK;
-  SGC_CUDA_TRY(cudaStreamSynchronize(c->stream));  // the replicas are zero between launches
+  SGC_CUDA_TRY(cudaStreamSynchronize(stream));  // the replicas are zero between launches
   cudaFree(c->d_rep);
   c->d_rep = nullptr;
   c->n_rep = 1;
   if (n_rep > 1) {
     SGC_CUDA_TRY(cudaMalloc(&c->d_rep, (size_t)n_rep * c->lib->n * sizeof(uint64_t)));
-    SGC_CUDA_TRY(cudaMemsetAsync(c->d_rep, 0, (size_t)n_rep * c->lib->n * sizeof(uint64_t), c->stream));
+    SGC_CUDA_TRY(cudaMemsetAsync(c->d_rep, 0, (size_t)n_rep * c->lib->n * sizeof(uint64_t), stream));
     c->n_rep = n_rep;
   }
   return SGC_OK;
@@ -1500,7 +1504,7 @@ int plan_skew(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const ui
   // shares among everything this counter has seen so far (earlier small batches included)
   const uint64_t seen = std::max<uint64_t>(top.total, 1), top_count = top.packed[0] >> 32;
   if (top_count * 256 < seen) return SGC_OK;  // no guide stands out
-  rc = alloc_replicas(c, 16);
+  rc = alloc_replicas(c, 16, stream);
   if (rc) return rc;
   int n_hot = 0;
   for (int j = 0; j < kHotGuides; ++j)
@@ -1534,18 +1538,7 @@ int sgc::count_gathered_lines(sgc_counter* c, const uint8_t* d_text, uint64_t n_
   return rc;
 }
 
-namespace {
-
-// an empty unmatched report
-int clear_unmatched(sgc_counter* c) {
-  const uint64_t blocks = std::min<uint64_t>((c->um_capacity + 255) / 256, (uint64_t)c->lib->sm_count * 8);
-  unmatched_clear_kernel<<<(unsigned)blocks, 256, 0, c->stream>>>(static_cast<ulonglong2*>(c->d_um_table), c->um_capacity);
-  SGC_CUDA_TRY(cudaGetLastError());
-  SGC_CUDA_TRY(cudaMemsetAsync(c->d_um_tally, 0, kTallyWords * sizeof(uint64_t), c->stream));
-  return SGC_OK;
-}
-
-int check_batch(const sgc_counter* c, const uint8_t* lines, uint64_t n_bytes, const uint32_t* line_off,
+int sgc::check_batch(const sgc_counter* c, const uint8_t* lines, uint64_t n_bytes, const uint32_t* line_off,
                 uint32_t stride, uint32_t read_len, uint64_t n_reads) {
   if (!c) return set_error(SGC_ERR_INVALID_ARG, "counter is NULL");
   if (n_reads == 0) return SGC_OK;
@@ -1557,6 +1550,125 @@ int check_batch(const sgc_counter* c, const uint8_t* lines, uint64_t n_bytes, co
     if ((n_reads - 1) * (uint64_t)stride + read_len > n_bytes)
       return set_error(SGC_ERR_INVALID_ARG, "fixed-stride batch does not fit n_bytes");
   }
+  return SGC_OK;
+}
+
+uint64_t sgc::assign_scratch_reads() {
+  uint64_t n = kUnmatchedLaunchReads;
+  if (const long long cap = env_ll("SGC_MAX_LAUNCH_TILES", 0); cap > 0) n = std::min<uint64_t>(n, (uint64_t)cap * kWarpReads);
+  return n;
+}
+
+int sgc::count_into_scratch(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const uint32_t* d_off, uint32_t off_base,
+                            uint32_t stride, uint32_t read_len, uint64_t n_reads, int32_t* d_assign, cudaStream_t stream) {
+  if (n_reads == 0) return SGC_OK;
+  if (n_reads > kAssignScratchReads) return set_error(SGC_ERR_INVALID_ARG, "batch larger than the assignment scratch");
+  c->pair_assign = d_assign;
+  const int rc = count_batch(c, d_lines, n_bytes, d_off, off_base, stride, read_len, n_reads, nullptr, stream);
+  c->pair_assign = nullptr;
+  return rc;
+}
+
+int sgc::ensure_staging(sgc_counter* c) {
+  if (c->copy_stream) return SGC_OK;
+  SGC_CUDA_TRY(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
+  for (int i = 0; i < 2; ++i) {
+    SGC_CUDA_TRY(cudaEventCreateWithFlags(&c->copy_done[i], cudaEventDisableTiming));
+    SGC_CUDA_TRY(cudaEventCreateWithFlags(&c->kernel_done[i], cudaEventDisableTiming));
+  }
+  return SGC_OK;
+}
+
+// chunk geometry: whole tiles of reads, about kChunkBytes each
+uint64_t sgc::host_chunk_end(const uint32_t* line_off, uint32_t stride, uint64_t r0, uint64_t n_reads) {
+  if (line_off) {
+    // advance until the chunk holds about kChunkBytes
+    uint64_t lo = r0, hi = n_reads;
+    const uint64_t limit = (uint64_t)line_off[r0] + kChunkBytes;
+    while (lo < hi) {  // last r with line_off[r] <= limit
+      uint64_t mid = (lo + hi + 1) / 2;
+      if (line_off[mid] <= limit) lo = mid; else hi = mid - 1;
+    }
+    return lo > r0 ? lo : r0 + 1;
+  }
+  const uint64_t per = std::max<uint64_t>(kChunkAlignReads, (kChunkBytes / stride) / kChunkAlignReads * kChunkAlignReads);
+  return std::min(n_reads, r0 + per);
+}
+
+int sgc::stage_host_chunk(sgc_counter* c, cudaStream_t stream, const uint8_t* lines, uint64_t n_bytes, const uint32_t* line_off,
+                          uint32_t stride, uint64_t r0, uint64_t r1, HostChunk* out) {
+  const int b = (int)(c->chunks_submitted & 1);
+  const uint64_t byte0 = line_off ? line_off[r0] : r0 * stride;
+  const uint64_t byte1 = line_off ? line_off[r1] : std::min<uint64_t>(n_bytes, r1 * stride);
+  const size_t bytes = byte1 - byte0;
+  // (re)size this staging buffer; +64 so bulk copies of the last tile stay inside the allocation
+  if (bytes + 64 > c->stage_cap) {
+    SGC_CUDA_TRY(cudaStreamSynchronize(stream));
+    SGC_CUDA_TRY(cudaStreamSynchronize(c->copy_stream));
+    size_t cap = std::max<size_t>(bytes + 64, std::min<size_t>(kChunkBytes + (1 << 20), n_bytes + 64));
+    for (int i = 0; i < 2; ++i) {
+      cudaFree(c->d_stage[i]);
+      c->d_stage[i] = nullptr;
+      SGC_CUDA_TRY(cudaMalloc(&c->d_stage[i], cap));
+    }
+    c->stage_cap = cap;
+  }
+  const size_t n_off = line_off ? (r1 - r0 + 1) : 0;
+  if (n_off > c->stage_off_cap) {
+    SGC_CUDA_TRY(cudaStreamSynchronize(stream));
+    SGC_CUDA_TRY(cudaStreamSynchronize(c->copy_stream));
+    size_t cap = n_off * 2;
+    for (int i = 0; i < 2; ++i) {
+      cudaFree(c->d_stage_off[i]);
+      c->d_stage_off[i] = nullptr;
+      SGC_CUDA_TRY(cudaMalloc(&c->d_stage_off[i], cap * sizeof(uint32_t)));
+    }
+    c->stage_off_cap = cap;
+  }
+  // copy stream: wait until the kernel that last read this buffer is done, then copy
+  if (c->chunks_submitted >= 2) SGC_CUDA_TRY(cudaStreamWaitEvent(c->copy_stream, c->kernel_done[b], 0));
+  SGC_CUDA_TRY(cudaMemcpyAsync(c->d_stage[b], lines + byte0, bytes, cudaMemcpyHostToDevice, c->copy_stream));
+  if (line_off)
+    SGC_CUDA_TRY(cudaMemcpyAsync(c->d_stage_off[b], line_off + r0, n_off * sizeof(uint32_t), cudaMemcpyHostToDevice,
+                                 c->copy_stream));
+  SGC_CUDA_TRY(cudaEventRecord(c->copy_done[b], c->copy_stream));
+  SGC_CUDA_TRY(cudaStreamWaitEvent(stream, c->copy_done[b], 0));
+  out->d_lines = c->d_stage[b];
+  out->d_off = line_off ? c->d_stage_off[b] : nullptr;
+  out->bytes = bytes;
+  out->off_base = (uint32_t)(line_off ? byte0 : 0);
+  out->buf = b;
+  return SGC_OK;
+}
+
+int sgc::end_host_chunk(sgc_counter* c, cudaStream_t stream, const HostChunk& ch) {
+  SGC_CUDA_TRY(cudaEventRecord(c->kernel_done[ch.buf], stream));
+  c->chunks_submitted += 1;
+  return SGC_OK;
+}
+
+// ticket of a submit call's copies (sgc_counter_wait_copies)
+int sgc::push_copy_ticket(sgc_counter* c) {
+  cudaEvent_t ticket = nullptr;
+  if (!c->free_tickets.empty()) {
+    ticket = c->free_tickets.back();
+    c->free_tickets.pop_back();
+  } else {
+    SGC_CUDA_TRY(cudaEventCreateWithFlags(&ticket, cudaEventDisableTiming));
+  }
+  c->copy_tickets.push_back(ticket);
+  SGC_CUDA_TRY(cudaEventRecord(ticket, c->copy_stream));
+  return SGC_OK;
+}
+
+namespace {
+
+// an empty unmatched report
+int clear_unmatched(sgc_counter* c) {
+  const uint64_t blocks = std::min<uint64_t>((c->um_capacity + 255) / 256, (uint64_t)c->lib->sm_count * 8);
+  unmatched_clear_kernel<<<(unsigned)blocks, 256, 0, c->stream>>>(static_cast<ulonglong2*>(c->d_um_table), c->um_capacity);
+  SGC_CUDA_TRY(cudaGetLastError());
+  SGC_CUDA_TRY(cudaMemsetAsync(c->d_um_tally, 0, kTallyWords * sizeof(uint64_t), c->stream));
   return SGC_OK;
 }
 
@@ -1686,85 +1798,19 @@ int sgc_counter_submit(sgc_counter* c, const uint8_t* lines, uint64_t n_bytes, c
   if (n_reads == 0) return SGC_OK;
   if (line_off && line_off[n_reads] > n_bytes) return set_error(SGC_ERR_INVALID_ARG, "line offsets exceed n_bytes");
   DeviceGuard guard(c->lib->device);
-  if (!c->copy_stream) {
-    SGC_CUDA_TRY(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < 2; ++i) {
-      SGC_CUDA_TRY(cudaEventCreateWithFlags(&c->copy_done[i], cudaEventDisableTiming));
-      SGC_CUDA_TRY(cudaEventCreateWithFlags(&c->kernel_done[i], cudaEventDisableTiming));
-    }
-  }
-  // chunk geometry: whole tiles of reads, about kChunkBytes each
+  if ((rc = ensure_staging(c))) return rc;
   uint64_t r0 = 0;
   while (r0 < n_reads) {
-    uint64_t r1;
-    if (line_off) {
-      // advance until the chunk holds about kChunkBytes
-      uint64_t lo = r0, hi = n_reads;
-      const uint64_t limit = (uint64_t)line_off[r0] + kChunkBytes;
-      while (lo < hi) {  // last r with line_off[r] <= limit
-        uint64_t mid = (lo + hi + 1) / 2;
-        if (line_off[mid] <= limit) lo = mid; else hi = mid - 1;
-      }
-      r1 = lo > r0 ? lo : r0 + 1;
-    } else {
-      uint64_t per = std::max<uint64_t>(kChunkAlignReads, (kChunkBytes / stride) / kChunkAlignReads * kChunkAlignReads);
-      r1 = std::min(n_reads, r0 + per);
-    }
-    const int b = (int)(c->chunks_submitted & 1);
-    const uint64_t byte0 = line_off ? line_off[r0] : r0 * stride;
-    const uint64_t byte1 = line_off ? line_off[r1] : std::min<uint64_t>(n_bytes, r1 * stride);
-    const size_t bytes = byte1 - byte0;
-    // (re)size this staging buffer; +64 so bulk copies of the last tile stay inside the allocation
-    if (bytes + 64 > c->stage_cap) {
-      SGC_CUDA_TRY(cudaStreamSynchronize(c->stream));
-      SGC_CUDA_TRY(cudaStreamSynchronize(c->copy_stream));
-      size_t cap = std::max<size_t>(bytes + 64, std::min<size_t>(kChunkBytes + (1 << 20), n_bytes + 64));
-      for (int i = 0; i < 2; ++i) {
-        cudaFree(c->d_stage[i]);
-        c->d_stage[i] = nullptr;
-        SGC_CUDA_TRY(cudaMalloc(&c->d_stage[i], cap));
-      }
-      c->stage_cap = cap;
-    }
-    const size_t n_off = line_off ? (r1 - r0 + 1) : 0;
-    if (n_off > c->stage_off_cap) {
-      SGC_CUDA_TRY(cudaStreamSynchronize(c->stream));
-      SGC_CUDA_TRY(cudaStreamSynchronize(c->copy_stream));
-      size_t cap = n_off * 2;
-      for (int i = 0; i < 2; ++i) {
-        cudaFree(c->d_stage_off[i]);
-        c->d_stage_off[i] = nullptr;
-        SGC_CUDA_TRY(cudaMalloc(&c->d_stage_off[i], cap * sizeof(uint32_t)));
-      }
-      c->stage_off_cap = cap;
-    }
-    // copy stream: wait until the kernel that last read this buffer is done, then copy
-    if (c->chunks_submitted >= 2) SGC_CUDA_TRY(cudaStreamWaitEvent(c->copy_stream, c->kernel_done[b], 0));
-    SGC_CUDA_TRY(cudaMemcpyAsync(c->d_stage[b], lines + byte0, bytes, cudaMemcpyHostToDevice, c->copy_stream));
-    if (line_off)
-      SGC_CUDA_TRY(cudaMemcpyAsync(c->d_stage_off[b], line_off + r0, n_off * sizeof(uint32_t), cudaMemcpyHostToDevice,
-                                   c->copy_stream));
-    SGC_CUDA_TRY(cudaEventRecord(c->copy_done[b], c->copy_stream));
-    SGC_CUDA_TRY(cudaStreamWaitEvent(c->stream, c->copy_done[b], 0));
+    const uint64_t r1 = host_chunk_end(line_off, stride, r0, n_reads);
+    HostChunk ch;
+    if ((rc = stage_host_chunk(c, c->stream, lines, n_bytes, line_off, stride, r0, r1, &ch))) return rc;
     // the chunk's offsets stay what they were in the batch: the kernel subtracts the chunk's base
-    rc = count_batch(c, c->d_stage[b], bytes, line_off ? c->d_stage_off[b] : nullptr, (uint32_t)(line_off ? byte0 : 0),
-                     stride, read_len, r1 - r0, nullptr, c->stream);
+    rc = count_batch(c, ch.d_lines, ch.bytes, ch.d_off, ch.off_base, stride, read_len, r1 - r0, nullptr, c->stream);
     if (rc) return rc;
-    SGC_CUDA_TRY(cudaEventRecord(c->kernel_done[b], c->stream));
-    c->chunks_submitted += 1;
+    if ((rc = end_host_chunk(c, c->stream, ch))) return rc;
     r0 = r1;
   }
-  // ticket of this call's copies (sgc_counter_wait_copies)
-  cudaEvent_t ticket = nullptr;
-  if (!c->free_tickets.empty()) {
-    ticket = c->free_tickets.back();
-    c->free_tickets.pop_back();
-  } else {
-    SGC_CUDA_TRY(cudaEventCreateWithFlags(&ticket, cudaEventDisableTiming));
-  }
-  c->copy_tickets.push_back(ticket);
-  SGC_CUDA_TRY(cudaEventRecord(ticket, c->copy_stream));
-  return SGC_OK;
+  return push_copy_ticket(c);
 }
 
 int sgc_counter_set_replicas(sgc_counter* c, uint32_t replicas) {
@@ -1774,11 +1820,11 @@ int sgc_counter_set_replicas(sgc_counter* c, uint32_t replicas) {
     c->auto_skew = true;
     c->skew_planned = false;
     for (int j = 0; j < kHotGuides; ++j) c->hot[j] = -2;
-    return alloc_replicas(c, 1);
+    return alloc_replicas(c, 1, c->stream);
   }
   c->auto_skew = false;
   for (int j = 0; j < kHotGuides; ++j) c->hot[j] = -2;
-  return alloc_replicas(c, replicas);
+  return alloc_replicas(c, replicas, c->stream);
 }
 
 int sgc_counter_set_max_shift(sgc_counter* c, uint32_t max_shift) {

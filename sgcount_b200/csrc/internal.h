@@ -102,6 +102,9 @@ struct sgc_counter {
   unsigned long long* d_um_tally = nullptr;
   // device-ingest streams that count into this counter (gzip.cu); released with it if still open
   std::vector<struct sgc_fastq_stream*> fastq_streams;
+  // pair.cu: set only while a pair counter counts one chunk of a mate (count_into_scratch): the line
+  // (shift, byte-keyed) kernel writes read r's assignment to pair_assign[r]; NULL for every other caller
+  int32_t* pair_assign = nullptr;
 };
 
 namespace sgc {
@@ -111,6 +114,32 @@ int count_gathered_lines(sgc_counter* c, const uint8_t* d_text, uint64_t n_bytes
 // gzip.cu: frees the device side of a stream whose counter is going away (the handle stays valid
 // for sgc_fastq_stream_destroy)
 void fastq_stream_release(struct sgc_fastq_stream* s);
+int check_batch(const sgc_counter* c, const uint8_t* lines, uint64_t n_bytes, const uint32_t* line_off, uint32_t stride,
+                uint32_t read_len, uint64_t n_reads);
+// entries of a fixed per-read assignment scratch (the unmatched report's, each mate's of a pair counter)
+constexpr uint64_t kAssignScratchReads = 1ull << 24;
+// count.cu: reads per launch of a counter whose assignments go to such a scratch: kAssignScratchReads, fewer
+// under SGC_MAX_LAUNCH_TILES (read from the environment at every call)
+uint64_t assign_scratch_reads();
+// count.cu: counts a device-resident batch of at most kAssignScratchReads reads on `stream` through the
+// line, shift or byte-keyed kernel (the skew plan included) and writes read r's assignment to d_assign[r]
+int count_into_scratch(sgc_counter* c, const uint8_t* d_lines, uint64_t n_bytes, const uint32_t* d_off, uint32_t off_base,
+                       uint32_t stride, uint32_t read_len, uint64_t n_reads, int32_t* d_assign, cudaStream_t stream);
+// count.cu: a host batch copied chunk by chunk into a counter's two staging buffers on its copy stream
+// (sgc_counter_submit); `stream` is the stream whose kernels read the chunk
+struct HostChunk {
+  const uint8_t* d_lines;
+  const uint32_t* d_off;
+  uint64_t bytes;
+  uint32_t off_base;
+  int buf;
+};
+int ensure_staging(sgc_counter* c);
+uint64_t host_chunk_end(const uint32_t* line_off, uint32_t stride, uint64_t r0, uint64_t n_reads);
+int stage_host_chunk(sgc_counter* c, cudaStream_t stream, const uint8_t* lines, uint64_t n_bytes, const uint32_t* line_off,
+                     uint32_t stride, uint64_t r0, uint64_t r1, HostChunk* out);
+int end_host_chunk(sgc_counter* c, cudaStream_t stream, const HostChunk& ch);  // after the chunk's kernels
+int push_copy_ticket(sgc_counter* c);  // at the end of a submit call
 }
 
 struct sgc_library {
